@@ -24,6 +24,10 @@ ImageConverter::imageCb (monoslam_ransac.cpp:404-557).
 
 Timing: W warm-up steps, then K steps each bracketed by CUDA events on the launching stream; L2 is
 flushed (256 MiB write) between timed steps, outside the event pairs; max over ranks.
+
+--dump-outputs DIR: after the timed steps, rank 0 writes what the headline path computed in its last step as
+DIR/<name>.npy (float32 / float64, at most 64 MB in all), so that two builds can be compared output for output
+on the same seeded inputs.
 """
 import argparse
 import hashlib
@@ -37,6 +41,7 @@ import types
 
 import numpy as np
 
+sys.dont_write_bytecode = True   # the tree may be read-only: nothing is cached in it
 ROOT = os.path.dirname(os.path.abspath(__file__))
 for _p in (ROOT, os.path.join(ROOT, "oracle"), os.path.join(ROOT, "tests")):
     if _p not in sys.path:
@@ -61,6 +66,7 @@ BATCH_FILTERS = 4096
 METRIC_BATCH = "batched EKF filter-steps/s (predict+match+update), 4096 independent filters x N=30 features per GPU"
 UNIT_BATCH = "filter-steps/s"
 PARITY_TOL = 1e-9
+DUMP_LIMIT = 64 << 20
 BENCH_DEPTH_RANGE = (1.5, 3.0)
 BENCH_RHO_0 = 0.5
 
@@ -210,6 +216,34 @@ def ctx_max(ctx, v):
     return float(t.item())
 
 
+def dump_outputs(directory, arrays):
+    """Writes every array as DIR/<name>.npy in float64 (float32 arrays stay float32)."""
+    arrays = {k: np.asarray(v) if np.asarray(v).dtype == np.float32 else np.asarray(v, dtype=np.float64) for k, v in arrays.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    assert total <= DUMP_LIMIT, f"outputs of {total} bytes exceed the {DUMP_LIMIT} byte limit"
+    os.makedirs(directory, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(directory, name + ".npy"), a)
+    log(f"dumped {len(arrays)} outputs ({total / 2**20:.1f} MiB) to {directory}")
+
+
+def filter_outputs(filt):
+    """What a caller of one filter step receives: the state, the covariance (whole when it fits half the dump limit,
+    else a fixed seeded sample of its rows, all columns) and the feature table."""
+    from helpers import INT_FIELDS
+    mu, S = filt.get_full()
+    n = S.shape[0]
+    rows = np.sort(np.random.default_rng(0).choice(n, min(n, (DUMP_LIMIT // 2) // (8 * n)), replace=False))
+    feats = [filt.feature(i) for i in range(filt.numOfFeatures())]
+    st = filt.stats()
+    return {"mu": mu, "sigma_rows": S[rows], "sigma_row_index": rows,
+            "feature_center": np.array([tuple(a.center) for a in feats], dtype=np.float32).reshape(-1, 2),
+            "feature_z": np.array([tuple(a.z) for a in feats]).reshape(-1, 2),
+            "feature_h": np.array([tuple(a.h) for a in feats]).reshape(-1, 2),
+            "feature_table": np.array([[getattr(a, k) for k in INT_FIELDS] for a in feats]).reshape(-1, len(INT_FIELDS)),
+            "step_stats": np.array([getattr(st, k) for k, _ in type(st)._fields_ if k != "kernel_launches"])}
+
+
 def state_digest(mu, S):
     hsh = hashlib.sha256()
     hsh.update(np.ascontiguousarray(mu).tobytes()); hsh.update(np.ascontiguousarray(S).tobytes())
@@ -296,7 +330,7 @@ def _numpy_finish(filt, cfg, mu0, S0, feats, st, mu1, S1, t0, numpy_stacked_upda
 # ------------------------------------------------------------------------------------------------
 # single-filter workloads (cfg1 / cfg2: replicas at N > 1; cfg4: row-block partitioned at N > 1)
 # ------------------------------------------------------------------------------------------------
-def bench_single(args, ctx, workload, K, Wm, with_cpu=True, with_clocks=True, with_parity=True):
+def bench_single(args, ctx, workload, K, Wm, with_cpu=True, with_clocks=True, with_parity=True, dump_dir=None):
     torch, dist, rank, world, local = ctx.torch, ctx.dist, ctx.rank, ctx.world, ctx.local
     import ekfb200
     pkg = ekfb200.load_package()
@@ -405,6 +439,11 @@ def bench_single(args, ctx, workload, K, Wm, with_cpu=True, with_clocks=True, wi
     stA = filt.stats()
     n_end = filt.state_dim()
     dist_bytes_A = filt.dist_info()["allgather_bytes"] if partitioned else 0
+    if dump_dir:
+        outputs = filter_outputs(filt)          # every rank: reading a row-partitioned filter is collective
+        if rank == 0:
+            dump_outputs(dump_dir, outputs)
+        del outputs
     del filt
     # ---- pass B: end to end through the public API with host buffers -----------------------------
     filt = new_filter()
@@ -521,7 +560,7 @@ def _dp4a_pipe(delta, n_features, ms, clocks):
     return {"warp_instr_per_feature": per_feature, "achieved_per_s": round(ach, 1), "peak_per_s": peak, "frac": round(ach / peak, 4)}
 
 
-def bench_match(args, ctx, workload, K, Wm):
+def bench_match(args, ctx, workload, K, Wm, dump_dir=None):
     """BASELINE configs[4]: the stateless batched matcher (ekf_match_batch), frames sharded across ranks."""
     torch, dist, rank, world, local = ctx.torch, ctx.dist, ctx.rank, ctx.world, ctx.local
     import ekfb200
@@ -569,6 +608,8 @@ def bench_match(args, ctx, workload, K, Wm):
     sampler = ClockSampler(local, enabled=(rank == 0))
     sampler.start()
     tA = timed(step_resident)
+    if dump_dir and rank == 0:
+        dump_outputs(dump_dir, {"uv": uv.cpu().numpy(), "score": sc.cpu().numpy()})
     tB = timed(step_e2e)
     clocks = sampler.stop()
     found = int((uv_h[:, 0] >= 0).sum())
@@ -623,7 +664,7 @@ def bench_match(args, ctx, workload, K, Wm):
 # ------------------------------------------------------------------------------------------------
 # cfg3: batch of independent filters, sharded by filter
 # ------------------------------------------------------------------------------------------------
-def bench_batch(args, ctx, workload, K, Wm, with_cpu=True, with_clocks=True, with_parity=True):
+def bench_batch(args, ctx, workload, K, Wm, with_cpu=True, with_clocks=True, with_parity=True, dump_dir=None):
     """BASELINE configs[2]: a Monte-Carlo ensemble of independent filters, sharded by filter across
     ranks with no data-path collective (weak scaling: BATCH_FILTERS filters per GPU)."""
     torch, dist, rank, world, local = ctx.torch, ctx.dist, ctx.rank, ctx.world, ctx.local
@@ -728,6 +769,9 @@ def bench_batch(args, ctx, workload, K, Wm, with_cpu=True, with_clocks=True, wit
     batch = new_batch()
     tA, launches, cls = timed(step_resident, batch)
     mu14, st = batch.camera_states()
+    if dump_dir and rank == 0:
+        _, sigma14, _ = batch.camera_states(want_sigma=True)
+        dump_outputs(dump_dir, {"camera_states": mu14, "camera_sigma": sigma14, "step_counters": st})
     n_state = batch.state_dim(0)
     n_min = min(batch.state_dim(i) for i in (0, B // 2, B - 1))
     li_mean = float(st[:, 2].mean())
@@ -972,6 +1016,8 @@ def main():
     ap.add_argument("--filters", type=int, default=BATCH_FILTERS, help="filters per GPU of the batched workload")
     ap.add_argument("--cpu-budget", type=float, default=30.0)
     ap.add_argument("--ref-budget", type=float, default=150.0)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the headline path computed in its last timed step to DIR/<name>.npy")
     args = ap.parse_args()
     if args.impl == "reference":
         run_reference(args)
@@ -980,11 +1026,11 @@ def main():
     K, Wm = args.steps, max(args.warmup, 3)
     parity = not args.no_parity
     if args.workload.startswith("cfg3"):
-        out = bench_batch(args, ctx, args.workload, K, Wm, with_parity=parity)
+        out = bench_batch(args, ctx, args.workload, K, Wm, with_parity=parity, dump_dir=args.dump_outputs)
     elif args.workload.startswith("cfg5"):
-        out = bench_match(args, ctx, args.workload, K, Wm)
+        out = bench_match(args, ctx, args.workload, K, Wm, dump_dir=args.dump_outputs)
     else:
-        out = bench_single(args, ctx, args.workload, K, Wm, with_parity=parity)
+        out = bench_single(args, ctx, args.workload, K, Wm, with_parity=parity, dump_dir=args.dump_outputs)
         if args.workload == "cfg2_n500" and not args.no_sharded and args.match_every <= 1:
             # the paths that shard, measured in the same run at this N (VERDICT r1 item 2)
             Ks = max(2, min(args.sharded_steps, K))

@@ -16,10 +16,6 @@ import ekfb200  # noqa: E402
 abi = ekfb200.load_package()._abi
 
 
-def available():
-    return os.path.isdir(os.environ.get("EKF_REFERENCE_ROOT", "/root/reference") + "/mono-slam/src")
-
-
 def build(force=False):
     sys.path.insert(0, _HERE)
     import build_ref

@@ -9,10 +9,6 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 _LIB = None
 
 
-def available():
-    return os.path.exists(os.path.join(_HERE, "_ref", "libref_selector_f64.so")) or os.path.isdir("/root/reference")
-
-
 def lib():
     global _LIB
     if _LIB is None:

@@ -4,18 +4,18 @@ unmodified source into oracle/_ref/libref_selector_f64.so (oracle/build_ref_sele
 trajectory into both: nodes_and_prjcts.txt, cams_cov.txt and cams_cov2.txt must be BYTE-IDENTICAL and the images
 written must carry the same names in the same order.  Trajectories are built so that every branch of the selector is
 taken (candidate in the half-threshold band, key frame = current frame, key frame = earlier candidate, the
-"frameId < 5" start-up rule, the reset of min_cov_for_pose).  Golden copies of the reference's files are committed under
-tests/golden/keyframes/ (oracle/gen_golden_keyframes.py) so that the comparison also runs where /root/reference does not
-exist.  What stays unpinned: Eigen's number formatting itself (the absent dependency; the shim follows its documented
+"frameId < 5" start-up rule, the reset of min_cov_for_pose).  The reference selector's files for these trajectories are
+stored under tests/golden/keyframes/ (oracle/gen_golden_keyframes.py), and every test here compares against them, so the
+comparison runs without the reference.  What stays unpinned: Eigen's number formatting itself (the absent dependency; the shim follows its documented
 default IOFormat)."""
 import os
+import shutil
 import struct
 import subprocess
 
 import numpy as np
 import pytest
 
-import refselbind
 from test_keyframes import Stub, _run_python, _trajectory
 
 GOLD = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "keyframes")
@@ -44,16 +44,21 @@ def trajectories():
     return out
 
 
-needs_ref = pytest.mark.skipif(not refselbind.available(), reason="neither /root/reference nor a built oracle/_ref selector")
+def reference_run(directory, name):
+    """The reference selector's output for trajectory `name`: its three files copied into `directory`; returns the
+    image names it wrote, in order."""
+    gold = os.path.join(GOLD, name)
+    for f in FILES:
+        shutil.copyfile(os.path.join(gold, f), os.path.join(directory, f))
+    return open(os.path.join(gold, "images.txt")).read().split()
 
 
-@needs_ref
 @pytest.mark.parametrize("name", sorted(trajectories()))
 def test_python_recorder_equals_reference_selector(pkg, tmp_path, name):
     traj = trajectories()[name]
     refdir = tmp_path / "ref"; pydir = tmp_path / "py"
     refdir.mkdir(); pydir.mkdir()
-    ref_images = refselbind.run(refdir, traj[0], traj[1], traj[2])
+    ref_images = reference_run(refdir, name)
     rec, saved = _run_python(pkg, pydir, traj)
     assert [os.path.basename(p) for p in saved] == ref_images
     assert len(ref_images) >= 3
@@ -61,13 +66,12 @@ def test_python_recorder_equals_reference_selector(pkg, tmp_path, name):
         assert (pydir / f).read_bytes() == (refdir / f).read_bytes(), f"{name}: {f} differs from the reference selector's"
 
 
-@needs_ref
 def test_every_branch_is_exercised(tmp_path):
     """The three trajectories together take both sub-branches of the key-frame case and the start-up rule."""
     seen_current, seen_candidate, seen_startup, seen_cov2 = False, False, False, False
-    for name, traj in trajectories().items():
+    for name in trajectories():
         d = tmp_path / name; d.mkdir()
-        imgs = refselbind.run(d, traj[0], traj[1], traj[2])
+        imgs = reference_run(d, name)
         text = (d / "nodes_and_prjcts.txt").read_text()
         seen_current |= "0  0  0" in text          # literal written with the CURRENT frame (:640, :672)
         seen_candidate |= "\n0 0 0\n" in text      # min_projs (MatrixX3i::Zero(1,3)) written with an EARLIER candidate (:650)
@@ -78,13 +82,12 @@ def test_every_branch_is_exercised(tmp_path):
     assert seen_current and seen_candidate and seen_startup and seen_cov2
 
 
-@needs_ref
 def test_cpp_recorder_equals_reference_selector(tmp_path):
     name = "walk11"
     traj = trajectories()[name]
     refdir = tmp_path / "ref"; cdir = tmp_path / "cpp"
     refdir.mkdir(); cdir.mkdir()
-    ref_images = refselbind.run(refdir, traj[0], traj[1], traj[2])
+    ref_images = reference_run(refdir, name)
     states, sigmas, covs, pts = traj
     blob = struct.pack("i", len(states))
     for s, S, c in zip(states, sigmas, covs):
