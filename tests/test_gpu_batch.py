@@ -4,7 +4,7 @@ bit-exact, state and covariance within 1e-9 relative per step from identical inp
 import numpy as np
 import pytest
 
-from helpers import INT_FIELDS, TOL, make_pair, relerr, seed_features
+from helpers import INT_FIELDS, TOL, assert_scaled_close, make_pair, relerr, seed_features
 
 pytestmark = pytest.mark.gpu
 
@@ -45,6 +45,7 @@ def _check(batch, oracles, ctx, tol=TOL):
         assert mg.shape == mo.shape, f"{ctx} filter {b}"
         em, es = relerr(mg, mo), relerr(Sg, So)
         assert em <= tol and es <= tol, f"{ctx} filter {b}: mu {em:.2e} Sigma {es:.2e}"
+        assert_scaled_close(mg, Sg, mo, So, f"{ctx} filter {b}", free_running=tol > TOL)
         worst = max(worst, em, es)
         for i in range(o.numOfFeatures()):
             a, c = batch.feature(b, i), o.feature(i)

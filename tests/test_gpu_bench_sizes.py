@@ -12,7 +12,7 @@ import numpy as np
 import pytest
 
 import bench
-from helpers import TOL, assert_state_close, assert_tables_equal, numpy_stacked_update, relerr
+from helpers import TOL, assert_scaled_close, assert_state_close, assert_tables_equal, numpy_stacked_update, relerr
 
 pytestmark = pytest.mark.gpu
 
@@ -80,6 +80,7 @@ def _numpy_check(gpu_pkg, workload, n_frames_checked=1, symmetric=True):
         ed = relerr(S1 - S0, S_ref - S0)
         out.append((st.n_li, em, es, ed))
         assert em <= TOL and es <= TOL, f"{workload} frame {t}: mu {em:.3e} Sigma {es:.3e}"
+        assert_scaled_close(mu1, S1, mu_ref, S_ref, f"{workload} frame {t} vs numpy")
         assert ed <= 1e-7, f"{workload} frame {t}: relative error of the covariance correction {ed:.3e}"
     return g.state_dim(), out
 

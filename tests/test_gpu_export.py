@@ -4,7 +4,7 @@ the feature archive and RosVSLAM::getPointsFeatures (RosVSLAMRansac.cpp:340-418)
 import numpy as np
 import pytest
 
-from helpers import TOL, assert_state_close, assert_tables_equal, make_pair, relerr, seed_features
+from helpers import TOL, assert_scaled_close, assert_state_close, assert_tables_equal, make_pair, relerr, seed_features
 
 pytestmark = pytest.mark.gpu
 
@@ -81,6 +81,7 @@ def test_rts_epoch(gpu_pkg, orc, seed, zero_w):
     mg, Sg = g.rts_epoch(mu, sg, mus, sgs, dts, drs, 1 / 30)
     mo, So = o.rts_epoch(mu, sg, mus, sgs, dts, drs, 1 / 30)
     assert relerr(mg, mo) <= TOL and relerr(Sg, So) <= TOL, f"mu {relerr(mg, mo):.2e} Sigma {relerr(Sg, So):.2e}"
+    assert_scaled_close(mg, Sg, mo, So, "rts_epoch")
     assert relerr(mg, mu) > 1e-6
     with pytest.raises(Exception):
         g.rts_epoch(mu, sg, mus, sgs, dts, drs, 0.0)

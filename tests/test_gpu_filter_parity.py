@@ -90,7 +90,7 @@ def test_free_running_trajectory(gpu_pkg, orc):
             f.predict()
             f.update(sc.picks(t, 40))
         assert_tables_equal(g, o, ctx=f"frame {t}")
-        assert_state_close(g, o, tol=1e-8, ctx=f"frame {t} free-running")
+        assert_state_close(g, o, tol=1e-8, ctx=f"frame {t} free-running", free_running=True)
     assert abs(g.Covariance_Parameter() - o.Covariance_Parameter()) <= 1e-9 * abs(o.Covariance_Parameter())
 
 

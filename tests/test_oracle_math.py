@@ -272,3 +272,55 @@ def test_sparse_numpy_update_matches_oracle(pkg, orc):
     mo, So = o.get_full()
     assert relerr(mo, mu1) < 1e-12 and relerr(So, S1) < 1e-12
     assert relerr(So - S, S1 - S) < 1e-10
+
+
+def test_scaled_bar_catches_what_the_norm_bar_misses(pkg, orc):
+    """tests/helpers.scaled_errors: errors in the small-variance parts of Sigma that the norm-wise bar (1e-9 of |Sigma|_F) lets
+    through — every anchor-xyz block off by 10 %, the quaternion block off by 5e-4 — fail the bar in the covariance's own
+    units, while two fp64 evaluations of the same update (the oracle and numpy / LAPACK) pass it."""
+    from helpers import TOL, TOL_SCALED_MU, TOL_SCALED_SIGMA, numpy_stacked_update, scaled_errors
+    N = 150
+    sc = _scene(pkg, n_features=N, n_frames=3, seed=6)
+    o = make_oracle(pkg, orc, sc, omp=True)
+    seed_features(o, sc)
+    o.captureNewFrame(sc.frame(1), sc.stamps[1]); o.predict(); o.update(sc.picks(1, N))
+    o.captureNewFrame(sc.frame(2), sc.stamps[2]); o.predict()
+    assert o.match() > 0
+    mu0, S0 = o.get_full()
+    feats = [o.feature(i) for i in range(o.numOfFeatures())]
+    o.update_after_match(sc.picks(2, N))
+    st = o.stats()
+    assert st.n_hi == 0 and st.n_removed == 0 and st.n_li > 100
+    sel = [i for i in range(o.numOfFeatures()) if o.feature(i).is_in_li]
+    mu_np, S_np = numpy_stacked_update(mu0, S0, feats, sel, 4.0)
+    mu, S = o.get_full()
+    sS, sm = scaled_errors(mu_np, S_np, mu, S)
+    assert sS <= TOL_SCALED_SIGMA / 10 and sm <= TOL_SCALED_MU / 10, (sS, sm)
+
+    anchors = S.copy()
+    for i in range(o.numOfFeatures()):
+        p = o.feature(i).position_in_state
+        anchors[p:p + 3, p:p + 3] *= 1.1
+    quat = S.copy()
+    quat[3:7, 3:7] *= 1 + 5e-4
+    for name, P, expect in (("anchor-xyz blocks x 1.1", anchors, 0.1), ("quaternion block x (1 + 5e-4)", quat, 5e-4)):
+        assert relerr(P, S) <= TOL, f"{name}: the norm-wise bar no longer passes it"
+        sS, sm = scaled_errors(mu, P, mu, S)
+        assert sm == 0.0
+        assert sS > TOL_SCALED_SIGMA, f"{name}: scaled error {sS:.2e} passes the bar"
+        assert abs(sS - expect) <= 0.01 * expect, f"{name}: scaled error {sS:.3e}, expected {expect}"
+
+
+def test_scaled_errors_zero_variance():
+    """Entries with Sigma_ii = 0 must agree exactly; any difference there is an infinite scaled error."""
+    from helpers import scaled_errors
+    S = np.diag([4.0, 0.0, 1.0]); mu = np.array([1.0, 2.0, 3.0])
+    assert scaled_errors(mu, S, mu, S) == (0.0, 0.0)
+    T = S.copy(); T[0, 2] = T[2, 0] = 1e-3
+    assert scaled_errors(mu, T, mu, S)[0] == 1e-3 / 2.0
+    T = S.copy(); T[1, 0] = T[0, 1] = 1e-300
+    assert scaled_errors(mu, T, mu, S)[0] == np.inf
+    m2 = mu.copy(); m2[1] = np.nextafter(m2[1], 3.0)
+    assert scaled_errors(m2, S, mu, S)[1] == np.inf
+    m2 = mu.copy(); m2[2] += 2.0 ** -40
+    assert scaled_errors(m2, S, mu, S)[1] == 2.0 ** -40
