@@ -69,6 +69,7 @@ SIGNATURES = {
     "ekf_batch_capture_frame": (_i, [_vp, _vp, _i, _i, _i, _d]),
     "ekf_batch_capture_frame_device": (_i, [_vp, _vp, _i, _i, _i, _d]),
     "ekf_batch_step": (_i, [_vp, _vp, _vp, _i, _vp, _i]),
+    "ekf_batch_convert2xyz_if_linear_all": (_i, [_vp]),
     "ekf_batch_get_camera_states": (_i, [_vp, _vp, _vp, _vp]),
     "ekf_batch_num_features": (_i, [_vp, _i]),
     "ekf_batch_state_dim": (_i, [_vp, _i]),

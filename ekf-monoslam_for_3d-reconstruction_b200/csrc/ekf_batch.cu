@@ -10,7 +10,9 @@
 //                                   W = Sigma H^T (n x k <= 64) and its Cholesky gain live in shared
 //                                   memory, the rank-k downdate Sigma -= V V^T runs on the fp64 tensor
 //                                   pipe (DMMA.8x8x4) straight from shared-memory V.
-// plus k_batch_compact when a filter flagged features for deletion.
+// plus k_batch_compact when a filter flagged features for deletion or, with cfg.xyz_conversion, has
+// inverse-depth features to convert to XYZ (convert2XYZ_ifLinearAll, V:1317): k_batch_update decides the
+// conversions, k_batch_compact applies removals and conversions in one pass over Sigma.
 // Every stage evaluates the same expressions as the single-filter kernels (same device functions).
 #include <algorithm>
 #include <cstdio>
@@ -39,7 +41,29 @@ struct BatchView {
   int* N;               // [B] feature count
   long long sstride;    // doubles between consecutive filters' Sigma
   int ld, Ncap, tstride;
+  // XYZ conversions decided for the next k_batch_compact, kept out of FeatTab (single filters have their own arrays)
+  int* xyz_flag;        // [B][Ncap] feature converts
+  double* xyz_J;        // [B][Ncap][18] its 3 x 6 Jacobian
+  double* xyz_y;        // [B][Ncap][3] its XYZ point
+  int* xyz_count;       // [B] conversions pending (k_batch_compact resets it)
 };
+
+// convert2XYZ_ifLinear's decision (V:741-772, xyz_linear_decide) for feature i = lane of filter b, if `eligible` and still
+// in inverse depth.  Called by the whole of warp 0 (N <= BNCAP = 32); lane 0 stores the filter's count.
+__device__ void warp_xyz_decide(const BatchView& bv, int b, const double* Sigma, const double* mu, const FeatTab& ft, int N,
+                                bool eligible, const DevCfg& cfg) {
+  const int i = threadIdx.x;
+  const size_t k = (size_t)b * bv.Ncap + i;
+  int conv = 0;
+  if (eligible && i < N && !ft.coding[i]) {
+    const int pos = ft.pos[i];
+    conv = xyz_linear_decide(mu + pos, mu, Sigma[(size_t)(pos + 5) * bv.ld + pos + 5], cfg.linearity_threshold,
+                             cfg.abs_int_quirk, bv.xyz_y + 3 * k, bv.xyz_J + 18 * k);
+  }
+  if (i < N) bv.xyz_flag[k] = conv;
+  const int cnt = __popc(__ballot_sync(0xffffffffu, conv));
+  if (i == 0) bv.xyz_count[b] = cnt;
+}
 
 // ------------------------------------------------------------------------------------------------
 // predict for one filter per CTA: same arithmetic as k_predict_cov / k_predict_features / k_predict_S2
@@ -385,7 +409,7 @@ __device__ void cta_stacked_update(const UpdSmem& sm, double* __restrict__ Sigma
 __global__ void __launch_bounds__(BUPD_THREADS, 1) k_batch_update(BatchView bv, DevCfg cfg, const uint32_t* __restrict__ picks,
                                                                   int n_picks, double* __restrict__ out_mu14,
                                                                   double* __restrict__ out_S14, int* __restrict__ out_stats,
-                                                                  int min_features, int max_features) {
+                                                                  int min_features, int max_features, int xyz_conversion) {
   extern __shared__ __align__(16) double usm[];
   UpdSmem sm;
   sm.W = usm;
@@ -488,39 +512,67 @@ __global__ void __launch_bounds__(BUPD_THREADS, 1) k_batch_update(BatchView bv, 
     st[EKF_BSTAT_HI] = n_hi; st[EKF_BSTAT_HYPS] = ctl->ransac_hyps; st[EKF_BSTAT_CHOL_FAIL] = ctl->chol_fail;
     st[EKF_BSTAT_REMOVED] = removed; st[EKF_BSTAT_TOPUP] = topup;
   }
+  // convert2XYZ_ifLinearAll (V:1317) of the features that survive this step: not flagged, and not the removeFeature(0)
+  // victim, the first unflagged feature (V:1312-1313).  The reference removes, then converts; deciding here, on the
+  // pre-removal state, gives the same decisions: removal moves entries without changing a value, and the linearity index
+  // reads only the feature's own mu entries, the camera position mu[0:3] and the feature's own rho variance.
+  // k_batch_compact then applies removals and conversions together.
+  if (xyz_conversion && tid < 32) {
+    const bool alive = tid < N && !ft.removef[tid];
+    const unsigned alive_mask = __ballot_sync(0xffffffffu, alive);
+    const bool drop_first = (n_vis < min_features) && (N - n_rem > max_features);
+    const int victim = drop_first ? __ffs(alive_mask) - 1 : -1;
+    warp_xyz_decide(bv, b, Sigma, mu, ft, N, alive && tid != victim, cfg);
+  }
 }
 
 // ------------------------------------------------------------------------------------------------
-// removeFeature (V:373-421) for every flagged feature of every filter that has any: Sigma / mu are
-// compacted through the filter's slice of the scratch buffer, the feature table through registers.
+// removeFeature (V:373-421) for every flagged feature (remove != 0) and convert2XYZ_ifLinear (V:741-772) for every
+// feature decided in bv.xyz_flag, of every filter that has either, in one pass: Sigma / mu are rebuilt through the
+// filter's slice of the scratch buffer, the feature table through registers.  The row map carries (src, code) as in
+// k_xyz_apply: code < 0 copies old entry src, code = 4 f + x is row x of converted feature f (old index).  Removal keeps
+// the order of the survivors, so J Sigma J^T over the survivors' rows (xyz_apply_entry) is bit for bit the reference's
+// removals followed by its one-at-a-time conversions.  A filter with nothing to do returns at once.
 // ------------------------------------------------------------------------------------------------
 #define BCMP_THREADS 256
 __global__ void __launch_bounds__(BCMP_THREADS) k_batch_compact(BatchView bv, double* __restrict__ scratch, int min_features,
-                                                                int max_features) {
-  __shared__ int keep[BNCAP], newpos[BNCAP], map[BNMAX];
+                                                                int max_features, int remove) {
+  __shared__ int keep[BNCAP], newpos[BNCAP], conv[BNCAP];
+  __shared__ int2 rmap[BNMAX];
   __shared__ int s_N2, s_n2;
   const int b = blockIdx.x, tid = threadIdx.x;
   DevCtl* ctl = bv.ctl + b;
-  if (ctl->n_remove <= 0) return;
-  const int n = bv.n[b], N = bv.N[b], ld = bv.ld;
+  const bool rem = remove && ctl->n_remove > 0;
+  const int nconv = bv.xyz_count[b];
+  if (!rem && nconv <= 0) return;
+  const int N = bv.N[b], ld = bv.ld;
   double* Sigma = bv.Sigma + (size_t)b * bv.sstride;
   double* tmp = scratch + (size_t)b * bv.sstride;
   double* mu = bv.mu + (size_t)b * ld;
   const FeatTab ft = feattab_slice(bv.ft, b, bv.Ncap, bv.tstride);
+  const int* cflag = bv.xyz_flag + (size_t)b * bv.Ncap;
+  const double* Jall = bv.xyz_J + (size_t)b * bv.Ncap * 18;
+  const double* yall = bv.xyz_y + (size_t)b * bv.Ncap * 3;
   if (tid == 0) {
     int flagged = 0;
-    for (int f = 0; f < N; ++f) flagged += ft.removef[f] ? 1 : 0;
+    if (rem)
+      for (int f = 0; f < N; ++f) flagged += ft.removef[f] ? 1 : 0;
     // removeFeature(0) after the flagged ones are gone (V:1312-1313): first survivor
-    const bool drop_first = (ctl->n_visible < min_features) && (N - flagged > max_features);
+    const bool drop_first = rem && (ctl->n_visible < min_features) && (N - flagged > max_features);
     int N2 = 0, n2 = EKF_CAM;
     bool dropped = false;
-    for (int i = 0; i < EKF_CAM; ++i) map[i] = i;
+    for (int i = 0; i < EKF_CAM; ++i) rmap[i] = make_int2(i, -1);
     for (int f = 0; f < N; ++f) {
-      if (ft.removef[f]) continue;
+      if (rem && ft.removef[f]) continue;
       if (drop_first && !dropped) { dropped = true; continue; }
-      const int fs = ft.coding[f] ? 3 : 6;
-      keep[N2] = f; newpos[N2] = n2; ++N2;
-      for (int c = 0; c < fs; ++c) map[n2++] = ft.pos[f] + c;
+      const int cv = nconv > 0 && cflag[f];
+      keep[N2] = f; newpos[N2] = n2; conv[N2] = cv; ++N2;
+      if (cv) {
+        for (int x = 0; x < 3; ++x) rmap[n2++] = make_int2(ft.pos[f], 4 * f + x);
+      } else {
+        const int fs = ft.coding[f] ? 3 : 6;
+        for (int c = 0; c < fs; ++c) rmap[n2++] = make_int2(ft.pos[f] + c, -1);
+      }
     }
     s_N2 = N2; s_n2 = n2;
   }
@@ -528,10 +580,13 @@ __global__ void __launch_bounds__(BCMP_THREADS) k_batch_compact(BatchView bv, do
   const int N2 = s_N2, n2 = s_n2;
   for (int e = tid; e < n2 * n2; e += BCMP_THREADS) {
     const int i = e / n2, j = e - i * n2;
-    tmp[(size_t)i * ld + j] = Sigma[(size_t)map[i] * ld + map[j]];
+    tmp[(size_t)i * ld + j] = xyz_apply_entry(Sigma, ld, rmap[i], rmap[j], Jall);
   }
   double mv = 0.0;
-  if (tid < n2) mv = mu[map[tid]];   // n2 <= 206 <= BCMP_THREADS
+  if (tid < n2) {   // n2 <= 206 <= BCMP_THREADS
+    const int2 r = rmap[tid];
+    mv = (r.y < 0) ? mu[r.x] : yall[3 * (r.y >> 2) + (r.y & 3)];
+  }
   __syncthreads();
   for (int e = tid; e < n2 * n2; e += BCMP_THREADS) {
     const int i = e / n2, j = e - i * n2;
@@ -553,7 +608,7 @@ __global__ void __launch_bounds__(BCMP_THREADS) k_batch_compact(BatchView bv, do
   }
   __syncthreads();
   if (tid < N2) {
-    ft.pos[tid] = newpos[tid]; ft.coding[tid] = iv[0]; ft.innov[tid] = iv[1]; ft.li[tid] = iv[2]; ft.hi[tid] = iv[3];
+    ft.pos[tid] = newpos[tid]; ft.coding[tid] = conv[tid] ? 1 : iv[0]; ft.innov[tid] = iv[1]; ft.li[tid] = iv[2]; ft.hi[tid] = iv[3];
     ft.removef[tid] = iv[4]; ft.n_tot[tid] = iv[5]; ft.n_find[tid] = iv[6]; ft.real_index[tid] = iv[7]; ft.pos_in_z[tid] = iv[8];
     ft.center[2 * tid] = fv[0]; ft.center[2 * tid + 1] = fv[1]; ft.quality[tid] = fv[2]; ft.last_ncc[tid] = fv[3];
     for (int c = 0; c < 2; ++c) { ft.z[2 * tid + c] = dv[c]; ft.h[2 * tid + c] = dv[2 + c]; }
@@ -576,7 +631,18 @@ __global__ void __launch_bounds__(BCMP_THREADS) k_batch_compact(BatchView bv, do
     }
     __syncthreads();
   }
-  if (tid == 0) { bv.n[b] = n2; bv.N[b] = N2; ctl->n_remove = 0; }
+  if (tid == 0) {
+    bv.n[b] = n2; bv.N[b] = N2; bv.xyz_count[b] = 0;
+    if (remove) ctl->n_remove = 0;
+  }
+}
+
+// convert2XYZ_ifLinearAll (V:776-780) outside a step: the decisions of every filter, one CTA per filter, one thread per
+// feature; k_batch_compact (remove = 0) applies them.
+__global__ void __launch_bounds__(BNCAP) k_batch_xyz_decide(BatchView bv, DevCfg cfg) {
+  const int b = blockIdx.x;
+  const FeatTab ft = feattab_slice(bv.ft, b, bv.Ncap, bv.tstride);
+  warp_xyz_decide(bv, b, bv.Sigma + (size_t)b * bv.sstride, bv.mu + (size_t)b * bv.ld, ft, bv.N[b], true, cfg);
 }
 
 // seed: every filter <- the single filter `src`
@@ -628,6 +694,7 @@ struct ekf_batch {
   int* out_stats = nullptr;
   double *h_mu14 = nullptr, *h_S14 = nullptr;   // pinned
   int* h_stats = nullptr;                       // pinned
+  int* h_xyz_count = nullptr;                   // pinned mirror of bv.xyz_count
   int *h_n = nullptr, *h_N = nullptr;           // pinned mirrors of bv.n / bv.N
   double* stage_mu14 = nullptr;                 // device staging for set_camera_states
   double dT = 1.0, old_ts = -1.0;
@@ -667,6 +734,7 @@ int ekf_batch_destroy(ekf_batch* b) {
   cudaFree(t.n_tot); cudaFree(t.n_find); cudaFree(t.real_index); cudaFree(t.pos_in_z); cudaFree(t.sel);
   cudaFree(t.center); cudaFree(t.quality); cudaFree(t.last_ncc); cudaFree(t.z); cudaFree(t.h); cudaFree(t.Hc);
   cudaFree(t.S2); cudaFree(t.patch); cudaFree(t.mpatch);
+  cudaFree(b->bv.xyz_flag); cudaFree(b->bv.xyz_J); cudaFree(b->bv.xyz_y); cudaFree(b->bv.xyz_count);
   cudaFree(b->bv.Sigma); cudaFree(b->bv.mu); cudaFree(b->bv.ctl); cudaFree(b->bv.n); cudaFree(b->bv.N);
   cudaFree(b->match_defer);
   cudaFree(b->scratch); cudaFree(b->frame); cudaFree(b->picks_dev); cudaFree(b->out_mu14); cudaFree(b->out_S14);
@@ -674,6 +742,7 @@ int ekf_batch_destroy(ekf_batch* b) {
   if (b->h_mu14) cudaFreeHost(b->h_mu14);
   if (b->h_S14) cudaFreeHost(b->h_S14);
   if (b->h_stats) cudaFreeHost(b->h_stats);
+  if (b->h_xyz_count) cudaFreeHost(b->h_xyz_count);
   if (b->h_n) cudaFreeHost(b->h_n);
   if (b->h_N) cudaFreeHost(b->h_N);
   for (auto& e : b->ev) if (e) cudaEventDestroy(e);
@@ -686,7 +755,7 @@ int ekf_batch_create(const ekf_config* cfg, int n_filters, int feature_capacity,
   if (!cfg || !out || n_filters < 1 || feature_capacity < 1) return EKF_ERR_ARG;
   *out = nullptr;
   if (feature_capacity > BNCAP) return EKF_ERR_CAPACITY;
-  if (cfg->kernel_size < 100000 || cfg->scale != 1 || cfg->forsePlane != 0 || cfg->xyz_conversion != 0) return EKF_ERR_UNSUPPORTED;
+  if (cfg->kernel_size < 100000 || cfg->scale != 1 || cfg->forsePlane != 0) return EKF_ERR_UNSUPPORTED;
   if (cfg->window_size < 3 || cfg->window_size > 31 || cfg->search_clamp > 20 || cfg->search_clamp < 0) return EKF_ERR_UNSUPPORTED;
   int ndev = 0;
   if (cudaGetDeviceCount(&ndev) != cudaSuccess || device < 0 || device >= ndev) return EKF_ERR_CUDA;
@@ -719,15 +788,18 @@ int ekf_batch_create(const ekf_config* cfg, int n_filters, int feature_capacity,
   TRY(balloc(&t.pos_in_z, cap)) TRY(balloc(&t.sel, cap)) TRY(balloc(&t.center, 2 * cap)) TRY(balloc(&t.quality, cap))
   TRY(balloc(&t.last_ncc, cap)) TRY(balloc(&t.z, 2 * cap)) TRY(balloc(&t.h, 2 * cap)) TRY(balloc(&t.Hc, 26 * cap))
   TRY(balloc(&t.S2, 4 * cap)) TRY(balloc(&t.patch, cap * w2)) TRY(balloc(&t.mpatch, cap * w2))
+  TRY(balloc(&v.xyz_flag, cap)) TRY(balloc(&v.xyz_J, 18 * cap)) TRY(balloc(&v.xyz_y, 3 * cap)) TRY(balloc(&v.xyz_count, Bn))
   TRY(balloc(&b->out_mu14, Bn * 14)) TRY(balloc(&b->out_S14, Bn * 196)) TRY(balloc(&b->out_stats, Bn * EKF_BATCH_STAT_FIELDS))
   TRY(balloc(&b->stage_mu14, Bn * 14))
   TRY(cudaMallocHost((void**)&b->h_mu14, sizeof(double) * Bn * 14)) TRY(cudaMallocHost((void**)&b->h_S14, sizeof(double) * Bn * 196))
   TRY(cudaMallocHost((void**)&b->h_stats, sizeof(int) * Bn * EKF_BATCH_STAT_FIELDS))
   TRY(cudaMallocHost((void**)&b->h_n, sizeof(int) * Bn)) TRY(cudaMallocHost((void**)&b->h_N, sizeof(int) * Bn))
+  TRY(cudaMallocHost((void**)&b->h_xyz_count, sizeof(int) * Bn))
   TRY(cudaMemsetAsync(v.Sigma, 0, sizeof(double) * Bn * v.sstride, b->stream))
   TRY(cudaMemsetAsync(v.mu, 0, sizeof(double) * Bn * b->ld, b->stream))
   TRY(cudaMemsetAsync(v.ctl, 0, sizeof(DevCtl) * Bn, b->stream))
   TRY(cudaMemsetAsync(v.n, 0, sizeof(int) * Bn, b->stream)) TRY(cudaMemsetAsync(v.N, 0, sizeof(int) * Bn, b->stream))
+  TRY(cudaMemsetAsync(v.xyz_count, 0, sizeof(int) * Bn, b->stream))
   for (auto& evn : b->ev) TRY(cudaEventCreate(&evn))
   TRY(cudaStreamSynchronize(b->stream))
 #undef TRY
@@ -852,22 +924,25 @@ int ekf_batch_step(ekf_batch* b, const double dv[3], const double dw[3], int vco
                             b->match_defer + (size_t)b->B * b->Ncap, &b->launches);
   BCHECK(cudaEventRecord(b->ev[2], st));
   k_batch_update<<<b->B, BUPD_THREADS, kUpdSmemBytes, st>>>(b->bv, b->dcfg, b->picks_dev, n_picks, b->out_mu14, b->out_S14,
-                                                            b->out_stats, b->cfg.min_features, b->cfg.max_features);
+                                                            b->out_stats, b->cfg.min_features, b->cfg.max_features,
+                                                            b->cfg.xyz_conversion);
   b->launches += 1;
   BCHECK(cudaEventRecord(b->ev[3], st));
   BCHECK(cudaGetLastError());
   const size_t Bn = (size_t)b->B;
   BCHECK(cudaMemcpyAsync(b->h_stats, b->out_stats, sizeof(int) * Bn * EKF_BATCH_STAT_FIELDS, cudaMemcpyDeviceToHost, st));
   BCHECK(cudaMemcpyAsync(b->h_mu14, b->out_mu14, sizeof(double) * Bn * 14, cudaMemcpyDeviceToHost, st));
+  if (b->cfg.xyz_conversion) BCHECK(cudaMemcpyAsync(b->h_xyz_count, b->bv.xyz_count, sizeof(int) * Bn, cudaMemcpyDeviceToHost, st));
   BCHECK(cudaStreamSynchronize(st));
   b->results_valid = true;
-  long long removed = 0, fails = 0;
+  long long removed = 0, converted = 0, fails = 0;
   for (size_t i = 0; i < Bn; ++i) {
     removed += b->h_stats[i * EKF_BATCH_STAT_FIELDS + EKF_BSTAT_REMOVED];
     fails += b->h_stats[i * EKF_BATCH_STAT_FIELDS + EKF_BSTAT_CHOL_FAIL];
+    if (b->cfg.xyz_conversion) converted += b->h_xyz_count[i];
   }
-  if (removed > 0) {
-    k_batch_compact<<<b->B, BCMP_THREADS, 0, st>>>(b->bv, b->scratch, b->cfg.min_features, b->cfg.max_features);
+  if (removed > 0 || converted > 0) {   // removals, then convert2XYZ_ifLinearAll (V:1312-1317), in one pass
+    k_batch_compact<<<b->B, BCMP_THREADS, 0, st>>>(b->bv, b->scratch, b->cfg.min_features, b->cfg.max_features, 1);
     b->launches += 1;
     BCHECK(cudaGetLastError());
     BCHECK(cudaMemcpyAsync(b->h_n, b->bv.n, sizeof(int) * Bn, cudaMemcpyDeviceToHost, st));
@@ -875,6 +950,29 @@ int ekf_batch_step(ekf_batch* b, const double dv[3], const double dw[3], int vco
     BCHECK(cudaStreamSynchronize(st));
   }
   if (fails > 0) return bfail(b, EKF_ERR_STATE, "innovation covariance not positive definite in at least one filter");
+  return EKF_OK;
+}
+
+int ekf_batch_convert2xyz_if_linear_all(ekf_batch* b) {
+  if (!b) return EKF_ERR_ARG;
+  if (!b->seeded) return bfail(b, EKF_ERR_STATE, "convert2XYZ_ifLinearAll before ekf_batch_seed_from");
+  BCHECK(cudaSetDevice(b->device));
+  cudaStream_t st = b->stream;
+  const size_t Bn = (size_t)b->B;
+  k_batch_xyz_decide<<<b->B, BNCAP, 0, st>>>(b->bv, b->dcfg);
+  b->launches += 1;
+  BCHECK(cudaGetLastError());
+  BCHECK(cudaMemcpyAsync(b->h_xyz_count, b->bv.xyz_count, sizeof(int) * Bn, cudaMemcpyDeviceToHost, st));
+  BCHECK(cudaStreamSynchronize(st));
+  long long converted = 0;
+  for (size_t i = 0; i < Bn; ++i) converted += b->h_xyz_count[i];
+  if (converted == 0) return EKF_OK;
+  k_batch_compact<<<b->B, BCMP_THREADS, 0, st>>>(b->bv, b->scratch, b->cfg.min_features, b->cfg.max_features, 0);
+  b->launches += 1;
+  BCHECK(cudaGetLastError());
+  BCHECK(cudaMemcpyAsync(b->h_n, b->bv.n, sizeof(int) * Bn, cudaMemcpyDeviceToHost, st));
+  BCHECK(cudaMemcpyAsync(b->h_N, b->bv.N, sizeof(int) * Bn, cudaMemcpyDeviceToHost, st));
+  BCHECK(cudaStreamSynchronize(st));
   return EKF_OK;
 }
 

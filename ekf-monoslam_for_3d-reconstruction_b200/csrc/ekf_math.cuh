@@ -299,3 +299,71 @@ __host__ __device__ __forceinline__ void d_inv2_pplu(const double A[4], double X
   for (int j = 0; j < 2; ++j) { x0[j] -= a01 * x1[j]; x0[j] = x0[j] / a00; }
   X[0] = x0[0]; X[1] = x0[1]; X[2] = x1[0]; X[3] = x1[1];
 }
+
+// ---- convert2XYZ_ifLinear (V:741-772) -----------------------------------------------------------------------------------
+// Shared by the single filter (k_xyz_decide / k_xyz_apply), the batched filters (ekf_batch.cu) and a host test harness.
+//
+// Linearity test of inverseDepth2XyzWorld (V:690-738) for the inverse-depth feature f[6] seen from the camera position r[3];
+// sigma_rho is Sigma(pos + 5, pos + 5).  Returns 1 if the feature converts and then writes its XYZ point y[3] and the 3 x 6
+// Jacobian J (row-major); otherwise writes nothing.  QUIRKS kept: the rho VARIANCE is used as a sigma (V:717); bare
+// abs(float) (V:719) is fabs unless abs_int_quirk.
+__host__ __device__ inline int xyz_linear_decide(const double* f, const double* r, double sigma_rho, double threshold,
+                                                 int abs_int_quirk, double* y, double* J) {
+  const double theta = f[3], phi = f[4], ro = f[5];
+  double m[3], yy[3], d[3];
+  m[0] = sin(theta) * cos(phi);
+  m[1] = -sin(phi);
+  m[2] = cos(theta) * cos(phi);
+  for (int c = 0; c < 3; ++c) yy[c] = f[c] + m[c] / ro;
+  for (int c = 0; c < 3; ++c) d[c] = yy[c] - r[c];
+  double t = 0;
+  for (int c = 0; c < 3; ++c) t += d[c] * m[c];
+  const double at = abs_int_quirk ? (double)abs((int)t) : fabs(t);
+  const double L_d = 4 * sigma_rho * at / (ro * ro * (d[0] * d[0] + d[1] * d[1] + d[2] * d[2]));
+  if (!(L_d < threshold)) return 0;
+  for (int c = 0; c < 18; ++c) J[c] = 0;
+  for (int c = 0; c < 3; ++c) J[c * 6 + c] = 1;
+  J[0 * 6 + 3] = cos(theta) * cos(phi) / ro;
+  J[1 * 6 + 3] = 0;
+  J[2 * 6 + 3] = -sin(theta) * cos(phi) / ro;
+  J[0 * 6 + 4] = -sin(theta) * sin(phi) / ro;
+  J[1 * 6 + 4] = -cos(phi) / ro;
+  J[2 * 6 + 4] = -cos(theta) * sin(phi) / ro;
+  for (int c = 0; c < 3; ++c) J[c * 6 + 5] = -m[c] / (ro * ro);
+  for (int c = 0; c < 3; ++c) y[c] = yy[c];
+  return 1;
+}
+
+// Entry (i, j) of Sigma' = J Sigma J^T for any number of conversions at once, in the reference's association (one
+// conversion after the other): the sum over the EARLIER-converted feature's six entries is the inner one.  ri / rj are the
+// row-map entries of i and j, (src, code): code < 0 is the plain state entry src; code = 4 f + x is row x of converted
+// feature f, whose old 6-entry block starts at src and whose Jacobian is Jall[18 f .. 18 f + 17].  Features keep their
+// relative order in the map, so "earlier" is the smaller f.
+__host__ __device__ inline double xyz_apply_entry(const double* src, int ld, int2 ri, int2 rj, const double* Jall) {
+  if (ri.y < 0 && rj.y < 0) return src[(size_t)ri.x * ld + rj.x];
+  double v = 0;
+  if (ri.y >= 0 && rj.y < 0) {                // (J Sigma)[i, j]
+    const double* Jr = Jall + 18 * (ri.y >> 2) + 6 * (ri.y & 3);
+    for (int a = 0; a < 6; ++a) v += Jr[a] * src[(size_t)(ri.x + a) * ld + rj.x];
+  } else if (ri.y < 0) {                      // (Sigma J^T)[i, j]
+    const double* Jc = Jall + 18 * (rj.y >> 2) + 6 * (rj.y & 3);
+    for (int b = 0; b < 6; ++b) v += src[(size_t)ri.x * ld + rj.x + b] * Jc[b];
+  } else {
+    const double* Jr = Jall + 18 * (ri.y >> 2) + 6 * (ri.y & 3);
+    const double* Jc = Jall + 18 * (rj.y >> 2) + 6 * (rj.y & 3);
+    if ((ri.y >> 2) <= (rj.y >> 2)) {         // row feature converted first (or diagonal block): (J_r Sigma) J_c^T
+      for (int b = 0; b < 6; ++b) {
+        double t = 0;
+        for (int a = 0; a < 6; ++a) t += Jr[a] * src[(size_t)(ri.x + a) * ld + rj.x + b];
+        v += t * Jc[b];
+      }
+    } else {                                  // column feature converted first: J_r (Sigma J_c^T)
+      for (int a = 0; a < 6; ++a) {
+        double t = 0;
+        for (int b = 0; b < 6; ++b) t += src[(size_t)(ri.x + a) * ld + rj.x + b] * Jc[b];
+        v += Jr[a] * t;
+      }
+    }
+  }
+  return v;
+}

@@ -513,8 +513,8 @@ __global__ void k_gather_features(FeatTab src, FeatTab dst, int N2, const int* _
 // Decisions for all inverse-depth features are taken at once from the pre-conversion state: a
 // conversion only touches its own 6 rows / columns (J is the identity elsewhere), so the linearity
 // index of a later feature (its own state, mu[0:3] and Sigma[pos+5,pos+5]) is unaffected by earlier
-// conversions of the same call.  QUIRKS kept: the rho VARIANCE is used as a sigma (V:717); bare
-// abs(float) (V:719) is fabs unless cfg.abs_int_quirk.
+// conversions of the same call.  The arithmetic (quirks included) is xyz_linear_decide / xyz_apply_entry
+// in ekf_math.cuh.
 // ------------------------------------------------------------------------------------------------
 __global__ void __launch_bounds__(128) k_xyz_decide(const double* __restrict__ Sigma, int ld, const double* __restrict__ mu,
                                                     FeatTab ft, int N, DevCfg cfg, int only, int* __restrict__ flag,
@@ -524,76 +524,21 @@ __global__ void __launch_bounds__(128) k_xyz_decide(const double* __restrict__ S
   int conv = 0;
   if (!ft.coding[i] && (only < 0 || only == i)) {
     const int pos = ft.pos[i];
-    double f[6];
+    double f[6], r[3];
     for (int c = 0; c < 6; ++c) f[c] = mu[pos + c];
-    const double theta = f[3], phi = f[4], ro = f[5];
-    double m[3], y[3], d[3];
-    m[0] = sin(theta) * cos(phi);
-    m[1] = -sin(phi);
-    m[2] = cos(theta) * cos(phi);
-    for (int c = 0; c < 3; ++c) y[c] = f[c] + m[c] / ro;
-    for (int c = 0; c < 3; ++c) d[c] = y[c] - mu[c];
-    const double sigma_rho = Sigma[(size_t)(pos + 5) * ld + pos + 5];
-    double t = 0;
-    for (int c = 0; c < 3; ++c) t += d[c] * m[c];
-    const double at = cfg.abs_int_quirk ? (double)abs((int)t) : fabs(t);
-    const double L_d = 4 * sigma_rho * at / (ro * ro * (d[0] * d[0] + d[1] * d[1] + d[2] * d[2]));
-    conv = (L_d < cfg.linearity_threshold) ? 1 : 0;
-    if (conv) {
-      double* J = Jout + 18 * i;
-      for (int c = 0; c < 18; ++c) J[c] = 0;
-      for (int c = 0; c < 3; ++c) J[c * 6 + c] = 1;
-      J[0 * 6 + 3] = cos(theta) * cos(phi) / ro;
-      J[1 * 6 + 3] = 0;
-      J[2 * 6 + 3] = -sin(theta) * cos(phi) / ro;
-      J[0 * 6 + 4] = -sin(theta) * sin(phi) / ro;
-      J[1 * 6 + 4] = -cos(phi) / ro;
-      J[2 * 6 + 4] = -cos(theta) * sin(phi) / ro;
-      for (int c = 0; c < 3; ++c) J[c * 6 + 5] = -m[c] / (ro * ro);
-      for (int c = 0; c < 3; ++c) yout[3 * i + c] = y[c];
-    }
+    for (int c = 0; c < 3; ++c) r[c] = mu[c];
+    conv = xyz_linear_decide(f, r, Sigma[(size_t)(pos + 5) * ld + pos + 5], cfg.linearity_threshold, cfg.abs_int_quirk,
+                             yout + 3 * i, Jout + 18 * i);
   }
   flag[i] = conv;
 }
-// Sigma' = J Sigma J^T for all converted features at once, in the reference's association: the sum
-// over the EARLIER-converted feature's six entries is the inner one.  rmap[i'] = (src, code):
-// code < 0: plain state entry src; code = 4 f + x: row x of converted feature f whose old block starts at src.
+// Sigma' = J Sigma J^T for all converted features at once (xyz_apply_entry); rmap[i'] = (src, code).
 __global__ void k_xyz_apply(const double* __restrict__ src, double* __restrict__ dst, int ld, int n2, const int2* __restrict__ rmap,
                             const double* __restrict__ Jall) {
   const int j = blockIdx.x * blockDim.x + threadIdx.x;
   const int i = blockIdx.y;
   if (j >= n2) return;
-  const int2 ri = rmap[i], rj = rmap[j];
-  double v;
-  if (ri.y < 0 && rj.y < 0) {
-    v = src[(size_t)ri.x * ld + rj.x];
-  } else if (ri.y >= 0 && rj.y < 0) {         // (J Sigma)[i, j]
-    const double* Jr = Jall + 18 * (ri.y >> 2) + 6 * (ri.y & 3);
-    v = 0;
-    for (int a = 0; a < 6; ++a) v += Jr[a] * src[(size_t)(ri.x + a) * ld + rj.x];
-  } else if (ri.y < 0 && rj.y >= 0) {         // (Sigma J^T)[i, j]
-    const double* Jc = Jall + 18 * (rj.y >> 2) + 6 * (rj.y & 3);
-    v = 0;
-    for (int b = 0; b < 6; ++b) v += src[(size_t)ri.x * ld + rj.x + b] * Jc[b];
-  } else {
-    const double* Jr = Jall + 18 * (ri.y >> 2) + 6 * (ri.y & 3);
-    const double* Jc = Jall + 18 * (rj.y >> 2) + 6 * (rj.y & 3);
-    v = 0;
-    if ((ri.y >> 2) <= (rj.y >> 2)) {        // row feature converted first (or diagonal block): (J_r Sigma) J_c^T
-      for (int b = 0; b < 6; ++b) {
-        double t = 0;
-        for (int a = 0; a < 6; ++a) t += Jr[a] * src[(size_t)(ri.x + a) * ld + rj.x + b];
-        v += t * Jc[b];
-      }
-    } else {                                  // column feature converted first: J_r (Sigma J_c^T)
-      for (int a = 0; a < 6; ++a) {
-        double t = 0;
-        for (int b = 0; b < 6; ++b) t += src[(size_t)(ri.x + a) * ld + rj.x + b] * Jc[b];
-        v += Jr[a] * t;
-      }
-    }
-  }
-  dst[(size_t)i * ld + j] = v;
+  dst[(size_t)i * ld + j] = xyz_apply_entry(src, ld, rmap[i], rmap[j], Jall);
 }
 __global__ void k_xyz_mu(const double* __restrict__ musrc, double* __restrict__ mudst, int n2, const int2* __restrict__ rmap,
                          const double* __restrict__ yall) {

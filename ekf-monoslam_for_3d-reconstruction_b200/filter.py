@@ -343,6 +343,10 @@ class FilterBatch:
         a = np.asarray(dv, dtype=np.float64); b = np.asarray(dw, dtype=np.float64)
         self._ck(self.L.ekf_batch_step(self.h, _ptr(a), _ptr(b), int(bool(vcontrol)), _ptr(p), int(p.size)))
 
+    def convert2XYZ_ifLinearAll(self):
+        """vslamRansac.cpp:775-780 on every filter of the batch."""
+        self._ck(self.L.ekf_batch_convert2xyz_if_linear_all(self.h))
+
     def camera_states(self, want_sigma=False):
         mu = np.zeros((self.B, 14)); st = np.zeros((self.B, _abi.BATCH_STAT_FIELDS), dtype=np.int32)
         S = np.zeros((self.B, 14, 14)) if want_sigma else None

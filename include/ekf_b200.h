@@ -222,7 +222,11 @@ int ekf_match_batch(const uint8_t* frames, int n_frames, int width, int height, 
  * for the active search (:870-880).  All filters see the same frame (one camera, many hypotheses).
  * Every filter runs exactly the single-filter algorithm; there is no exchange between filters, so a
  * batch shards across GPUs by filter index with no collective (one ekf_batch per device / rank).
- * feature_capacity <= 32 (the stacked update of one filter is kept in shared memory). */
+ * A step ends like the single filter's update: feature deletion, then, when cfg.xyz_conversion is set,
+ * convert2XYZ_ifLinearAll (vslamRansac.cpp:1317) on every filter.  New features (findNewFeatures) are
+ * the caller's; EKF_BSTAT_TOPUP reports how many each filter asks for.
+ * feature_capacity <= 32 (the stacked update of one filter is kept in shared memory).  Motion blur
+ * (kernel_size < 100000), scale != 1 and forsePlane are not supported (EKF_ERR_UNSUPPORTED). */
 typedef struct ekf_batch ekf_batch;
 typedef struct ekf_batch_desc {
   int32_t n_filters, feature_capacity, state_capacity /* 14 + 6 * feature_capacity */, ld /* Sigma row stride */;
@@ -249,10 +253,12 @@ int ekf_batch_set_camera_states(ekf_batch* b, const double* mu14);
 /* captureNewFrame for the whole batch (vslamRansac.cpp:226-245): HOST / DEVICE source. */
 int ekf_batch_capture_frame(ekf_batch* b, const uint8_t* gray, int width, int height, int stride, double stamp);
 int ekf_batch_capture_frame_device(ekf_batch* b, const uint8_t* gray_dev, int width, int height, int stride, double stamp);
-/* predict + update (match, 1-point RANSAC, both corrections, book-keeping, feature deletion) for
- * every filter.  dv / dw / vcontrol as ekf_predict; picks as ekf_update (every filter draws from the
+/* predict + update (match, 1-point RANSAC, both corrections, book-keeping, feature deletion, XYZ
+ * conversion if cfg.xyz_conversion) for every filter.  dv / dw / vcontrol as ekf_predict; picks as ekf_update (every filter draws from the
  * same sequence).  Returns after the per-filter counters have reached the host. */
 int ekf_batch_step(ekf_batch* b, const double dv[3], const double dw[3], int vcontrol, const uint32_t* picks, int n_picks);
+/* convert2XYZ_ifLinearAll (vslamRansac.cpp:776-780) on every filter of the batch. */
+int ekf_batch_convert2xyz_if_linear_all(ekf_batch* b);
 /* Results of the last step, HOST output arrays: camera state (n_filters x 14), 14 x 14 covariance
  * block (n_filters x 196, may be NULL), counters (n_filters x EKF_BATCH_STAT_FIELDS, may be NULL). */
 int ekf_batch_get_camera_states(ekf_batch* b, double* mu14, double* sigma14, int32_t* stats);
