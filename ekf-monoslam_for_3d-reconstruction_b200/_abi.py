@@ -72,4 +72,5 @@ class EkfBatchDesc(C.Structure):
 
 
 BATCH_STAT_FIELDS = 8
+BATCH_MAX_CORNERS = 32   # EKF_BATCH_MAX_CORNERS
 BSTAT = dict(innov=0, matched=1, li=2, hi=3, hyps=4, chol_fail=5, removed=6, topup=7)

@@ -76,6 +76,12 @@ SIGNATURES = {
     "ekf_batch_get_full": (_i, [_vp, _i, _vp, _vp, _i]),
     "ekf_batch_set_full": (_i, [_vp, _i, _vp, _vp, _i]),
     "ekf_batch_get_feature": (_i, [_vp, _i, _i, _P(_abi.EkfFeatureInfo)]),
+    "ekf_batch_add_feature": (_i, [_vp, _i, _f, _f]),
+    "ekf_batch_detect_corners": (_i, [_vp, _vp, _vp, _vp]),
+    "ekf_batch_find_new_features": (_i, [_vp, _vp, _vp]),
+    "ekf_batch_set_topup": (_i, [_vp, _i]),
+    "ekf_batch_last_added": (_i, [_vp, _vp]),
+    "ekf_batch_get_template": (_i, [_vp, _i, _i, _i, _vp]),
     "ekf_batch_kernel_launches": (C.c_int64, [_vp]),
     "ekf_batch_last_step_ms": (_i, [_vp, _vp]),
     "ekf_batch_last_match_deferred": (_i, [_vp]),

@@ -13,7 +13,7 @@ from concurrent.futures import ThreadPoolExecutor
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 OUT = os.path.join(HERE, "libekf_b200.so")
-SOURCES = ["ekf_api.cu", "ekf_predict.cu", "ekf_match.cu", "ekf_update.cu", "ekf_gemm.cu", "ekf_batch.cu", "ekf_dist.cu", "ekf_detect.cu", "ekf_export.cu"]
+SOURCES = ["ekf_api.cu", "ekf_predict.cu", "ekf_match.cu", "ekf_update.cu", "ekf_gemm.cu", "ekf_batch.cu", "ekf_batch_detect.cu", "ekf_dist.cu", "ekf_detect.cu", "ekf_export.cu"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "--fmad=false", "-std=c++17",
               "-Xcompiler", "-fPIC", "-Xcompiler", "-Wall", "-diag-suppress", "550"]
 

@@ -12,7 +12,9 @@
 //                                   pipe (DMMA.8x8x4) straight from shared-memory V.
 // plus k_batch_compact when a filter flagged features for deletion or, with cfg.xyz_conversion, has
 // inverse-depth features to convert to XYZ (convert2XYZ_ifLinearAll, V:1317): k_batch_update decides the
-// conversions, k_batch_compact applies removals and conversions in one pass over Sigma.
+// conversions, k_batch_compact applies removals and conversions in one pass over Sigma.  With top-up on and a
+// filter asking for features (V:1312-1315), that filter's pass removes only; the batched detector
+// (ekf_batch_detect.cu) and k_batch_add then add its new features, and a second k_batch_compact converts.
 // Every stage evaluates the same expressions as the single-filter kernels (same device functions).
 #include <algorithm>
 #include <cstdio>
@@ -46,6 +48,7 @@ struct BatchView {
   double* xyz_J;        // [B][Ncap][18] its 3 x 6 Jacobian
   double* xyz_y;        // [B][Ncap][3] its XYZ point
   int* xyz_count;       // [B] conversions pending (k_batch_compact resets it)
+  int* patchnumbre;     // [B] real_index of the filter's next new feature (VSlamFilter::patchnumbre)
 };
 
 // convert2XYZ_ifLinear's decision (V:741-772, xyz_linear_decide) for feature i = lane of filter b, if `eligible` and still
@@ -535,24 +538,27 @@ __global__ void __launch_bounds__(BUPD_THREADS, 1) k_batch_update(BatchView bv, 
 // removals followed by its one-at-a-time conversions.  A filter with nothing to do returns at once.
 // ------------------------------------------------------------------------------------------------
 #define BCMP_THREADS 256
+// hold (stats of the step, or NULL): a filter whose EKF_BSTAT_TOPUP is set only removes here, and its pending decisions move
+// with the surviving records; the conversions follow its new features (ekf_batch_step).
 __global__ void __launch_bounds__(BCMP_THREADS) k_batch_compact(BatchView bv, double* __restrict__ scratch, int min_features,
-                                                                int max_features, int remove) {
+                                                                int max_features, int remove, const int* __restrict__ hold_stats) {
   __shared__ int keep[BNCAP], newpos[BNCAP], conv[BNCAP];
   __shared__ int2 rmap[BNMAX];
   __shared__ int s_N2, s_n2;
   const int b = blockIdx.x, tid = threadIdx.x;
   DevCtl* ctl = bv.ctl + b;
   const bool rem = remove && ctl->n_remove > 0;
-  const int nconv = bv.xyz_count[b];
+  const bool hold = hold_stats && hold_stats[(size_t)b * EKF_BATCH_STAT_FIELDS + EKF_BSTAT_TOPUP] > 0;
+  const int nconv = hold ? 0 : bv.xyz_count[b];
   if (!rem && nconv <= 0) return;
   const int N = bv.N[b], ld = bv.ld;
   double* Sigma = bv.Sigma + (size_t)b * bv.sstride;
   double* tmp = scratch + (size_t)b * bv.sstride;
   double* mu = bv.mu + (size_t)b * ld;
   const FeatTab ft = feattab_slice(bv.ft, b, bv.Ncap, bv.tstride);
-  const int* cflag = bv.xyz_flag + (size_t)b * bv.Ncap;
-  const double* Jall = bv.xyz_J + (size_t)b * bv.Ncap * 18;
-  const double* yall = bv.xyz_y + (size_t)b * bv.Ncap * 3;
+  int* cflag = bv.xyz_flag + (size_t)b * bv.Ncap;
+  double* Jall = bv.xyz_J + (size_t)b * bv.Ncap * 18;
+  double* yall = bv.xyz_y + (size_t)b * bv.Ncap * 3;
   if (tid == 0) {
     int flagged = 0;
     if (rem)
@@ -597,6 +603,7 @@ __global__ void __launch_bounds__(BCMP_THREADS) k_batch_compact(BatchView bv, do
   const int w16 = bv.tstride >> 4;
   int o = -1;
   int iv[10]; float fv[4]; double dv[8 + 26];
+  int hflag = 0; double hJ[18], hy[3];   // held decision of the record (hold only)
   if (tid < N2) {
     o = keep[tid];
     iv[0] = ft.coding[o]; iv[1] = ft.innov[o]; iv[2] = ft.li[o]; iv[3] = ft.hi[o]; iv[4] = ft.removef[o];
@@ -605,6 +612,11 @@ __global__ void __launch_bounds__(BCMP_THREADS) k_batch_compact(BatchView bv, do
     for (int c = 0; c < 2; ++c) { dv[c] = ft.z[2 * o + c]; dv[2 + c] = ft.h[2 * o + c]; }
     for (int c = 0; c < 4; ++c) dv[4 + c] = ft.S2[4 * o + c];
     for (int c = 0; c < 26; ++c) dv[8 + c] = ft.Hc[26 * o + c];
+    if (hold) {
+      hflag = cflag[o];
+      for (int c = 0; c < 18; ++c) hJ[c] = Jall[18 * o + c];
+      for (int c = 0; c < 3; ++c) hy[c] = yall[3 * o + c];
+    }
   }
   __syncthreads();
   if (tid < N2) {
@@ -614,6 +626,11 @@ __global__ void __launch_bounds__(BCMP_THREADS) k_batch_compact(BatchView bv, do
     for (int c = 0; c < 2; ++c) { ft.z[2 * tid + c] = dv[c]; ft.h[2 * tid + c] = dv[2 + c]; }
     for (int c = 0; c < 4; ++c) ft.S2[4 * tid + c] = dv[4 + c];
     for (int c = 0; c < 26; ++c) ft.Hc[26 * tid + c] = dv[8 + c];
+    if (hold) {
+      cflag[tid] = hflag;
+      for (int c = 0; c < 18; ++c) Jall[18 * tid + c] = hJ[c];
+      for (int c = 0; c < 3; ++c) yall[3 * tid + c] = hy[c];
+    }
   }
   // templates: records only move towards lower indices, in ascending order
   for (int f = 0; f < N2; ++f) {
@@ -632,7 +649,8 @@ __global__ void __launch_bounds__(BCMP_THREADS) k_batch_compact(BatchView bv, do
     __syncthreads();
   }
   if (tid == 0) {
-    bv.n[b] = n2; bv.N[b] = N2; bv.xyz_count[b] = 0;
+    bv.n[b] = n2; bv.N[b] = N2;
+    if (!hold) bv.xyz_count[b] = 0;
     if (remove) ctl->n_remove = 0;
   }
 }
@@ -645,9 +663,60 @@ __global__ void __launch_bounds__(BNCAP) k_batch_xyz_decide(BatchView bv, DevCfg
   warp_xyz_decide(bv, b, bv.Sigma + (size_t)b * bv.sstride, bv.mu + (size_t)b * bv.ld, ft, bv.N[b], true, cfg);
 }
 
+// addFeature (V:309-371) for the corners of every filter that has some (cnt[b] of them at xy + 2 * EKF_BATCH_MAX_CORNERS * b),
+// one CTA per filter, one add after the other in corner order with a barrier between adds: add j reads the rows add j - 1
+// wrote, exactly as consecutive ekf_add_feature calls do, and through the same device functions (ekf_math.cuh), so the
+// result is the single filter's bit for bit.  n <= 200 before an add, so one CTA covers every row.  one >= 0: filter `one`
+// adds the pixel (u, v) instead.  decide: the new features' convert2XYZ_ifLinear decisions join the ones k_batch_update
+// took for the filter's older features (adds change no entry their linearity test reads), for k_batch_compact to apply.
+#define BADD_THREADS 256
+__global__ void __launch_bounds__(BADD_THREADS) k_batch_add(BatchView bv, FrameView fr, DevCfg cfg, const float* __restrict__ xy,
+                                                            const int* __restrict__ cnt, int one, float u, float v, int decide) {
+  __shared__ double A[6 * 7], Ap[6 * 3], fnew[6], Tc[6 * 7];
+  const int b = one >= 0 ? one : blockIdx.x, tid = threadIdx.x;
+  const int k = one >= 0 ? 1 : cnt[b];
+  if (k <= 0) return;
+  const int ld = bv.ld, w = cfg.window, w2 = w * w;
+  double* Sigma = bv.Sigma + (size_t)b * bv.sstride;
+  double* mu = bv.mu + (size_t)b * ld;
+  const FeatTab ft = feattab_slice(bv.ft, b, bv.Ncap, bv.tstride);
+  int n = bv.n[b], N = bv.N[b], real = bv.patchnumbre[b];
+  const int N0 = N;
+  for (int j = 0; j < k; ++j) {
+    const float px = one >= 0 ? u : xy[(size_t)b * 2 * EKF_BATCH_MAX_CORNERS + 2 * j];
+    const float py = one >= 0 ? v : xy[(size_t)b * 2 * EKF_BATCH_MAX_CORNERS + 2 * j + 1];
+    if (tid == 0) add_feature_jacobians(cfg.cam, mu, px, py, cfg.rho_0, A, Ap, fnew);
+    __syncthreads();
+    if (tid < n) add_feature_cross(Sigma, ld, n, tid, A);
+    for (int e = tid; e < 42; e += BADD_THREADS) Tc[e] = add_feature_corner_T(Sigma, ld, A, e);   // rows / columns < 7: not written above
+    __syncthreads();
+    for (int e = tid; e < 36; e += BADD_THREADS)
+      Sigma[(size_t)(n + e / 6) * ld + n + e % 6] = add_feature_corner(Tc, A, Ap, e, cfg.sigma_pixel_2, cfg.sigma_rho_0);
+    if (tid < 6) mu[n + tid] = fnew[tid];
+    for (int e = tid; e < w2; e += BADD_THREADS) ft.patch[(size_t)N * cfg.tstride + e] = add_feature_template_px(fr, w, px, py, e);
+    if (tid == 0) add_feature_record(ft, N, n, px, py, real);
+    __syncthreads();
+    n += 6; N += 1; real += 1;
+  }
+  if (tid == 0) { bv.n[b] = n; bv.N[b] = N; bv.patchnumbre[b] = real; }
+  if (decide && tid < 32) {   // N <= BNCAP = 32
+    const int i = tid;
+    const size_t kk = (size_t)b * bv.Ncap + i;
+    int conv = 0;
+    if (i >= N0 && i < N) {
+      const int pos = ft.pos[i];
+      conv = xyz_linear_decide(mu + pos, mu, Sigma[(size_t)(pos + 5) * ld + pos + 5], cfg.linearity_threshold, cfg.abs_int_quirk,
+                               bv.xyz_y + 3 * kk, bv.xyz_J + 18 * kk);
+      bv.xyz_flag[kk] = conv;
+    }
+    const int c = __popc(__ballot_sync(0xffffffffu, conv));
+    if (i == 0) bv.xyz_count[b] += c;
+  }
+}
+
 // seed: every filter <- the single filter `src`
 __global__ void __launch_bounds__(256) k_batch_seed(BatchView bv, const double* __restrict__ Ssrc, int ld_src,
-                                                    const double* __restrict__ musrc, FeatTab src, int n, int N) {
+                                                    const double* __restrict__ musrc, FeatTab src, int n, int N, int patchnumbre) {
   const int b = blockIdx.x, tid = threadIdx.x;
   double* Sigma = bv.Sigma + (size_t)b * bv.sstride;
   double* mu = bv.mu + (size_t)b * bv.ld;
@@ -666,7 +735,7 @@ __global__ void __launch_bounds__(256) k_batch_seed(BatchView bv, const double* 
     for (int c = 0; c < 26; ++c) ft.Hc[26 * f + c] = src.Hc[26 * f + c];
   }
   for (int e = tid; e < N * bv.tstride; e += 256) { ft.patch[e] = src.patch[e]; ft.mpatch[e] = src.mpatch[e]; }
-  if (tid == 0) { bv.n[b] = n; bv.N[b] = N; bv.ctl[b] = DevCtl{}; }
+  if (tid == 0) { bv.n[b] = n; bv.N[b] = N; bv.ctl[b] = DevCtl{}; bv.patchnumbre[b] = patchnumbre; }
 }
 __global__ void k_batch_set_cam(BatchView bv, const double* __restrict__ mu14, int B) {
   const int e = blockIdx.x * blockDim.x + threadIdx.x;
@@ -697,8 +766,14 @@ struct ekf_batch {
   int* h_xyz_count = nullptr;                   // pinned mirror of bv.xyz_count
   int *h_n = nullptr, *h_N = nullptr;           // pinned mirrors of bv.n / bv.N
   double* stage_mu14 = nullptr;                 // device staging for set_camera_states
+  BatchDetectBufs det;                          // batched corner detection (ekf_batch_detect.cu)
+  float* det_xy = nullptr;                      // [B][EKF_BATCH_MAX_CORNERS][2] corners of the last detection
+  int *det_n = nullptr, *det_num = nullptr;     // [B] their count; [B] corners asked for (host num staged)
+  float* h_det_xy = nullptr;                    // pinned
+  int *h_det_n = nullptr, *h_num = nullptr;     // pinned
+  int* h_added = nullptr;                       // pinned: features each filter added in the last step / top-up call
   double dT = 1.0, old_ts = -1.0;
-  bool have_frame = false, seeded = false, results_valid = false;
+  bool have_frame = false, seeded = false, results_valid = false, topup = false;
   long long launches = 0;
   cudaEvent_t ev[4] = {nullptr, nullptr, nullptr, nullptr};
   std::string err;
@@ -738,7 +813,13 @@ int ekf_batch_destroy(ekf_batch* b) {
   cudaFree(b->bv.Sigma); cudaFree(b->bv.mu); cudaFree(b->bv.ctl); cudaFree(b->bv.n); cudaFree(b->bv.N);
   cudaFree(b->match_defer);
   cudaFree(b->scratch); cudaFree(b->frame); cudaFree(b->picks_dev); cudaFree(b->out_mu14); cudaFree(b->out_S14);
-  cudaFree(b->out_stats); cudaFree(b->stage_mu14);
+  cudaFree(b->out_stats); cudaFree(b->stage_mu14); cudaFree(b->bv.patchnumbre);
+  batch_detect_free(b->det);
+  cudaFree(b->det_xy); cudaFree(b->det_n); cudaFree(b->det_num);
+  if (b->h_det_xy) cudaFreeHost(b->h_det_xy);
+  if (b->h_det_n) cudaFreeHost(b->h_det_n);
+  if (b->h_num) cudaFreeHost(b->h_num);
+  if (b->h_added) cudaFreeHost(b->h_added);
   if (b->h_mu14) cudaFreeHost(b->h_mu14);
   if (b->h_S14) cudaFreeHost(b->h_S14);
   if (b->h_stats) cudaFreeHost(b->h_stats);
@@ -790,7 +871,11 @@ int ekf_batch_create(const ekf_config* cfg, int n_filters, int feature_capacity,
   TRY(balloc(&t.S2, 4 * cap)) TRY(balloc(&t.patch, cap * w2)) TRY(balloc(&t.mpatch, cap * w2))
   TRY(balloc(&v.xyz_flag, cap)) TRY(balloc(&v.xyz_J, 18 * cap)) TRY(balloc(&v.xyz_y, 3 * cap)) TRY(balloc(&v.xyz_count, Bn))
   TRY(balloc(&b->out_mu14, Bn * 14)) TRY(balloc(&b->out_S14, Bn * 196)) TRY(balloc(&b->out_stats, Bn * EKF_BATCH_STAT_FIELDS))
-  TRY(balloc(&b->stage_mu14, Bn * 14))
+  TRY(balloc(&b->stage_mu14, Bn * 14)) TRY(balloc(&v.patchnumbre, Bn))
+  TRY(balloc(&b->det_xy, Bn * 2 * EKF_BATCH_MAX_CORNERS)) TRY(balloc(&b->det_n, Bn)) TRY(balloc(&b->det_num, Bn))
+  TRY(cudaMallocHost((void**)&b->h_det_xy, sizeof(float) * Bn * 2 * EKF_BATCH_MAX_CORNERS))
+  TRY(cudaMallocHost((void**)&b->h_det_n, sizeof(int) * Bn)) TRY(cudaMallocHost((void**)&b->h_num, sizeof(int) * Bn))
+  TRY(cudaMallocHost((void**)&b->h_added, sizeof(int) * Bn))
   TRY(cudaMallocHost((void**)&b->h_mu14, sizeof(double) * Bn * 14)) TRY(cudaMallocHost((void**)&b->h_S14, sizeof(double) * Bn * 196))
   TRY(cudaMallocHost((void**)&b->h_stats, sizeof(int) * Bn * EKF_BATCH_STAT_FIELDS))
   TRY(cudaMallocHost((void**)&b->h_n, sizeof(int) * Bn)) TRY(cudaMallocHost((void**)&b->h_N, sizeof(int) * Bn))
@@ -803,7 +888,7 @@ int ekf_batch_create(const ekf_config* cfg, int n_filters, int feature_capacity,
   for (auto& evn : b->ev) TRY(cudaEventCreate(&evn))
   TRY(cudaStreamSynchronize(b->stream))
 #undef TRY
-  for (size_t i = 0; i < Bn; ++i) { b->h_n[i] = 0; b->h_N[i] = 0; }
+  for (size_t i = 0; i < Bn; ++i) { b->h_n[i] = 0; b->h_N[i] = 0; b->h_added[i] = 0; }
   DevCfg& d = b->dcfg;
   d.cam = CamParams{cfg->fx, cfg->fy, cfg->u0, cfg->v0, cfg->k1, cfg->k2, cfg->k3, cfg->p1, cfg->p2};
   d.Vmax[0] = cfg->sigma_vx * cfg->sigma_vx; d.Vmax[1] = cfg->sigma_vy * cfg->sigma_vy; d.Vmax[2] = cfg->sigma_vz * cfg->sigma_vz;
@@ -850,7 +935,7 @@ int ekf_batch_seed_from(ekf_batch* b, ekf_handle* src) {
   if (src->cfg.window_size != b->cfg.window_size) return bfail(b, EKF_ERR_ARG, "window_size differs");
   BCHECK(cudaSetDevice(b->device));
   BCHECK(cudaStreamSynchronize(src->stream));
-  k_batch_seed<<<b->B, 256, 0, b->stream>>>(b->bv, src->Sigma, src->ld, src->mu, src->ft, src->n, src->N);
+  k_batch_seed<<<b->B, 256, 0, b->stream>>>(b->bv, src->Sigma, src->ld, src->mu, src->ft, src->n, src->N, src->patchnumbre);
   b->launches += 1;
   BCHECK(cudaGetLastError());
   BCHECK(cudaStreamSynchronize(b->stream));
@@ -899,6 +984,29 @@ static int bcapture(ekf_batch* b, const uint8_t* gray, int width, int height, in
 int ekf_batch_capture_frame(ekf_batch* b, const uint8_t* g, int w, int h, int s, double stamp) { return bcapture(b, g, w, h, s, stamp, false); }
 int ekf_batch_capture_frame_device(ekf_batch* b, const uint8_t* g, int w, int h, int s, double stamp) { return bcapture(b, g, w, h, s, stamp, true); }
 
+// detection + adds for every filter, filter b asking for num[b * num_stride] corners (<= 0: none); decide: also take the new
+// features' XYZ decisions (in-step top-up).  Enqueued only.
+static int batch_topup(ekf_batch* b, const int* num, int num_stride, int decide) {
+  cudaStream_t st = b->stream;
+  BCHECK(batch_detect_reserve(b->det, (size_t)b->fv.w * b->fv.h, b->B));
+  BCHECK(launch_batch_detect(st, b->det, b->fv, b->bv.ft.center, b->bv.N, b->Ncap, b->B, b->cfg.window_size, num, num_stride, 1,
+                             b->det_xy, b->det_n, &b->launches));
+  k_batch_add<<<b->B, BADD_THREADS, 0, st>>>(b->bv, b->fv, b->dcfg, b->det_xy, b->det_n, -1, 0.0f, 0.0f, decide);
+  b->launches += 1;
+  BCHECK(cudaGetLastError());
+  return EKF_OK;
+}
+// n / N mirrors (and the per-filter add counts) back to the host: the one synchronisation of a top-up
+static int batch_readback(ekf_batch* b, bool added) {
+  cudaStream_t st = b->stream;
+  const size_t Bn = (size_t)b->B;
+  BCHECK(cudaMemcpyAsync(b->h_n, b->bv.n, sizeof(int) * Bn, cudaMemcpyDeviceToHost, st));
+  BCHECK(cudaMemcpyAsync(b->h_N, b->bv.N, sizeof(int) * Bn, cudaMemcpyDeviceToHost, st));
+  if (added) BCHECK(cudaMemcpyAsync(b->h_added, b->det_n, sizeof(int) * Bn, cudaMemcpyDeviceToHost, st));
+  BCHECK(cudaStreamSynchronize(st));
+  return EKF_OK;
+}
+
 int ekf_batch_step(ekf_batch* b, const double dv[3], const double dw[3], int vcontrol, const uint32_t* picks, int n_picks) {
   if (!b || n_picks < 0 || (n_picks > 0 && !picks)) return EKF_ERR_ARG;
   if (!b->seeded) return bfail(b, EKF_ERR_STATE, "batch step before ekf_batch_seed_from");
@@ -935,19 +1043,41 @@ int ekf_batch_step(ekf_batch* b, const double dv[3], const double dw[3], int vco
   if (b->cfg.xyz_conversion) BCHECK(cudaMemcpyAsync(b->h_xyz_count, b->bv.xyz_count, sizeof(int) * Bn, cudaMemcpyDeviceToHost, st));
   BCHECK(cudaStreamSynchronize(st));
   b->results_valid = true;
-  long long removed = 0, converted = 0, fails = 0;
+  long long removed = 0, converted = 0, fails = 0, topups = 0;
   for (size_t i = 0; i < Bn; ++i) {
     removed += b->h_stats[i * EKF_BATCH_STAT_FIELDS + EKF_BSTAT_REMOVED];
     fails += b->h_stats[i * EKF_BATCH_STAT_FIELDS + EKF_BSTAT_CHOL_FAIL];
+    topups += b->h_stats[i * EKF_BATCH_STAT_FIELDS + EKF_BSTAT_TOPUP] > 0;
     if (b->cfg.xyz_conversion) converted += b->h_xyz_count[i];
   }
-  if (removed > 0 || converted > 0) {   // removals, then convert2XYZ_ifLinearAll (V:1312-1317), in one pass
-    k_batch_compact<<<b->B, BCMP_THREADS, 0, st>>>(b->bv, b->scratch, b->cfg.min_features, b->cfg.max_features, 1);
-    b->launches += 1;
+  std::fill(b->h_added, b->h_added + Bn, 0);
+  if (!b->topup || topups == 0) {
+    if (removed > 0 || converted > 0) {   // removals, then convert2XYZ_ifLinearAll (V:1312-1317), in one pass
+      k_batch_compact<<<b->B, BCMP_THREADS, 0, st>>>(b->bv, b->scratch, b->cfg.min_features, b->cfg.max_features, 1, nullptr);
+      b->launches += 1;
+      BCHECK(cudaGetLastError());
+      BCHECK(cudaMemcpyAsync(b->h_n, b->bv.n, sizeof(int) * Bn, cudaMemcpyDeviceToHost, st));
+      BCHECK(cudaMemcpyAsync(b->h_N, b->bv.N, sizeof(int) * Bn, cudaMemcpyDeviceToHost, st));
+      BCHECK(cudaStreamSynchronize(st));
+    }
+  } else {
+    // The reference order (V:1312-1317): removals, findNewFeatures, convert2XYZ_ifLinearAll.  A filter that tops up must
+    // convert after its adds: the new feature's cross-covariance with a converted feature f is J (A Sigma[cam, f]) there,
+    // and converting first would give A (J Sigma[cam, f]), equal only up to rounding.  So its compaction removes only;
+    // every other filter keeps the fused pass.
+    if (removed > 0 || converted > 0) {
+      k_batch_compact<<<b->B, BCMP_THREADS, 0, st>>>(b->bv, b->scratch, b->cfg.min_features, b->cfg.max_features, 1, b->out_stats);
+      b->launches += 1;
+    }
+    int rc = batch_topup(b, b->out_stats + EKF_BSTAT_TOPUP, EKF_BATCH_STAT_FIELDS, b->cfg.xyz_conversion);
+    if (rc) return rc;
+    if (b->cfg.xyz_conversion) {   // the held conversions and the new features' (filters with none return at once)
+      k_batch_compact<<<b->B, BCMP_THREADS, 0, st>>>(b->bv, b->scratch, b->cfg.min_features, b->cfg.max_features, 0, nullptr);
+      b->launches += 1;
+    }
     BCHECK(cudaGetLastError());
-    BCHECK(cudaMemcpyAsync(b->h_n, b->bv.n, sizeof(int) * Bn, cudaMemcpyDeviceToHost, st));
-    BCHECK(cudaMemcpyAsync(b->h_N, b->bv.N, sizeof(int) * Bn, cudaMemcpyDeviceToHost, st));
-    BCHECK(cudaStreamSynchronize(st));
+    rc = batch_readback(b, true);
+    if (rc) return rc;
   }
   if (fails > 0) return bfail(b, EKF_ERR_STATE, "innovation covariance not positive definite in at least one filter");
   return EKF_OK;
@@ -967,7 +1097,7 @@ int ekf_batch_convert2xyz_if_linear_all(ekf_batch* b) {
   long long converted = 0;
   for (size_t i = 0; i < Bn; ++i) converted += b->h_xyz_count[i];
   if (converted == 0) return EKF_OK;
-  k_batch_compact<<<b->B, BCMP_THREADS, 0, st>>>(b->bv, b->scratch, b->cfg.min_features, b->cfg.max_features, 0);
+  k_batch_compact<<<b->B, BCMP_THREADS, 0, st>>>(b->bv, b->scratch, b->cfg.min_features, b->cfg.max_features, 0, nullptr);
   b->launches += 1;
   BCHECK(cudaGetLastError());
   BCHECK(cudaMemcpyAsync(b->h_n, b->bv.n, sizeof(int) * Bn, cudaMemcpyDeviceToHost, st));
@@ -1046,6 +1176,90 @@ int ekf_batch_get_feature(ekf_batch* b, int f, int idx, ekf_feature_info* o) {
   BCHECK(cudaStreamSynchronize(st));
   for (int a = 0; a < fs; ++a)
     for (int c = 0; c < fs; ++c) o->cov[a * 6 + c] = blk[a * fs + c];
+  return EKF_OK;
+}
+
+int ekf_batch_add_feature(ekf_batch* b, int f, float u, float v) {
+  if (!b || f < 0 || f >= b->B) return EKF_ERR_ARG;
+  if (!b->seeded) return bfail(b, EKF_ERR_STATE, "addFeature before ekf_batch_seed_from");
+  if (!b->have_frame) return bfail(b, EKF_ERR_STATE, "addFeature before captureNewFrame");
+  BCHECK(cudaSetDevice(b->device));
+  const int half = b->cfg.window_size / 2;
+  // isInsideImage (vslamRansac.cpp:314,1644-1652), as ekf_add_feature
+  const double x = (double)u, y = (double)v;
+  if (!(x > half && y > half && x < b->fv.w - half && y < b->fv.h - half)) return 0;
+  if (b->h_N[f] >= b->Ncap || b->h_n[f] + 6 > b->ncap) return bfail(b, EKF_ERR_CAPACITY, "feature capacity exceeded");
+  k_batch_add<<<1, BADD_THREADS, 0, b->stream>>>(b->bv, b->fv, b->dcfg, nullptr, nullptr, f, u, v, 0);
+  b->launches += 1;
+  BCHECK(cudaGetLastError());
+  b->h_N[f] += 1;
+  b->h_n[f] += 6;
+  return 1;
+}
+
+static int batch_stage_num(ekf_batch* b, const int32_t* num) {
+  std::copy(num, num + b->B, b->h_num);
+  BCHECK(cudaMemcpyAsync(b->det_num, b->h_num, sizeof(int) * b->B, cudaMemcpyHostToDevice, b->stream));
+  return EKF_OK;
+}
+
+int ekf_batch_detect_corners(ekf_batch* b, const int32_t* num, float* out_xy, int32_t* out_n) {
+  if (!b || !num || !out_xy || !out_n) return EKF_ERR_ARG;
+  if (!b->seeded) return bfail(b, EKF_ERR_STATE, "findNewFeatures before ekf_batch_seed_from");
+  if (!b->have_frame) return bfail(b, EKF_ERR_STATE, "findNewFeatures before captureNewFrame");
+  BCHECK(cudaSetDevice(b->device));
+  cudaStream_t st = b->stream;
+  const size_t Bn = (size_t)b->B;
+  int rc = batch_stage_num(b, num);
+  if (rc) return rc;
+  BCHECK(batch_detect_reserve(b->det, (size_t)b->fv.w * b->fv.h, b->B));
+  BCHECK(launch_batch_detect(st, b->det, b->fv, b->bv.ft.center, b->bv.N, b->Ncap, b->B, b->cfg.window_size, b->det_num, 1, 0,
+                             b->det_xy, b->det_n, &b->launches));
+  BCHECK(cudaMemcpyAsync(b->h_det_xy, b->det_xy, sizeof(float) * Bn * 2 * EKF_BATCH_MAX_CORNERS, cudaMemcpyDeviceToHost, st));
+  BCHECK(cudaMemcpyAsync(b->h_det_n, b->det_n, sizeof(int) * Bn, cudaMemcpyDeviceToHost, st));
+  BCHECK(cudaStreamSynchronize(st));
+  std::copy(b->h_det_xy, b->h_det_xy + Bn * 2 * EKF_BATCH_MAX_CORNERS, out_xy);
+  std::copy(b->h_det_n, b->h_det_n + Bn, out_n);
+  return EKF_OK;
+}
+
+int ekf_batch_find_new_features(ekf_batch* b, const int32_t* num, int32_t* added) {
+  if (!b) return EKF_ERR_ARG;
+  if (!b->seeded) return bfail(b, EKF_ERR_STATE, "findNewFeatures before ekf_batch_seed_from");
+  if (!b->have_frame) return bfail(b, EKF_ERR_STATE, "findNewFeatures before captureNewFrame");
+  if (!num && !b->results_valid) return bfail(b, EKF_ERR_STATE, "findNewFeatures(EKF_BSTAT_TOPUP) without a completed step");
+  BCHECK(cudaSetDevice(b->device));
+  int rc = num ? batch_stage_num(b, num) : EKF_OK;
+  if (rc) return rc;
+  rc = num ? batch_topup(b, b->det_num, 1, 0) : batch_topup(b, b->out_stats + EKF_BSTAT_TOPUP, EKF_BATCH_STAT_FIELDS, 0);
+  if (rc) return rc;
+  rc = batch_readback(b, true);
+  if (rc) return rc;
+  long long total = 0;
+  for (int i = 0; i < b->B; ++i) total += b->h_added[i];
+  if (added) std::copy(b->h_added, b->h_added + b->B, added);
+  return (int)total;
+}
+
+int ekf_batch_set_topup(ekf_batch* b, int on) {
+  if (!b) return EKF_ERR_ARG;
+  b->topup = on != 0;
+  return EKF_OK;
+}
+
+int ekf_batch_last_added(ekf_batch* b, int32_t* added) {
+  if (!b || !added) return EKF_ERR_ARG;
+  std::copy(b->h_added, b->h_added + b->B, added);
+  return EKF_OK;
+}
+
+int ekf_batch_get_template(ekf_batch* b, int f, int idx, int which, uint8_t* out) {
+  if (!b || f < 0 || f >= b->B || !out || idx < 0 || idx >= b->h_N[f]) return EKF_ERR_ARG;
+  BCHECK(cudaSetDevice(b->device));
+  const FeatTab t = feattab_slice(b->bv.ft, f, b->Ncap, b->bv.tstride);
+  const uint8_t* src = (which ? t.mpatch : t.patch) + (size_t)idx * b->bv.tstride;
+  BCHECK(cudaMemcpyAsync(out, src, (size_t)b->cfg.window_size * b->cfg.window_size, cudaMemcpyDeviceToHost, b->stream));
+  BCHECK(cudaStreamSynchronize(b->stream));
   return EKF_OK;
 }
 

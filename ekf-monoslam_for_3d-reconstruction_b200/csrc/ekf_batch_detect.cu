@@ -1,0 +1,145 @@
+// csrc/ekf_batch_detect.cu — findNewFeatures' detection (vslamRansac.cpp:783-831) for every filter of a batch at once.
+//
+// All filters see one frame, so the min-eigenvalue map (k_det_eig) is computed once per call.  What differs per filter is
+// the mask (the base border minus a box around each of the filter's patches) and with it the threshold
+// thr_b = 0.01 * max(eig over mask_b).  The single filter's candidates are the pixels p that
+//   (1) lie in rows / columns 1 .. size-2 and are 3x3 local maxima of THRESH_TOZERO(eig, thr_b),
+//   (2) have eig[p] > thr_b, and (3) are set in mask_b.
+// Given (2), (1) is the same as "no raw neighbour exceeds eig[p]": a neighbour above eig[p] is above thr_b and survives the
+// threshold, one at or below eig[p] cannot beat it whether zeroed or not.  So (1) does not depend on the filter, and one
+// list of every local maximum with eig > 0 inside the base mask, sorted once by the single filter's key (score bits << 32 |
+// pixel index), holds every filter's candidates as a subsequence in the same order.  Each filter then walks that list
+// (det_select_walk), skipping its boxes and stopping at its threshold or its corner limit.  The list is dense (one slot per
+// pixel, zero where there is no candidate), so it can never be truncated and its length is known on the host.
+//
+// The masked maximum must be exact: the frame's pixel keys (base mask, eig > 0) are sorted once, and one warp per filter
+// walks down that order until the first pixel outside the filter's boxes.  The walk is long only as far as the top pixels
+// sit inside the filter's own boxes (at most 32 (2 w + 1)^2 pixels).
+//
+// Early stop: every pixel inside the mask is at least window_size from the border, more than the window_size / 2 of
+// isInsideImage, so addFeature accepts every detected corner and the single filter's loop over them (V:832-835) stops only
+// on its capacity: taking min(num_b, Ncap - N_b) corners is exactly what it adds.
+#include <cub/device/device_radix_sort.cuh>
+
+#include "../../include/ekf_b200.h"
+#include "ekf_detect.cuh"
+#include "ekf_kernels.h"
+
+// pixel keys (base mask, eig > 0) and candidate keys (those that are also raw 3x3 local maxima), one slot per pixel
+__global__ void k_bdet_keys(const float* __restrict__ eig, int W, int H, int estrem, unsigned long long* __restrict__ kp,
+                            unsigned long long* __restrict__ kc) {
+  const int x = blockIdx.x * blockDim.x + threadIdx.x, y = blockIdx.y;
+  if (x >= W) return;
+  const size_t i = (size_t)y * W + x;
+  const float v = eig[i];
+  unsigned long long p = 0ull, c = 0ull;
+  if (v > 0.0f && det_in_base(x, y, W, H, estrem)) {
+    p = det_key(__float_as_uint(v), (unsigned)i);
+    if (x >= 1 && x < W - 1 && y >= 1 && y < H - 1) {
+      bool mx = true;
+      for (int dy = -1; dy <= 1; ++dy)
+        for (int dx = -1; dx <= 1; ++dx) mx = mx && !(eig[(size_t)(y + dy) * W + x + dx] > v);
+      if (mx) c = p;
+    }
+  }
+  kp[i] = p;
+  kc[i] = c;
+}
+
+// One warp per filter: its boxes, its corner limit and thr_b from the first sorted pixel outside its boxes.
+#define BDET_WARPS 8
+__global__ void __launch_bounds__(32 * BDET_WARPS) k_bdet_threshold(const unsigned long long* __restrict__ kp, int npx, int W, int H,
+                                                                     int window, const float* __restrict__ centers,
+                                                                     const int* __restrict__ N, int Ncap, int B,
+                                                                     const int* __restrict__ num, int num_stride, int cap_mode,
+                                                                     DetBox* __restrict__ boxes, unsigned* __restrict__ thr_bits,
+                                                                     int* __restrict__ limit) {
+  __shared__ DetBox sb[BDET_WARPS][EKF_BATCH_MAX_CORNERS];
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const int b = blockIdx.x * BDET_WARPS + warp;
+  if (b >= B) return;   // the whole warp
+  const int nb = N[b];
+  int lim = min(num[(size_t)b * num_stride], cap_mode ? Ncap - nb : EKF_BATCH_MAX_CORNERS);
+  lim = max(0, min(lim, EKF_BATCH_MAX_CORNERS));
+  DetBox bx{0, 0, 0, 0};
+  if (lane < nb) bx = det_patch_box(centers[2 * ((size_t)b * Ncap + lane)], centers[2 * ((size_t)b * Ncap + lane) + 1], W, H, window);
+  sb[warp][lane] = bx;
+  boxes[(size_t)b * EKF_BATCH_MAX_CORNERS + lane] = bx;
+  __syncwarp();
+  if (lane == 0) limit[b] = lim;
+  if (lim == 0) return;
+  unsigned maxbits = 0;   // no pixel of the mask above 0: threshold 0, as k_det_max leaves it
+  for (int i0 = 0; i0 < npx; i0 += 32) {
+    const int i = i0 + lane;
+    const unsigned long long k = i < npx ? kp[i] : 0ull;
+    bool stop = (k == 0ull);
+    if (!stop) {
+      const unsigned idx = (unsigned)(k & 0xffffffffull);
+      stop = !det_in_boxes((int)(idx % (unsigned)W), (int)(idx / (unsigned)W), sb[warp], nb);
+    }
+    const unsigned m = __ballot_sync(0xffffffffu, stop);
+    if (m) {
+      maxbits = (unsigned)(__shfl_sync(0xffffffffu, k, __ffs(m) - 1) >> 32);
+      break;
+    }
+  }
+  if (lane == 0) thr_bits[b] = __float_as_uint((float)((double)__uint_as_float(maxbits) * 0.01));
+}
+
+// One thread per filter: goodFeaturesToTrack's greedy selection over the shared candidate list.
+__global__ void k_bdet_select(const unsigned long long* __restrict__ kc, int nkeys, int W, const DetBox* __restrict__ boxes,
+                              const int* __restrict__ N, const unsigned* __restrict__ thr_bits, const int* __restrict__ limit, int B,
+                              float* __restrict__ out_xy, int* __restrict__ out_n) {
+  const int b = blockIdx.x * blockDim.x + threadIdx.x;
+  if (b >= B) return;
+  const int lim = limit[b];
+  out_n[b] = lim > 0 ? det_select_walk(kc, nkeys, W, thr_bits[b], boxes + (size_t)b * EKF_BATCH_MAX_CORNERS, N[b], 144.0f, lim,
+                                       out_xy + (size_t)b * 2 * EKF_BATCH_MAX_CORNERS)
+                     : 0;
+}
+
+cudaError_t batch_detect_reserve(BatchDetectBufs& d, size_t px, int B) {
+  cudaError_t e;
+  if (!d.boxes) {
+    if ((e = cudaMalloc((void**)&d.boxes, sizeof(DetBox) * EKF_BATCH_MAX_CORNERS * (size_t)B)) != cudaSuccess) return e;
+    if ((e = cudaMalloc((void**)&d.thr_bits, sizeof(unsigned) * (size_t)B)) != cudaSuccess) return e;
+    if ((e = cudaMalloc((void**)&d.limit, sizeof(int) * (size_t)B)) != cudaSuccess) return e;
+  }
+  if (px <= d.cap) return cudaSuccess;
+  cudaFree(d.eig); cudaFree(d.keys); cudaFree(d.tmp);
+  d.eig = nullptr; d.keys = nullptr; d.tmp = nullptr; d.cap = 0;
+  size_t tmp = 0;
+  if ((e = cub::DeviceRadixSort::SortKeysDescending(nullptr, tmp, (const unsigned long long*)nullptr, (unsigned long long*)nullptr,
+                                                    (int)px)) != cudaSuccess)
+    return e;
+  if ((e = cudaMalloc((void**)&d.eig, sizeof(float) * px)) != cudaSuccess) return e;
+  if ((e = cudaMalloc((void**)&d.keys, sizeof(unsigned long long) * 4 * px)) != cudaSuccess) return e;
+  if ((e = cudaMalloc(&d.tmp, tmp)) != cudaSuccess) return e;
+  d.tmp_bytes = tmp;
+  d.cap = px;
+  return cudaSuccess;
+}
+
+void batch_detect_free(BatchDetectBufs& d) {
+  cudaFree(d.eig); cudaFree(d.keys); cudaFree(d.tmp); cudaFree(d.boxes); cudaFree(d.thr_bits); cudaFree(d.limit);
+  d = BatchDetectBufs{};
+}
+
+cudaError_t launch_batch_detect(cudaStream_t st, BatchDetectBufs& d, FrameView fr, const float* centers, const int* N, int Ncap, int B,
+                                int window, const int* num, int num_stride, int cap_mode, float* out_xy, int* out_n, long long* launches) {
+  const int W = fr.w, H = fr.h, npx = W * H;
+  unsigned long long *kp = d.keys, *kc = d.keys + d.cap, *kp_s = d.keys + 2 * d.cap, *kc_s = d.keys + 3 * d.cap;
+  launch_det_eig(st, fr, d.eig, launches);
+  k_bdet_keys<<<dim3((W + 255) / 256, H), 256, 0, st>>>(d.eig, W, H, window, kp, kc);
+  size_t tmp = d.tmp_bytes;
+  cudaError_t e = cub::DeviceRadixSort::SortKeysDescending(d.tmp, tmp, kp, kp_s, npx, 0, 64, st);
+  if (e != cudaSuccess) return e;
+  tmp = d.tmp_bytes;
+  e = cub::DeviceRadixSort::SortKeysDescending(d.tmp, tmp, kc, kc_s, npx, 0, 64, st);
+  if (e != cudaSuccess) return e;
+  k_bdet_threshold<<<(B + BDET_WARPS - 1) / BDET_WARPS, 32 * BDET_WARPS, 0, st>>>(kp_s, npx, W, H, window, centers, N, Ncap, B, num,
+                                                                                  num_stride, cap_mode, d.boxes, d.thr_bits, d.limit);
+  k_bdet_select<<<(B + 127) / 128, 128, 0, st>>>(kc_s, npx, W, d.boxes, N, d.thr_bits, d.limit, B, out_xy, out_n);
+  *launches += 5;   // keys, the two sorts (counted once each), threshold, select; the eig map counts itself
+  return cudaGetLastError();
+}

@@ -1,6 +1,7 @@
 // csrc/ekf_kernels.h — host-side launch wrappers of the kernels in ekf_*.cu (internal to libekf_b200).
 #pragma once
 #include "ekf_common.cuh"
+#include "ekf_detect.cuh"
 
 #define EKF_UB 128  // rows per update block (64 features): K of the rank-b downdate GEMM
 
@@ -117,5 +118,23 @@ int gemm_kernels_preload();
 // ekf_detect.cu
 int launch_detect_corners(cudaStream_t st, FrameView fr, FeatTab ft, int N, int window, uint8_t* mask, float* eig,
                           unsigned long long* keys, int key_cap, int* counters, int max_corners, float* out_xy, long long* launches);
+// the min-eigenvalue map of goodFeaturesToTrack for a whole frame (k_det_eig)
+void launch_det_eig(cudaStream_t st, FrameView fr, float* eig, long long* launches);
 void launch_capture_resize_gray(cudaStream_t st, const uint8_t* src, int sw, int sh, int sstride, int cn, uint8_t* dst, int dw, int dh,
                                 int dstride, long long* launches);
+// ekf_batch_detect.cu: findNewFeatures' detection for every filter of a batch (one frame, per-filter masks)
+struct BatchDetectBufs {
+  float* eig = nullptr;                 // [cap] min-eigenvalue map
+  unsigned long long* keys = nullptr;   // [4][cap] pixel keys, candidate keys, both sorted
+  void* tmp = nullptr;                  // CUB radix-sort workspace
+  size_t tmp_bytes = 0, cap = 0;        // cap: pixels the buffers hold
+  DetBox* boxes = nullptr;              // [B][EKF_BATCH_MAX_CORNERS] mask boxes per filter
+  unsigned* thr_bits = nullptr;         // [B] per-filter threshold (float bits)
+  int* limit = nullptr;                 // [B] corners each filter may take
+};
+cudaError_t batch_detect_reserve(BatchDetectBufs& d, size_t px, int B);
+void batch_detect_free(BatchDetectBufs& d);
+// num[b * num_stride] corners for filter b, capped at EKF_BATCH_MAX_CORNERS (cap_mode 0) or at Ncap - N[b] (cap_mode 1);
+// out_xy [B][EKF_BATCH_MAX_CORNERS][2], out_n [B]
+cudaError_t launch_batch_detect(cudaStream_t st, BatchDetectBufs& d, FrameView fr, const float* centers, const int* N, int Ncap, int B,
+                                int window, const int* num, int num_stride, int cap_mode, float* out_xy, int* out_n, long long* launches);

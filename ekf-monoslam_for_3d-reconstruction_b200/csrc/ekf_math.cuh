@@ -300,6 +300,104 @@ __host__ __device__ __forceinline__ void d_inv2_pplu(const double A[4], double X
   X[0] = x0[0]; X[1] = x0[1]; X[2] = x1[0]; X[3] = x1[1];
 }
 
+// ---- addFeature (V:309-371) ---------------------------------------------------------------------------------------------
+// Shared by the single filter (k_add_feature) and the batched filters (k_batch_add).  New state entries and the 6 new rows /
+// columns of Sigma' = Js blkdiag(Sigma, sigma_px^2 I2, sigma_rho_0) Js^T, evaluated in the reference's association
+// (Js*S)*Js^T with the exact-zero terms dropped (SURVEY.md §3.2):
+//   rows  n+a, j<n : sum_{c<7} A[a,c] Sigma[c,j]          cols i<n, n+b : sum_{c<7} Sigma[i,c] A[b,c]
+//   corner         : sum_{c<7} T[a,c] A[b,c] + sum_e (Ap[a,e] s_e) Ap[b,e]
+// A = [I3 0 ; Jf*Jq (rows theta,phi) ; 0], Ap = [Jf*R*J2d | e6].
+//
+// A (6 x 7), Ap (6 x 3) and the new state entries fnew[6] from the camera r, q = mu[0:7] and the pixel.
+__device__ inline void add_feature_jacobians(const CamParams& cam, const double* mu, float pfx, float pfy, double rho_0, double* A,
+                                             double* Ap, double* fnew) {
+  double r[3] = {mu[0], mu[1], mu[2]}, q[4] = {mu[3], mu[4], mu[5], mu[6]};
+  const double hd[2] = {(double)pfx, (double)pfy};
+  double hC[3], J2d[6], Rot[9], hW[3];
+  d_cam_unproject_J(cam, hd, hC, J2d);
+  d_quat2rot(q, Rot);
+  for (int i = 0; i < 3; ++i) {
+    double s = 0;
+    for (int k = 0; k < 3; ++k) s += Rot[i * 3 + k] * hC[k];
+    hW[i] = s;
+  }
+  const double hx = hW[0], hy = hW[1], hz = hW[2];
+  fnew[0] = r[0]; fnew[1] = r[1]; fnew[2] = r[2];
+  fnew[3] = atan2(hx, hz);
+  fnew[4] = atan2(-hy, sqrt(hx * hx + hz * hz));
+  fnew[5] = rho_0;
+  double Jt[3], Jp[3], Jq[12];
+  d_jac_f_hW(hW, Jt, Jp);
+  d_jac_hW_q(q, hC, Jq);
+  for (int i = 0; i < 42; ++i) A[i] = 0;
+  for (int i = 0; i < 18; ++i) Ap[i] = 0;
+  for (int i = 0; i < 3; ++i) A[i * 7 + i] = 1;
+  // (Jf*Jq): rows 3,4 = Jt*Jq, Jp*Jq (other rows are sums of exact zeros)
+  for (int b = 0; b < 4; ++b) {
+    double s3 = 0, s4 = 0;
+    for (int k = 0; k < 3; ++k) { s3 += Jt[k] * Jq[k * 4 + b]; s4 += Jp[k] * Jq[k * 4 + b]; }
+    A[3 * 7 + 3 + b] = s3; A[4 * 7 + 3 + b] = s4;
+  }
+  // (Jf*Rot)*J2d
+  double JR3[3], JR4[3];
+  for (int b = 0; b < 3; ++b) {
+    double s3 = 0, s4 = 0;
+    for (int k = 0; k < 3; ++k) { s3 += Jt[k] * Rot[k * 3 + b]; s4 += Jp[k] * Rot[k * 3 + b]; }
+    JR3[b] = s3; JR4[b] = s4;
+  }
+  for (int b = 0; b < 2; ++b) {
+    double s3 = 0, s4 = 0;
+    for (int k = 0; k < 3; ++k) { s3 += JR3[k] * J2d[k * 2 + b]; s4 += JR4[k] * J2d[k * 2 + b]; }
+    Ap[3 * 3 + b] = s3; Ap[4 * 3 + b] = s4;
+  }
+  Ap[5 * 3 + 2] = 1;
+}
+// New row n + a, column t and new column n + a, row t of an n x n Sigma (t < n), for a = 0..5.
+__device__ inline void add_feature_cross(double* Sigma, int ld, int n, int t, const double* A) {
+  double col[7], rowv[7];
+  for (int c = 0; c < 7; ++c) { col[c] = Sigma[(size_t)c * ld + t]; rowv[c] = Sigma[(size_t)t * ld + c]; }
+  for (int a = 0; a < 6; ++a) {
+    double s = 0, u = 0;
+    for (int c = 0; c < 7; ++c) { s += A[a * 7 + c] * col[c]; u += rowv[c] * A[a * 7 + c]; }
+    Sigma[(size_t)(n + a) * ld + t] = s;
+    Sigma[(size_t)t * ld + n + a] = u;
+  }
+}
+// Entry e = 7 a + c of T = A Sigma[0:7, 0:7] (6 x 7), the left factor of the 6 x 6 corner.
+__device__ inline double add_feature_corner_T(const double* Sigma, int ld, const double* A, int e) {
+  const int a = e / 7, c = e % 7;
+  double s = 0;
+  for (int k = 0; k < 7; ++k) s += A[a * 7 + k] * Sigma[(size_t)k * ld + c];
+  return s;
+}
+// Entry e = 6 a + b of the 6 x 6 corner Sigma'[n + a, n + b].
+__device__ inline double add_feature_corner(const double* T, const double* A, const double* Ap, int e, double sigma_pixel_2,
+                                            double sigma_rho_0) {
+  const int a = e / 6, b = e % 6;
+  double s = 0;
+  for (int c = 0; c < 7; ++c) s += T[a * 7 + c] * A[b * 7 + c];
+  for (int k = 0; k < 3; ++k) {
+    const double sd = (k < 2) ? sigma_pixel_2 : sigma_rho_0;  // V:362,365
+    s += (Ap[a * 3 + k] * sd) * Ap[b * 3 + k];
+  }
+  return s;
+}
+// Template byte e of the Patch constructor (Patch.cpp:78-103): the frame ROI at (int)(pf - w/2).
+__device__ __forceinline__ uint8_t add_feature_template_px(const FrameView& fr, int w, float pfx, float pfy, int e) {
+  const int x0 = (int)(pfx - w / 2), y0 = (int)(pfy - w / 2);
+  return fr.px[(size_t)(y0 + e / w) * fr.stride + x0 + (e % w)];
+}
+// Feature-table record fidx of a new inverse-depth feature at state position n.
+__device__ inline void add_feature_record(const FeatTab& ft, int fidx, int n, float pfx, float pfy, int real_index) {
+  ft.pos[fidx] = n; ft.coding[fidx] = 0; ft.innov[fidx] = 0; ft.li[fidx] = 0; ft.hi[fidx] = 0;
+  ft.removef[fidx] = 0; ft.n_tot[fidx] = 1; ft.n_find[fidx] = 1; ft.real_index[fidx] = real_index;
+  ft.pos_in_z[fidx] = 0; ft.center[2 * fidx] = pfx; ft.center[2 * fidx + 1] = pfy;
+  ft.quality[fidx] = 0.0f; ft.last_ncc[fidx] = -1.0f;
+  ft.z[2 * fidx] = 0; ft.z[2 * fidx + 1] = 0; ft.h[2 * fidx] = 0; ft.h[2 * fidx + 1] = 0;
+  for (int c = 0; c < 26; ++c) ft.Hc[26 * fidx + c] = 0;
+  for (int c = 0; c < 4; ++c) ft.S2[4 * fidx + c] = 0;
+}
+
 // ---- convert2XYZ_ifLinear (V:741-772) -----------------------------------------------------------------------------------
 // Shared by the single filter (k_xyz_decide / k_xyz_apply), the batched filters (ekf_batch.cu) and a host test harness.
 //

@@ -377,6 +377,46 @@ class FilterBatch:
         self._ck(self.L.ekf_batch_get_feature(self.h, int(f), int(i), C.byref(o)))
         return o
 
+    def addFeature(self, f, u, v):
+        """vslamRansac.cpp:309-371 on filter f; 1 added, 0 rejected by isInsideImage."""
+        return self._ck(self.L.ekf_batch_add_feature(self.h, int(f), float(u), float(v)))
+
+    def _num(self, num):
+        return np.ascontiguousarray(np.broadcast_to(np.asarray(num, dtype=np.int32), (self.B,)))
+
+    def detect_corners(self, num):
+        """findNewFeatures' detection alone (vslamRansac.cpp:783-831) on every filter; num is one count or one per filter
+        (capped at 32).  Returns a list of (k_b, 2) float32 arrays."""
+        a = self._num(num)
+        xy = np.zeros((self.B, _abi.BATCH_MAX_CORNERS, 2), dtype=np.float32); n = np.zeros(self.B, dtype=np.int32)
+        self._ck(self.L.ekf_batch_detect_corners(self.h, _ptr(a), _ptr(xy), _ptr(n)))
+        return [xy[b, :n[b]].copy() for b in range(self.B)]
+
+    def findNewFeatures(self, num=None):
+        """vslamRansac.cpp:783-839 on every filter: num is one count or one per filter (<= 0: none — unlike the single
+        filter's nInitFeatures); None takes each filter's EKF_BSTAT_TOPUP of the last step.  Returns the features each
+        filter added."""
+        added = np.zeros(self.B, dtype=np.int32)
+        a = self._num(num) if num is not None else None
+        self._ck(self.L.ekf_batch_find_new_features(self.h, _ptr(a) if a is not None else None, _ptr(added)))
+        return added
+
+    def set_topup(self, on=True):
+        """on: step() ends like ekf_update_after_match — removals, findNewFeatures(EKF_BSTAT_TOPUP), XYZ conversion."""
+        self._ck(self.L.ekf_batch_set_topup(self.h, int(bool(on))))
+
+    def last_added(self):
+        """Features each filter added in the last step."""
+        out = np.zeros(self.B, dtype=np.int32)
+        self._ck(self.L.ekf_batch_last_added(self.h, _ptr(out)))
+        return out
+
+    def template(self, f, i, which=0):
+        w = self.cfg.window_size
+        out = np.zeros((w, w), dtype=np.uint8)
+        self._ck(self.L.ekf_batch_get_template(self.h, int(f), int(i), int(which), _ptr(out)))
+        return out
+
     def kernel_launches(self):
         return int(self.L.ekf_batch_kernel_launches(self.h))
 
