@@ -81,6 +81,8 @@ SIGNATURES = {
     "ekf_batch_find_new_features": (_i, [_vp, _vp, _vp]),
     "ekf_batch_set_topup": (_i, [_vp, _i]),
     "ekf_batch_last_added": (_i, [_vp, _vp]),
+    "ekf_batch_set_motion_blur": (_i, [_vp, _i]),
+    "ekf_batch_last_blur_counts": (_i, [_vp, _vp]),
     "ekf_batch_get_template": (_i, [_vp, _i, _i, _i, _vp]),
     "ekf_batch_kernel_launches": (C.c_int64, [_vp]),
     "ekf_batch_last_step_ms": (_i, [_vp, _vp]),

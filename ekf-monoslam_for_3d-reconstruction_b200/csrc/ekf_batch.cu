@@ -5,6 +5,7 @@
 // step (148 concurrent filters x 310 KB = 46 MB of the 126 MB L2), so HBM sees each Sigma once in and
 // once out.  Three launches per step:
 //   k_batch_predict  (B CTAs)       motion model, block covariance propagation, h / H / gate, S blocks
+//   (k_batch_predict_blur (B CTAs)  motion-blur templates, only once ekf_batch_set_motion_blur switched them on)
 //   k_match_filter_batch (N x B)    active search, shared frame (ekf_match.cu)
 //   k_batch_update   (B CTAs)       1-point RANSAC, Li update, Hi rescue, Hi update, book-keeping:
 //                                   W = Sigma H^T (n x k <= 64) and its Cholesky gain live in shared
@@ -22,6 +23,7 @@
 #include <vector>
 
 #include "../../include/ekf_b200.h"
+#include "ekf_blur.cuh"
 #include "ekf_cta.cuh"
 #include "ekf_factor.cuh"
 #include "ekf_handle.h"
@@ -192,6 +194,79 @@ __global__ void __launch_bounds__(BPRED_THREADS, 4) k_batch_predict(BatchView bv
       ft.S2[4 * f + 0] = s00 + cfg.sigma_pixel_2; ft.S2[4 * f + 1] = s01;
       ft.S2[4 * f + 2] = s10; ft.S2[4 * f + 3] = s11 + cfg.sigma_pixel_2;
     }
+  }
+}
+
+// ------------------------------------------------------------------------------------------------
+// motion-blur template prediction (Patch::blur, Patch.cpp:50-57; libblur.cpp:17-81) for one filter per CTA, after
+// k_batch_predict: same arithmetic as k_predict_blur (ekf_blur.cuh), another shape.  Warp 0 takes the blur decision with
+// lane = feature; then every blurred template goes to one warp, which stages it in shared memory, rasterises the line
+// with lane = point, keeps each distinct coefficient once, orders them by (row, column) and has every output pixel walk
+// that list: the terms and their order are the bit mask walk's, without the zeros.  out[b] = templates blurred,
+// out[B + b] = 1 when a kernel exceeded BLUR_MAXK (that template stays unblurred, as in k_predict_blur).
+// ------------------------------------------------------------------------------------------------
+#define BBLUR_WARPS 4
+__global__ void __launch_bounds__(BBLUR_WARPS * 32) k_batch_predict_blur(BatchView bv, DevCfg cfg, double dT, int* __restrict__ out) {
+  __shared__ int s_feat[BNCAP], s_rows[BNCAP], s_cols[BNCAP], s_nblur;
+  __shared__ double s_dx[BNCAP], s_dy[BNCAP];
+  __shared__ __align__(16) uint8_t s_tmpl[BBLUR_WARPS][1024];
+  __shared__ int s_seq[BBLUR_WARPS][BLUR_MAXPTS], s_coef[BBLUR_WARPS][BLUR_MAXPTS];
+  const int b = blockIdx.x, lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  const int N = bv.N[b], ld = bv.ld;
+  const double* mu = bv.mu + (size_t)b * ld;
+  const FeatTab ft = feattab_slice(bv.ft, b, bv.Ncap, bv.tstride);
+  if (warp == 0) {   // N <= BNCAP = 32: one feature per lane
+    const int f = lane;
+    int d = 0, krows = 0, kcols = 0;
+    double ddx = 0.0, ddy = 0.0;
+    if (f < N && ft.innov[f]) {
+      double cam[13], rb[3], Rb[9];
+      for (int c = 0; c < 13; ++c) cam[c] = mu[c];   // predicted camera state, committed by k_batch_predict
+      blur_pose(cam, cfg.T_camera, dT, rb, Rb);
+      const int pos = ft.pos[f], coding = ft.coding[f];
+      double fs[6];
+      for (int c = 0; c < (coding ? 3 : 6); ++c) fs[c] = mu[pos + c];
+      blur_displacement(cfg.cam, fs, coding, rb, Rb, ft.h[2 * f], ft.h[2 * f + 1], &ddx, &ddy);
+      d = blur_decide(ddx, ddy, cfg.kernel_min_size, &krows, &kcols);
+    }
+    const unsigned blur = __ballot_sync(0xffffffffu, d > 0), big = __ballot_sync(0xffffffffu, d < 0);
+    if (d > 0) {
+      const int k = __popc(blur & ((1u << lane) - 1u));
+      s_feat[k] = f; s_rows[k] = krows; s_cols[k] = kcols; s_dx[k] = ddx; s_dy[k] = ddy;
+    }
+    if (lane == 0) {
+      s_nblur = __popc(blur);
+      out[b] = __popc(blur);
+      out[gridDim.x + b] = big != 0u;
+    }
+  }
+  __syncthreads();
+  const int w = cfg.window, w2 = w * w;
+  uint8_t* tm = s_tmpl[warp];
+  int* seq = s_seq[warp];
+  int* coef = s_coef[warp];
+  for (int k = warp; k < s_nblur; k += BBLUR_WARPS) {
+    const int f = s_feat[k], krows = s_rows[k], kcols = s_cols[k];
+    const uint4* src = reinterpret_cast<const uint4*>(ft.patch + (size_t)f * bv.tstride);
+    for (int c = lane; c < (bv.tstride >> 4); c += 32) reinterpret_cast<uint4*>(tm)[c] = src[c];
+    // the distinct coefficients in line order: lane = point i of evaluateKernel's loop (libblur.cpp:25-43)
+    const BlurLine L = blur_line(s_dx[k], s_dy[k]);
+    int m = 0;
+    for (int base = 0; base < L.length; base += 32) {
+      const int i = base + lane;
+      int x = 0, y = 0;
+      const bool nw = i < L.length && blur_line_point_new(L, i, krows, kcols, &x, &y);
+      const unsigned bal = __ballot_sync(0xffffffffu, nw);
+      if (nw) seq[m + __popc(bal & ((1u << lane) - 1u))] = blur_pack(x, y);
+      m += __popc(bal);
+    }
+    __syncwarp();
+    for (int j = lane; j < m; j += 32) coef[blur_rank(seq, m, j)] = seq[j];
+    __syncwarp();
+    const double kf = 1.0 / (double)m;   // kernel / sum(kernel): every set coefficient is 1 / count
+    uint8_t* dst = ft.mpatch + (size_t)f * bv.tstride;
+    for (int e = lane; e < w2; e += 32) dst[e] = blur_pixel_list(tm, w, e, coef, m, krows, kcols, kf);
+    __syncwarp();   // tm, seq and coef are reused by the warp's next template
   }
 }
 
@@ -772,8 +847,10 @@ struct ekf_batch {
   float* h_det_xy = nullptr;                    // pinned
   int *h_det_n = nullptr, *h_num = nullptr;     // pinned
   int* h_added = nullptr;                       // pinned: features each filter added in the last step / top-up call
+  int* blur_out = nullptr;                      // [2][B] k_batch_predict_blur: templates blurred, kernel too large
+  int* h_blur = nullptr;                        // pinned mirror of blur_out
   double dT = 1.0, old_ts = -1.0;
-  bool have_frame = false, seeded = false, results_valid = false, topup = false;
+  bool have_frame = false, seeded = false, results_valid = false, topup = false, blur = false;
   long long launches = 0;
   cudaEvent_t ev[4] = {nullptr, nullptr, nullptr, nullptr};
   std::string err;
@@ -820,6 +897,8 @@ int ekf_batch_destroy(ekf_batch* b) {
   if (b->h_det_n) cudaFreeHost(b->h_det_n);
   if (b->h_num) cudaFreeHost(b->h_num);
   if (b->h_added) cudaFreeHost(b->h_added);
+  cudaFree(b->blur_out);
+  if (b->h_blur) cudaFreeHost(b->h_blur);
   if (b->h_mu14) cudaFreeHost(b->h_mu14);
   if (b->h_S14) cudaFreeHost(b->h_S14);
   if (b->h_stats) cudaFreeHost(b->h_stats);
@@ -876,6 +955,7 @@ int ekf_batch_create(const ekf_config* cfg, int n_filters, int feature_capacity,
   TRY(cudaMallocHost((void**)&b->h_det_xy, sizeof(float) * Bn * 2 * EKF_BATCH_MAX_CORNERS))
   TRY(cudaMallocHost((void**)&b->h_det_n, sizeof(int) * Bn)) TRY(cudaMallocHost((void**)&b->h_num, sizeof(int) * Bn))
   TRY(cudaMallocHost((void**)&b->h_added, sizeof(int) * Bn))
+  TRY(balloc(&b->blur_out, 2 * Bn)) TRY(cudaMallocHost((void**)&b->h_blur, sizeof(int) * 2 * Bn))
   TRY(cudaMallocHost((void**)&b->h_mu14, sizeof(double) * Bn * 14)) TRY(cudaMallocHost((void**)&b->h_S14, sizeof(double) * Bn * 196))
   TRY(cudaMallocHost((void**)&b->h_stats, sizeof(int) * Bn * EKF_BATCH_STAT_FIELDS))
   TRY(cudaMallocHost((void**)&b->h_n, sizeof(int) * Bn)) TRY(cudaMallocHost((void**)&b->h_N, sizeof(int) * Bn))
@@ -889,6 +969,7 @@ int ekf_batch_create(const ekf_config* cfg, int n_filters, int feature_capacity,
   TRY(cudaStreamSynchronize(b->stream))
 #undef TRY
   for (size_t i = 0; i < Bn; ++i) { b->h_n[i] = 0; b->h_N[i] = 0; b->h_added[i] = 0; }
+  std::fill(b->h_blur, b->h_blur + 2 * Bn, 0);
   DevCfg& d = b->dcfg;
   d.cam = CamParams{cfg->fx, cfg->fy, cfg->u0, cfg->v0, cfg->k1, cfg->k2, cfg->k3, cfg->p1, cfg->p2};
   d.Vmax[0] = cfg->sigma_vx * cfg->sigma_vx; d.Vmax[1] = cfg->sigma_vy * cfg->sigma_vy; d.Vmax[2] = cfg->sigma_vz * cfg->sigma_vz;
@@ -1027,6 +1108,10 @@ int ekf_batch_step(ekf_batch* b, const double dv[3], const double dw[3], int vco
   k_batch_predict<<<b->B, BPRED_THREADS, 0, st>>>(b->bv, b->fv, b->dcfg, b->dT, make_double3(a[0], a[1], a[2]),
                                                    make_double3(w[0], w[1], w[2]), vcontrol);
   b->launches += 1;
+  if (b->blur) {   // matching_patch <- blurred patch where the prediction moves far enough (k_batch_predict copied patch)
+    k_batch_predict_blur<<<b->B, BBLUR_WARPS * 32, 0, st>>>(b->bv, b->dcfg, b->dT, b->blur_out);
+    b->launches += 1;
+  }
   BCHECK(cudaEventRecord(b->ev[1], st));
   launch_match_filter_batch(st, b->bv.ft, b->Ncap, b->bv.N, b->B, b->fv, b->dcfg, &b->frame_map, b->match_defer,
                             b->match_defer + (size_t)b->B * b->Ncap, &b->launches);
@@ -1041,6 +1126,7 @@ int ekf_batch_step(ekf_batch* b, const double dv[3], const double dw[3], int vco
   BCHECK(cudaMemcpyAsync(b->h_stats, b->out_stats, sizeof(int) * Bn * EKF_BATCH_STAT_FIELDS, cudaMemcpyDeviceToHost, st));
   BCHECK(cudaMemcpyAsync(b->h_mu14, b->out_mu14, sizeof(double) * Bn * 14, cudaMemcpyDeviceToHost, st));
   if (b->cfg.xyz_conversion) BCHECK(cudaMemcpyAsync(b->h_xyz_count, b->bv.xyz_count, sizeof(int) * Bn, cudaMemcpyDeviceToHost, st));
+  if (b->blur) BCHECK(cudaMemcpyAsync(b->h_blur, b->blur_out, sizeof(int) * 2 * Bn, cudaMemcpyDeviceToHost, st));
   BCHECK(cudaStreamSynchronize(st));
   b->results_valid = true;
   long long removed = 0, converted = 0, fails = 0, topups = 0;
@@ -1080,6 +1166,9 @@ int ekf_batch_step(ekf_batch* b, const double dv[3], const double dw[3], int vco
     if (rc) return rc;
   }
   if (fails > 0) return bfail(b, EKF_ERR_STATE, "innovation covariance not positive definite in at least one filter");
+  for (size_t i = 0; b->blur && i < Bn; ++i)
+    if (b->h_blur[Bn + i])
+      return bfail(b, EKF_ERR_UNSUPPORTED, "filter " + std::to_string(i) + ": a motion-blur kernel exceeded 256 x 256 pixels");
   return EKF_OK;
 }
 
@@ -1244,6 +1333,20 @@ int ekf_batch_find_new_features(ekf_batch* b, const int32_t* num, int32_t* added
 int ekf_batch_set_topup(ekf_batch* b, int on) {
   if (!b) return EKF_ERR_ARG;
   b->topup = on != 0;
+  return EKF_OK;
+}
+
+int ekf_batch_set_motion_blur(ekf_batch* b, int32_t kernel_size) {
+  if (!b) return EKF_ERR_ARG;
+  b->dcfg.kernel_min_size = kernel_size;
+  b->blur = kernel_size < 100000;
+  if (!b->blur) std::fill(b->h_blur, b->h_blur + 2 * (size_t)b->B, 0);   // steps without blur leave the counts at zero
+  return EKF_OK;
+}
+
+int ekf_batch_last_blur_counts(ekf_batch* b, int32_t* out) {
+  if (!b || !out) return EKF_ERR_ARG;
+  std::copy(b->h_blur, b->h_blur + b->B, out);
   return EKF_OK;
 }
 

@@ -411,6 +411,17 @@ class FilterBatch:
         self._ck(self.L.ekf_batch_last_added(self.h, _ptr(out)))
         return out
 
+    def set_motion_blur(self, kernel_size):
+        """Patch::blur (Patch.cpp:50-57) in every filter's predict: kernel_size as EkfConfig.kernel_size (>= 100000: off,
+        the default); T_camera is the batch configuration's."""
+        self._ck(self.L.ekf_batch_set_motion_blur(self.h, int(kernel_size)))
+
+    def last_blur_counts(self):
+        """Templates each filter blurred in the last step (int32, zeros with blur off)."""
+        out = np.zeros(self.B, dtype=np.int32)
+        self._ck(self.L.ekf_batch_last_blur_counts(self.h, _ptr(out)))
+        return out
+
     def template(self, f, i, which=0):
         w = self.cfg.window_size
         out = np.zeros((w, w), dtype=np.uint8)

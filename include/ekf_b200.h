@@ -227,8 +227,9 @@ int ekf_match_batch(const uint8_t* frames, int n_frames, int width, int height, 
  * min_features features, then, when cfg.xyz_conversion is set, convert2XYZ_ifLinearAll (:1317) on every
  * filter.  Top-up is off by default: the step then only reports in EKF_BSTAT_TOPUP how many features
  * each filter asks for, and ekf_batch_find_new_features serves those requests when the caller wants.
- * feature_capacity <= 32 (the stacked update of one filter is kept in shared memory).  Motion blur
- * (kernel_size < 100000), scale != 1 and forsePlane are not supported (EKF_ERR_UNSUPPORTED). */
+ * feature_capacity <= 32 (the stacked update of one filter is kept in shared memory).  ekf_batch_create
+ * refuses motion blur (kernel_size < 100000), scale != 1 and forsePlane (EKF_ERR_UNSUPPORTED); motion-blur
+ * template prediction is switched on after creation with ekf_batch_set_motion_blur. */
 typedef struct ekf_batch ekf_batch;
 typedef struct ekf_batch_desc {
   int32_t n_filters, feature_capacity, state_capacity /* 14 + 6 * feature_capacity */, ld /* Sigma row stride */;
@@ -291,6 +292,14 @@ int ekf_batch_find_new_features(ekf_batch* b, const int32_t* num, int32_t* added
 int ekf_batch_set_topup(ekf_batch* b, int on);
 /* Features each filter added in the last step (n_filters entries; zeros with top-up off). */
 int ekf_batch_last_added(ekf_batch* b, int32_t* added);
+/* Patch::blur (Patch.cpp:50-57, libblur.cpp:17-81) in every filter's predict: kernel_size has the meaning of
+ * ekf_config.kernel_size for a single filter (a template is blurred when the prediction moves by more than kernel_size px
+ * over T_camera * dT; >= 100000 = off, the default).  ekf_batch_create still refuses a configuration with blur on.
+ * T_camera is the batch configuration's.  A kernel above 256 x 256 px leaves that template unblurred; the step then runs
+ * to its end and returns EKF_ERR_UNSUPPORTED, and ekf_batch_last_error names the first such filter. */
+int ekf_batch_set_motion_blur(ekf_batch* b, int32_t kernel_size);
+/* Templates each filter blurred in the last step (n_filters entries; zeros with blur off). */
+int ekf_batch_last_blur_counts(ekf_batch* b, int32_t* out);
 /* which: 0 = Patch::patch, 1 = Patch::matching_patch of feature idx of one filter; out holds window_size^2 bytes */
 int ekf_batch_get_template(ekf_batch* b, int filter, int idx, int which, uint8_t* out);
 /* Kernels of this library launched on the batch so far. */
