@@ -68,6 +68,10 @@ SIGNATURES = {
     "ekf_batch_set_camera_states": (_i, [_vp, _vp]),
     "ekf_batch_capture_frame": (_i, [_vp, _vp, _i, _i, _i, _d]),
     "ekf_batch_capture_frame_device": (_i, [_vp, _vp, _i, _i, _i, _d]),
+    "ekf_batch_capture_frame_bgr": (_i, [_vp, _vp, _i, _i, _i, _d]),
+    "ekf_batch_get_frame": (_i, [_vp, _vp, _P(_i), _P(_i)]),
+    "ekf_batch_set_scale": (_i, [_vp, _i]),
+    "ekf_batch_set_force_plane": (_i, [_vp, _i]),
     "ekf_batch_step": (_i, [_vp, _vp, _vp, _i, _vp, _i]),
     "ekf_batch_convert2xyz_if_linear_all": (_i, [_vp]),
     "ekf_batch_get_camera_states": (_i, [_vp, _vp, _vp, _vp]),

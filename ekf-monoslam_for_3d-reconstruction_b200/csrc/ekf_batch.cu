@@ -10,12 +10,14 @@
 //   k_batch_update   (B CTAs)       1-point RANSAC, Li update, Hi rescue, Hi update, book-keeping:
 //                                   W = Sigma H^T (n x k <= 64) and its Cholesky gain live in shared
 //                                   memory, the rank-k downdate Sigma -= V V^T runs on the fp64 tensor
-//                                   pipe (DMMA.8x8x4) straight from shared-memory V.
+//                                   pipe (DMMA.8x8x4) straight from shared-memory V.  With forsePlane
+//                                   (ekf_batch_set_force_plane) the second update adds the plane block.
 // plus k_batch_compact when a filter flagged features for deletion or, with cfg.xyz_conversion, has
 // inverse-depth features to convert to XYZ (convert2XYZ_ifLinearAll, V:1317): k_batch_update decides the
 // conversions, k_batch_compact applies removals and conversions in one pass over Sigma.  With top-up on and a
 // filter asking for features (V:1312-1315), that filter's pass removes only; the batched detector
 // (ekf_batch_detect.cu) and k_batch_add then add its new features, and a second k_batch_compact converts.
+// Frames are captured once for the whole batch, resized and converted to gray when ekf_batch_set_scale / a BGR source ask.
 // Every stage evaluates the same expressions as the single-filter kernels (same device functions).
 #include <algorithm>
 #include <cstdio>
@@ -291,10 +293,15 @@ static constexpr size_t kUpdSmemDoubles =
     (size_t)BNMAX * BLDW + kFactDoubles + (BK / 32) * 32 * BLDD + (size_t)BK * BLDW + BK + BK + BNMAX + BNCAP * 27 + 48 + (4 * BNCAP) / 2;
 static constexpr size_t kUpdSmemBytes = kUpdSmemDoubles * sizeof(double);
 
-// One stacked update over the `cnt` features listed in ft.sel (V:1036-1064 / V:1245-1284).
-__device__ void cta_stacked_update(const UpdSmem& sm, double* __restrict__ Sigma, int ld, int n, double* __restrict__ mu,
-                                   const FeatTab& ft, int cnt, const DevCfg& cfg, DevCtl* ctl) {
-  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5, g = lane >> 2, t4 = lane & 3;
+// One stacked update block is a gather (W, S, nu in shared memory), then cta_block_gain_downdate, and the update ends with one
+// cta_normalize_quaternion.  cta_stacked_update is the usual single block; with forsePlane the second update is the Hi block, the
+// plane block (cta_gather_plane), then the normalisation, as the single filter's stacked_update / launch_finish_update.
+//
+// Gather of the Hi / Li block over the `cnt` features listed in ft.sel (V:1036-1064 / V:1245-1284): W = Sigma H^T, S = H W + R
+// padded with identity to BK, nu = z - h.
+__device__ void cta_gather_features(const UpdSmem& sm, const double* __restrict__ Sigma, int ld, int n, const FeatTab& ft, int cnt,
+                                    const DevCfg& cfg) {
+  const int tid = threadIdx.x;
   const int k = 2 * cnt;
   int* fids = sm.ibuf + BNCAP; int* poss = fids + BNCAP; int* nds = poss + BNCAP;
   for (int a = tid; a < BNCAP; a += BUPD_THREADS) {
@@ -375,6 +382,37 @@ __device__ void cta_stacked_update(const UpdSmem& sm, double* __restrict__ Sigma
     sm.Sb[r * BLDW + s] = v;
   }
   __syncthreads();
+}
+
+// forsePlane (V:1245-1263): the pseudo-measurements mu[1] = mu[4] = mu[6] = 0 with R = 1e-5 I3 as one more block of k = 3 rows, the
+// unit rows e1, e4, e6 (k_plane_gather / k_plane_S): W[:, j] = Sigma[:, k_j], nu_j = 0 - mu[k_j] with mu already corrected by the
+// Hi block (the single filter's (0 - mu[k_j]) - delta[k_j] over the same sequential blocks), S = W[{1, 4, 6}, :] + 1e-5 I.
+__device__ void cta_gather_plane(const UpdSmem& sm, const double* __restrict__ Sigma, int ld, int n, const double* __restrict__ mu,
+                                 DevCtl* ctl) {
+  const int tid = threadIdx.x;
+  for (int e = tid; e < BNMAX * (BK / 2); e += BUPD_THREADS) {
+    const int i = e / (BK / 2), c = 2 * (e % (BK / 2));
+    double2 v = make_double2(0.0, 0.0);
+    if (i < n && c == 0) v = make_double2(Sigma[(size_t)i * ld + 1], Sigma[(size_t)i * ld + 4]);
+    if (i < n && c == 2) v.x = Sigma[(size_t)i * ld + 6];
+    *reinterpret_cast<double2*>(sm.W + (size_t)i * BLDW + c) = v;
+  }
+  if (tid < BK) sm.nu[tid] = (tid < 3) ? 0.0 - mu[tid == 0 ? 1 : (tid == 1 ? 4 : 6)] : 0.0;
+  if (tid == 0) ctl->k_rows += 3;
+  __syncthreads();
+  for (int e = tid; e < BK * BK; e += BUPD_THREADS) {
+    const int r = e / BK, s = e % BK;
+    double v = (r == s) ? 1.0 : 0.0;
+    if (r < 3 && s < 3) v = sm.W[(size_t)(r == 0 ? 1 : (r == 1 ? 4 : 6)) * BLDW + s] + ((r == s) ? 0.00001 : 0.0);
+    sm.Sb[r * BLDW + s] = v;
+  }
+  __syncthreads();
+}
+
+// Gain and downdate of the gathered block of k rows: L = chol(S), V = W L^-T, mu += V L^-1 nu, Sigma -= V V^T.
+__device__ void cta_block_gain_downdate(const UpdSmem& sm, double* __restrict__ Sigma, int ld, int n, double* __restrict__ mu, int k,
+                                        DevCtl* ctl) {
+  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5, g = lane >> 2, t4 = lane & 3;
   cta_chol_panel<BK>(sm.fact, sm.Sb, BLDW, sm.nu, sm.Sb, BLDW, sm.Dv, BLDD, sm.y, &ctl->chol_fail);
   // V = W L^-T in place: every warp owns 8-row tiles for the whole blocked triangular solve
   for (int rt = warp; rt < BNMAX / 8; rt += BUPD_THREADS / 32) {
@@ -436,7 +474,11 @@ __device__ void cta_stacked_update(const UpdSmem& sm, double* __restrict__ Sigma
     }
   }
   __syncthreads();
-  // normalizeQuaternion (V:1625-1642): 4 rows + 4 columns
+}
+
+// normalizeQuaternion (V:1625-1642): 4 rows + 4 columns
+__device__ void cta_normalize_quaternion(const UpdSmem& sm, double* __restrict__ Sigma, int ld, int n, double* __restrict__ mu) {
+  const int tid = threadIdx.x;
   double* J = sm.qj; double* Cq = J + 16; double* Tq = Cq + 16;
   if (tid == 0) {
     double q[4];
@@ -484,6 +526,16 @@ __device__ void cta_stacked_update(const UpdSmem& sm, double* __restrict__ Sigma
   __syncthreads();
 }
 
+// One stacked update over the `cnt` features listed in ft.sel (V:1036-1064 / V:1245-1284).
+__device__ void cta_stacked_update(const UpdSmem& sm, double* __restrict__ Sigma, int ld, int n, double* __restrict__ mu,
+                                   const FeatTab& ft, int cnt, const DevCfg& cfg, DevCtl* ctl) {
+  cta_gather_features(sm, Sigma, ld, n, ft, cnt, cfg);
+  cta_block_gain_downdate(sm, Sigma, ld, n, mu, 2 * cnt, ctl);
+  cta_normalize_quaternion(sm, Sigma, ld, n, mu);
+}
+
+// PLANE: forsePlane (ekf_batch_set_force_plane), a separate instantiation so that the plane-off kernel is the same code as without it.
+template <bool PLANE>
 __global__ void __launch_bounds__(BUPD_THREADS, 1) k_batch_update(BatchView bv, DevCfg cfg, const uint32_t* __restrict__ picks,
                                                                   int n_picks, double* __restrict__ out_mu14,
                                                                   double* __restrict__ out_S14, int* __restrict__ out_stats,
@@ -558,7 +610,17 @@ __global__ void __launch_bounds__(BUPD_THREADS, 1) k_batch_update(BatchView bv, 
   const int n_hi = block_compact(ft.hi, N, ft.sel, ft.pos_in_z);
   if (tid == 0) { ctl->n_hi = n_hi; ctl->k_rows = 2 * n_hi; }
   __syncthreads();
-  if (n_hi > 0) cta_stacked_update(sm, Sigma, ld, n, mu, ft, n_hi, cfg, ctl);
+  if constexpr (PLANE) {   // the second update runs with or without Hi rows (z_hi.rows() > 0 with the plane rows, V:1245-1272)
+    if (n_hi > 0) {
+      cta_gather_features(sm, Sigma, ld, n, ft, n_hi, cfg);
+      cta_block_gain_downdate(sm, Sigma, ld, n, mu, 2 * n_hi, ctl);
+    }
+    cta_gather_plane(sm, Sigma, ld, n, mu, ctl);
+    cta_block_gain_downdate(sm, Sigma, ld, n, mu, 3, ctl);
+    cta_normalize_quaternion(sm, Sigma, ld, n, mu);
+  } else {
+    if (n_hi > 0) cta_stacked_update(sm, Sigma, ld, n, mu, ft, n_hi, cfg, ctl);
+  }
   // book-keeping (k_bookkeeping) + visibility count (V:1296-1315)
   int my_remove = 0, my_vis = 0;
   for (int i = tid; i < N; i += BUPD_THREADS) {
@@ -829,6 +891,8 @@ struct ekf_batch {
   double* scratch = nullptr;
   uint8_t* frame = nullptr;
   size_t frame_cap = 0;
+  uint8_t* raw = nullptr;                       // device staging of a host frame that is resized or converted (cfg.scale > 1 or BGR)
+  size_t raw_cap = 0;
   FrameView fv{nullptr, 0, 0, 0};
   EkfTensorMap frame_map{};
   int* match_defer = nullptr;   // [B * Ncap] (filter, feature) pairs the warp matcher left to the CTA matcher, then the count
@@ -889,7 +953,7 @@ int ekf_batch_destroy(ekf_batch* b) {
   cudaFree(b->bv.xyz_flag); cudaFree(b->bv.xyz_J); cudaFree(b->bv.xyz_y); cudaFree(b->bv.xyz_count);
   cudaFree(b->bv.Sigma); cudaFree(b->bv.mu); cudaFree(b->bv.ctl); cudaFree(b->bv.n); cudaFree(b->bv.N);
   cudaFree(b->match_defer);
-  cudaFree(b->scratch); cudaFree(b->frame); cudaFree(b->picks_dev); cudaFree(b->out_mu14); cudaFree(b->out_S14);
+  cudaFree(b->scratch); cudaFree(b->frame); cudaFree(b->raw); cudaFree(b->picks_dev); cudaFree(b->out_mu14); cudaFree(b->out_S14);
   cudaFree(b->out_stats); cudaFree(b->stage_mu14); cudaFree(b->bv.patchnumbre);
   batch_detect_free(b->det);
   cudaFree(b->det_xy); cudaFree(b->det_n); cudaFree(b->det_num);
@@ -934,7 +998,8 @@ int ekf_batch_create(const ekf_config* cfg, int n_filters, int feature_capacity,
   TRY(cudaSetDevice(device))
   TRY(cudaStreamCreateWithFlags(&b->own_stream, cudaStreamNonBlocking))
   b->stream = b->own_stream;
-  TRY(cudaFuncSetAttribute(k_batch_update, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kUpdSmemBytes))
+  TRY(cudaFuncSetAttribute(k_batch_update<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kUpdSmemBytes))
+  TRY(cudaFuncSetAttribute(k_batch_update<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kUpdSmemBytes))
   const size_t Bn = (size_t)n_filters, cap = Bn * feature_capacity;
   BatchView& v = b->bv;
   v.ld = b->ld; v.Ncap = feature_capacity; v.tstride = w2;
@@ -1038,15 +1103,21 @@ int ekf_batch_set_camera_states(ekf_batch* b, const double* mu14) {
   return EKF_OK;
 }
 
-static int bcapture(ekf_batch* b, const uint8_t* gray, int width, int height, int stride, double stamp, bool dev) {
-  if (!b || !gray || width < 8 || height < 8 || stride < width) return EKF_ERR_ARG;
+// captureNewFrame (vslamRansac.cpp:226-245) for every filter, as the single filter's capture_common: time stamp, then with
+// cfg.scale == 1 and a gray frame one copy; otherwise a resize to (width / scale) x (height / scale) and BGR -> gray in
+// k_capture_resize_gray, from a device frame directly and from a host frame through the staging buffer `raw`.
+static int bcapture(ekf_batch* b, const uint8_t* img, int width, int height, int stride, int channels, double stamp, bool dev) {
+  if (!b || !img || width < 8 || height < 8 || stride < width * channels) return EKF_ERR_ARG;
+  const int scale = b->cfg.scale;
+  const int dw = width / scale, dh = height / scale;   // cv::Size(width / scale, height / scale), integer division
+  if (dw < 8 || dh < 8) return bfail(b, EKF_ERR_ARG, "resized frame smaller than 8 x 8 pixels");
   BCHECK(cudaSetDevice(b->device));
   if (stamp >= 0) {
     if (b->old_ts > 0) b->dT = (stamp - b->old_ts);
     b->old_ts = stamp;
   }
-  const int dstride = (width + 15) & ~15;
-  const size_t need = (size_t)dstride * height;
+  const int dstride = (dw + 15) & ~15;
+  const size_t need = (size_t)dstride * dh;
   if (need > b->frame_cap) {
     BCHECK(cudaStreamSynchronize(b->stream));
     cudaFree(b->frame);
@@ -1054,16 +1125,62 @@ static int bcapture(ekf_batch* b, const uint8_t* gray, int width, int height, in
     BCHECK(cudaMalloc((void**)&b->frame, need));
     b->frame_cap = need;
   }
-  BCHECK(cudaMemcpy2DAsync(b->frame, dstride, gray, stride, width, height, dev ? cudaMemcpyDeviceToDevice : cudaMemcpyHostToDevice,
-                           b->stream));
-  if (b->fv.px != b->frame || b->fv.w != width || b->fv.h != height || b->fv.stride != dstride)
-    match_make_tensor_map(&b->frame_map, b->frame, width, height, dstride, 1, b->cfg.window_size, (int)b->cfg.search_clamp);
-  b->fv = FrameView{b->frame, width, height, dstride};
+  if (scale == 1 && channels == 1) {
+    BCHECK(cudaMemcpy2DAsync(b->frame, dstride, img, stride, width, height, dev ? cudaMemcpyDeviceToDevice : cudaMemcpyHostToDevice,
+                             b->stream));
+  } else {
+    const uint8_t* src = img;
+    int sstride = stride;
+    if (!dev) {
+      const size_t rawneed = (size_t)width * channels * height;
+      if (rawneed > b->raw_cap) {
+        BCHECK(cudaStreamSynchronize(b->stream));
+        cudaFree(b->raw);
+        b->raw = nullptr;
+        BCHECK(cudaMalloc((void**)&b->raw, rawneed));
+        b->raw_cap = rawneed;
+      }
+      BCHECK(cudaMemcpy2DAsync(b->raw, (size_t)width * channels, img, stride, (size_t)width * channels, height, cudaMemcpyHostToDevice,
+                               b->stream));
+      src = b->raw; sstride = width * channels;
+    }
+    launch_capture_resize_gray(b->stream, src, width, height, sstride, channels, b->frame, dw, dh, dstride, &b->launches);
+    BCHECK(cudaGetLastError());
+  }
+  if (b->fv.px != b->frame || b->fv.w != dw || b->fv.h != dh || b->fv.stride != dstride)
+    match_make_tensor_map(&b->frame_map, b->frame, dw, dh, dstride, 1, b->cfg.window_size, (int)b->cfg.search_clamp);
+  b->fv = FrameView{b->frame, dw, dh, dstride};
   b->have_frame = true;
   return EKF_OK;
 }
-int ekf_batch_capture_frame(ekf_batch* b, const uint8_t* g, int w, int h, int s, double stamp) { return bcapture(b, g, w, h, s, stamp, false); }
-int ekf_batch_capture_frame_device(ekf_batch* b, const uint8_t* g, int w, int h, int s, double stamp) { return bcapture(b, g, w, h, s, stamp, true); }
+int ekf_batch_capture_frame(ekf_batch* b, const uint8_t* g, int w, int h, int s, double stamp) { return bcapture(b, g, w, h, s, 1, stamp, false); }
+int ekf_batch_capture_frame_device(ekf_batch* b, const uint8_t* g, int w, int h, int s, double stamp) { return bcapture(b, g, w, h, s, 1, stamp, true); }
+int ekf_batch_capture_frame_bgr(ekf_batch* b, const uint8_t* bgr, int w, int h, int s, double stamp) { return bcapture(b, bgr, w, h, s, 3, stamp, false); }
+
+int ekf_batch_get_frame(ekf_batch* b, uint8_t* out, int* width, int* height) {   // returnGrayImg (vslamRansac.cpp:1364)
+  if (!b || !width || !height) return EKF_ERR_ARG;
+  if (!b->have_frame) return bfail(b, EKF_ERR_STATE, "no frame captured");
+  *width = b->fv.w; *height = b->fv.h;
+  if (out) {
+    BCHECK(cudaSetDevice(b->device));
+    BCHECK(cudaMemcpy2DAsync(out, b->fv.w, b->frame, b->fv.stride, b->fv.w, b->fv.h, cudaMemcpyDeviceToHost, b->stream));
+    BCHECK(cudaStreamSynchronize(b->stream));
+  }
+  return EKF_OK;
+}
+
+int ekf_batch_set_scale(ekf_batch* b, int32_t scale) {
+  if (!b || scale < 1 || scale > 64) return EKF_ERR_ARG;   // the range ekf_create accepts
+  b->cfg.scale = scale;
+  return EKF_OK;
+}
+
+int ekf_batch_set_force_plane(ekf_batch* b, int on) {
+  if (!b) return EKF_ERR_ARG;
+  b->cfg.forsePlane = on != 0;
+  b->dcfg.forsePlane = on != 0;
+  return EKF_OK;
+}
 
 // detection + adds for every filter, filter b asking for num[b * num_stride] corners (<= 0: none); decide: also take the new
 // features' XYZ decisions (in-step top-up).  Enqueued only.
@@ -1116,9 +1233,10 @@ int ekf_batch_step(ekf_batch* b, const double dv[3], const double dw[3], int vco
   launch_match_filter_batch(st, b->bv.ft, b->Ncap, b->bv.N, b->B, b->fv, b->dcfg, &b->frame_map, b->match_defer,
                             b->match_defer + (size_t)b->B * b->Ncap, &b->launches);
   BCHECK(cudaEventRecord(b->ev[2], st));
-  k_batch_update<<<b->B, BUPD_THREADS, kUpdSmemBytes, st>>>(b->bv, b->dcfg, b->picks_dev, n_picks, b->out_mu14, b->out_S14,
-                                                            b->out_stats, b->cfg.min_features, b->cfg.max_features,
-                                                            b->cfg.xyz_conversion);
+  auto* const update = b->cfg.forsePlane ? k_batch_update<true> : k_batch_update<false>;
+  update<<<b->B, BUPD_THREADS, kUpdSmemBytes, st>>>(b->bv, b->dcfg, b->picks_dev, n_picks, b->out_mu14, b->out_S14,
+                                                    b->out_stats, b->cfg.min_features, b->cfg.max_features,
+                                                    b->cfg.xyz_conversion);
   b->launches += 1;
   BCHECK(cudaEventRecord(b->ev[3], st));
   BCHECK(cudaGetLastError());

@@ -294,6 +294,21 @@ class FilterBatch:
         self.h = h
         self.B = int(n_filters)
 
+    @classmethod
+    def from_config(cls, cfg, n_filters, feature_capacity=32, device=0):
+        """A batch from the configuration a VSlamFilter takes: created with motion blur, resize and forsePlane off (which
+        ekf_batch_create requires), then set_motion_blur(cfg.kernel_size) when blur is on, set_scale(cfg.scale) and
+        set_force_plane(cfg.forsePlane)."""
+        base = _abi.EkfConfig.from_buffer_copy(cfg)
+        base.kernel_size, base.scale, base.forsePlane = _abi.default_config().kernel_size, 1, 0
+        batch = cls(base, n_filters, feature_capacity=feature_capacity, device=device)
+        batch.cfg = cfg
+        if cfg.kernel_size < 100000:
+            batch.set_motion_blur(cfg.kernel_size)
+        batch.set_scale(cfg.scale)
+        batch.set_force_plane(cfg.forsePlane)
+        return batch
+
     def close(self):
         if getattr(self, "h", None):
             self.L.ekf_batch_destroy(self.h)
@@ -331,11 +346,30 @@ class FilterBatch:
         self._ck(self.L.ekf_batch_set_camera_states(self.h, _ptr(a)))
 
     def captureNewFrame(self, img, stamp=-1.0):
+        """As VSlamFilter.captureNewFrame: img is an HxW (gray) or HxWx3 (BGR) uint8 host array, resized by 1 / scale
+        (set_scale) and converted to gray inside the call."""
         img = np.ascontiguousarray(img, dtype=np.uint8)
-        self._ck(self.L.ekf_batch_capture_frame(self.h, _ptr(img), img.shape[1], img.shape[0], img.strides[0], float(stamp)))
+        fn = self.L.ekf_batch_capture_frame_bgr if img.ndim == 3 else self.L.ekf_batch_capture_frame
+        self._ck(fn(self.h, _ptr(img), img.shape[1], img.shape[0], img.strides[0], float(stamp)))
 
     def captureNewFrame_device(self, dev_ptr, width, height, stride, stamp=-1.0):
         self._ck(self.L.ekf_batch_capture_frame_device(self.h, C.c_void_p(int(dev_ptr)), width, height, stride, float(stamp)))
+
+    def returnGrayImg(self):
+        """vslamRansac.cpp:1364: the gray frame every filter works on (after resize)."""
+        w, h = C.c_int(0), C.c_int(0)
+        self._ck(self.L.ekf_batch_get_frame(self.h, None, C.byref(w), C.byref(h)))
+        out = np.zeros((h.value, w.value), dtype=np.uint8)
+        self._ck(self.L.ekf_batch_get_frame(self.h, _ptr(out), C.byref(w), C.byref(h)))
+        return out
+
+    def set_scale(self, scale):
+        """EkfConfig.scale for the batch's captures (default 1); the configuration's intrinsics are the resized image's."""
+        self._ck(self.L.ekf_batch_set_scale(self.h, int(scale)))
+
+    def set_force_plane(self, on=True):
+        """EkfConfig.forsePlane for every filter (vslamRansac.cpp:1245-1272; default off)."""
+        self._ck(self.L.ekf_batch_set_force_plane(self.h, int(bool(on))))
 
     def step(self, picks=None, dv=(0.0, 0.0, 0.0), dw=(0.0, 0.0, 0.0), vcontrol=False):
         """predict + update of every filter."""

@@ -96,6 +96,9 @@ class Scene:
     noise_sigma: float = 20.0
     visible_every: int = 1    # > 1: after frame 0 only every visible_every-th feature's template is in the image (m = N / visible_every matches)
     template_smooth: float = 0.0  # > 0: low-pass templates (Gaussian sigma in px) that survive motion-blur prediction
+    planar: bool = False      # a ground robot's camera: y = 0, q = (w, 0, q_y, 0) (identity at frame 0), moving in the x-z plane and
+                              # turning about y only, so that forsePlane's pseudo-measurements (vslamRansac.cpp:1245-1272) hold;
+                              # the filter's prior orientation is Q0, so set its camera state to (r[0], q[0]) before adding features
 
     def __post_init__(self):
         rng = np.random.default_rng(self.seed)
@@ -106,11 +109,15 @@ class Scene:
         v = np.zeros((T, 3)); w = np.zeros((T, 3))
         d = rng.normal(size=3); d /= np.linalg.norm(d)
         e = rng.normal(size=3); e /= np.linalg.norm(e)
+        in_plane = np.array([1.0, 0.0, 1.0]) if self.planar else np.ones(3)      # v components kept
+        about_y = np.array([0.0, 1.0, 0.0]) if self.planar else np.ones(3)       # w components kept
+        if self.planar:
+            d = d * in_plane / np.linalg.norm(d * in_plane); e = np.array([0.0, np.sign(e[1]) or 1.0, 0.0])
         v[0] = self.speed * d; w[0] = self.omega * e
         for t in range(1, T):
-            v[t] = v[t - 1] + rng.normal(scale=self.accel_sigma, size=3)
-            w[t] = w[t - 1] + rng.normal(scale=self.accel_sigma, size=3)
-        r = np.zeros((T, 3)); q = np.zeros((T, 4)); q[0] = Q0
+            v[t] = v[t - 1] + rng.normal(scale=self.accel_sigma, size=3) * in_plane
+            w[t] = w[t - 1] + rng.normal(scale=self.accel_sigma, size=3) * about_y
+        r = np.zeros((T, 3)); q = np.zeros((T, 4)); q[0] = np.array([1.0, 0.0, 0.0, 0.0]) if self.planar else Q0
         for t in range(1, T):
             r[t] = r[t - 1] + dT * v[t]
             q[t] = quat_mul(q[t - 1], vec2quat(dT * w[t]))
