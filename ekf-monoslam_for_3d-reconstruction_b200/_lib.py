@@ -59,6 +59,8 @@ SIGNATURES = {
     "ekf_get_S_blocks": (_i, [_vp, _vp]),
     "ekf_match_batch": (_i, [_vp, _i, _i, _i, _i, _vp, _i, _i, _vp, _vp, _f, _f, _f, _vp, _vp, _vp]),
     "ekf_batch_create": (_i, [_P(_abi.EkfConfig), _i, _i, _i, _P(_vp)]),
+    "ekf_batch_create_large": (_i, [_P(_abi.EkfConfig), _i, _i, _i, _P(_vp)]),
+    "ekf_batch_update_clusters": (_i, [_vp, _P(_i), _P(_i)]),
     "ekf_batch_destroy": (_i, [_vp]),
     "ekf_batch_describe": (_i, [_vp, _P(_abi.EkfBatchDesc)]),
     "ekf_batch_set_stream": (_i, [_vp, _vp]),

@@ -18,11 +18,16 @@
 // filter asking for features (V:1312-1315), that filter's pass removes only; the batched detector
 // (ekf_batch_detect.cu) and k_batch_add then add its new features, and a second k_batch_compact converts.
 // Frames are captured once for the whole batch, resized and converted to gray when ekf_batch_set_scale / a BGR source ask.
+// ekf_batch_create_large: up to BNCAP_L = 128 features (n <= 782); the update then runs on a cluster of 2 to 4 CTAs per filter
+// (k_batch_update_cluster) and the other kernels take their BNCAP_L instantiations.  Sigma and the compaction scratch are
+// B x ncap x ld doubles each: 4.9 MB per filter each at capacity 128, 40 GB in total for 4096 filters.
 // Every stage evaluates the same expressions as the single-filter kernels (same device functions).
 #include <algorithm>
 #include <cstdio>
 #include <string>
 #include <vector>
+
+#include <cooperative_groups.h>
 
 #include "../../include/ekf_b200.h"
 #include "ekf_blur.cuh"
@@ -32,8 +37,11 @@
 #include "ekf_kernels.h"
 #include "ekf_math.cuh"
 
+namespace cg = cooperative_groups;
+
 #define BK 64                 // measurement rows of one stacked update (<= 32 features)
-#define BNCAP 32              // feature capacity of a batched filter
+#define BNCAP 32              // feature capacity of a batched filter created by ekf_batch_create
+#define BNCAP_L EKF_BATCH_MAX_FEATURES   // 128: feature capacity of one from ekf_batch_create_large
 #define BNMAX (EKF_CAM + 6 * BNCAP + 2)  // 208: state rows rounded up to a multiple of 8
 #define BLDW (BK + 4)         // row stride of W / V / Linv in shared memory (conflict-free fragment reads)
 #define BUPD_THREADS FACT_THREADS
@@ -69,6 +77,24 @@ __device__ void warp_xyz_decide(const BatchView& bv, int b, const double* Sigma,
   }
   if (i < N) bv.xyz_flag[k] = conv;
   const int cnt = __popc(__ballot_sync(0xffffffffu, conv));
+  if (i == 0) bv.xyz_count[b] = cnt;
+}
+
+// The same decisions for up to blockDim.x features, one thread per feature (large batches).  use_alive: only features not
+// flagged for removal and other than `victim` are eligible (in a step); otherwise every one (convert2XYZ_ifLinearAll).
+// Called by the whole CTA; thread 0 stores the filter's count.
+__device__ void cta_xyz_decide(const BatchView& bv, int b, const double* Sigma, const double* mu, const FeatTab& ft, int N,
+                               bool use_alive, int victim, const DevCfg& cfg) {
+  const int i = threadIdx.x;
+  const size_t k = (size_t)b * bv.Ncap + i;
+  int conv = 0;
+  if (i < N && !ft.coding[i] && (!use_alive || (!ft.removef[i] && i != victim))) {
+    const int pos = ft.pos[i];
+    conv = xyz_linear_decide(mu + pos, mu, Sigma[(size_t)(pos + 5) * bv.ld + pos + 5], cfg.linearity_threshold,
+                             cfg.abs_int_quirk, bv.xyz_y + 3 * k, bv.xyz_J + 18 * k);
+  }
+  if (i < N) bv.xyz_flag[k] = conv;
+  const int cnt = __syncthreads_count(conv);
   if (i == 0) bv.xyz_count[b] = cnt;
 }
 
@@ -208,38 +234,47 @@ __global__ void __launch_bounds__(BPRED_THREADS, 4) k_batch_predict(BatchView bv
 // out[B + b] = 1 when a kernel exceeded BLUR_MAXK (that template stays unblurred, as in k_predict_blur).
 // ------------------------------------------------------------------------------------------------
 #define BBLUR_WARPS 4
+// NC: feature capacity (BNCAP or BNCAP_L); warp 0 takes the decisions 32 features at a time, in ascending order.
+template <int NC>
 __global__ void __launch_bounds__(BBLUR_WARPS * 32) k_batch_predict_blur(BatchView bv, DevCfg cfg, double dT, int* __restrict__ out) {
-  __shared__ int s_feat[BNCAP], s_rows[BNCAP], s_cols[BNCAP], s_nblur;
-  __shared__ double s_dx[BNCAP], s_dy[BNCAP];
+  __shared__ int s_feat[NC], s_rows[NC], s_cols[NC], s_nblur;
+  __shared__ double s_dx[NC], s_dy[NC];
   __shared__ __align__(16) uint8_t s_tmpl[BBLUR_WARPS][1024];
   __shared__ int s_seq[BBLUR_WARPS][BLUR_MAXPTS], s_coef[BBLUR_WARPS][BLUR_MAXPTS];
   const int b = blockIdx.x, lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   const int N = bv.N[b], ld = bv.ld;
   const double* mu = bv.mu + (size_t)b * ld;
   const FeatTab ft = feattab_slice(bv.ft, b, bv.Ncap, bv.tstride);
-  if (warp == 0) {   // N <= BNCAP = 32: one feature per lane
-    const int f = lane;
-    int d = 0, krows = 0, kcols = 0;
-    double ddx = 0.0, ddy = 0.0;
-    if (f < N && ft.innov[f]) {
-      double cam[13], rb[3], Rb[9];
-      for (int c = 0; c < 13; ++c) cam[c] = mu[c];   // predicted camera state, committed by k_batch_predict
-      blur_pose(cam, cfg.T_camera, dT, rb, Rb);
-      const int pos = ft.pos[f], coding = ft.coding[f];
-      double fs[6];
-      for (int c = 0; c < (coding ? 3 : 6); ++c) fs[c] = mu[pos + c];
-      blur_displacement(cfg.cam, fs, coding, rb, Rb, ft.h[2 * f], ft.h[2 * f + 1], &ddx, &ddy);
-      d = blur_decide(ddx, ddy, cfg.kernel_min_size, &krows, &kcols);
-    }
-    const unsigned blur = __ballot_sync(0xffffffffu, d > 0), big = __ballot_sync(0xffffffffu, d < 0);
-    if (d > 0) {
-      const int k = __popc(blur & ((1u << lane) - 1u));
-      s_feat[k] = f; s_rows[k] = krows; s_cols[k] = kcols; s_dx[k] = ddx; s_dy[k] = ddy;
+  if (warp == 0) {   // one feature per lane, NC / 32 rounds
+    int nblur = 0;
+    unsigned anybig = 0u;
+#pragma unroll
+    for (int f0 = 0; f0 < NC; f0 += 32) {
+      const int f = f0 + lane;
+      int d = 0, krows = 0, kcols = 0;
+      double ddx = 0.0, ddy = 0.0;
+      if (f < N && ft.innov[f]) {
+        double cam[13], rb[3], Rb[9];
+        for (int c = 0; c < 13; ++c) cam[c] = mu[c];   // predicted camera state, committed by k_batch_predict
+        blur_pose(cam, cfg.T_camera, dT, rb, Rb);
+        const int pos = ft.pos[f], coding = ft.coding[f];
+        double fs[6];
+        for (int c = 0; c < (coding ? 3 : 6); ++c) fs[c] = mu[pos + c];
+        blur_displacement(cfg.cam, fs, coding, rb, Rb, ft.h[2 * f], ft.h[2 * f + 1], &ddx, &ddy);
+        d = blur_decide(ddx, ddy, cfg.kernel_min_size, &krows, &kcols);
+      }
+      const unsigned blur = __ballot_sync(0xffffffffu, d > 0), big = __ballot_sync(0xffffffffu, d < 0);
+      if (d > 0) {
+        const int k = nblur + __popc(blur & ((1u << lane) - 1u));
+        s_feat[k] = f; s_rows[k] = krows; s_cols[k] = kcols; s_dx[k] = ddx; s_dy[k] = ddy;
+      }
+      nblur += __popc(blur);
+      anybig |= big;
     }
     if (lane == 0) {
-      s_nblur = __popc(blur);
-      out[b] = __popc(blur);
-      out[gridDim.x + b] = big != 0u;
+      s_nblur = nblur;
+      out[b] = nblur;
+      out[gridDim.x + b] = anybig != 0u;
     }
   }
   __syncthreads();
@@ -667,6 +702,419 @@ __global__ void __launch_bounds__(BUPD_THREADS, 1) k_batch_update(BatchView bv, 
 }
 
 // ------------------------------------------------------------------------------------------------
+// update for one filter per CLUSTER of C = ceil(ld / BSTRIP) CTAs (2 to 4; ekf_batch_create_large, capacity 33 to 128).
+// Every CTA has k_batch_update's 512 threads and UpdSmem layout; CTA r owns rows [BSTRIP r, BSTRIP r + BSTRIP) of W / V, of
+// Sigma and of the correction delta (sm.mu_i), and reads the other CTAs' W / V panels and delta strips through distributed
+// shared memory.  BSTRIP = 208 = 13 x 16, so the downdate's 16 x 16 tiles never straddle two CTAs.
+//   * rank 0 runs 1-point RANSAC (mu_i in its idle Cholesky workspace), the Hi rescue and the book-keeping; the others wait at
+//     the cluster barrier.
+//   * an update over cnt features runs as ceil(cnt / 32) blocks of at most BK rows, block b with the innovation
+//     (z_b - h_b) - H_b delta, delta the correction of the earlier blocks (the single filter's blocked schedules,
+//     ekf_update.cu); mu += delta and one quaternion normalisation follow the last block.
+//   * per block: each CTA gathers its rows of W = Sigma H^T; barrier; every CTA forms the same S = H W + R and nu from the
+//     owners' W rows and delta entries; barrier; every CTA factors S (same inputs, same code: the same L bits everywhere), solves
+//     V = W L^-T and accumulates delta += V y on its rows; barrier; each CTA downdates its row strip over all columns, the
+//     b-fragments of a column tile from its owner's V; barrier.
+// ------------------------------------------------------------------------------------------------
+#define BSTRIP BNMAX
+#define BCL_MAX 4
+
+static __device__ __forceinline__ void cl_sync() { cg::this_cluster().sync(); }
+// row `row` of the panel `p` (W or the delta strip, row stride ldp) of the CTA owning it
+static __device__ __forceinline__ double* cl_row(double* p, int row, int ldp) {
+  return cg::this_cluster().map_shared_rank(p + (size_t)(row % BSTRIP) * ldp, row / BSTRIP);
+}
+
+// One block of the features ft.sel[a0 .. a0 + m) (m <= BK / 2): W own rows, S, nu; ends with the S / nu cluster barrier.
+__device__ void cl_gather_features(const UpdSmem& sm, int rank, double* Sigma, int ld, int n, const FeatTab& ft, int a0, int m,
+                                   const DevCfg& cfg) {
+  const int tid = threadIdx.x, k = 2 * m, row0 = rank * BSTRIP;
+  int* fids = sm.ibuf + BNCAP; int* poss = fids + BNCAP; int* nds = poss + BNCAP;
+  for (int a = tid; a < BNCAP; a += BUPD_THREADS) {
+    if (a < m) {
+      const int f = ft.sel[a0 + a];
+      fids[a] = f; poss[a] = ft.pos[f]; nds[a] = 7 + (ft.coding[f] ? 3 : 6);
+    } else { fids[a] = -1; poss[a] = 0; nds[a] = 0; }
+  }
+  __syncthreads();
+  for (int e = tid; e < BNCAP * 26; e += BUPD_THREADS) {
+    const int a = e / 26, c = e % 26;
+    sm.Hs[a * 27 + c] = (a < m) ? ft.Hc[26 * fids[a] + c] : 0.0;
+  }
+  __syncthreads();
+  // W = Sigma H^T on the CTA's rows: thread = (row, feature), 16 rows x 32 features a pass, the 13 loads of a row in flight
+  {
+    const int rl = tid >> 5, a = tid & 31;
+    const int pos = poss[a], nd = nds[a];
+    const double* hs = sm.Hs + a * 27;
+    for (int r0 = 0; r0 < BSTRIP; r0 += 16) {
+      const int il = r0 + rl, i = row0 + il;
+      double w0 = 0, w1 = 0;
+      if (i < n && a < m) {
+        const double* row = Sigma + (size_t)i * ld;
+        double sg[13];
+#pragma unroll
+        for (int c = 0; c < 13; ++c) sg[c] = (c < nd) ? row[ekf_idx13(c, pos)] : 0.0;
+#pragma unroll
+        for (int c = 0; c < 13; ++c)
+          if (c < nd) { w0 += sg[c] * hs[c]; w1 += sg[c] * hs[13 + c]; }
+      }
+      *reinterpret_cast<double2*>(sm.W + (size_t)il * BLDW + 2 * a) = make_double2(w0, w1);
+    }
+  }
+  __syncthreads();
+  cl_sync();   // every CTA's W rows and delta strip are final
+  if (tid < BK) {   // nu = (z - h) - H delta
+    double v = 0.0;
+    if (tid < k) {
+      const int a = tid >> 1, f = fids[a];
+      v = ft.z[2 * f + (tid & 1)] - ft.h[2 * f + (tid & 1)];
+      if (a0 > 0) {
+        const int pos = poss[a], nd = nds[a];
+        const double* hc = sm.Hs + a * 27 + 13 * (tid & 1);
+        double acc = 0;
+        for (int c = 0; c < nd; ++c) acc += hc[c] * *cl_row(sm.mu_i, ekf_idx13(c, pos), 1);
+        v = v - acc;
+      }
+    }
+    sm.nu[tid] = v;
+  }
+  // S = H W + sigma_px^2 I from the owners' W rows; rows / columns past k are identity
+  for (int e = tid; e < BK * BK; e += BUPD_THREADS) {
+    const int r = e / BK, s = e % BK;
+    double v = (r == s) ? 1.0 : 0.0;
+    if (r < k && s < k) {
+      const int a = r >> 1;
+      const int pos = poss[a], nd = nds[a];
+      const double* hc = sm.Hs + a * 27 + 13 * (r & 1);
+      double acc = 0;
+      for (int c = 0; c < nd; ++c) acc += hc[c] * cl_row(sm.W, ekf_idx13(c, pos), BLDW)[s];
+      v = acc + ((r == s) ? cfg.sigma_pixel_2 : 0.0);
+    }
+    sm.Sb[r * BLDW + s] = v;
+  }
+  __syncthreads();
+  cl_sync();   // no CTA reads another's W or delta any more: V may overwrite W
+}
+
+// The plane block (cta_gather_plane) in a cluster: W[:, j] = Sigma[:, k_j] on the CTA's rows, nu_j = (0 - mu[k_j]) - delta[k_j],
+// S = W[{1, 4, 6}, :] + 1e-5 I from rank 0's rows.
+__device__ void cl_gather_plane(const UpdSmem& sm, int rank, double* Sigma, int ld, int n, const double* mu, DevCtl* ctl) {
+  const int tid = threadIdx.x, row0 = rank * BSTRIP;
+  for (int e = tid; e < BSTRIP * (BK / 2); e += BUPD_THREADS) {
+    const int il = e / (BK / 2), c = 2 * (e % (BK / 2)), i = row0 + il;
+    double2 v = make_double2(0.0, 0.0);
+    if (i < n && c == 0) v = make_double2(Sigma[(size_t)i * ld + 1], Sigma[(size_t)i * ld + 4]);
+    if (i < n && c == 2) v.x = Sigma[(size_t)i * ld + 6];
+    *reinterpret_cast<double2*>(sm.W + (size_t)il * BLDW + c) = v;
+  }
+  if (rank == 0 && tid == 0) ctl->k_rows += 3;
+  __syncthreads();
+  cl_sync();
+  if (tid < BK) {
+    double v = 0.0;
+    if (tid < 3) {
+      const int kj = tid == 0 ? 1 : (tid == 1 ? 4 : 6);
+      v = (0.0 - mu[kj]) - *cl_row(sm.mu_i, kj, 1);
+    }
+    sm.nu[tid] = v;
+  }
+  for (int e = tid; e < BK * BK; e += BUPD_THREADS) {
+    const int r = e / BK, s = e % BK;
+    double v = (r == s) ? 1.0 : 0.0;
+    if (r < 3 && s < 3) v = cl_row(sm.W, r == 0 ? 1 : (r == 1 ? 4 : 6), BLDW)[s] + ((r == s) ? 0.00001 : 0.0);
+    sm.Sb[r * BLDW + s] = v;
+  }
+  __syncthreads();
+  cl_sync();
+}
+
+// Gain and downdate of the gathered block of k rows: L = chol(S) in every CTA, V = W L^-T and delta += V y on the CTA's rows,
+// Sigma -= V V^T on its row strip over all columns (b-fragments from the column tile's owner).  Ends with a cluster barrier.
+__device__ void cl_block_gain_downdate(const UpdSmem& sm, int rank, double* __restrict__ Sigma, int ld, int n, int k, DevCtl* ctl) {
+  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5, g = lane >> 2, t4 = lane & 3;
+  const int row0 = rank * BSTRIP;
+  cta_chol_panel<BK>(sm.fact, sm.Sb, BLDW, sm.nu, sm.Sb, BLDW, sm.Dv, BLDD, sm.y, &ctl->chol_fail);
+  for (int rt = warp; rt < BSTRIP / 8; rt += BUPD_THREADS / 32) {
+    double part = warp_trsm_tile<BK>(sm.W + (size_t)rt * 8 * BLDW, BLDW, sm.Sb, BLDW, sm.Dv, BLDD, sm.y);
+    part += __shfl_xor_sync(0xffffffffu, part, 1);
+    part += __shfl_xor_sync(0xffffffffu, part, 2);
+    const int il = rt * 8 + g;
+    if (t4 == 0 && row0 + il < n) sm.mu_i[il] += part;
+  }
+  __syncthreads();
+  cl_sync();   // every CTA's V is final
+  {
+    const int rows = min(max(n - row0, 0), BSTRIP);
+    const int nt = (n + 15) >> 4, rtl = (rows + 15) >> 4, ksteps = (k + 3) >> 2, ntile = rtl * nt;
+    auto load_c = [&](int t, double (&c)[2][2][2]) {
+      const int ti = t / nt, tj = t - ti * nt;
+#pragma unroll
+      for (int a = 0; a < 2; ++a)
+#pragma unroll
+        for (int cc = 0; cc < 2; ++cc) {
+          const int r = row0 + ti * 16 + a * 8 + g, col = tj * 16 + cc * 8 + 2 * t4;
+          double2 v = make_double2(0.0, 0.0);
+          if (t < ntile) {
+            if (r < n && col + 1 < n) v = *reinterpret_cast<const double2*>(Sigma + (size_t)r * ld + col);
+            else if (r < n && col < n) v.x = Sigma[(size_t)r * ld + col];
+          }
+          c[a][cc][0] = v.x; c[a][cc][1] = v.y;
+        }
+    };
+    double nxt[2][2][2];
+    load_c(warp, nxt);
+    for (int t = warp; t < ntile; t += BUPD_THREADS / 32) {
+      const int ti = t / nt, tj = t - ti * nt;
+      double acc[2][2][2];
+#pragma unroll
+      for (int a = 0; a < 2; ++a)
+#pragma unroll
+        for (int cc = 0; cc < 2; ++cc) { acc[a][cc][0] = nxt[a][cc][0]; acc[a][cc][1] = nxt[a][cc][1]; }
+      load_c(t + BUPD_THREADS / 32, nxt);
+      const double* va = sm.W + (size_t)(ti * 16 + g) * BLDW + t4;
+      const double* vb = cl_row(sm.W, tj * 16 + g, BLDW) + t4;   // the owner's V (tiles never straddle two CTAs)
+      for (int q = 0; q < ksteps; ++q) {
+        const double a0 = va[4 * q], a1 = va[8 * BLDW + 4 * q];
+        const double b0 = -vb[4 * q], b1 = -vb[8 * BLDW + 4 * q];
+        dmma884f(acc[0][0][0], acc[0][0][1], a0, b0);
+        dmma884f(acc[0][1][0], acc[0][1][1], a0, b1);
+        dmma884f(acc[1][0][0], acc[1][0][1], a1, b0);
+        dmma884f(acc[1][1][0], acc[1][1][1], a1, b1);
+      }
+#pragma unroll
+      for (int a = 0; a < 2; ++a)
+#pragma unroll
+        for (int cc = 0; cc < 2; ++cc) {
+          const int r = row0 + ti * 16 + a * 8 + g, col = tj * 16 + cc * 8 + 2 * t4;
+          if (r < n && col + 1 < n) *reinterpret_cast<double2*>(Sigma + (size_t)r * ld + col) = make_double2(acc[a][cc][0], acc[a][cc][1]);
+          else if (r < n && col < n) Sigma[(size_t)r * ld + col] = acc[a][cc][0];
+        }
+    }
+  }
+  __syncthreads();
+  cl_sync();   // no CTA reads another's V any more: the next block may overwrite W
+}
+
+// End of an update: mu += delta on every CTA's rows, then normalizeQuaternion (V:1625-1642): every CTA takes J from mu[3..6]
+// and applies it to columns 3..6 of its rows; rank 0, the owner of rows 3..6, also to those rows and the 4 x 4 corner.  Ends
+// with a cluster barrier: Sigma and mu are final for every CTA.
+__device__ void cl_finish_update(const UpdSmem& sm, int rank, double* __restrict__ Sigma, int ld, int n, double* __restrict__ mu) {
+  const int tid = threadIdx.x, row0 = rank * BSTRIP, rows = min(max(n - row0, 0), BSTRIP);
+  for (int il = tid; il < rows; il += BUPD_THREADS) { mu[row0 + il] += sm.mu_i[il]; sm.mu_i[il] = 0.0; }
+  __syncthreads();
+  cl_sync();   // mu[3..6] final
+  double* J = sm.qj; double* Cq = J + 16; double* Tq = Cq + 16;
+  double q[4] = {0.0, 0.0, 0.0, 0.0}, norma = 0.0;
+  if (tid == 0) {
+    for (int i = 0; i < 4; ++i) q[i] = mu[3 + i];
+    norma = sqrt(q[0] * q[0] + q[1] * q[1] + q[2] * q[2] + q[3] * q[3]);
+    const double sc = 1 / (norma * norma * norma);
+    for (int i = 0; i < 4; ++i)
+      for (int j = 0; j < 4; ++j) J[i * 4 + j] = ((norma * norma) * (i == j ? 1.0 : 0.0) - q[i] * q[j]) * sc;
+  }
+  if (rank == 0 && tid >= 32 && tid < 48) Cq[tid - 32] = Sigma[(size_t)(3 + (tid - 32) / 4) * ld + 3 + ((tid - 32) % 4)];
+  __syncthreads();
+  cl_sync();   // every CTA has read mu[3..6]
+  if (rank == 0) {
+    if (tid == 0)
+      for (int i = 0; i < 4; ++i) mu[3 + i] = q[i] / norma;
+    if (tid < 16) {
+      const int a = tid / 4, c = tid % 4;
+      double t = 0;
+      for (int kk = 0; kk < 4; ++kk) t += J[a * 4 + kk] * Cq[kk * 4 + c];
+      Tq[tid] = t;
+    }
+    __syncthreads();
+    if (tid < 16) {
+      const int a = tid / 4, c = tid % 4;
+      double s = 0;
+      for (int kk = 0; kk < 4; ++kk) s += Tq[a * 4 + kk] * J[c * 4 + kk];
+      Sigma[(size_t)(3 + a) * ld + 3 + c] = s;
+    }
+    for (int jj = tid; jj < n - 4; jj += BUPD_THREADS) {   // rows 3..6, every column but 3..6
+      const int j = jj >= 3 ? jj + 4 : jj;
+      double x[4], yv[4];
+      for (int c = 0; c < 4; ++c) x[c] = Sigma[(size_t)(3 + c) * ld + j];
+      for (int a = 0; a < 4; ++a) {
+        double s = 0;
+        for (int c = 0; c < 4; ++c) s += J[a * 4 + c] * x[c];
+        yv[a] = s;
+      }
+      for (int a = 0; a < 4; ++a) Sigma[(size_t)(3 + a) * ld + j] = yv[a];
+    }
+  }
+  for (int il = tid; il < rows; il += BUPD_THREADS) {   // columns 3..6 of the CTA's rows but 3..6
+    const int j = row0 + il;
+    if (j >= 3 && j < 7) continue;
+    double x[4], yv[4];
+    double* row = Sigma + (size_t)j * ld + 3;
+    for (int c = 0; c < 4; ++c) x[c] = row[c];
+    for (int a = 0; a < 4; ++a) {
+      double s = 0;
+      for (int c = 0; c < 4; ++c) s += x[c] * J[a * 4 + c];
+      yv[a] = s;
+    }
+    for (int a = 0; a < 4; ++a) row[a] = yv[a];
+  }
+  __syncthreads();
+  cl_sync();
+}
+
+// A stacked update over the `cnt` features listed in ft.sel, in blocks of at most BK / 2 features.
+__device__ void cl_feature_blocks(const UpdSmem& sm, int rank, double* Sigma, int ld, int n, const FeatTab& ft, int cnt,
+                                  const DevCfg& cfg, DevCtl* ctl) {
+  for (int a0 = 0; a0 < cnt; a0 += BK / 2) {
+    const int m = min(BK / 2, cnt - a0);
+    cl_gather_features(sm, rank, Sigma, ld, n, ft, a0, m, cfg);
+    cl_block_gain_downdate(sm, rank, Sigma, ld, n, 2 * m, ctl);
+  }
+}
+
+// high-innovation rescue (k_hi_rescue) by rank 0: pose from the old mu, feature parameters from mu_tmp; sets ft.hi, ft.sel, n_hi
+static __device__ __noinline__ void cl_hi_rescue(double* Sigma, int ld, const double* mu, FeatTab ft, int N, DevCtl* ctl,
+                                                 const DevCfg& cfg) {
+  const int tid = threadIdx.x;
+  for (int i = tid; i < N; i += BUPD_THREADS) {
+    int flag = 0;
+    if (!ft.li[i] && ft.innov[i]) {
+      const int pos = ft.pos[i], coding = ft.coding[i];
+      const int fsz = coding ? 3 : 6, nd = 7 + fsz;
+      double fs[6], r[3], qc[4], Rcw[9], hi[2], Hc[26], hcz;
+      for (int c = 0; c < fsz; ++c) fs[c] = mu[pos + c];
+      for (int c = 0; c < 3; ++c) r[c] = ctl->cam_old[c];
+      qc[0] = ctl->cam_old[3]; qc[1] = -ctl->cam_old[4]; qc[2] = -ctl->cam_old[5]; qc[3] = -ctl->cam_old[6];
+      d_quat2rot(qc, Rcw);
+      d_feature_hH(cfg.cam, fs, coding, r, qc, Rcw, hi, Hc, &hcz);
+      ft.h[2 * i] = hi[0]; ft.h[2 * i + 1] = hi[1];
+      for (int c = 0; c < 26; ++c) ft.Hc[26 * i + c] = Hc[c];
+      double Tm[26];
+      for (int bb = 0; bb < nd; ++bb) {
+        const int jb = ekf_idx13(bb, pos);
+        double sg[13];
+#pragma unroll
+        for (int c = 0; c < 13; ++c) sg[c] = (c < nd) ? Sigma[(size_t)ekf_idx13(c, pos) * ld + jb] : 0.0;
+        double t0 = 0, t1 = 0;
+#pragma unroll
+        for (int c = 0; c < 13; ++c)
+          if (c < nd) { t0 += Hc[c] * sg[c]; t1 += Hc[13 + c] * sg[c]; }
+        Tm[bb] = t0; Tm[13 + bb] = t1;
+      }
+      double S[4] = {0, 0, 0, 0};
+      for (int bb = 0; bb < nd; ++bb) {
+        S[0] += Tm[bb] * Hc[bb]; S[1] += Tm[bb] * Hc[13 + bb];
+        S[2] += Tm[13 + bb] * Hc[bb]; S[3] += Tm[13 + bb] * Hc[13 + bb];
+      }
+      const double det = S[0] * S[3] - S[2] * S[1];
+      const double invdet = 1.0 / det;
+      const double i00 = S[3] * invdet, i10 = -S[2] * invdet, i01 = -S[1] * invdet, i11 = S[0] * invdet;
+      const double e0 = hi[0] - ft.z[2 * i], e1 = hi[1] - ft.z[2 * i + 1];
+      const double t0 = e0 * i00 + e1 * i10;
+      const double t1 = e0 * i01 + e1 * i11;
+      const double chi = t0 * e0 + t1 * e1;
+      flag = (chi <= cfg.th_hi) ? 1 : 0;
+    }
+    ft.hi[i] = flag;
+  }
+  __syncthreads();
+  const int nh = block_compact(ft.hi, N, ft.sel, ft.pos_in_z);
+  if (tid == 0) { ctl->n_hi = nh; ctl->k_rows = 2 * nh; }
+}
+
+template <bool PLANE>
+__global__ void __launch_bounds__(BUPD_THREADS, 1) k_batch_update_cluster(BatchView bv, DevCfg cfg, const uint32_t* __restrict__ picks,
+                                                                          int n_picks, double* __restrict__ out_mu14,
+                                                                          double* __restrict__ out_S14, int* __restrict__ out_stats,
+                                                                          int min_features, int max_features, int xyz_conversion) {
+  extern __shared__ __align__(16) double usm[];
+  UpdSmem sm;
+  sm.W = usm;
+  sm.fact = sm.W + (size_t)BNMAX * BLDW;
+  sm.Dv = sm.fact + kFactDoubles;
+  sm.Sb = sm.Dv + (BK / 32) * 32 * BLDD;
+  sm.nu = sm.Sb + (size_t)BK * BLDW;
+  sm.y = sm.nu + BK;
+  sm.mu_i = sm.y + BK;   // here: the correction delta of the CTA's rows
+  sm.Hs = sm.mu_i + BNMAX;
+  sm.qj = sm.Hs + BNCAP * 27;
+  sm.ibuf = reinterpret_cast<int*>(sm.qj + 48);
+  const int C = (int)cg::this_cluster().num_blocks(), rank = (int)cg::this_cluster().block_rank();
+  const int b = blockIdx.x / C, tid = threadIdx.x;
+  const int n = bv.n[b], N = bv.N[b], ld = bv.ld;
+  double* Sigma = bv.Sigma + (size_t)b * bv.sstride;
+  double* mu = bv.mu + (size_t)b * ld;
+  const FeatTab ft = feattab_slice(bv.ft, b, bv.Ncap, bv.tstride);
+  DevCtl* ctl = bv.ctl + b;
+  for (int i = tid; i < BSTRIP; i += BUPD_THREADS) sm.mu_i[i] = 0.0;
+  if (rank == 0) {   // 1-point RANSAC: mu_i (n <= 782) in the Cholesky workspace, the candidates (N <= 128) in ibuf
+    if (tid == 0) ctl->chol_fail = 0;
+    cta_ransac(Sigma, ld, n, mu, ft, N, ctl, cfg, picks, n_picks, sm.fact, sm.ibuf);
+  }
+  __syncthreads();
+  cl_sync();
+  const int n_li = *(volatile int*)&ctl->n_li;
+  if (n_li > 0) {
+    cl_feature_blocks(sm, rank, Sigma, ld, n, ft, n_li, cfg, ctl);
+    cl_finish_update(sm, rank, Sigma, ld, n, mu);
+  }
+  if (rank == 0) cl_hi_rescue(Sigma, ld, mu, ft, N, ctl, cfg);
+  __syncthreads();
+  cl_sync();
+  const int n_hi = *(volatile int*)&ctl->n_hi;
+  if constexpr (PLANE) {   // the Hi blocks, the plane block, one normalisation
+    if (n_hi > 0) cl_feature_blocks(sm, rank, Sigma, ld, n, ft, n_hi, cfg, ctl);
+    cl_gather_plane(sm, rank, Sigma, ld, n, mu, ctl);
+    cl_block_gain_downdate(sm, rank, Sigma, ld, n, 3, ctl);
+    cl_finish_update(sm, rank, Sigma, ld, n, mu);
+  } else {
+    if (n_hi > 0) {
+      cl_feature_blocks(sm, rank, Sigma, ld, n, ft, n_hi, cfg, ctl);
+      cl_finish_update(sm, rank, Sigma, ld, n, mu);
+    }
+  }
+  if (rank != 0) return;   // the last cluster barrier is behind every CTA: nobody reads this CTA's shared memory any more
+  // book-keeping (k_bookkeeping) + visibility count (V:1296-1315), as k_batch_update
+  int my_remove = 0, my_vis = 0;
+  for (int i = tid; i < N; i += BUPD_THREADS) {
+    int nfind = ft.n_find[i];
+    const int ntot = ft.n_tot[i];
+    if (ft.hi[i] || ft.li[i]) nfind++;
+    ft.n_find[i] = nfind;
+    const float qi = (float)(ntot - nfind) / ((float)nfind);
+    ft.quality[i] = qi;
+    if (qi > cfg.quality_ratio) ft.removef[i] = 1;
+    if (ft.removef[i]) my_remove++;
+    else if (ft.innov[i]) my_vis++;
+  }
+  const int n_rem = __syncthreads_count(my_remove);   // N <= 128 <= blockDim: one feature per thread
+  const int n_vis = __syncthreads_count(my_vis);
+  for (int e = tid; e < 14; e += BUPD_THREADS) out_mu14[(size_t)b * 14 + e] = mu[e];
+  if (out_S14)
+    for (int e = tid; e < 196; e += BUPD_THREADS) out_S14[(size_t)b * 196 + e] = Sigma[(size_t)(e / 14) * ld + (e % 14)];
+  const bool drop_first = (n_vis < min_features) && (N - n_rem > max_features);
+  if (tid == 0) {
+    int* st = out_stats + (size_t)b * EKF_BATCH_STAT_FIELDS;
+    int removed = n_rem, topup = 0;
+    if (n_vis < min_features) {
+      if (N - n_rem > max_features) removed += 1;   // removeFeature(0) (V:1313), applied by k_batch_compact
+      topup = min_features - n_vis;
+    }
+    ctl->n_remove = removed;
+    ctl->n_visible = n_vis;
+    st[EKF_BSTAT_INNOV] = ctl->m_innov; st[EKF_BSTAT_MATCHED] = ctl->n_matched; st[EKF_BSTAT_LI] = n_li;
+    st[EKF_BSTAT_HI] = n_hi; st[EKF_BSTAT_HYPS] = ctl->ransac_hyps; st[EKF_BSTAT_CHOL_FAIL] = ctl->chol_fail;
+    st[EKF_BSTAT_REMOVED] = removed; st[EKF_BSTAT_TOPUP] = topup;
+    int victim = -1;   // removeFeature(0)'s victim: the first feature not flagged (k_batch_update's decision)
+    if (drop_first)
+      for (int f = 0; f < N && victim < 0; ++f)
+        if (!ft.removef[f]) victim = f;
+    sm.ibuf[0] = victim;
+  }
+  __syncthreads();
+  if (xyz_conversion) cta_xyz_decide(bv, b, Sigma, mu, ft, N, true, sm.ibuf[0], cfg);
+}
+
+// ------------------------------------------------------------------------------------------------
 // removeFeature (V:373-421) for every flagged feature (remove != 0) and convert2XYZ_ifLinear (V:741-772) for every
 // feature decided in bv.xyz_flag, of every filter that has either, in one pass: Sigma / mu are rebuilt through the
 // filter's slice of the scratch buffer, the feature table through registers.  The row map carries (src, code) as in
@@ -676,11 +1124,14 @@ __global__ void __launch_bounds__(BUPD_THREADS, 1) k_batch_update(BatchView bv, 
 // ------------------------------------------------------------------------------------------------
 #define BCMP_THREADS 256
 // hold (stats of the step, or NULL): a filter whose EKF_BSTAT_TOPUP is set only removes here, and its pending decisions move
-// with the surviving records; the conversions follow its new features (ekf_batch_step).
+// with the surviving records; the conversions follow its new features (ekf_batch_step).  NC: feature capacity (BNCAP or
+// BNCAP_L); one CTA covers every entry of n2 x n2 either way, and every record (N2 <= 128 <= BCMP_THREADS).
+template <int NC>
 __global__ void __launch_bounds__(BCMP_THREADS) k_batch_compact(BatchView bv, double* __restrict__ scratch, int min_features,
                                                                 int max_features, int remove, const int* __restrict__ hold_stats) {
-  __shared__ int keep[BNCAP], newpos[BNCAP], conv[BNCAP];
-  __shared__ int2 rmap[BNMAX];
+  constexpr int MV = (EKF_CAM + 6 * NC + BCMP_THREADS - 1) / BCMP_THREADS;   // state entries a thread moves: 1 at NC = 32
+  __shared__ int keep[NC], newpos[NC], conv[NC];
+  __shared__ int2 rmap[EKF_CAM + 6 * NC + 2];
   __shared__ int s_N2, s_n2;
   const int b = blockIdx.x, tid = threadIdx.x;
   DevCtl* ctl = bv.ctl + b;
@@ -725,17 +1176,24 @@ __global__ void __launch_bounds__(BCMP_THREADS) k_batch_compact(BatchView bv, do
     const int i = e / n2, j = e - i * n2;
     tmp[(size_t)i * ld + j] = xyz_apply_entry(Sigma, ld, rmap[i], rmap[j], Jall);
   }
-  double mv = 0.0;
-  if (tid < n2) {   // n2 <= 206 <= BCMP_THREADS
-    const int2 r = rmap[tid];
-    mv = (r.y < 0) ? mu[r.x] : yall[3 * (r.y >> 2) + (r.y & 3)];
+  double mv[MV];
+#pragma unroll
+  for (int q = 0; q < MV; ++q) {
+    const int i = tid + q * BCMP_THREADS;
+    mv[q] = 0.0;
+    if (i < n2) {
+      const int2 r = rmap[i];
+      mv[q] = (r.y < 0) ? mu[r.x] : yall[3 * (r.y >> 2) + (r.y & 3)];
+    }
   }
   __syncthreads();
   for (int e = tid; e < n2 * n2; e += BCMP_THREADS) {
     const int i = e / n2, j = e - i * n2;
     Sigma[(size_t)i * ld + j] = tmp[(size_t)i * ld + j];
   }
-  if (tid < n2) mu[tid] = mv;
+#pragma unroll
+  for (int q = 0; q < MV; ++q)
+    if (tid + q * BCMP_THREADS < n2) mu[tid + q * BCMP_THREADS] = mv[q];
   // feature table: thread f < N2 moves record keep[f] -> f through registers
   const int w16 = bv.tstride >> 4;
   int o = -1;
@@ -799,6 +1257,12 @@ __global__ void __launch_bounds__(BNCAP) k_batch_xyz_decide(BatchView bv, DevCfg
   const FeatTab ft = feattab_slice(bv.ft, b, bv.Ncap, bv.tstride);
   warp_xyz_decide(bv, b, bv.Sigma + (size_t)b * bv.sstride, bv.mu + (size_t)b * bv.ld, ft, bv.N[b], true, cfg);
 }
+// The same for a large batch (capacity up to BNCAP_L): one thread per feature, BNCAP_L threads.
+__global__ void __launch_bounds__(BNCAP_L) k_batch_xyz_decide_large(BatchView bv, DevCfg cfg) {
+  const int b = blockIdx.x;
+  const FeatTab ft = feattab_slice(bv.ft, b, bv.Ncap, bv.tstride);
+  cta_xyz_decide(bv, b, bv.Sigma + (size_t)b * bv.sstride, bv.mu + (size_t)b * bv.ld, ft, bv.N[b], false, -1, cfg);
+}
 
 // addFeature (V:309-371) for the corners of every filter that has some (cnt[b] of them at xy + 2 * EKF_BATCH_MAX_CORNERS * b),
 // one CTA per filter, one add after the other in corner order with a barrier between adds: add j reads the rows add j - 1
@@ -806,9 +1270,13 @@ __global__ void __launch_bounds__(BNCAP) k_batch_xyz_decide(BatchView bv, DevCfg
 // result is the single filter's bit for bit.  n <= 200 before an add, so one CTA covers every row.  one >= 0: filter `one`
 // adds the pixel (u, v) instead.  decide: the new features' convert2XYZ_ifLinear decisions join the ones k_batch_update
 // took for the filter's older features (adds change no entry their linearity test reads), for k_batch_compact to apply.
+// LARGE (capacity up to BNCAP_L): the corners sit at xy + 2 * BNCAP_L * b, the rows (n <= 776 before an add) are taken
+// BADD_THREADS at a time and the decisions one thread per feature.
 #define BADD_THREADS 256
+template <bool LARGE>
 __global__ void __launch_bounds__(BADD_THREADS) k_batch_add(BatchView bv, FrameView fr, DevCfg cfg, const float* __restrict__ xy,
                                                             const int* __restrict__ cnt, int one, float u, float v, int decide) {
+  constexpr int CS = LARGE ? BNCAP_L : EKF_BATCH_MAX_CORNERS;   // corner stride of xy
   __shared__ double A[6 * 7], Ap[6 * 3], fnew[6], Tc[6 * 7];
   const int b = one >= 0 ? one : blockIdx.x, tid = threadIdx.x;
   const int k = one >= 0 ? 1 : cnt[b];
@@ -820,11 +1288,15 @@ __global__ void __launch_bounds__(BADD_THREADS) k_batch_add(BatchView bv, FrameV
   int n = bv.n[b], N = bv.N[b], real = bv.patchnumbre[b];
   const int N0 = N;
   for (int j = 0; j < k; ++j) {
-    const float px = one >= 0 ? u : xy[(size_t)b * 2 * EKF_BATCH_MAX_CORNERS + 2 * j];
-    const float py = one >= 0 ? v : xy[(size_t)b * 2 * EKF_BATCH_MAX_CORNERS + 2 * j + 1];
+    const float px = one >= 0 ? u : xy[(size_t)b * 2 * CS + 2 * j];
+    const float py = one >= 0 ? v : xy[(size_t)b * 2 * CS + 2 * j + 1];
     if (tid == 0) add_feature_jacobians(cfg.cam, mu, px, py, cfg.rho_0, A, Ap, fnew);
     __syncthreads();
-    if (tid < n) add_feature_cross(Sigma, ld, n, tid, A);
+    if constexpr (LARGE) {
+      for (int r = tid; r < n; r += BADD_THREADS) add_feature_cross(Sigma, ld, n, r, A);
+    } else {
+      if (tid < n) add_feature_cross(Sigma, ld, n, tid, A);
+    }
     for (int e = tid; e < 42; e += BADD_THREADS) Tc[e] = add_feature_corner_T(Sigma, ld, A, e);   // rows / columns < 7: not written above
     __syncthreads();
     for (int e = tid; e < 36; e += BADD_THREADS)
@@ -836,6 +1308,22 @@ __global__ void __launch_bounds__(BADD_THREADS) k_batch_add(BatchView bv, FrameV
     n += 6; N += 1; real += 1;
   }
   if (tid == 0) { bv.n[b] = n; bv.N[b] = N; bv.patchnumbre[b] = real; }
+  if constexpr (LARGE) {
+    if (decide) {   // one thread per feature (N <= BNCAP_L <= BADD_THREADS)
+      const int i = tid;
+      const size_t kk = (size_t)b * bv.Ncap + i;
+      int conv = 0;
+      if (i >= N0 && i < N) {
+        const int pos = ft.pos[i];
+        conv = xyz_linear_decide(mu + pos, mu, Sigma[(size_t)(pos + 5) * ld + pos + 5], cfg.linearity_threshold, cfg.abs_int_quirk,
+                                 bv.xyz_y + 3 * kk, bv.xyz_J + 18 * kk);
+        bv.xyz_flag[kk] = conv;
+      }
+      const int c = __syncthreads_count(conv);
+      if (i == 0) bv.xyz_count[b] += c;
+    }
+    return;
+  }
   if (decide && tid < 32) {   // N <= BNCAP = 32
     const int i = tid;
     const size_t kk = (size_t)b * bv.Ncap + i;
@@ -906,7 +1394,7 @@ struct ekf_batch {
   int *h_n = nullptr, *h_N = nullptr;           // pinned mirrors of bv.n / bv.N
   double* stage_mu14 = nullptr;                 // device staging for set_camera_states
   BatchDetectBufs det;                          // batched corner detection (ekf_batch_detect.cu)
-  float* det_xy = nullptr;                      // [B][EKF_BATCH_MAX_CORNERS][2] corners of the last detection
+  float* det_xy = nullptr;                      // [B][cstride][2] corners of the last detection
   int *det_n = nullptr, *det_num = nullptr;     // [B] their count; [B] corners asked for (host num staged)
   float* h_det_xy = nullptr;                    // pinned
   int *h_det_n = nullptr, *h_num = nullptr;     // pinned
@@ -915,6 +1403,9 @@ struct ekf_batch {
   int* h_blur = nullptr;                        // pinned mirror of blur_out
   double dT = 1.0, old_ts = -1.0;
   bool have_frame = false, seeded = false, results_valid = false, topup = false, blur = false;
+  bool large = false;                           // ekf_batch_create_large with capacity > 32: the cluster update, BNCAP_L kernels
+  int cl_ctas = 1, cl_resident = 0;             // CTAs per filter in the update; clusters resident at once (large only)
+  int cstride = EKF_BATCH_MAX_CORNERS;          // corners per filter in det_xy (BNCAP_L when large)
   long long launches = 0;
   cudaEvent_t ev[4] = {nullptr, nullptr, nullptr, nullptr};
   std::string err;
@@ -975,10 +1466,21 @@ int ekf_batch_destroy(ekf_batch* b) {
   return EKF_OK;
 }
 
-int ekf_batch_create(const ekf_config* cfg, int n_filters, int feature_capacity, int device, ekf_batch** out) {
-  if (!cfg || !out || n_filters < 1 || feature_capacity < 1) return EKF_ERR_ARG;
-  *out = nullptr;
-  if (feature_capacity > BNCAP) return EKF_ERR_CAPACITY;
+// launch configuration of k_batch_update_cluster for B filters of C CTAs each
+static cudaLaunchConfig_t cluster_config(int B, int C, cudaStream_t st, cudaLaunchAttribute* attr) {
+  cudaLaunchConfig_t lc = {};
+  lc.gridDim = dim3((unsigned)(B * C), 1, 1);
+  lc.blockDim = dim3(BUPD_THREADS, 1, 1);
+  lc.dynamicSmemBytes = kUpdSmemBytes;
+  lc.stream = st;
+  attr[0].id = cudaLaunchAttributeClusterDimension;
+  attr[0].val.clusterDim.x = (unsigned)C; attr[0].val.clusterDim.y = 1; attr[0].val.clusterDim.z = 1;
+  lc.attrs = attr;
+  lc.numAttrs = 1;
+  return lc;
+}
+
+static int batch_create(const ekf_config* cfg, int n_filters, int feature_capacity, int device, bool large, ekf_batch** out) {
   if (cfg->kernel_size < 100000 || cfg->scale != 1 || cfg->forsePlane != 0) return EKF_ERR_UNSUPPORTED;
   if (cfg->window_size < 3 || cfg->window_size > 31 || cfg->search_clamp > 20 || cfg->search_clamp < 0) return EKF_ERR_UNSUPPORTED;
   int ndev = 0;
@@ -987,6 +1489,11 @@ int ekf_batch_create(const ekf_config* cfg, int n_filters, int feature_capacity,
   b->cfg = *cfg; b->device = device; b->B = n_filters; b->Ncap = feature_capacity;
   b->ncap = EKF_CAM + 6 * feature_capacity;
   b->ld = (b->ncap + 7) & ~7;
+  b->large = large;
+  if (large) {
+    b->cl_ctas = (b->ld + BSTRIP - 1) / BSTRIP;
+    b->cstride = BNCAP_L;
+  }
   const int w2 = (cfg->window_size * cfg->window_size + 15) & ~15;
   auto fail = [&](cudaError_t e, const char* what) {
     fprintf(stderr, "ekf_batch_create: %s: %s\n", what, cudaGetErrorString(e));
@@ -1000,7 +1507,23 @@ int ekf_batch_create(const ekf_config* cfg, int n_filters, int feature_capacity,
   b->stream = b->own_stream;
   TRY(cudaFuncSetAttribute(k_batch_update<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kUpdSmemBytes))
   TRY(cudaFuncSetAttribute(k_batch_update<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kUpdSmemBytes))
-  const size_t Bn = (size_t)n_filters, cap = Bn * feature_capacity;
+  if (large) {
+    TRY(cudaFuncSetAttribute(k_batch_update_cluster<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kUpdSmemBytes))
+    TRY(cudaFuncSetAttribute(k_batch_update_cluster<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kUpdSmemBytes))
+    cudaLaunchAttribute attr[1];
+    for (int plane = 0; plane < 2; ++plane) {
+      const cudaLaunchConfig_t lc = cluster_config(1, b->cl_ctas, nullptr, attr);
+      int ncl = 0;
+      TRY(cudaOccupancyMaxActiveClusters(&ncl, plane ? (void*)k_batch_update_cluster<true> : (void*)k_batch_update_cluster<false>, &lc))
+      if (ncl < 1) {
+        fprintf(stderr, "ekf_batch_create_large: the device cannot hold one cluster of %d CTAs with %zu bytes of shared memory each\n",
+                b->cl_ctas, kUpdSmemBytes);
+        ekf_batch_destroy(b);
+        return EKF_ERR_UNSUPPORTED;
+      }
+      b->cl_resident = plane ? std::min(b->cl_resident, ncl) : ncl;
+    }
+  }  const size_t Bn = (size_t)n_filters, cap = Bn * feature_capacity;
   BatchView& v = b->bv;
   v.ld = b->ld; v.Ncap = feature_capacity; v.tstride = w2;
   v.sstride = (long long)b->ncap * b->ld;
@@ -1016,7 +1539,7 @@ int ekf_batch_create(const ekf_config* cfg, int n_filters, int feature_capacity,
   TRY(balloc(&v.xyz_flag, cap)) TRY(balloc(&v.xyz_J, 18 * cap)) TRY(balloc(&v.xyz_y, 3 * cap)) TRY(balloc(&v.xyz_count, Bn))
   TRY(balloc(&b->out_mu14, Bn * 14)) TRY(balloc(&b->out_S14, Bn * 196)) TRY(balloc(&b->out_stats, Bn * EKF_BATCH_STAT_FIELDS))
   TRY(balloc(&b->stage_mu14, Bn * 14)) TRY(balloc(&v.patchnumbre, Bn))
-  TRY(balloc(&b->det_xy, Bn * 2 * EKF_BATCH_MAX_CORNERS)) TRY(balloc(&b->det_n, Bn)) TRY(balloc(&b->det_num, Bn))
+  TRY(balloc(&b->det_xy, Bn * 2 * b->cstride)) TRY(balloc(&b->det_n, Bn)) TRY(balloc(&b->det_num, Bn))
   TRY(cudaMallocHost((void**)&b->h_det_xy, sizeof(float) * Bn * 2 * EKF_BATCH_MAX_CORNERS))
   TRY(cudaMallocHost((void**)&b->h_det_n, sizeof(int) * Bn)) TRY(cudaMallocHost((void**)&b->h_num, sizeof(int) * Bn))
   TRY(cudaMallocHost((void**)&b->h_added, sizeof(int) * Bn))
@@ -1052,6 +1575,27 @@ int ekf_batch_create(const ekf_config* cfg, int n_filters, int feature_capacity,
   d.forsePlane = cfg->forsePlane; d.abs_int_quirk = cfg->abs_int_quirk;
   d.tstride = w2;
   *out = b;
+  return EKF_OK;
+}
+
+int ekf_batch_create(const ekf_config* cfg, int n_filters, int feature_capacity, int device, ekf_batch** out) {
+  if (!cfg || !out || n_filters < 1 || feature_capacity < 1) return EKF_ERR_ARG;
+  *out = nullptr;
+  if (feature_capacity > BNCAP) return EKF_ERR_CAPACITY;
+  return batch_create(cfg, n_filters, feature_capacity, device, false, out);
+}
+
+int ekf_batch_create_large(const ekf_config* cfg, int n_filters, int feature_capacity, int device, ekf_batch** out) {
+  if (!cfg || !out || n_filters < 1 || feature_capacity < 1) return EKF_ERR_ARG;
+  *out = nullptr;
+  if (feature_capacity > BNCAP_L) return EKF_ERR_CAPACITY;
+  return batch_create(cfg, n_filters, feature_capacity, device, feature_capacity > BNCAP, out);
+}
+
+int ekf_batch_update_clusters(const ekf_batch* b, int32_t* ctas_per_filter, int32_t* resident) {
+  if (!b) return EKF_ERR_ARG;
+  if (ctas_per_filter) *ctas_per_filter = b->cl_ctas;
+  if (resident) *resident = b->cl_resident;
   return EKF_OK;
 }
 
@@ -1182,14 +1726,26 @@ int ekf_batch_set_force_plane(ekf_batch* b, int on) {
   return EKF_OK;
 }
 
+// k_batch_compact at the batch's capacity
+static void launch_compact(ekf_batch* b, int remove, const int* hold_stats) {
+  if (b->large)
+    k_batch_compact<BNCAP_L><<<b->B, BCMP_THREADS, 0, b->stream>>>(b->bv, b->scratch, b->cfg.min_features, b->cfg.max_features, remove,
+                                                                   hold_stats);
+  else
+    k_batch_compact<BNCAP><<<b->B, BCMP_THREADS, 0, b->stream>>>(b->bv, b->scratch, b->cfg.min_features, b->cfg.max_features, remove,
+                                                                 hold_stats);
+  b->launches += 1;
+}
+
 // detection + adds for every filter, filter b asking for num[b * num_stride] corners (<= 0: none); decide: also take the new
 // features' XYZ decisions (in-step top-up).  Enqueued only.
 static int batch_topup(ekf_batch* b, const int* num, int num_stride, int decide) {
   cudaStream_t st = b->stream;
-  BCHECK(batch_detect_reserve(b->det, (size_t)b->fv.w * b->fv.h, b->B));
+  BCHECK(batch_detect_reserve(b->det, (size_t)b->fv.w * b->fv.h, b->B, b->cstride));
   BCHECK(launch_batch_detect(st, b->det, b->fv, b->bv.ft.center, b->bv.N, b->Ncap, b->B, b->cfg.window_size, num, num_stride, 1,
-                             b->det_xy, b->det_n, &b->launches));
-  k_batch_add<<<b->B, BADD_THREADS, 0, st>>>(b->bv, b->fv, b->dcfg, b->det_xy, b->det_n, -1, 0.0f, 0.0f, decide);
+                             b->cstride, b->det_xy, b->det_n, &b->launches));
+  if (b->large) k_batch_add<true><<<b->B, BADD_THREADS, 0, st>>>(b->bv, b->fv, b->dcfg, b->det_xy, b->det_n, -1, 0.0f, 0.0f, decide);
+  else k_batch_add<false><<<b->B, BADD_THREADS, 0, st>>>(b->bv, b->fv, b->dcfg, b->det_xy, b->det_n, -1, 0.0f, 0.0f, decide);
   b->launches += 1;
   BCHECK(cudaGetLastError());
   return EKF_OK;
@@ -1226,17 +1782,26 @@ int ekf_batch_step(ekf_batch* b, const double dv[3], const double dw[3], int vco
                                                    make_double3(w[0], w[1], w[2]), vcontrol);
   b->launches += 1;
   if (b->blur) {   // matching_patch <- blurred patch where the prediction moves far enough (k_batch_predict copied patch)
-    k_batch_predict_blur<<<b->B, BBLUR_WARPS * 32, 0, st>>>(b->bv, b->dcfg, b->dT, b->blur_out);
+    if (b->large) k_batch_predict_blur<BNCAP_L><<<b->B, BBLUR_WARPS * 32, 0, st>>>(b->bv, b->dcfg, b->dT, b->blur_out);
+    else k_batch_predict_blur<BNCAP><<<b->B, BBLUR_WARPS * 32, 0, st>>>(b->bv, b->dcfg, b->dT, b->blur_out);
     b->launches += 1;
   }
   BCHECK(cudaEventRecord(b->ev[1], st));
   launch_match_filter_batch(st, b->bv.ft, b->Ncap, b->bv.N, b->B, b->fv, b->dcfg, &b->frame_map, b->match_defer,
                             b->match_defer + (size_t)b->B * b->Ncap, &b->launches);
   BCHECK(cudaEventRecord(b->ev[2], st));
-  auto* const update = b->cfg.forsePlane ? k_batch_update<true> : k_batch_update<false>;
-  update<<<b->B, BUPD_THREADS, kUpdSmemBytes, st>>>(b->bv, b->dcfg, b->picks_dev, n_picks, b->out_mu14, b->out_S14,
-                                                    b->out_stats, b->cfg.min_features, b->cfg.max_features,
-                                                    b->cfg.xyz_conversion);
+  if (b->large) {   // one cluster of cl_ctas CTAs per filter
+    cudaLaunchAttribute attr[1];
+    const cudaLaunchConfig_t lc = cluster_config(b->B, b->cl_ctas, st, attr);
+    auto* const update = b->cfg.forsePlane ? k_batch_update_cluster<true> : k_batch_update_cluster<false>;
+    BCHECK(cudaLaunchKernelEx(&lc, update, b->bv, b->dcfg, (const uint32_t*)b->picks_dev, n_picks, b->out_mu14, b->out_S14,
+                              b->out_stats, (int)b->cfg.min_features, (int)b->cfg.max_features, (int)b->cfg.xyz_conversion));
+  } else {
+    auto* const update = b->cfg.forsePlane ? k_batch_update<true> : k_batch_update<false>;
+    update<<<b->B, BUPD_THREADS, kUpdSmemBytes, st>>>(b->bv, b->dcfg, b->picks_dev, n_picks, b->out_mu14, b->out_S14,
+                                                      b->out_stats, b->cfg.min_features, b->cfg.max_features,
+                                                      b->cfg.xyz_conversion);
+  }
   b->launches += 1;
   BCHECK(cudaEventRecord(b->ev[3], st));
   BCHECK(cudaGetLastError());
@@ -1257,8 +1822,7 @@ int ekf_batch_step(ekf_batch* b, const double dv[3], const double dw[3], int vco
   std::fill(b->h_added, b->h_added + Bn, 0);
   if (!b->topup || topups == 0) {
     if (removed > 0 || converted > 0) {   // removals, then convert2XYZ_ifLinearAll (V:1312-1317), in one pass
-      k_batch_compact<<<b->B, BCMP_THREADS, 0, st>>>(b->bv, b->scratch, b->cfg.min_features, b->cfg.max_features, 1, nullptr);
-      b->launches += 1;
+      launch_compact(b, 1, nullptr);
       BCHECK(cudaGetLastError());
       BCHECK(cudaMemcpyAsync(b->h_n, b->bv.n, sizeof(int) * Bn, cudaMemcpyDeviceToHost, st));
       BCHECK(cudaMemcpyAsync(b->h_N, b->bv.N, sizeof(int) * Bn, cudaMemcpyDeviceToHost, st));
@@ -1270,14 +1834,12 @@ int ekf_batch_step(ekf_batch* b, const double dv[3], const double dw[3], int vco
     // and converting first would give A (J Sigma[cam, f]), equal only up to rounding.  So its compaction removes only;
     // every other filter keeps the fused pass.
     if (removed > 0 || converted > 0) {
-      k_batch_compact<<<b->B, BCMP_THREADS, 0, st>>>(b->bv, b->scratch, b->cfg.min_features, b->cfg.max_features, 1, b->out_stats);
-      b->launches += 1;
+      launch_compact(b, 1, b->out_stats);
     }
     int rc = batch_topup(b, b->out_stats + EKF_BSTAT_TOPUP, EKF_BATCH_STAT_FIELDS, b->cfg.xyz_conversion);
     if (rc) return rc;
     if (b->cfg.xyz_conversion) {   // the held conversions and the new features' (filters with none return at once)
-      k_batch_compact<<<b->B, BCMP_THREADS, 0, st>>>(b->bv, b->scratch, b->cfg.min_features, b->cfg.max_features, 0, nullptr);
-      b->launches += 1;
+      launch_compact(b, 0, nullptr);
     }
     BCHECK(cudaGetLastError());
     rc = batch_readback(b, true);
@@ -1296,7 +1858,8 @@ int ekf_batch_convert2xyz_if_linear_all(ekf_batch* b) {
   BCHECK(cudaSetDevice(b->device));
   cudaStream_t st = b->stream;
   const size_t Bn = (size_t)b->B;
-  k_batch_xyz_decide<<<b->B, BNCAP, 0, st>>>(b->bv, b->dcfg);
+  if (b->large) k_batch_xyz_decide_large<<<b->B, BNCAP_L, 0, st>>>(b->bv, b->dcfg);
+  else k_batch_xyz_decide<<<b->B, BNCAP, 0, st>>>(b->bv, b->dcfg);
   b->launches += 1;
   BCHECK(cudaGetLastError());
   BCHECK(cudaMemcpyAsync(b->h_xyz_count, b->bv.xyz_count, sizeof(int) * Bn, cudaMemcpyDeviceToHost, st));
@@ -1304,8 +1867,7 @@ int ekf_batch_convert2xyz_if_linear_all(ekf_batch* b) {
   long long converted = 0;
   for (size_t i = 0; i < Bn; ++i) converted += b->h_xyz_count[i];
   if (converted == 0) return EKF_OK;
-  k_batch_compact<<<b->B, BCMP_THREADS, 0, st>>>(b->bv, b->scratch, b->cfg.min_features, b->cfg.max_features, 0, nullptr);
-  b->launches += 1;
+  launch_compact(b, 0, nullptr);
   BCHECK(cudaGetLastError());
   BCHECK(cudaMemcpyAsync(b->h_n, b->bv.n, sizeof(int) * Bn, cudaMemcpyDeviceToHost, st));
   BCHECK(cudaMemcpyAsync(b->h_N, b->bv.N, sizeof(int) * Bn, cudaMemcpyDeviceToHost, st));
@@ -1396,7 +1958,8 @@ int ekf_batch_add_feature(ekf_batch* b, int f, float u, float v) {
   const double x = (double)u, y = (double)v;
   if (!(x > half && y > half && x < b->fv.w - half && y < b->fv.h - half)) return 0;
   if (b->h_N[f] >= b->Ncap || b->h_n[f] + 6 > b->ncap) return bfail(b, EKF_ERR_CAPACITY, "feature capacity exceeded");
-  k_batch_add<<<1, BADD_THREADS, 0, b->stream>>>(b->bv, b->fv, b->dcfg, nullptr, nullptr, f, u, v, 0);
+  if (b->large) k_batch_add<true><<<1, BADD_THREADS, 0, b->stream>>>(b->bv, b->fv, b->dcfg, nullptr, nullptr, f, u, v, 0);
+  else k_batch_add<false><<<1, BADD_THREADS, 0, b->stream>>>(b->bv, b->fv, b->dcfg, nullptr, nullptr, f, u, v, 0);
   b->launches += 1;
   BCHECK(cudaGetLastError());
   b->h_N[f] += 1;
@@ -1419,10 +1982,14 @@ int ekf_batch_detect_corners(ekf_batch* b, const int32_t* num, float* out_xy, in
   const size_t Bn = (size_t)b->B;
   int rc = batch_stage_num(b, num);
   if (rc) return rc;
-  BCHECK(batch_detect_reserve(b->det, (size_t)b->fv.w * b->fv.h, b->B));
+  BCHECK(batch_detect_reserve(b->det, (size_t)b->fv.w * b->fv.h, b->B, b->cstride));
   BCHECK(launch_batch_detect(st, b->det, b->fv, b->bv.ft.center, b->bv.N, b->Ncap, b->B, b->cfg.window_size, b->det_num, 1, 0,
-                             b->det_xy, b->det_n, &b->launches));
-  BCHECK(cudaMemcpyAsync(b->h_det_xy, b->det_xy, sizeof(float) * Bn * 2 * EKF_BATCH_MAX_CORNERS, cudaMemcpyDeviceToHost, st));
+                             b->cstride, b->det_xy, b->det_n, &b->launches));
+  if (b->cstride == EKF_BATCH_MAX_CORNERS)
+    BCHECK(cudaMemcpyAsync(b->h_det_xy, b->det_xy, sizeof(float) * Bn * 2 * EKF_BATCH_MAX_CORNERS, cudaMemcpyDeviceToHost, st));
+  else   // the public layout: EKF_BATCH_MAX_CORNERS corners a filter (cap_mode 0 detects no more)
+    BCHECK(cudaMemcpy2DAsync(b->h_det_xy, sizeof(float) * 2 * EKF_BATCH_MAX_CORNERS, b->det_xy, sizeof(float) * 2 * b->cstride,
+                             sizeof(float) * 2 * EKF_BATCH_MAX_CORNERS, Bn, cudaMemcpyDeviceToHost, st));
   BCHECK(cudaMemcpyAsync(b->h_det_n, b->det_n, sizeof(int) * Bn, cudaMemcpyDeviceToHost, st));
   BCHECK(cudaStreamSynchronize(st));
   std::copy(b->h_det_xy, b->h_det_xy + Bn * 2 * EKF_BATCH_MAX_CORNERS, out_xy);

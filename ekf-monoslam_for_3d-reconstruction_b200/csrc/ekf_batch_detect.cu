@@ -14,7 +14,7 @@
 //
 // The masked maximum must be exact: the frame's pixel keys (base mask, eig > 0) are sorted once, and one warp per filter
 // walks down that order until the first pixel outside the filter's boxes.  The walk is long only as far as the top pixels
-// sit inside the filter's own boxes (at most 32 (2 w + 1)^2 pixels).
+// sit inside the filter's own boxes (at most N (2 w + 1)^2 pixels, N <= 32, or <= 128 in a large batch).
 //
 // Early stop: every pixel inside the mask is at least window_size from the border, more than the window_size / 2 of
 // isInsideImage, so addFeature accepts every detected corner and the single filter's loop over them (V:832-835) stops only
@@ -46,25 +46,30 @@ __global__ void k_bdet_keys(const float* __restrict__ eig, int W, int H, int est
   kc[i] = c;
 }
 
-// One warp per filter: its boxes, its corner limit and thr_b from the first sorted pixel outside its boxes.
+// One warp per filter: its boxes, its corner limit and thr_b from the first sorted pixel outside its boxes.  CS: boxes and
+// corners a filter has room for (EKF_BATCH_MAX_CORNERS, or EKF_BATCH_MAX_FEATURES in a large batch).
 #define BDET_WARPS 8
+template <int CS>
 __global__ void __launch_bounds__(32 * BDET_WARPS) k_bdet_threshold(const unsigned long long* __restrict__ kp, int npx, int W, int H,
                                                                      int window, const float* __restrict__ centers,
                                                                      const int* __restrict__ N, int Ncap, int B,
                                                                      const int* __restrict__ num, int num_stride, int cap_mode,
                                                                      DetBox* __restrict__ boxes, unsigned* __restrict__ thr_bits,
                                                                      int* __restrict__ limit) {
-  __shared__ DetBox sb[BDET_WARPS][EKF_BATCH_MAX_CORNERS];
+  __shared__ DetBox sb[BDET_WARPS][CS];
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int b = blockIdx.x * BDET_WARPS + warp;
   if (b >= B) return;   // the whole warp
   const int nb = N[b];
   int lim = min(num[(size_t)b * num_stride], cap_mode ? Ncap - nb : EKF_BATCH_MAX_CORNERS);
-  lim = max(0, min(lim, EKF_BATCH_MAX_CORNERS));
-  DetBox bx{0, 0, 0, 0};
-  if (lane < nb) bx = det_patch_box(centers[2 * ((size_t)b * Ncap + lane)], centers[2 * ((size_t)b * Ncap + lane) + 1], W, H, window);
-  sb[warp][lane] = bx;
-  boxes[(size_t)b * EKF_BATCH_MAX_CORNERS + lane] = bx;
+  lim = max(0, min(lim, CS));
+#pragma unroll
+  for (int i = lane; i < CS; i += 32) {
+    DetBox bx{0, 0, 0, 0};
+    if (i < nb) bx = det_patch_box(centers[2 * ((size_t)b * Ncap + i)], centers[2 * ((size_t)b * Ncap + i) + 1], W, H, window);
+    sb[warp][i] = bx;
+    boxes[(size_t)b * CS + i] = bx;
+  }
   __syncwarp();
   if (lane == 0) limit[b] = lim;
   if (lim == 0) return;
@@ -87,21 +92,22 @@ __global__ void __launch_bounds__(32 * BDET_WARPS) k_bdet_threshold(const unsign
 }
 
 // One thread per filter: goodFeaturesToTrack's greedy selection over the shared candidate list.
+template <int CS>
 __global__ void k_bdet_select(const unsigned long long* __restrict__ kc, int nkeys, int W, const DetBox* __restrict__ boxes,
                               const int* __restrict__ N, const unsigned* __restrict__ thr_bits, const int* __restrict__ limit, int B,
                               float* __restrict__ out_xy, int* __restrict__ out_n) {
   const int b = blockIdx.x * blockDim.x + threadIdx.x;
   if (b >= B) return;
   const int lim = limit[b];
-  out_n[b] = lim > 0 ? det_select_walk(kc, nkeys, W, thr_bits[b], boxes + (size_t)b * EKF_BATCH_MAX_CORNERS, N[b], 144.0f, lim,
-                                       out_xy + (size_t)b * 2 * EKF_BATCH_MAX_CORNERS)
+  out_n[b] = lim > 0 ? det_select_walk(kc, nkeys, W, thr_bits[b], boxes + (size_t)b * CS, N[b], 144.0f, lim,
+                                       out_xy + (size_t)b * 2 * CS)
                      : 0;
 }
 
-cudaError_t batch_detect_reserve(BatchDetectBufs& d, size_t px, int B) {
+cudaError_t batch_detect_reserve(BatchDetectBufs& d, size_t px, int B, int cstride) {
   cudaError_t e;
   if (!d.boxes) {
-    if ((e = cudaMalloc((void**)&d.boxes, sizeof(DetBox) * EKF_BATCH_MAX_CORNERS * (size_t)B)) != cudaSuccess) return e;
+    if ((e = cudaMalloc((void**)&d.boxes, sizeof(DetBox) * cstride * (size_t)B)) != cudaSuccess) return e;
     if ((e = cudaMalloc((void**)&d.thr_bits, sizeof(unsigned) * (size_t)B)) != cudaSuccess) return e;
     if ((e = cudaMalloc((void**)&d.limit, sizeof(int) * (size_t)B)) != cudaSuccess) return e;
   }
@@ -126,7 +132,8 @@ void batch_detect_free(BatchDetectBufs& d) {
 }
 
 cudaError_t launch_batch_detect(cudaStream_t st, BatchDetectBufs& d, FrameView fr, const float* centers, const int* N, int Ncap, int B,
-                                int window, const int* num, int num_stride, int cap_mode, float* out_xy, int* out_n, long long* launches) {
+                                int window, const int* num, int num_stride, int cap_mode, int cstride, float* out_xy, int* out_n,
+                                long long* launches) {
   const int W = fr.w, H = fr.h, npx = W * H;
   unsigned long long *kp = d.keys, *kc = d.keys + d.cap, *kp_s = d.keys + 2 * d.cap, *kc_s = d.keys + 3 * d.cap;
   launch_det_eig(st, fr, d.eig, launches);
@@ -137,9 +144,16 @@ cudaError_t launch_batch_detect(cudaStream_t st, BatchDetectBufs& d, FrameView f
   tmp = d.tmp_bytes;
   e = cub::DeviceRadixSort::SortKeysDescending(d.tmp, tmp, kc, kc_s, npx, 0, 64, st);
   if (e != cudaSuccess) return e;
-  k_bdet_threshold<<<(B + BDET_WARPS - 1) / BDET_WARPS, 32 * BDET_WARPS, 0, st>>>(kp_s, npx, W, H, window, centers, N, Ncap, B, num,
-                                                                                  num_stride, cap_mode, d.boxes, d.thr_bits, d.limit);
-  k_bdet_select<<<(B + 127) / 128, 128, 0, st>>>(kc_s, npx, W, d.boxes, N, d.thr_bits, d.limit, B, out_xy, out_n);
+  const unsigned gt = (B + BDET_WARPS - 1) / BDET_WARPS, gs = (B + 127) / 128;
+  if (cstride == EKF_BATCH_MAX_CORNERS) {
+    k_bdet_threshold<EKF_BATCH_MAX_CORNERS><<<gt, 32 * BDET_WARPS, 0, st>>>(kp_s, npx, W, H, window, centers, N, Ncap, B, num,
+                                                                           num_stride, cap_mode, d.boxes, d.thr_bits, d.limit);
+    k_bdet_select<EKF_BATCH_MAX_CORNERS><<<gs, 128, 0, st>>>(kc_s, npx, W, d.boxes, N, d.thr_bits, d.limit, B, out_xy, out_n);
+  } else {
+    k_bdet_threshold<EKF_BATCH_MAX_FEATURES><<<gt, 32 * BDET_WARPS, 0, st>>>(kp_s, npx, W, H, window, centers, N, Ncap, B, num,
+                                                                            num_stride, cap_mode, d.boxes, d.thr_bits, d.limit);
+    k_bdet_select<EKF_BATCH_MAX_FEATURES><<<gs, 128, 0, st>>>(kc_s, npx, W, d.boxes, N, d.thr_bits, d.limit, B, out_xy, out_n);
+  }
   *launches += 5;   // keys, the two sorts (counted once each), threshold, select; the eig map counts itself
   return cudaGetLastError();
 }

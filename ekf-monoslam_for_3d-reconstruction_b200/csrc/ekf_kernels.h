@@ -128,13 +128,15 @@ struct BatchDetectBufs {
   unsigned long long* keys = nullptr;   // [4][cap] pixel keys, candidate keys, both sorted
   void* tmp = nullptr;                  // CUB radix-sort workspace
   size_t tmp_bytes = 0, cap = 0;        // cap: pixels the buffers hold
-  DetBox* boxes = nullptr;              // [B][EKF_BATCH_MAX_CORNERS] mask boxes per filter
+  DetBox* boxes = nullptr;              // [B][cstride] mask boxes per filter
   unsigned* thr_bits = nullptr;         // [B] per-filter threshold (float bits)
   int* limit = nullptr;                 // [B] corners each filter may take
 };
-cudaError_t batch_detect_reserve(BatchDetectBufs& d, size_t px, int B);
+cudaError_t batch_detect_reserve(BatchDetectBufs& d, size_t px, int B, int cstride);
 void batch_detect_free(BatchDetectBufs& d);
-// num[b * num_stride] corners for filter b, capped at EKF_BATCH_MAX_CORNERS (cap_mode 0) or at Ncap - N[b] (cap_mode 1);
-// out_xy [B][EKF_BATCH_MAX_CORNERS][2], out_n [B]
+// num[b * num_stride] corners for filter b, capped at EKF_BATCH_MAX_CORNERS (cap_mode 0) or at Ncap - N[b] (cap_mode 1), and at
+// cstride, the boxes and corners a filter has room for: EKF_BATCH_MAX_CORNERS, or EKF_BATCH_MAX_FEATURES for a large batch;
+// out_xy [B][cstride][2], out_n [B]
 cudaError_t launch_batch_detect(cudaStream_t st, BatchDetectBufs& d, FrameView fr, const float* centers, const int* N, int Ncap, int B,
-                                int window, const int* num, int num_stride, int cap_mode, float* out_xy, int* out_n, long long* launches);
+                                int window, const int* num, int num_stride, int cap_mode, int cstride, float* out_xy, int* out_n,
+                                long long* launches);

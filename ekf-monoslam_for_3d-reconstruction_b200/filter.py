@@ -284,24 +284,27 @@ class FilterBatch:
     Seed it from a single VSlamFilter, optionally perturb the camera states, then call
     captureNewFrame / step once per frame."""
 
-    def __init__(self, cfg, n_filters, feature_capacity=32, device=0):
+    def __init__(self, cfg, n_filters, feature_capacity=32, device=0, large=False):
+        """large: up to 128 features per filter (ekf_batch_create_large; the update of a filter above 32 features runs on a
+        cluster of CTAs).  Without it the capacity is at most 32."""
         self.L = lib()
         self.cfg = cfg
         h = C.c_void_p()
-        rc = self.L.ekf_batch_create(C.byref(cfg), int(n_filters), int(feature_capacity), int(device), C.byref(h))
+        create = self.L.ekf_batch_create_large if large else self.L.ekf_batch_create
+        rc = create(C.byref(cfg), int(n_filters), int(feature_capacity), int(device), C.byref(h))
         if rc != 0:
-            raise EkfError(f"ekf_batch_create failed with {rc}")
+            raise EkfError(f"{'ekf_batch_create_large' if large else 'ekf_batch_create'} failed with {rc}")
         self.h = h
         self.B = int(n_filters)
 
     @classmethod
-    def from_config(cls, cfg, n_filters, feature_capacity=32, device=0):
+    def from_config(cls, cfg, n_filters, feature_capacity=32, device=0, large=False):
         """A batch from the configuration a VSlamFilter takes: created with motion blur, resize and forsePlane off (which
         ekf_batch_create requires), then set_motion_blur(cfg.kernel_size) when blur is on, set_scale(cfg.scale) and
         set_force_plane(cfg.forsePlane)."""
         base = _abi.EkfConfig.from_buffer_copy(cfg)
         base.kernel_size, base.scale, base.forsePlane = _abi.default_config().kernel_size, 1, 0
-        batch = cls(base, n_filters, feature_capacity=feature_capacity, device=device)
+        batch = cls(base, n_filters, feature_capacity=feature_capacity, device=device, large=large)
         batch.cfg = cfg
         if cfg.kernel_size < 100000:
             batch.set_motion_blur(cfg.kernel_size)
@@ -464,6 +467,12 @@ class FilterBatch:
 
     def kernel_launches(self):
         return int(self.L.ekf_batch_kernel_launches(self.h))
+
+    def update_clusters(self):
+        """(CTAs per filter in the update, clusters the device holds at once; 0 for a one-CTA update)."""
+        c, r = C.c_int(0), C.c_int(0)
+        self._ck(self.L.ekf_batch_update_clusters(self.h, C.byref(c), C.byref(r)))
+        return c.value, r.value
 
     def last_match_deferred(self):
         """(filter, feature) pairs of the last step that the warp-per-feature matcher left to the CTA matcher."""

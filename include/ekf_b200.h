@@ -227,7 +227,8 @@ int ekf_match_batch(const uint8_t* frames, int n_frames, int width, int height, 
  * min_features features, then, when cfg.xyz_conversion is set, convert2XYZ_ifLinearAll (:1317) on every
  * filter.  Top-up is off by default: the step then only reports in EKF_BSTAT_TOPUP how many features
  * each filter asks for, and ekf_batch_find_new_features serves those requests when the caller wants.
- * feature_capacity <= 32 (the stacked update of one filter is kept in shared memory).  ekf_batch_create
+ * ekf_batch_create takes feature_capacity <= 32 (the stacked update of one filter is kept in one CTA's shared memory);
+ * ekf_batch_create_large takes up to 128 (the update of one filter on a cluster of CTAs).  ekf_batch_create
  * refuses motion blur (kernel_size < 100000), scale != 1 and forsePlane (EKF_ERR_UNSUPPORTED); each of them is
  * switched on after creation instead, with ekf_batch_set_motion_blur, ekf_batch_set_scale and
  * ekf_batch_set_force_plane, so that a batch honours every ConfigVSLAM switch a single filter honours. */
@@ -243,6 +244,17 @@ enum { EKF_BSTAT_INNOV = 0, EKF_BSTAT_MATCHED = 1, EKF_BSTAT_LI = 2, EKF_BSTAT_H
        EKF_BSTAT_CHOL_FAIL = 5, EKF_BSTAT_REMOVED = 6, EKF_BSTAT_TOPUP = 7 };
 
 int ekf_batch_create(const ekf_config* cfg, int n_filters, int feature_capacity, int device, ekf_batch** out);
+/* A batch of up to EKF_BATCH_MAX_FEATURES features per filter (1 <= feature_capacity <= 128; EKF_ERR_CAPACITY above).
+ * With feature_capacity <= 32 it is exactly what ekf_batch_create builds.  Above 32, each filter's update runs on a
+ * thread-block cluster of ceil(ld / 208) CTAs (2 to 4) that share the stacked update through distributed shared memory;
+ * EKF_ERR_UNSUPPORTED when the device cannot hold one such cluster.  Every other ekf_batch_* entry works on it unchanged.
+ * Memory: Sigma and the compaction scratch are n_filters x state_capacity x ld doubles each, 4.9 MB per filter each at
+ * capacity 128 (40 GB in total for 4096 filters). */
+#define EKF_BATCH_MAX_FEATURES 128
+int ekf_batch_create_large(const ekf_config* cfg, int n_filters, int feature_capacity, int device, ekf_batch** out);
+/* CTAs per filter in the batch's update (1 for capacity <= 32) and, for a cluster update, how many clusters the device holds
+ * at once (0 otherwise); either pointer may be NULL. */
+int ekf_batch_update_clusters(const ekf_batch* b, int32_t* ctas_per_filter, int32_t* resident);
 int ekf_batch_destroy(ekf_batch* b);
 int ekf_batch_describe(const ekf_batch* b, ekf_batch_desc* out);
 int ekf_batch_set_stream(ekf_batch* b, void* cuda_stream);
