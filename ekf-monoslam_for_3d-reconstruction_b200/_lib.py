@@ -89,6 +89,11 @@ SIGNATURES = {
     "ekf_batch_last_added": (_i, [_vp, _vp]),
     "ekf_batch_set_motion_blur": (_i, [_vp, _i]),
     "ekf_batch_last_blur_counts": (_i, [_vp, _vp]),
+    "ekf_batch_set_archive": (_i, [_vp, _i]),
+    "ekf_batch_remove_feature": (_i, [_vp, _i, _i]),
+    "ekf_batch_num_deleted": (_i, [_vp, _vp]),
+    "ekf_batch_get_deleted": (_i, [_vp, _i, _vp, _i, _P(_i)]),
+    "ekf_batch_get_points_features": (_i, [_vp, _i, _i, _vp, _i, _vp]),
     "ekf_batch_get_template": (_i, [_vp, _i, _i, _i, _vp]),
     "ekf_batch_kernel_launches": (C.c_int64, [_vp]),
     "ekf_batch_last_step_ms": (_i, [_vp, _vp]),

@@ -36,6 +36,7 @@
 #include "ekf_handle.h"
 #include "ekf_kernels.h"
 #include "ekf_math.cuh"
+#include "ekf_points.cuh"
 
 namespace cg = cooperative_groups;
 
@@ -1123,20 +1124,39 @@ __global__ void __launch_bounds__(BUPD_THREADS, 1) k_batch_update_cluster(BatchV
 // removals followed by its one-at-a-time conversions.  A filter with nothing to do returns at once.
 // ------------------------------------------------------------------------------------------------
 #define BCMP_THREADS 256
+// The feature archive of a batch (VSlamFilter::deleted_patches, ekf_batch_set_archive): cap records per filter, each a
+// real_index and PTS_COLS doubles (ekf_points.cuh).  cap = 0: off, and nothing is archived.
+struct BatchArchive {
+  double* rec;       // [B][cap][PTS_COLS]
+  int* real_index;   // [B][cap]
+  int* count;        // [B] records held
+  int* overflow;     // [B] records dropped for want of room, ever (ekf_batch_step compares it with its last read-back)
+  int cap;
+};
+
 // hold (stats of the step, or NULL): a filter whose EKF_BSTAT_TOPUP is set only removes here, and its pending decisions move
 // with the surviving records; the conversions follow its new features (ekf_batch_step).  NC: feature capacity (BNCAP or
 // BNCAP_L); one CTA covers every entry of n2 x n2 either way, and every record (N2 <= 128 <= BCMP_THREADS).
+// one >= 0 (grid of one CTA): removeFeature(one_idx) on filter `one` alone (ekf_batch_remove_feature): no other removal, no
+// max_features rule, no conversion; pending decisions move with the records as under hold.
+// With the archive on, every removed feature that removeFeature archives (XYZ, n_find > 5) is appended to the filter's archive
+// in the single filter's order: the flagged features in ascending index (ekf_update_after_match's victims), then the
+// removeFeature(0) victim.  The records are read from Sigma and mu before the pass overwrites them.  A conversion fused into
+// the same pass never touches a removed feature's block: the reference removes before it converts, the decisions exclude the
+// removed features, and J is the identity on every row but the converted feature's.
 template <int NC>
-__global__ void __launch_bounds__(BCMP_THREADS) k_batch_compact(BatchView bv, double* __restrict__ scratch, int min_features,
-                                                                int max_features, int remove, const int* __restrict__ hold_stats) {
+__global__ void __launch_bounds__(BCMP_THREADS, 1) k_batch_compact(BatchView bv, double* __restrict__ scratch, int min_features,
+                                                                int max_features, int remove, const int* __restrict__ hold_stats,
+                                                                BatchArchive ar, int one, int one_idx) {
   constexpr int MV = (EKF_CAM + 6 * NC + BCMP_THREADS - 1) / BCMP_THREADS;   // state entries a thread moves: 1 at NC = 32
-  __shared__ int keep[NC], newpos[NC], conv[NC];
+  __shared__ int keep[NC], newpos[NC], conv[NC], arch[NC];
   __shared__ int2 rmap[EKF_CAM + 6 * NC + 2];
-  __shared__ int s_N2, s_n2;
-  const int b = blockIdx.x, tid = threadIdx.x;
+  __shared__ int s_N2, s_n2, s_narch, s_abase;
+  const bool single = one >= 0;
+  const int b = single ? one : blockIdx.x, tid = threadIdx.x;
   DevCtl* ctl = bv.ctl + b;
-  const bool rem = remove && ctl->n_remove > 0;
-  const bool hold = hold_stats && hold_stats[(size_t)b * EKF_BATCH_STAT_FIELDS + EKF_BSTAT_TOPUP] > 0;
+  const bool rem = single || (remove && ctl->n_remove > 0);
+  const bool hold = single || (hold_stats && hold_stats[(size_t)b * EKF_BATCH_STAT_FIELDS + EKF_BSTAT_TOPUP] > 0);
   const int nconv = hold ? 0 : bv.xyz_count[b];
   if (!rem && nconv <= 0) return;
   const int N = bv.N[b], ld = bv.ld;
@@ -1148,17 +1168,28 @@ __global__ void __launch_bounds__(BCMP_THREADS) k_batch_compact(BatchView bv, do
   double* Jall = bv.xyz_J + (size_t)b * bv.Ncap * 18;
   double* yall = bv.xyz_y + (size_t)b * bv.Ncap * 3;
   if (tid == 0) {
+#define DEAD(f) (single ? (f) == one_idx : (rem && ft.removef[f] != 0))
     int flagged = 0;
-    if (rem)
-      for (int f = 0; f < N; ++f) flagged += ft.removef[f] ? 1 : 0;
+    for (int f = 0; f < N; ++f) flagged += DEAD(f) ? 1 : 0;
     // removeFeature(0) after the flagged ones are gone (V:1312-1313): first survivor
-    const bool drop_first = rem && (ctl->n_visible < min_features) && (N - flagged > max_features);
+    const bool drop_first = !single && rem && (ctl->n_visible < min_features) && (N - flagged > max_features);
+    int victim = -1;
+    for (int f = 0; drop_first && f < N && victim < 0; ++f)
+      if (!DEAD(f)) victim = f;
+    if (ar.cap > 0) {   // archive order: the flagged features ascending, then the victim
+      int na = 0;
+      for (int f = 0; f < N; ++f)
+        if (DEAD(f) && pts_archived(ft.coding[f], ft.n_find[f])) arch[na++] = f;
+      if (victim >= 0 && pts_archived(ft.coding[victim], ft.n_find[victim])) arch[na++] = victim;
+      const int base = ar.count[b], room = base < ar.cap ? ar.cap - base : 0, kept = na < room ? na : room;
+      ar.count[b] = base + kept;
+      if (na > kept) ar.overflow[b] += na - kept;
+      s_narch = kept; s_abase = base;
+    }
     int N2 = 0, n2 = EKF_CAM;
-    bool dropped = false;
     for (int i = 0; i < EKF_CAM; ++i) rmap[i] = make_int2(i, -1);
     for (int f = 0; f < N; ++f) {
-      if (rem && ft.removef[f]) continue;
-      if (drop_first && !dropped) { dropped = true; continue; }
+      if (DEAD(f) || f == victim) continue;
       const int cv = nconv > 0 && cflag[f];
       keep[N2] = f; newpos[N2] = n2; conv[N2] = cv; ++N2;
       if (cv) {
@@ -1169,9 +1200,17 @@ __global__ void __launch_bounds__(BCMP_THREADS) k_batch_compact(BatchView bv, do
       }
     }
     s_N2 = N2; s_n2 = n2;
+#undef DEAD
   }
   __syncthreads();
   const int N2 = s_N2, n2 = s_n2;
+  if (ar.cap > 0)   // before Sigma, mu and the table are rewritten (barriers below)
+    for (int k = tid; k < s_narch; k += BCMP_THREADS) {
+      const int f = arch[k];
+      const size_t slot = (size_t)b * ar.cap + s_abase + k;
+      pts_record(mu, Sigma, ld, ft.pos[f], ar.rec + slot * PTS_COLS);
+      ar.real_index[slot] = ft.real_index[f];
+    }
   for (int e = tid; e < n2 * n2; e += BCMP_THREADS) {
     const int i = e / n2, j = e - i * n2;
     tmp[(size_t)i * ld + j] = xyz_apply_entry(Sigma, ld, rmap[i], rmap[j], Jall);
@@ -1362,6 +1401,59 @@ __global__ void __launch_bounds__(256) k_batch_seed(BatchView bv, const double* 
   for (int e = tid; e < N * bv.tstride; e += 256) { ft.patch[e] = src.patch[e]; ft.mpatch[e] = src.mpatch[e]; }
   if (tid == 0) { bv.n[b] = n; bv.N[b] = N; bv.ctl[b] = DevCtl{}; bv.patchnumbre[b] = patchnumbre; }
 }
+// deleted_patches of the seed filter into every filter's archive (ekf_batch_seed_from with the archive on): n records staged at
+// rec / ri.
+__global__ void __launch_bounds__(256) k_batch_seed_archive(BatchArchive ar, const double* __restrict__ rec, const int* __restrict__ ri,
+                                                            int n) {
+  const int b = blockIdx.x, tid = threadIdx.x;
+  double* dst = ar.rec + (size_t)b * ar.cap * PTS_COLS;
+  for (int e = tid; e < n * PTS_COLS; e += 256) dst[e] = rec[e];
+  for (int e = tid; e < n; e += 256) ar.real_index[(size_t)b * ar.cap + e] = ri[e];
+  if (tid == 0) ar.count[b] = n;
+}
+
+// RosVSLAM::getPointsFeatures (RosVSLAMRansac.cpp:340-418) for filters [first, first + gridDim.x), one CTA per filter, with the
+// row assembly of ekf_points.cuh: rows_out / held_out receive each filter's row count and archive size.  With out (a
+// rows_cap x PTS_COLS slice per filter, zeroed here) and the filter's rows within rows_cap: the live XYZ rows, one thread per
+// feature, then the archived records in archive order, warp 0 taking 32 at a time (of records with the same real_index the
+// later one writes, as sequential overwrites would leave it).  map_scale is the filter's mu[13].  The clear rule
+// (pts_clears) is the caller's, once every requested filter is known to fit.
+#define BPTS_THREADS 256
+__global__ void __launch_bounds__(BPTS_THREADS) k_batch_points_features(BatchView bv, BatchArchive ar, int first, int rows_cap,
+                                                                        double* __restrict__ out, int* __restrict__ rows_out,
+                                                                        int* __restrict__ held_out) {
+  const int k = blockIdx.x, b = first + k, tid = threadIdx.x;
+  const int N = bv.N[b];
+  const FeatTab ft = feattab_slice(bv.ft, b, bv.Ncap, bv.tstride);
+  const int rows = pts_row_count(N, ft.real_index);
+  const int held = ar.cap > 0 ? ar.count[b] : 0;
+  if (tid == 0) { rows_out[k] = rows; held_out[k] = held; }
+  if (!out || rows > rows_cap) return;
+  double* o = out + (size_t)k * rows_cap * PTS_COLS;
+  for (size_t e = tid; e < (size_t)rows * PTS_COLS; e += BPTS_THREADS) o[e] = 0.0;
+  for (size_t e = (size_t)rows * PTS_COLS + tid; e < (size_t)rows_cap * PTS_COLS; e += BPTS_THREADS) o[e] = 0.0;
+  __syncthreads();
+  const double* mu = bv.mu + (size_t)b * bv.ld;
+  const double* Sigma = bv.Sigma + (size_t)b * bv.sstride;
+  const double map_scale = mu[13];
+  for (int i = tid; i < N; i += BPTS_THREADS) {
+    const int ri = ft.real_index[i];
+    if (pts_archive_in_range(ri, rows)) pts_live_row(ft.coding[i], ft.pos[i], mu, Sigma, bv.ld, map_scale, o + (size_t)ri * PTS_COLS);
+  }
+  __syncthreads();
+  if (tid < 32) {
+    for (int k0 = 0; k0 < held; k0 += 32) {
+      const int kk = k0 + tid;
+      const size_t slot = (size_t)b * ar.cap + kk;
+      const int ri = kk < held ? ar.real_index[slot] : -1;
+      const bool in = kk < held && pts_archive_in_range(ri, rows);
+      const unsigned same = __match_any_sync(0xffffffffu, in ? ri : -1);
+      if (in && (same & ~((2u << tid) - 1u)) == 0u) pts_archive_row(ar.rec + slot * PTS_COLS, map_scale, o + (size_t)ri * PTS_COLS);
+      __syncwarp();
+    }
+  }
+}
+
 __global__ void k_batch_set_cam(BatchView bv, const double* __restrict__ mu14, int B) {
   const int e = blockIdx.x * blockDim.x + threadIdx.x;
   if (e < B * 14) bv.mu[(size_t)(e / 14) * bv.ld + (e % 14)] = mu14[e];
@@ -1407,6 +1499,10 @@ struct ekf_batch {
   int cl_ctas = 1, cl_resident = 0;             // CTAs per filter in the update; clusters resident at once (large only)
   int cstride = EKF_BATCH_MAX_CORNERS;          // corners per filter in det_xy (BNCAP_L when large)
   long long launches = 0;
+  BatchArchive ar{};                            // feature archive (ekf_batch_set_archive; cap 0: off)
+  int* h_over = nullptr;                        // pinned mirror of ar.overflow, read back with the step's n / N
+  std::vector<int> over_seen;                   // ar.overflow at the last check
+  int *pts_dev = nullptr, *h_pts = nullptr;     // [2][B] row counts and archive sizes of ekf_batch_get_points_features; pinned mirror
   cudaEvent_t ev[4] = {nullptr, nullptr, nullptr, nullptr};
   std::string err;
 };
@@ -1460,6 +1556,9 @@ int ekf_batch_destroy(ekf_batch* b) {
   if (b->h_xyz_count) cudaFreeHost(b->h_xyz_count);
   if (b->h_n) cudaFreeHost(b->h_n);
   if (b->h_N) cudaFreeHost(b->h_N);
+  cudaFree(b->ar.rec); cudaFree(b->ar.real_index); cudaFree(b->ar.count); cudaFree(b->ar.overflow); cudaFree(b->pts_dev);
+  if (b->h_over) cudaFreeHost(b->h_over);
+  if (b->h_pts) cudaFreeHost(b->h_pts);
   for (auto& e : b->ev) if (e) cudaEventDestroy(e);
   if (b->own_stream) cudaStreamDestroy(b->own_stream);
   delete b;
@@ -1623,11 +1722,35 @@ int ekf_batch_seed_from(ekf_batch* b, ekf_handle* src) {
   if (src->device != b->device) return bfail(b, EKF_ERR_ARG, "seed filter lives on another device");
   if (src->N > b->Ncap || src->n > b->ncap) return bfail(b, EKF_ERR_CAPACITY, "seed filter holds more features than the batch capacity");
   if (src->cfg.window_size != b->cfg.window_size) return bfail(b, EKF_ERR_ARG, "window_size differs");
+  const int nd = (int)src->deleted.size();
+  if (b->ar.cap > 0 && nd > b->ar.cap)
+    return bfail(b, EKF_ERR_CAPACITY, "seed filter's feature archive holds more records than the batch's archive capacity");
   BCHECK(cudaSetDevice(b->device));
   BCHECK(cudaStreamSynchronize(src->stream));
   k_batch_seed<<<b->B, 256, 0, b->stream>>>(b->bv, src->Sigma, src->ld, src->mu, src->ft, src->n, src->N, src->patchnumbre);
   b->launches += 1;
   BCHECK(cudaGetLastError());
+  if (b->ar.cap > 0) {   // deleted_patches travels with the filter: every filter starts from the source's archive
+    std::vector<double> rec((size_t)std::max(nd, 1) * PTS_COLS);
+    std::vector<int> ri((size_t)std::max(nd, 1));
+    for (int i = 0; i < nd; ++i) {
+      const DeletedPatch& dp = src->deleted[i];
+      ri[i] = dp.real_index;
+      for (int c = 0; c < 3; ++c) rec[(size_t)i * PTS_COLS + c] = dp.XYZ_pos[c];
+      for (int c = 0; c < 9; ++c) rec[(size_t)i * PTS_COLS + 3 + c] = dp.cov_4_delete[c];
+    }
+    double* d_rec = nullptr;
+    int* d_ri = nullptr;
+    BCHECK(cudaMallocAsync((void**)&d_rec, sizeof(double) * rec.size(), b->stream));
+    BCHECK(cudaMallocAsync((void**)&d_ri, sizeof(int) * ri.size(), b->stream));
+    BCHECK(cudaMemcpyAsync(d_rec, rec.data(), sizeof(double) * rec.size(), cudaMemcpyHostToDevice, b->stream));
+    BCHECK(cudaMemcpyAsync(d_ri, ri.data(), sizeof(int) * ri.size(), cudaMemcpyHostToDevice, b->stream));
+    k_batch_seed_archive<<<b->B, 256, 0, b->stream>>>(b->ar, d_rec, d_ri, nd);
+    b->launches += 1;
+    BCHECK(cudaGetLastError());
+    BCHECK(cudaFreeAsync(d_rec, b->stream));
+    BCHECK(cudaFreeAsync(d_ri, b->stream));
+  }
   BCHECK(cudaStreamSynchronize(b->stream));
   for (int i = 0; i < b->B; ++i) { b->h_n[i] = src->n; b->h_N[i] = src->N; }
   b->dT = src->dT; b->old_ts = src->old_ts;
@@ -1726,15 +1849,35 @@ int ekf_batch_set_force_plane(ekf_batch* b, int on) {
   return EKF_OK;
 }
 
-// k_batch_compact at the batch's capacity
-static void launch_compact(ekf_batch* b, int remove, const int* hold_stats) {
+// k_batch_compact at the batch's capacity; one >= 0: removeFeature(one_idx) on filter `one` alone (one CTA)
+static void launch_compact(ekf_batch* b, int remove, const int* hold_stats, int one = -1, int one_idx = -1) {
+  const unsigned grid = one >= 0 ? 1u : (unsigned)b->B;
   if (b->large)
-    k_batch_compact<BNCAP_L><<<b->B, BCMP_THREADS, 0, b->stream>>>(b->bv, b->scratch, b->cfg.min_features, b->cfg.max_features, remove,
-                                                                   hold_stats);
+    k_batch_compact<BNCAP_L><<<grid, BCMP_THREADS, 0, b->stream>>>(b->bv, b->scratch, b->cfg.min_features, b->cfg.max_features, remove,
+                                                                   hold_stats, b->ar, one, one_idx);
   else
-    k_batch_compact<BNCAP><<<b->B, BCMP_THREADS, 0, b->stream>>>(b->bv, b->scratch, b->cfg.min_features, b->cfg.max_features, remove,
-                                                                 hold_stats);
+    k_batch_compact<BNCAP><<<grid, BCMP_THREADS, 0, b->stream>>>(b->bv, b->scratch, b->cfg.min_features, b->cfg.max_features, remove,
+                                                                 hold_stats, b->ar, one, one_idx);
   b->launches += 1;
+}
+
+// With the archive on: enqueue the overflow counters' read-back beside a read-back of n / N, and after its synchronisation name
+// the first filter whose archive dropped records since the last check (EKF_ERR_CAPACITY).
+static int archive_readback(ekf_batch* b) {
+  if (b->ar.cap > 0)
+    BCHECK(cudaMemcpyAsync(b->h_over, b->ar.overflow, sizeof(int) * b->B, cudaMemcpyDeviceToHost, b->stream));
+  return EKF_OK;
+}
+static int archive_check(ekf_batch* b) {
+  if (b->ar.cap <= 0) return EKF_OK;
+  int first = -1;
+  for (int i = 0; i < b->B; ++i) {
+    if (b->h_over[i] != b->over_seen[i] && first < 0) first = i;
+    b->over_seen[i] = b->h_over[i];
+  }
+  if (first < 0) return EKF_OK;
+  return bfail(b, EKF_ERR_CAPACITY, "filter " + std::to_string(first) + ": feature archive full (capacity " + std::to_string(b->ar.cap) +
+                                        "), removed features were not archived");
 }
 
 // detection + adds for every filter, filter b asking for num[b * num_stride] corners (<= 0: none); decide: also take the new
@@ -1757,6 +1900,8 @@ static int batch_readback(ekf_batch* b, bool added) {
   BCHECK(cudaMemcpyAsync(b->h_n, b->bv.n, sizeof(int) * Bn, cudaMemcpyDeviceToHost, st));
   BCHECK(cudaMemcpyAsync(b->h_N, b->bv.N, sizeof(int) * Bn, cudaMemcpyDeviceToHost, st));
   if (added) BCHECK(cudaMemcpyAsync(b->h_added, b->det_n, sizeof(int) * Bn, cudaMemcpyDeviceToHost, st));
+  const int rc = archive_readback(b);
+  if (rc) return rc;
   BCHECK(cudaStreamSynchronize(st));
   return EKF_OK;
 }
@@ -1824,9 +1969,8 @@ int ekf_batch_step(ekf_batch* b, const double dv[3], const double dw[3], int vco
     if (removed > 0 || converted > 0) {   // removals, then convert2XYZ_ifLinearAll (V:1312-1317), in one pass
       launch_compact(b, 1, nullptr);
       BCHECK(cudaGetLastError());
-      BCHECK(cudaMemcpyAsync(b->h_n, b->bv.n, sizeof(int) * Bn, cudaMemcpyDeviceToHost, st));
-      BCHECK(cudaMemcpyAsync(b->h_N, b->bv.N, sizeof(int) * Bn, cudaMemcpyDeviceToHost, st));
-      BCHECK(cudaStreamSynchronize(st));
+      const int rc = batch_readback(b, false);
+      if (rc) return rc;
     }
   } else {
     // The reference order (V:1312-1317): removals, findNewFeatures, convert2XYZ_ifLinearAll.  A filter that tops up must
@@ -1849,7 +1993,7 @@ int ekf_batch_step(ekf_batch* b, const double dv[3], const double dw[3], int vco
   for (size_t i = 0; b->blur && i < Bn; ++i)
     if (b->h_blur[Bn + i])
       return bfail(b, EKF_ERR_UNSUPPORTED, "filter " + std::to_string(i) + ": a motion-blur kernel exceeded 256 x 256 pixels");
-  return EKF_OK;
+  return archive_check(b);
 }
 
 int ekf_batch_convert2xyz_if_linear_all(ekf_batch* b) {
@@ -2048,6 +2192,119 @@ int ekf_batch_get_template(ekf_batch* b, int f, int idx, int which, uint8_t* out
   const uint8_t* src = (which ? t.mpatch : t.patch) + (size_t)idx * b->bv.tstride;
   BCHECK(cudaMemcpyAsync(out, src, (size_t)b->cfg.window_size * b->cfg.window_size, cudaMemcpyDeviceToHost, b->stream));
   BCHECK(cudaStreamSynchronize(b->stream));
+  return EKF_OK;
+}
+
+int ekf_batch_set_archive(ekf_batch* b, int32_t capacity) {
+  if (!b || capacity < 0) return EKF_ERR_ARG;
+  BCHECK(cudaSetDevice(b->device));
+  BCHECK(cudaStreamSynchronize(b->stream));
+  cudaFree(b->ar.rec); cudaFree(b->ar.real_index); cudaFree(b->ar.count); cudaFree(b->ar.overflow);
+  b->ar = BatchArchive{};
+  if (capacity == 0) return EKF_OK;
+  const size_t Bn = (size_t)b->B, slots = Bn * (size_t)capacity;
+  BatchArchive a{};
+  cudaError_t e = balloc(&a.rec, slots * PTS_COLS);
+  if (e == cudaSuccess) e = balloc(&a.real_index, slots);
+  if (e == cudaSuccess) e = balloc(&a.count, Bn);
+  if (e == cudaSuccess) e = balloc(&a.overflow, Bn);
+  if (e == cudaSuccess && !b->h_over) e = cudaMallocHost((void**)&b->h_over, sizeof(int) * Bn);
+  if (e != cudaSuccess) {
+    cudaFree(a.rec); cudaFree(a.real_index); cudaFree(a.count); cudaFree(a.overflow);
+    return bfail(b, EKF_ERR_CUDA, std::string("feature archive allocation: ") + cudaGetErrorString(e));
+  }
+  a.cap = capacity;
+  BCHECK(cudaMemsetAsync(a.count, 0, sizeof(int) * Bn, b->stream));
+  BCHECK(cudaMemsetAsync(a.overflow, 0, sizeof(int) * Bn, b->stream));
+  BCHECK(cudaStreamSynchronize(b->stream));
+  std::fill(b->h_over, b->h_over + Bn, 0);
+  b->over_seen.assign(Bn, 0);
+  b->ar = a;
+  return EKF_OK;
+}
+
+int ekf_batch_remove_feature(ekf_batch* b, int f, int index) {
+  if (!b || f < 0 || f >= b->B) return EKF_ERR_ARG;
+  if (!b->seeded) return bfail(b, EKF_ERR_STATE, "removeFeature before ekf_batch_seed_from");
+  if (index < 0 || index >= b->h_N[f]) return bfail(b, EKF_ERR_ARG, "feature index out of range");
+  BCHECK(cudaSetDevice(b->device));
+  launch_compact(b, 0, nullptr, f, index);
+  BCHECK(cudaGetLastError());
+  const int rc = batch_readback(b, false);
+  if (rc) return rc;
+  return archive_check(b);
+}
+
+int ekf_batch_num_deleted(ekf_batch* b, int32_t* counts) {
+  if (!b || !counts) return EKF_ERR_ARG;
+  if (b->ar.cap <= 0) {
+    std::fill(counts, counts + b->B, 0);
+    return EKF_OK;
+  }
+  BCHECK(cudaSetDevice(b->device));
+  BCHECK(cudaMemcpyAsync(counts, b->ar.count, sizeof(int) * b->B, cudaMemcpyDeviceToHost, b->stream));
+  BCHECK(cudaStreamSynchronize(b->stream));
+  return EKF_OK;
+}
+
+int ekf_batch_get_deleted(ekf_batch* b, int f, ekf_deleted_info* out, int cap, int* n) {
+  if (!b || f < 0 || f >= b->B || !n || cap < 0 || (cap > 0 && !out)) return EKF_ERR_ARG;
+  *n = 0;
+  if (b->ar.cap <= 0) return EKF_OK;
+  BCHECK(cudaSetDevice(b->device));
+  cudaStream_t st = b->stream;
+  int held = 0;
+  BCHECK(cudaMemcpyAsync(&held, b->ar.count + f, sizeof(int), cudaMemcpyDeviceToHost, st));
+  BCHECK(cudaStreamSynchronize(st));
+  *n = held;
+  const int k = std::min(held, cap);
+  if (k <= 0) return EKF_OK;
+  std::vector<double> rec((size_t)k * PTS_COLS);
+  std::vector<int> ri(k);
+  const size_t slot = (size_t)f * b->ar.cap;
+  BCHECK(cudaMemcpyAsync(rec.data(), b->ar.rec + slot * PTS_COLS, sizeof(double) * rec.size(), cudaMemcpyDeviceToHost, st));
+  BCHECK(cudaMemcpyAsync(ri.data(), b->ar.real_index + slot, sizeof(int) * k, cudaMemcpyDeviceToHost, st));
+  BCHECK(cudaStreamSynchronize(st));
+  for (int i = 0; i < k; ++i) {
+    ekf_deleted_info& o = out[i];
+    o.real_index = ri[i]; o._pad = 0;
+    for (int c = 0; c < 3; ++c) o.xyz_pos[c] = rec[(size_t)i * PTS_COLS + c];
+    for (int c = 0; c < 9; ++c) o.cov_4_delete[c] = rec[(size_t)i * PTS_COLS + 3 + c];
+  }
+  return EKF_OK;
+}
+
+int ekf_batch_get_points_features(ekf_batch* b, int first, int count, double* out, int rows_cap, int32_t* rows) {
+  if (!b || !rows || first < 0 || count < 1 || first > b->B - count || (out && rows_cap < 1)) return EKF_ERR_ARG;
+  BCHECK(cudaSetDevice(b->device));
+  cudaStream_t st = b->stream;
+  const size_t Bn = (size_t)b->B;
+  if (!b->pts_dev) {
+    BCHECK(balloc(&b->pts_dev, 2 * Bn));
+    BCHECK(cudaMallocHost((void**)&b->h_pts, sizeof(int) * 2 * Bn));
+  }
+  const size_t bytes = out ? sizeof(double) * PTS_COLS * (size_t)rows_cap * count : 0;
+  double* dev = nullptr;
+  if (out) BCHECK(cudaMallocAsync((void**)&dev, bytes, st));
+  k_batch_points_features<<<count, BPTS_THREADS, 0, st>>>(b->bv, b->ar, first, rows_cap, dev, b->pts_dev, b->pts_dev + count);
+  b->launches += 1;
+  BCHECK(cudaGetLastError());
+  BCHECK(cudaMemcpyAsync(b->h_pts, b->pts_dev, sizeof(int) * 2 * count, cudaMemcpyDeviceToHost, st));
+  BCHECK(cudaStreamSynchronize(st));
+  int most = 0;
+  for (int k = 0; k < count; ++k) most = std::max(most, b->h_pts[k]);
+  std::copy(b->h_pts, b->h_pts + count, rows);
+  if (!out) return EKF_OK;
+  if (most > rows_cap) {
+    BCHECK(cudaFreeAsync(dev, st));
+    BCHECK(cudaStreamSynchronize(st));
+    return bfail(b, EKF_ERR_ARG, "rows_cap " + std::to_string(rows_cap) + " below the largest row count " + std::to_string(most));
+  }
+  BCHECK(cudaMemcpyAsync(out, dev, bytes, cudaMemcpyDeviceToHost, st));
+  BCHECK(cudaFreeAsync(dev, st));
+  for (int k = 0; k < count; ++k)   // the clear rule (R:395-403), on the device's archive of every exported filter
+    if (pts_clears(b->h_pts[count + k])) BCHECK(cudaMemsetAsync(b->ar.count + first + k, 0, sizeof(int), st));
+  BCHECK(cudaStreamSynchronize(st));
   return EKF_OK;
 }
 

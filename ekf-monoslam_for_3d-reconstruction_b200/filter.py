@@ -296,12 +296,13 @@ class FilterBatch:
             raise EkfError(f"{'ekf_batch_create_large' if large else 'ekf_batch_create'} failed with {rc}")
         self.h = h
         self.B = int(n_filters)
+        self._cams = None   # (mu14, Sigma14) of every filter, read once per step for the views
 
     @classmethod
-    def from_config(cls, cfg, n_filters, feature_capacity=32, device=0, large=False):
+    def from_config(cls, cfg, n_filters, feature_capacity=32, device=0, large=False, archive=0):
         """A batch from the configuration a VSlamFilter takes: created with motion blur, resize and forsePlane off (which
-        ekf_batch_create requires), then set_motion_blur(cfg.kernel_size) when blur is on, set_scale(cfg.scale) and
-        set_force_plane(cfg.forsePlane)."""
+        ekf_batch_create requires), then set_motion_blur(cfg.kernel_size) when blur is on, set_scale(cfg.scale),
+        set_force_plane(cfg.forsePlane) and, when archive > 0, set_archive(archive)."""
         base = _abi.EkfConfig.from_buffer_copy(cfg)
         base.kernel_size, base.scale, base.forsePlane = _abi.default_config().kernel_size, 1, 0
         batch = cls(base, n_filters, feature_capacity=feature_capacity, device=device, large=large)
@@ -310,6 +311,8 @@ class FilterBatch:
             batch.set_motion_blur(cfg.kernel_size)
         batch.set_scale(cfg.scale)
         batch.set_force_plane(cfg.forsePlane)
+        if archive:
+            batch.set_archive(archive)
         return batch
 
     def close(self):
@@ -340,12 +343,14 @@ class FilterBatch:
         self._ck(self.L.ekf_batch_sync(self.h))
 
     def seed_from(self, filt):
+        self._cams = None
         self._ck(self.L.ekf_batch_seed_from(self.h, filt.h))
 
     def set_camera_states(self, mu14):
         a = np.ascontiguousarray(mu14, dtype=np.float64)
         if a.shape != (self.B, 14):
             raise ValueError("set_camera_states expects (n_filters, 14)")
+        self._cams = None
         self._ck(self.L.ekf_batch_set_camera_states(self.h, _ptr(a)))
 
     def captureNewFrame(self, img, stamp=-1.0):
@@ -378,6 +383,7 @@ class FilterBatch:
         """predict + update of every filter."""
         p = np.ascontiguousarray(picks if picks is not None else np.zeros(0), dtype=np.uint32)
         a = np.asarray(dv, dtype=np.float64); b = np.asarray(dw, dtype=np.float64)
+        self._cams = None
         self._ck(self.L.ekf_batch_step(self.h, _ptr(a), _ptr(b), int(bool(vcontrol)), _ptr(p), int(p.size)))
 
     def convert2XYZ_ifLinearAll(self):
@@ -407,6 +413,7 @@ class FilterBatch:
         n = self.state_dim(f)
         if mu.size != n or S.shape != (n, n):
             raise ValueError("set_full: shape mismatch")
+        self._cams = None
         self._ck(self.L.ekf_batch_set_full(self.h, int(f), _ptr(mu), _ptr(S), n))
 
     def feature(self, f, i):
@@ -417,6 +424,56 @@ class FilterBatch:
     def addFeature(self, f, u, v):
         """vslamRansac.cpp:309-371 on filter f; 1 added, 0 rejected by isInsideImage."""
         return self._ck(self.L.ekf_batch_add_feature(self.h, int(f), float(u), float(v)))
+
+    def removeFeature(self, f, i):
+        """vslamRansac.cpp:373-421 on feature i of filter f (archived under the rule of set_archive)."""
+        self._ck(self.L.ekf_batch_remove_feature(self.h, int(f), int(i)))
+
+    # ---- the feature archive and the map export ---------------------------------------------------
+    def set_archive(self, capacity):
+        """Keep every filter's VSlamFilter::deleted_patches (vslamRansac.cpp:394-404), up to `capacity` records per filter
+        (0: off, the default).  Empties every archive."""
+        self._ck(self.L.ekf_batch_set_archive(self.h, int(capacity)))
+
+    def num_deleted(self):
+        """Records in each filter's archive (int32, n_filters)."""
+        out = np.zeros(self.B, dtype=np.int32)
+        self._ck(self.L.ekf_batch_num_deleted(self.h, _ptr(out)))
+        return out
+
+    def deleted(self, f):
+        """Filter f's archive as VSlamFilter.deleted(): list of (real_index, XYZ_pos[3], cov_4_delete[9])."""
+        n = C.c_int(0)
+        self._ck(self.L.ekf_batch_get_deleted(self.h, int(f), None, 0, C.byref(n)))
+        recs = (_abi.EkfDeletedInfo * max(n.value, 1))()
+        self._ck(self.L.ekf_batch_get_deleted(self.h, int(f), recs, n.value, C.byref(n)))
+        return [(o.real_index, np.array(o.xyz_pos), np.array(o.cov_4_delete)) for o in recs[:n.value]]
+
+    def points_features(self, first=0, count=None):
+        """RosVSLAM::getPointsFeatures (RosVSLAMRansac.cpp:340-418) for filters [first, first + count) from one export:
+        a list of (rows_f, 12) matrices, as VSlamFilter.getPointsFeatures() returns them."""
+        count = self.B - int(first) if count is None else int(count)
+        rows = np.zeros(max(count, 1), dtype=np.int32)
+        self._ck(self.L.ekf_batch_get_points_features(self.h, int(first), count, None, 0, _ptr(rows)))
+        cap = int(rows[:count].max())
+        out = np.zeros((count, cap, 12))
+        self._ck(self.L.ekf_batch_get_points_features(self.h, int(first), count, _ptr(out), cap, _ptr(rows)))
+        return [out[k, :rows[k]].copy() for k in range(count)]
+
+    def getPointsFeatures(self, f):
+        """Filter f's (rows, 12) matrix, as VSlamFilter.getPointsFeatures()."""
+        return self.points_features(f, 1)[0]
+
+    def view(self, f):
+        """Filter f as the object keyframes.KeyframeRecorder drives (getState, getSigma, Covariance_Parameter,
+        getPointsFeatures, Point4sba).  Every view of the batch reads its camera state from one cached read-back per step."""
+        return BatchFilterView(self, int(f))
+
+    def _camera_cache(self):
+        if self._cams is None:
+            mu, S, _ = self.camera_states(want_sigma=True)
+            self._cams = (mu, S)
+        return self._cams
 
     def _num(self, num):
         return np.ascontiguousarray(np.broadcast_to(np.asarray(num, dtype=np.int32), (self.B,)))
@@ -482,3 +539,29 @@ class FilterBatch:
         out = np.zeros(3, dtype=np.float32)
         self._ck(self.L.ekf_batch_last_step_ms(self.h, _ptr(out)))
         return dict(predict=float(out[0]), match=float(out[1]), update=float(out[2]))
+
+
+class BatchFilterView:
+    """One filter of a FilterBatch with the accessors of VSlamFilter that keyframes.KeyframeRecorder reads."""
+
+    Point4sba = np.zeros((1, 3), dtype=np.int32)   # the node's projection list stays empty (monoslam_ransac.cpp:689-752 is dead)
+
+    def __init__(self, batch, f):
+        self.batch, self.f = batch, f
+
+    def getState(self):
+        return self.batch._camera_cache()[0][self.f].copy()
+
+    def getSigma(self):
+        return self.batch._camera_cache()[1][self.f].copy()
+
+    def Covariance_Parameter(self):
+        """ekf_covariance_parameter (vslamRansac.cpp:854-855), the same sums in the same order."""
+        S = self.batch._camera_cache()[1][self.f]
+        P = 0.0
+        P += float(S[0, 0]) + float(S[1, 1]) + float(S[2, 2])
+        P += float(S[4, 4]) + float(S[5, 5]) + float(S[6, 6]) + float(S[3, 3])
+        return P
+
+    def getPointsFeatures(self):
+        return self.batch.getPointsFeatures(self.f)

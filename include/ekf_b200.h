@@ -326,6 +326,34 @@ int ekf_batch_last_added(ekf_batch* b, int32_t* added);
 int ekf_batch_set_motion_blur(ekf_batch* b, int32_t kernel_size);
 /* Templates each filter blurred in the last step (n_filters entries; zeros with blur off). */
 int ekf_batch_last_blur_counts(ekf_batch* b, int32_t* out);
+/* The feature archive of every filter (VSlamFilter::deleted_patches, vslamRansac.cpp:394-404), off by default.
+ * capacity > 0 turns it on with room for `capacity` records per filter and empties every filter's archive; 0 turns it off.
+ * Device memory: n_filters x capacity x 100 bytes (real_index + 12 doubles), e.g. 4096 filters x 7001 records = 2.9 GB.  The
+ * reference keeps its archive bounded only through the export's clear rule (more than 7000 records are cleared), so a capacity of
+ * at least 7001 lets an exporting caller never run out.  With the archive on, every removal (the step's quality deletions in
+ * ascending index, then its max_features removeFeature(0), and ekf_batch_remove_feature) archives each XYZ feature with
+ * n_find > 5, as ekf_get_deleted reports them for a single filter.  When a filter's archive is full its record is dropped: the
+ * step (or removal) still runs to its end, then returns EKF_ERR_CAPACITY and ekf_batch_last_error names the first filter that
+ * dropped one.  ekf_batch_seed_from copies the source's archive into every filter (EKF_ERR_CAPACITY if it holds more than
+ * capacity records).  EKF_ERR_ARG for a negative capacity. */
+int ekf_batch_set_archive(ekf_batch* b, int32_t capacity);
+/* VSlamFilter::removeFeature (vslamRansac.cpp:373-421) on feature `index` of one filter, on the device: exactly that feature
+ * goes (archived under the rule above), without the step's max_features rule.  EKF_ERR_ARG for a bad filter or index,
+ * EKF_ERR_STATE before seeding. */
+int ekf_batch_remove_feature(ekf_batch* b, int filter, int index);
+/* Records in each filter's archive (counts: n_filters entries; zeros with the archive off). */
+int ekf_batch_num_deleted(ekf_batch* b, int32_t* counts);
+/* One filter's archive in archive order, in ekf_get_deleted's layout: *n receives the record count, and the first
+ * min(*n, cap) records go to out (which may be NULL with cap = 0 to query the count). */
+int ekf_batch_get_deleted(ekf_batch* b, int filter, ekf_deleted_info* out, int cap, int* n);
+/* ekf_get_points_features (RosVSLAM::getPointsFeatures, RosVSLAMRansac.cpp:340-418) for filters [first, first + count) in one
+ * launch.  rows[k] receives filter first + k's row count (real_index of its last live feature + 1, or 1 without features).
+ * out holds count x rows_cap x 12 doubles: filter first + k's matrix starts at out + k * rows_cap * 12, and its rows past rows[k]
+ * are zero.  out == NULL only queries rows; EKF_ERR_ARG when rows_cap is below the largest row count.  Rows as for a single
+ * filter: live XYZ features write position * map_scale and their 3 x 3 block, inverse-depth rows stay zero, then archived
+ * records overwrite theirs in archive order (position * the filter's current map_scale = mu[13]; records past the last live
+ * real_index are dropped).  After the export every exported filter whose archive holds more than 7000 records has it cleared. */
+int ekf_batch_get_points_features(ekf_batch* b, int first, int count, double* out, int rows_cap, int32_t* rows);
 /* which: 0 = Patch::patch, 1 = Patch::matching_patch of feature idx of one filter; out holds window_size^2 bytes */
 int ekf_batch_get_template(ekf_batch* b, int filter, int idx, int which, uint8_t* out);
 /* Kernels of this library launched on the batch so far. */
