@@ -98,6 +98,14 @@ SIGNATURES = {
     "ekf_batch_kernel_launches": (C.c_int64, [_vp]),
     "ekf_batch_last_step_ms": (_i, [_vp, _vp]),
     "ekf_batch_last_match_deferred": (_i, [_vp]),
+    "ekf_batch_set_cameras": (_i, [_vp, _i, _vp]),
+    "ekf_batch_capture_frames": (_i, [_vp, _vp, _i, _i, _i, _vp]),
+    "ekf_batch_capture_frames_device": (_i, [_vp, _vp, _i, _i, _i, _vp]),
+    "ekf_batch_capture_frames_bgr": (_i, [_vp, _vp, _i, _i, _i, _vp]),
+    "ekf_batch_get_camera_frame": (_i, [_vp, _i, _vp, _P(_i), _P(_i)]),
+    "ekf_batch_get_dt": (_i, [_vp, _vp]),
+    "ekf_batch_set_detect_budget": (_i, [_vp, C.c_int64]),
+    "ekf_batch_step_controls": (_i, [_vp, _vp, _vp, _vp, _vp, _i]),
     "ekf_dist_load_nccl": (_i, [C.c_char_p]),
     "ekf_dist_unique_id": (_i, [_vp]),
     "ekf_dist_attach": (_i, [_vp, _vp, _i, _i]),

@@ -19,17 +19,29 @@
 // Early stop: every pixel inside the mask is at least window_size from the border, more than the window_size / 2 of
 // isInsideImage, so addFeature accepts every detected corner and the single filter's loop over them (V:832-835) stops only
 // on its capacity: taking min(num_b, Ncap - N_b) corners is exactly what it adds.
+//
+// Cameras (ekf_batch_set_cameras): the argument holds per frame, so each camera that at least one filter asks corners from
+// gets its own eig map, keys and sorted lists (one segment of npx slots), and each filter walks its camera's segment.  The
+// cameras asked from are processed in chunks whose scratch (44 bytes a pixel a camera, the sort's workspace included) fits a fixed
+// budget and whose C * npx keys stay within int range; a segmented radix
+// sort orders every segment of a chunk by the same key, so each camera's order is exactly the single filter's.
 #include <cub/device/device_radix_sort.cuh>
+#include <cub/device/device_segmented_radix_sort.cuh>
+
+#include <vector>
 
 #include "../../include/ekf_b200.h"
 #include "ekf_detect.cuh"
 #include "ekf_kernels.h"
 
 // pixel keys (base mask, eig > 0) and candidate keys (those that are also raw 3x3 local maxima), one slot per pixel
+// (blockIdx.z: the camera's segment of a chunk)
 __global__ void k_bdet_keys(const float* __restrict__ eig, int W, int H, int estrem, unsigned long long* __restrict__ kp,
                             unsigned long long* __restrict__ kc) {
   const int x = blockIdx.x * blockDim.x + threadIdx.x, y = blockIdx.y;
   if (x >= W) return;
+  const size_t seg = (size_t)blockIdx.z * W * H;
+  eig += seg; kp += seg; kc += seg;
   const size_t i = (size_t)y * W + x;
   const float v = eig[i];
   unsigned long long p = 0ull, c = 0ull;
@@ -46,6 +58,14 @@ __global__ void k_bdet_keys(const float* __restrict__ eig, int W, int H, int est
   kc[i] = c;
 }
 
+// Segment of filter b in a chunk of cameras: cam_of == nullptr (one camera) gives segment 0 for every filter; otherwise filter b
+// belongs to the chunk when its camera's slot among the cameras asked from lies in [lo, hi), and -1 is returned when it does not.
+__device__ __forceinline__ int bdet_segment(const int* __restrict__ cam_of, const int* __restrict__ slot_of_cam, int lo, int hi, int b) {
+  if (!cam_of) return 0;
+  const int s = slot_of_cam[cam_of[b]];
+  return (s >= lo && s < hi) ? s - lo : -1;
+}
+
 // One warp per filter: its boxes, its corner limit and thr_b from the first sorted pixel outside its boxes.  CS: boxes and
 // corners a filter has room for (EKF_BATCH_MAX_CORNERS, or EKF_BATCH_MAX_FEATURES in a large batch).
 #define BDET_WARPS 8
@@ -55,11 +75,15 @@ __global__ void __launch_bounds__(32 * BDET_WARPS) k_bdet_threshold(const unsign
                                                                      const int* __restrict__ N, int Ncap, int B,
                                                                      const int* __restrict__ num, int num_stride, int cap_mode,
                                                                      DetBox* __restrict__ boxes, unsigned* __restrict__ thr_bits,
-                                                                     int* __restrict__ limit) {
+                                                                     int* __restrict__ limit, const int* __restrict__ cam_of,
+                                                                     const int* __restrict__ slot_of_cam, int lo, int hi) {
   __shared__ DetBox sb[BDET_WARPS][CS];
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int b = blockIdx.x * BDET_WARPS + warp;
   if (b >= B) return;   // the whole warp
+  const int seg = bdet_segment(cam_of, slot_of_cam, lo, hi, b);
+  if (seg < 0) return;
+  kp += (size_t)seg * npx;
   const int nb = N[b];
   int lim = min(num[(size_t)b * num_stride], cap_mode ? Ncap - nb : EKF_BATCH_MAX_CORNERS);
   lim = max(0, min(lim, CS));
@@ -95,9 +119,13 @@ __global__ void __launch_bounds__(32 * BDET_WARPS) k_bdet_threshold(const unsign
 template <int CS>
 __global__ void k_bdet_select(const unsigned long long* __restrict__ kc, int nkeys, int W, const DetBox* __restrict__ boxes,
                               const int* __restrict__ N, const unsigned* __restrict__ thr_bits, const int* __restrict__ limit, int B,
-                              float* __restrict__ out_xy, int* __restrict__ out_n) {
+                              float* __restrict__ out_xy, int* __restrict__ out_n, const int* __restrict__ cam_of,
+                              const int* __restrict__ slot_of_cam, int lo, int hi) {
   const int b = blockIdx.x * blockDim.x + threadIdx.x;
   if (b >= B) return;
+  const int seg = bdet_segment(cam_of, slot_of_cam, lo, hi, b);
+  if (seg < 0) return;
+  kc += (size_t)seg * nkeys;
   const int lim = limit[b];
   out_n[b] = lim > 0 ? det_select_walk(kc, nkeys, W, thr_bits[b], boxes + (size_t)b * CS, N[b], 144.0f, lim,
                                        out_xy + (size_t)b * 2 * CS)
@@ -126,8 +154,34 @@ cudaError_t batch_detect_reserve(BatchDetectBufs& d, size_t px, int B, int cstri
   return cudaSuccess;
 }
 
+// scratch for chunks of up to `chunk` cameras of npx pixels each: the per-camera buffers, the segment offsets and the larger of
+// the two sorts' workspaces
+cudaError_t batch_detect_reserve_cams(BatchDetectBufs& d, size_t npx, int chunk, int B, int cstride) {
+  cudaError_t e = batch_detect_reserve(d, npx * (size_t)chunk, B, cstride);
+  if (e != cudaSuccess) return e;
+  size_t tmp = 0;
+  if ((e = cub::DeviceSegmentedRadixSort::SortKeysDescending(nullptr, tmp, (const unsigned long long*)nullptr, (unsigned long long*)nullptr,
+                                                             (int)(npx * chunk), chunk, (const int*)nullptr, (const int*)nullptr)) != cudaSuccess)
+    return e;
+  if (tmp > d.tmp_bytes) {
+    cudaFree(d.tmp);
+    d.tmp = nullptr; d.tmp_bytes = 0;
+    if ((e = cudaMalloc(&d.tmp, tmp)) != cudaSuccess) return e;
+    d.tmp_bytes = tmp;
+  }
+  if (d.offs_chunk == chunk && d.offs_npx == npx) return cudaSuccess;
+  std::vector<int> offs((size_t)chunk + 1);
+  for (int s = 0; s <= chunk; ++s) offs[s] = (int)(s * npx);
+  cudaFree(d.offs);
+  d.offs = nullptr; d.offs_chunk = 0;
+  if ((e = cudaMalloc((void**)&d.offs, sizeof(int) * offs.size())) != cudaSuccess) return e;
+  if ((e = cudaMemcpy(d.offs, offs.data(), sizeof(int) * offs.size(), cudaMemcpyHostToDevice)) != cudaSuccess) return e;
+  d.offs_chunk = chunk; d.offs_npx = npx;
+  return cudaSuccess;
+}
+
 void batch_detect_free(BatchDetectBufs& d) {
-  cudaFree(d.eig); cudaFree(d.keys); cudaFree(d.tmp); cudaFree(d.boxes); cudaFree(d.thr_bits); cudaFree(d.limit);
+  cudaFree(d.eig); cudaFree(d.keys); cudaFree(d.tmp); cudaFree(d.boxes); cudaFree(d.thr_bits); cudaFree(d.limit); cudaFree(d.offs);
   d = BatchDetectBufs{};
 }
 
@@ -147,13 +201,57 @@ cudaError_t launch_batch_detect(cudaStream_t st, BatchDetectBufs& d, FrameView f
   const unsigned gt = (B + BDET_WARPS - 1) / BDET_WARPS, gs = (B + 127) / 128;
   if (cstride == EKF_BATCH_MAX_CORNERS) {
     k_bdet_threshold<EKF_BATCH_MAX_CORNERS><<<gt, 32 * BDET_WARPS, 0, st>>>(kp_s, npx, W, H, window, centers, N, Ncap, B, num,
-                                                                           num_stride, cap_mode, d.boxes, d.thr_bits, d.limit);
-    k_bdet_select<EKF_BATCH_MAX_CORNERS><<<gs, 128, 0, st>>>(kc_s, npx, W, d.boxes, N, d.thr_bits, d.limit, B, out_xy, out_n);
+                                                                           num_stride, cap_mode, d.boxes, d.thr_bits, d.limit,
+                                                                           nullptr, nullptr, 0, 0);
+    k_bdet_select<EKF_BATCH_MAX_CORNERS><<<gs, 128, 0, st>>>(kc_s, npx, W, d.boxes, N, d.thr_bits, d.limit, B, out_xy, out_n,
+                                                             nullptr, nullptr, 0, 0);
   } else {
     k_bdet_threshold<EKF_BATCH_MAX_FEATURES><<<gt, 32 * BDET_WARPS, 0, st>>>(kp_s, npx, W, H, window, centers, N, Ncap, B, num,
-                                                                            num_stride, cap_mode, d.boxes, d.thr_bits, d.limit);
-    k_bdet_select<EKF_BATCH_MAX_FEATURES><<<gs, 128, 0, st>>>(kc_s, npx, W, d.boxes, N, d.thr_bits, d.limit, B, out_xy, out_n);
+                                                                            num_stride, cap_mode, d.boxes, d.thr_bits, d.limit,
+                                                                            nullptr, nullptr, 0, 0);
+    k_bdet_select<EKF_BATCH_MAX_FEATURES><<<gs, 128, 0, st>>>(kc_s, npx, W, d.boxes, N, d.thr_bits, d.limit, B, out_xy, out_n,
+                                                              nullptr, nullptr, 0, 0);
   }
   *launches += 5;   // keys, the two sorts (counted once each), threshold, select; the eig map counts itself
   return cudaGetLastError();
+}
+
+cudaError_t launch_batch_detect_cams(cudaStream_t st, BatchDetectBufs& d, FrameView fr, const int* cams, int n_req, int chunk,
+                                     const int* cam_of, const int* slot_of_cam, const float* centers, const int* N, int Ncap, int B,
+                                     int window, const int* num, int num_stride, int cap_mode, int cstride, float* out_xy, int* out_n,
+                                     long long* launches) {
+  const int W = fr.w, H = fr.h, npx = W * H;
+  const size_t fstep = (size_t)fr.h * fr.stride;
+  cudaError_t e = cudaMemsetAsync(out_n, 0, sizeof(int) * (size_t)B, st);   // filters of cameras nobody asks from find nothing
+  if (e != cudaSuccess) return e;
+  unsigned long long *kp = d.keys, *kc = d.keys + d.cap, *kp_s = d.keys + 2 * d.cap, *kc_s = d.keys + 3 * d.cap;
+  const unsigned gt = (B + BDET_WARPS - 1) / BDET_WARPS, gs = (B + 127) / 128;
+  for (int lo = 0; lo < n_req; lo += chunk) {
+    const int C = std::min(chunk, n_req - lo), hi = lo + C;
+    for (int s = 0; s < C; ++s)
+      launch_det_eig(st, FrameView{fr.px + (size_t)cams[lo + s] * fstep, W, H, fr.stride}, d.eig + (size_t)s * npx, launches);
+    k_bdet_keys<<<dim3((W + 255) / 256, H, C), 256, 0, st>>>(d.eig, W, H, window, kp, kc);
+    size_t tmp = d.tmp_bytes;
+    e = cub::DeviceSegmentedRadixSort::SortKeysDescending(d.tmp, tmp, kp, kp_s, C * npx, C, d.offs, d.offs + 1, 0, 64, st);
+    if (e != cudaSuccess) return e;
+    tmp = d.tmp_bytes;
+    e = cub::DeviceSegmentedRadixSort::SortKeysDescending(d.tmp, tmp, kc, kc_s, C * npx, C, d.offs, d.offs + 1, 0, 64, st);
+    if (e != cudaSuccess) return e;
+    if (cstride == EKF_BATCH_MAX_CORNERS) {
+      k_bdet_threshold<EKF_BATCH_MAX_CORNERS><<<gt, 32 * BDET_WARPS, 0, st>>>(kp_s, npx, W, H, window, centers, N, Ncap, B, num,
+                                                                             num_stride, cap_mode, d.boxes, d.thr_bits, d.limit,
+                                                                             cam_of, slot_of_cam, lo, hi);
+      k_bdet_select<EKF_BATCH_MAX_CORNERS><<<gs, 128, 0, st>>>(kc_s, npx, W, d.boxes, N, d.thr_bits, d.limit, B, out_xy, out_n,
+                                                               cam_of, slot_of_cam, lo, hi);
+    } else {
+      k_bdet_threshold<EKF_BATCH_MAX_FEATURES><<<gt, 32 * BDET_WARPS, 0, st>>>(kp_s, npx, W, H, window, centers, N, Ncap, B, num,
+                                                                              num_stride, cap_mode, d.boxes, d.thr_bits, d.limit,
+                                                                              cam_of, slot_of_cam, lo, hi);
+      k_bdet_select<EKF_BATCH_MAX_FEATURES><<<gs, 128, 0, st>>>(kc_s, npx, W, d.boxes, N, d.thr_bits, d.limit, B, out_xy, out_n,
+                                                                cam_of, slot_of_cam, lo, hi);
+    }
+    *launches += 5;
+    if ((e = cudaGetLastError()) != cudaSuccess) return e;
+  }
+  return cudaSuccess;
 }

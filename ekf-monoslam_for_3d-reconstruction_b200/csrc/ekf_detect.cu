@@ -204,6 +204,8 @@ __global__ void k_capture_resize_gray(const uint8_t* __restrict__ src, int sw, i
                                       int dw, int dh, int dstride) {
   const int x = blockIdx.x * blockDim.x + threadIdx.x, y = blockIdx.y;
   if (x >= dw || y >= dh) return;
+  src += (size_t)blockIdx.z * sh * sstride;   // frame z of a stack (batched cameras)
+  dst += (size_t)blockIdx.z * dh * dstride;
   int ch[3] = {0, 0, 0};
   if (sw == dw && sh == dh) {
     for (int c = 0; c < cn; ++c) ch[c] = src[(size_t)y * sstride + x * cn + c];
@@ -232,7 +234,7 @@ __global__ void k_capture_resize_gray(const uint8_t* __restrict__ src, int sw, i
   dst[(size_t)y * dstride + x] = (uint8_t)min(max(g, 0), 255);
 }
 void launch_capture_resize_gray(cudaStream_t st, const uint8_t* src, int sw, int sh, int sstride, int cn, uint8_t* dst, int dw, int dh,
-                                int dstride, long long* launches) {
-  k_capture_resize_gray<<<dim3((dw + 255) / 256, dh), 256, 0, st>>>(src, sw, sh, sstride, cn, dst, dw, dh, dstride);
+                                int dstride, long long* launches, int n_frames) {
+  k_capture_resize_gray<<<dim3((dw + 255) / 256, dh, n_frames), 256, 0, st>>>(src, sw, sh, sstride, cn, dst, dw, dh, dstride);
   *launches += 1;
 }

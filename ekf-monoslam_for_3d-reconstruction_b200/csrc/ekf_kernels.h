@@ -33,7 +33,8 @@ struct alignas(64) EkfTensorMap {
 void match_make_tensor_map(EkfTensorMap* out, const uint8_t* frames, int width, int height, int stride, int n_frames, int w, int clamp);
 void launch_match_filter(cudaStream_t st, FeatTab ft, int N, FrameView fr, const DevCfg& cfg, const EkfTensorMap* tmap, long long* launches);
 void launch_match_filter_batch(cudaStream_t st, FeatTab base, int Ncap, const int* Nper, int B, FrameView fr, const DevCfg& cfg,
-                               const EkfTensorMap* tmap, int* defer_list, int* defer_cnt, long long* launches);
+                               const EkfTensorMap* tmap, int* defer_list, int* defer_cnt, long long* launches,
+                               const int* cam_of = nullptr);   // cam_of [B]: filter b searches frame cam_of[b] of the stack fr
 int launch_match_batch(cudaStream_t st, const uint8_t* frames, int n_frames, int width, int height, int stride,
                        const uint8_t* templates, int fpf, int w, const double* h, const double* S, float sigma_size,
                        float thr, float clampv, int32_t* out_uv, float* out_score);
@@ -121,7 +122,7 @@ int launch_detect_corners(cudaStream_t st, FrameView fr, FeatTab ft, int N, int 
 // the min-eigenvalue map of goodFeaturesToTrack for a whole frame (k_det_eig)
 void launch_det_eig(cudaStream_t st, FrameView fr, float* eig, long long* launches);
 void launch_capture_resize_gray(cudaStream_t st, const uint8_t* src, int sw, int sh, int sstride, int cn, uint8_t* dst, int dw, int dh,
-                                int dstride, long long* launches);
+                                int dstride, long long* launches, int n_frames = 1);   // n_frames: a contiguous stack, frame z in blockIdx.z
 // ekf_batch_detect.cu: findNewFeatures' detection for every filter of a batch (one frame, per-filter masks)
 struct BatchDetectBufs {
   float* eig = nullptr;                 // [cap] min-eigenvalue map
@@ -131,6 +132,9 @@ struct BatchDetectBufs {
   DetBox* boxes = nullptr;              // [B][cstride] mask boxes per filter
   unsigned* thr_bits = nullptr;         // [B] per-filter threshold (float bits)
   int* limit = nullptr;                 // [B] corners each filter may take
+  int* offs = nullptr;                  // [offs_chunk + 1] segment offsets s * offs_npx of the per-camera sorts
+  int offs_chunk = 0;
+  size_t offs_npx = 0;
 };
 cudaError_t batch_detect_reserve(BatchDetectBufs& d, size_t px, int B, int cstride);
 void batch_detect_free(BatchDetectBufs& d);
@@ -140,3 +144,11 @@ void batch_detect_free(BatchDetectBufs& d);
 cudaError_t launch_batch_detect(cudaStream_t st, BatchDetectBufs& d, FrameView fr, const float* centers, const int* N, int Ncap, int B,
                                 int window, const int* num, int num_stride, int cap_mode, int cstride, float* out_xy, int* out_n,
                                 long long* launches);
+// Per camera (ekf_batch_set_cameras): the frames of the n_req cameras listed in HOST cams, frame c at fr.px + c * fr.h * fr.stride,
+// in chunks of `chunk` cameras (scratch from batch_detect_reserve_cams); filter b walks the segment of camera cam_of[b], whose
+// position in cams is slot_of_cam[cam_of[b]] (-1: nobody asks from it; the filter finds nothing).  Same outputs as above.
+cudaError_t batch_detect_reserve_cams(BatchDetectBufs& d, size_t npx, int chunk, int B, int cstride);
+cudaError_t launch_batch_detect_cams(cudaStream_t st, BatchDetectBufs& d, FrameView fr, const int* cams, int n_req, int chunk,
+                                     const int* cam_of, const int* slot_of_cam, const float* centers, const int* N, int Ncap, int B,
+                                     int window, const int* num, int num_stride, int cap_mode, int cstride, float* out_xy, int* out_n,
+                                     long long* launches);

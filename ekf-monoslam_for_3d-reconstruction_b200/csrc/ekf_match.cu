@@ -495,10 +495,10 @@ __device__ bool match_one_tile_cta(const MatchJob& jb, float sigma_size, float c
 // Filter-attached matcher: the loop V:870-880 with one CTA per feature.
 __device__ __forceinline__ void match_filter_feature(FeatTab ft, int f, FrameView fr, const DevCfg& cfg, unsigned char* smem_raw,
                                                      const CUtensorMap* tmap, unsigned* phase_io = nullptr, bool init_bar = true,
-                                                     bool try_tile = false) {
+                                                     bool try_tile = false, int frame_index = 0) {
   const int w = cfg.window, w2 = w * w;
   MatchJob jb;
-  jb.tmap = tmap; jb.frame_index = 0;
+  jb.tmap = tmap; jb.frame_index = frame_index;
   jb.frame = fr.px; jb.fw = fr.w; jb.fh = fr.h; jb.fstride = fr.stride;
   jb.tmpl = ft.mpatch + (size_t)f * cfg.tstride;
   jb.hu = ft.h[2 * f]; jb.hv = ft.h[2 * f + 1];
@@ -1039,11 +1039,19 @@ __device__ __forceinline__ void match_warp_commit(FeatTab ft, int f, FrameView f
   }
 }
 
+// The frame filter b searches: camera cam_of[b] of the batch's contiguous frame stack.  The camera is also the z coordinate of
+// the stack's tensor map, which only the CTA matcher reads.  The batched matcher kernels take CAMS = false with one camera, and
+// then compile to the code that reads the one frame from the kernel's parameters.
+__device__ __forceinline__ FrameView batch_frame(FrameView fr, int cam) {
+  fr.px += (size_t)cam * fr.h * fr.stride;
+  return fr;
+}
+
 // Batched filters, pass 1 with the full-window warp matcher (template side 11): one warp per (filter, feature)
-template <int MINB, bool TSMEM, bool SLIDE>
+template <int MINB, bool TSMEM, bool SLIDE, bool CAMS>
 __global__ void __launch_bounds__(MW2_WARPS * 32, MINB) k_match_filter_batch_warp2(FeatTab base, int Ncap, const int* __restrict__ Nper, int B,
                                                                                 FrameView fr, DevCfg cfg, int* __restrict__ defer_list,
-                                                                                int* __restrict__ defer_cnt) {
+                                                                                int* __restrict__ defer_cnt, const int* __restrict__ cam_of) {
   __shared__ MatchWarp2Smem<11> wsm[MW2_WARPS];
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const long long pair = (long long)blockIdx.x * MW2_WARPS + warp;
@@ -1052,6 +1060,7 @@ __global__ void __launch_bounds__(MW2_WARPS * 32, MINB) k_match_filter_batch_war
   const FeatTab ft = feattab_slice(base, b, Ncap, cfg.tstride);
   if (f >= Nper[b] || !ft.innov[f]) return;
   MatchJob jb;
+  if constexpr (CAMS) fr = batch_frame(fr, cam_of[b]);
   jb.tmap = nullptr; jb.frame_index = 0;
   jb.frame = fr.px; jb.fw = fr.w; jb.fh = fr.h; jb.fstride = fr.stride;
   jb.tmpl = ft.mpatch + (size_t)f * cfg.tstride;
@@ -1069,9 +1078,11 @@ __global__ void __launch_bounds__(MW2_WARPS * 32, MINB) k_match_filter_batch_war
 }
 
 // Batched filters, pass 1: one warp per (filter, feature); features that do not fit go to defer_list.
+template <bool CAMS>
 __global__ void __launch_bounds__(MW_WARPS * 32) k_match_filter_batch_warp(FeatTab base, int Ncap, const int* __restrict__ Nper, int B,
                                                                            FrameView fr, DevCfg cfg, int* __restrict__ defer_list,
-                                                                           int* __restrict__ defer_cnt, int warp_path) {
+                                                                           int* __restrict__ defer_cnt, int warp_path,
+                                                                           const int* __restrict__ cam_of) {
   __shared__ MatchWarpSmem wsm[MW_WARPS];
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const long long pair = (long long)blockIdx.x * MW_WARPS + warp;
@@ -1081,6 +1092,7 @@ __global__ void __launch_bounds__(MW_WARPS * 32) k_match_filter_batch_warp(FeatT
   if (f >= Nper[b] || !ft.innov[f]) return;
   const int w = cfg.window, w2 = w * w;
   MatchJob jb;
+  if constexpr (CAMS) fr = batch_frame(fr, cam_of[b]);
   jb.tmap = nullptr; jb.frame_index = 0;
   jb.frame = fr.px; jb.fw = fr.w; jb.fh = fr.h; jb.fstride = fr.stride;
   jb.tmpl = ft.mpatch + (size_t)f * cfg.tstride;
@@ -1113,10 +1125,12 @@ __global__ void __launch_bounds__(MW_WARPS * 32) k_match_filter_batch_warp(FeatT
   }
 }
 // pass 2: a persistent grid of CTAs works off the deferred (filter, feature) pairs with match_one
+template <bool CAMS>
 __global__ void __launch_bounds__(MATCH_THREADS) k_match_filter_batch_deferred(FeatTab base, int Ncap, FrameView fr, DevCfg cfg,
                                                                                const __grid_constant__ CUtensorMap tmap, int use_tma,
                                                                                const int* __restrict__ defer_list,
-                                                                               const int* __restrict__ defer_cnt) {
+                                                                               const int* __restrict__ defer_cnt,
+                                                                               const int* __restrict__ cam_of) {
   extern __shared__ __align__(128) unsigned char smem_raw[];
   const int n = *defer_cnt;
   unsigned phase = 0;
@@ -1125,7 +1139,8 @@ __global__ void __launch_bounds__(MATCH_THREADS) k_match_filter_batch_deferred(F
     const int pair = defer_list[i];
     const int b = pair / Ncap, f = pair - b * Ncap;
     const FeatTab ft = feattab_slice(base, b, Ncap, cfg.tstride);
-    match_filter_feature(ft, f, fr, cfg, smem_raw, use_tma ? &tmap : nullptr, &phase, first);
+    const int cam = (CAMS && cam_of) ? cam_of[b] : 0;
+    match_filter_feature(ft, f, CAMS ? batch_frame(fr, cam) : fr, cfg, smem_raw, use_tma ? &tmap : nullptr, &phase, first, false, cam);
     first = false;
     __syncthreads();
   }
@@ -1248,12 +1263,15 @@ void launch_match_filter(cudaStream_t st, FeatTab ft, int N, FrameView fr, const
 }
 
 void launch_match_filter_batch(cudaStream_t st, FeatTab base, int Ncap, const int* Nper, int B, FrameView fr, const DevCfg& cfg,
-                               const EkfTensorMap* tmap, int* defer_list, int* defer_cnt, long long* launches) {
+                               const EkfTensorMap* tmap, int* defer_list, int* defer_cnt, long long* launches, const int* cam_of) {
   if (B <= 0 || Ncap <= 0) return;
   static PerDeviceOnce once;   // opt in to the largest supported window once per device
   const size_t smem = match_smem_bytes(cfg.window, cfg.search_clamp);
-  if (once.ensure([] { return cudaFuncSetAttribute(k_match_filter_batch_deferred, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                                   (int)match_smem_bytes(MATCH_MAX_W, 20.0f)); }) != cudaSuccess) return;   // the error stays in cudaGetLastError() for the caller
+  if (once.ensure([] {
+        const int bytes = (int)match_smem_bytes(MATCH_MAX_W, 20.0f);
+        const cudaError_t e = cudaFuncSetAttribute(k_match_filter_batch_deferred<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes);
+        return e != cudaSuccess ? e : cudaFuncSetAttribute(k_match_filter_batch_deferred<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes);
+      }) != cudaSuccess) return;   // the error stays in cudaGetLastError() for the caller
   static const EkfTensorMap none{};
   const EkfTensorMap& tm = (tmap && tmap->ok) ? *tmap : none;
   // pass 1: a warp per (filter, feature) for small windows; pass 2: a persistent grid of CTAs for the deferred rest
@@ -1265,7 +1283,9 @@ void launch_match_filter_batch(cudaStream_t st, FeatTab base, int Ncap, const in
   if (warp_path >= 2 && cfg.window == 11 && cfg.search_clamp <= 20.0f) {
     const unsigned grid = (unsigned)((pairs + MW2_WARPS - 1) / MW2_WARPS);
     const int var = match_w2_variant();
-#define MW2_LAUNCH(MINB, TS, SL) k_match_filter_batch_warp2<MINB, TS, SL><<<grid, MW2_WARPS * 32, 0, st>>>(base, Ncap, Nper, B, fr, cfg, defer_list, defer_cnt)
+#define MW2_LAUNCH(MINB, TS, SL)                                                                                                        \
+  if (cam_of) k_match_filter_batch_warp2<MINB, TS, SL, true><<<grid, MW2_WARPS * 32, 0, st>>>(base, Ncap, Nper, B, fr, cfg, defer_list, defer_cnt, cam_of); \
+  else k_match_filter_batch_warp2<MINB, TS, SL, false><<<grid, MW2_WARPS * 32, 0, st>>>(base, Ncap, Nper, B, fr, cfg, defer_list, defer_cnt, cam_of)
     switch (var) {
       case 0: MW2_LAUNCH(2, false, false); break;
       case 2: MW2_LAUNCH(3, true, false); break;
@@ -1275,17 +1295,20 @@ void launch_match_filter_batch(cudaStream_t st, FeatTab base, int Ncap, const in
       default: MW2_LAUNCH(2, true, false); break;   // 1
     }
 #undef MW2_LAUNCH
-  } else
-    k_match_filter_batch_warp<<<(unsigned)((pairs + MW_WARPS - 1) / MW_WARPS), MW_WARPS * 32, 0, st>>>(base, Ncap, Nper, B, fr, cfg, defer_list, defer_cnt,
-                                                                                                       warp_path);
+  } else {
+    const unsigned grid = (unsigned)((pairs + MW_WARPS - 1) / MW_WARPS);
+    if (cam_of) k_match_filter_batch_warp<true><<<grid, MW_WARPS * 32, 0, st>>>(base, Ncap, Nper, B, fr, cfg, defer_list, defer_cnt, warp_path, cam_of);
+    else k_match_filter_batch_warp<false><<<grid, MW_WARPS * 32, 0, st>>>(base, Ncap, Nper, B, fr, cfg, defer_list, defer_cnt, warp_path, cam_of);
+  }
   int dev = 0, sms = 148;
   if (cudaGetDevice(&dev) == cudaSuccess) cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
   int per_sm = 4;   // persistent grid: as many CTAs as are resident at this shared-memory footprint
-  if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_match_filter_batch_deferred, MATCH_THREADS, smem) != cudaSuccess || per_sm < 1) {
+  auto* const deferred = cam_of ? k_match_filter_batch_deferred<true> : k_match_filter_batch_deferred<false>;   // the one launched
+  if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, deferred, MATCH_THREADS, smem) != cudaSuccess || per_sm < 1) {
     cudaGetLastError();
     per_sm = 4;
   }
-  k_match_filter_batch_deferred<<<sms * per_sm, MATCH_THREADS, smem, st>>>(base, Ncap, fr, cfg, as_cu(tm), tm.ok, defer_list, defer_cnt);
+  deferred<<<sms * per_sm, MATCH_THREADS, smem, st>>>(base, Ncap, fr, cfg, as_cu(tm), tm.ok, defer_list, defer_cnt, cam_of);
   *launches += 2;
 }
 
