@@ -105,6 +105,8 @@ SIGNATURES = {
     "ekf_batch_get_camera_frame": (_i, [_vp, _i, _vp, _P(_i), _P(_i)]),
     "ekf_batch_get_dt": (_i, [_vp, _vp]),
     "ekf_batch_set_detect_budget": (_i, [_vp, C.c_int64]),
+    "ekf_batch_set_intrinsics": (_i, [_vp, _vp]),
+    "ekf_batch_set_frame_sizes": (_i, [_vp, _vp]),
     "ekf_batch_step_controls": (_i, [_vp, _vp, _vp, _vp, _vp, _i]),
     "ekf_dist_load_nccl": (_i, [C.c_char_p]),
     "ekf_dist_unique_id": (_i, [_vp]),

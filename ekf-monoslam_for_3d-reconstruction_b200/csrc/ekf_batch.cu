@@ -26,6 +26,7 @@
 // Every stage evaluates the same expressions as the single-filter kernels (same device functions).
 #include <algorithm>
 #include <climits>
+#include <cmath>
 #include <cstdio>
 #include <string>
 #include <vector>
@@ -65,7 +66,17 @@ struct BatchView {
   double* xyz_y;        // [B][Ncap][3] its XYZ point
   int* xyz_count;       // [B] conversions pending (k_batch_compact resets it)
   int* patchnumbre;     // [B] real_index of the filter's next new feature (VSlamFilter::patchnumbre)
+  const CamParams* cam; // [B] intrinsics of each filter (ekf_batch_set_intrinsics); null: every filter uses cfg.cam
 };
+
+// The intrinsics filter b projects, linearises and unprojects with.  INTR: the batch has a table (kernels that project take it
+// as a template parameter, so that a batch without one runs the code it ran before).  A reference, so that the fields load
+// where they are used.
+template <bool INTR>
+__device__ __forceinline__ const CamParams& filter_cam(const BatchView& bv, const DevCfg& cfg, int b) {
+  if constexpr (INTR) return bv.cam[b];
+  else return cfg.cam;
+}
 
 // convert2XYZ_ifLinear's decision (V:741-772, xyz_linear_decide) for feature i = lane of filter b, if `eligible` and still
 // in inverse depth.  Called by the whole of warp 0 (N <= BNCAP = 32); lane 0 stores the filter's count.
@@ -109,6 +120,7 @@ struct BatchStepIn {
   const double* dT;        // [n_cameras] each camera's dT
   const double* ctl;       // [B][6] dv, dw of each filter (ekf_batch_step_controls)
   const int* vcontrol;     // [B]
+  const int* fsize;        // [n_cameras][4] frame sizes (ekf_batch_set_frame_sizes): the gate uses [2], [3] of the filter's camera
 };
 __device__ __forceinline__ double step_dT(const BatchStepIn& in, int b, double dT) {
   return in.dT ? in.dT[in.cam_of ? in.cam_of[b] : 0] : dT;
@@ -118,6 +130,7 @@ __device__ __forceinline__ double step_dT(const BatchStepIn& in, int b, double d
 // predict for one filter per CTA: same arithmetic as k_predict_cov / k_predict_features / k_predict_S2
 // ------------------------------------------------------------------------------------------------
 #define BPRED_THREADS 128
+template <bool INTR>
 __global__ void __launch_bounds__(BPRED_THREADS, 4) k_batch_predict(BatchView bv, FrameView fr, DevCfg cfg, double dT, double3 dv,
                                                                  double3 dw, int vcontrol, BatchStepIn in) {
   __shared__ double F[169], C[169], T[169], Q[169], cam[13];
@@ -197,9 +210,14 @@ __global__ void __launch_bounds__(BPRED_THREADS, 4) k_batch_predict(BatchView bv
       for (int c = 0; c < 13; ++c) cm[c] = cam[c];
       double qc[4] = {cm[3], -cm[4], -cm[5], -cm[6]}, Rcw[9], hi[2], Hc[26], hcz;
       d_quat2rot(qc, Rcw);
-      d_feature_hH(cfg.cam, fs, coding, cm, qc, Rcw, hi, Hc, &hcz);
+      d_feature_hH(filter_cam<INTR>(bv, cfg, b), fs, coding, cm, qc, Rcw, hi, Hc, &hcz);
       const int half = cfg.window / 2;
-      ok = (hi[0] > half && hi[1] > half && hi[0] < fr.w - half && hi[1] < fr.h - half) && (hcz >= 0);
+      int fw = fr.w, fh = fr.h;
+      if (in.fsize) {
+        const int c = in.cam_of ? in.cam_of[b] : 0;
+        fw = in.fsize[4 * c + 2]; fh = in.fsize[4 * c + 3];
+      }
+      ok = (hi[0] > half && hi[1] > half && hi[0] < fw - half && hi[1] < fh - half) && (hcz >= 0);
       if (ok) {
         ft.h[2 * i] = hi[0]; ft.h[2 * i + 1] = hi[1];
         for (int c = 0; c < 26; ++c) ft.Hc[26 * i + c] = Hc[c];
@@ -257,7 +275,7 @@ __global__ void __launch_bounds__(BPRED_THREADS, 4) k_batch_predict(BatchView bv
 // ------------------------------------------------------------------------------------------------
 #define BBLUR_WARPS 4
 // NC: feature capacity (BNCAP or BNCAP_L); warp 0 takes the decisions 32 features at a time, in ascending order.
-template <int NC>
+template <int NC, bool INTR>
 __global__ void __launch_bounds__(BBLUR_WARPS * 32) k_batch_predict_blur(BatchView bv, DevCfg cfg, double dT, int* __restrict__ out,
                                                                      BatchStepIn in) {
   __shared__ int s_feat[NC], s_rows[NC], s_cols[NC], s_nblur;
@@ -284,7 +302,7 @@ __global__ void __launch_bounds__(BBLUR_WARPS * 32) k_batch_predict_blur(BatchVi
         const int pos = ft.pos[f], coding = ft.coding[f];
         double fs[6];
         for (int c = 0; c < (coding ? 3 : 6); ++c) fs[c] = mu[pos + c];
-        blur_displacement(cfg.cam, fs, coding, rb, Rb, ft.h[2 * f], ft.h[2 * f + 1], &ddx, &ddy);
+        blur_displacement(filter_cam<INTR>(bv, cfg, b), fs, coding, rb, Rb, ft.h[2 * f], ft.h[2 * f + 1], &ddx, &ddy);
         d = blur_decide(ddx, ddy, cfg.kernel_min_size, &krows, &kcols);
       }
       const unsigned blur = __ballot_sync(0xffffffffu, d > 0), big = __ballot_sync(0xffffffffu, d < 0);
@@ -594,7 +612,7 @@ __device__ void cta_stacked_update(const UpdSmem& sm, double* __restrict__ Sigma
 }
 
 // PLANE: forsePlane (ekf_batch_set_force_plane), a separate instantiation so that the plane-off kernel is the same code as without it.
-template <bool PLANE>
+template <bool PLANE, bool INTR>
 __global__ void __launch_bounds__(BUPD_THREADS, 1) k_batch_update(BatchView bv, DevCfg cfg, const uint32_t* __restrict__ picks,
                                                                   int n_picks, double* __restrict__ out_mu14,
                                                                   double* __restrict__ out_S14, int* __restrict__ out_stats,
@@ -619,7 +637,13 @@ __global__ void __launch_bounds__(BUPD_THREADS, 1) k_batch_update(BatchView bv, 
   DevCtl* ctl = bv.ctl + b;
   if (tid == 0) ctl->chol_fail = 0;
   // 1-point RANSAC, low-innovation update
-  cta_ransac(Sigma, ld, n, mu, ft, N, ctl, cfg, picks, n_picks, sm.mu_i, sm.ibuf);
+  if constexpr (INTR) {   // a configuration with the filter's intrinsics for cta_ransac; the Hi rescue below reads the row itself
+    DevCfg rcfg = cfg;
+    rcfg.cam = bv.cam[b];
+    cta_ransac(Sigma, ld, n, mu, ft, N, ctl, rcfg, picks, n_picks, sm.mu_i, sm.ibuf);
+  } else {
+    cta_ransac(Sigma, ld, n, mu, ft, N, ctl, cfg, picks, n_picks, sm.mu_i, sm.ibuf);
+  }
   __syncthreads();
   const int n_li = ctl->n_li;
   if (n_li > 0) cta_stacked_update(sm, Sigma, ld, n, mu, ft, n_li, cfg, ctl);
@@ -634,7 +658,7 @@ __global__ void __launch_bounds__(BUPD_THREADS, 1) k_batch_update(BatchView bv, 
       for (int c = 0; c < 3; ++c) r[c] = ctl->cam_old[c];
       qc[0] = ctl->cam_old[3]; qc[1] = -ctl->cam_old[4]; qc[2] = -ctl->cam_old[5]; qc[3] = -ctl->cam_old[6];
       d_quat2rot(qc, Rcw);
-      d_feature_hH(cfg.cam, fs, coding, r, qc, Rcw, hi, Hc, &hcz);
+      d_feature_hH(filter_cam<INTR>(bv, cfg, b), fs, coding, r, qc, Rcw, hi, Hc, &hcz);
       ft.h[2 * i] = hi[0]; ft.h[2 * i + 1] = hi[1];
       for (int c = 0; c < 26; ++c) ft.Hc[26 * i + c] = Hc[c];
       double Tm[26];
@@ -1045,7 +1069,7 @@ static __device__ __noinline__ void cl_hi_rescue(double* Sigma, int ld, const do
   if (tid == 0) { ctl->n_hi = nh; ctl->k_rows = 2 * nh; }
 }
 
-template <bool PLANE>
+template <bool PLANE, bool INTR>
 __global__ void __launch_bounds__(BUPD_THREADS, 1) k_batch_update_cluster(BatchView bv, DevCfg cfg, const uint32_t* __restrict__ picks,
                                                                           int n_picks, double* __restrict__ out_mu14,
                                                                           double* __restrict__ out_S14, int* __restrict__ out_stats,
@@ -1069,6 +1093,7 @@ __global__ void __launch_bounds__(BUPD_THREADS, 1) k_batch_update_cluster(BatchV
   double* mu = bv.mu + (size_t)b * ld;
   const FeatTab ft = feattab_slice(bv.ft, b, bv.Ncap, bv.tstride);
   DevCtl* ctl = bv.ctl + b;
+  if constexpr (INTR) cfg.cam = bv.cam[b];   // every device function below projects with the filter's intrinsics
   for (int i = tid; i < BSTRIP; i += BUPD_THREADS) sm.mu_i[i] = 0.0;
   if (rank == 0) {   // 1-point RANSAC: mu_i (n <= 782) in the Cholesky workspace, the candidates (N <= 128) in ibuf
     if (tid == 0) ctl->chol_fail = 0;
@@ -1336,7 +1361,7 @@ __global__ void __launch_bounds__(BNCAP_L) k_batch_xyz_decide_large(BatchView bv
 // BADD_THREADS at a time and the decisions one thread per feature.  Templates come from frame cam_of[b] of the stack fr
 // (cam_of null: frame 0).
 #define BADD_THREADS 256
-template <bool LARGE>
+template <bool LARGE, bool INTR>
 __global__ void __launch_bounds__(BADD_THREADS) k_batch_add(BatchView bv, FrameView fr, DevCfg cfg, const float* __restrict__ xy,
                                                             const int* __restrict__ cnt, int one, float u, float v, int decide,
                                                             const int* __restrict__ cam_of) {
@@ -1355,7 +1380,7 @@ __global__ void __launch_bounds__(BADD_THREADS) k_batch_add(BatchView bv, FrameV
   for (int j = 0; j < k; ++j) {
     const float px = one >= 0 ? u : xy[(size_t)b * 2 * CS + 2 * j];
     const float py = one >= 0 ? v : xy[(size_t)b * 2 * CS + 2 * j + 1];
-    if (tid == 0) add_feature_jacobians(cfg.cam, mu, px, py, cfg.rho_0, A, Ap, fnew);
+    if (tid == 0) add_feature_jacobians(filter_cam<INTR>(bv, cfg, b), mu, px, py, cfg.rho_0, A, Ap, fnew);
     __syncthreads();
     if constexpr (LARGE) {
       for (int r = tid; r < n; r += BADD_THREADS) add_feature_cross(Sigma, ld, n, r, A);
@@ -1503,6 +1528,11 @@ struct ekf_batch {
   int* cam_dev = nullptr;                       // [B] camera of each filter; null with one camera
   std::vector<int> cam_host;                    // [B] the same on the host
   std::vector<double> cam_dT, cam_ts;           // [n_cam] each camera's dT / old_ts (captureNewFrame's clock)
+  std::vector<int> size_in;                     // [n_cam][2] input frame sizes (ekf_batch_set_frame_sizes); empty: the whole slot
+  std::vector<int> fsize_host;                  // [n_cam][4] in w, in h, resized w, h of the last capture with sizes (fsize_dev)
+  int* fsize_dev = nullptr;
+  bool fsize_on = false;                        // the captured stack has per-camera sizes
+  CamParams* intr_dev = nullptr;                // [B] intrinsics of each filter (ekf_batch_set_intrinsics); bv.cam, null without
   int* det_slot = nullptr;                      // [n_cam] position of each camera among those a detection asks from, or -1
   int* h_det_slot = nullptr;                    // pinned
   size_t det_budget = (size_t)1 << 30;          // scratch of one chunk of cameras of the per-camera detector
@@ -1577,7 +1607,7 @@ int ekf_batch_destroy(ekf_batch* b) {
   cudaFree(b->match_defer);
   cudaFree(b->scratch); cudaFree(b->frame); cudaFree(b->raw); cudaFree(b->picks_dev); cudaFree(b->out_mu14); cudaFree(b->out_S14);
   cudaFree(b->out_stats); cudaFree(b->stage_mu14); cudaFree(b->bv.patchnumbre);
-  cudaFree(b->cam_dev); cudaFree(b->det_slot); cudaFree(b->step_dev);
+  cudaFree(b->cam_dev); cudaFree(b->det_slot); cudaFree(b->step_dev); cudaFree(b->intr_dev); cudaFree(b->fsize_dev);
   if (b->h_det_slot) cudaFreeHost(b->h_det_slot);
   if (b->step_host) cudaFreeHost(b->step_host);
   batch_detect_free(b->det);
@@ -1642,23 +1672,25 @@ static int batch_create(const ekf_config* cfg, int n_filters, int feature_capaci
   TRY(cudaSetDevice(device))
   TRY(cudaStreamCreateWithFlags(&b->own_stream, cudaStreamNonBlocking))
   b->stream = b->own_stream;
-  TRY(cudaFuncSetAttribute(k_batch_update<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kUpdSmemBytes))
-  TRY(cudaFuncSetAttribute(k_batch_update<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kUpdSmemBytes))
+  for (void* k : {(void*)k_batch_update<false, false>, (void*)k_batch_update<true, false>, (void*)k_batch_update<false, true>,
+                  (void*)k_batch_update<true, true>})
+    TRY(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kUpdSmemBytes))
   if (large) {
-    TRY(cudaFuncSetAttribute(k_batch_update_cluster<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kUpdSmemBytes))
-    TRY(cudaFuncSetAttribute(k_batch_update_cluster<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kUpdSmemBytes))
+    void* const cl[4] = {(void*)k_batch_update_cluster<false, false>, (void*)k_batch_update_cluster<true, false>,
+                         (void*)k_batch_update_cluster<false, true>, (void*)k_batch_update_cluster<true, true>};
+    for (void* k : cl) TRY(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kUpdSmemBytes))
     cudaLaunchAttribute attr[1];
-    for (int plane = 0; plane < 2; ++plane) {
+    for (int i = 0; i < 4; ++i) {   // forsePlane x intrinsics table
       const cudaLaunchConfig_t lc = cluster_config(1, b->cl_ctas, nullptr, attr);
       int ncl = 0;
-      TRY(cudaOccupancyMaxActiveClusters(&ncl, plane ? (void*)k_batch_update_cluster<true> : (void*)k_batch_update_cluster<false>, &lc))
+      TRY(cudaOccupancyMaxActiveClusters(&ncl, cl[i], &lc))
       if (ncl < 1) {
         fprintf(stderr, "ekf_batch_create_large: the device cannot hold one cluster of %d CTAs with %zu bytes of shared memory each\n",
                 b->cl_ctas, kUpdSmemBytes);
         ekf_batch_destroy(b);
         return EKF_ERR_UNSUPPORTED;
       }
-      b->cl_resident = plane ? std::min(b->cl_resident, ncl) : ncl;
+      b->cl_resident = i ? std::min(b->cl_resident, ncl) : ncl;
     }
   }  const size_t Bn = (size_t)n_filters, cap = Bn * feature_capacity;
   BatchView& v = b->bv;
@@ -1685,7 +1717,7 @@ static int batch_create(const ekf_config* cfg, int n_filters, int feature_capaci
   TRY(cudaMallocHost((void**)&b->h_stats, sizeof(int) * Bn * EKF_BATCH_STAT_FIELDS))
   TRY(cudaMallocHost((void**)&b->h_n, sizeof(int) * Bn)) TRY(cudaMallocHost((void**)&b->h_N, sizeof(int) * Bn))
   TRY(cudaMallocHost((void**)&b->h_xyz_count, sizeof(int) * Bn))
-  TRY(balloc(&b->det_slot, 1)) TRY(cudaMallocHost((void**)&b->h_det_slot, sizeof(int)))
+  TRY(balloc(&b->det_slot, 2)) TRY(cudaMallocHost((void**)&b->h_det_slot, sizeof(int) * 2))
   TRY(cudaMemsetAsync(v.Sigma, 0, sizeof(double) * Bn * v.sstride, b->stream))
   TRY(cudaMemsetAsync(v.mu, 0, sizeof(double) * Bn * b->ld, b->stream))
   TRY(cudaMemsetAsync(v.ctl, 0, sizeof(DevCtl) * Bn, b->stream))
@@ -1817,11 +1849,34 @@ int ekf_batch_set_camera_states(ekf_batch* b, const double* mu14) {
 // the staging buffer `raw`, a chunk of cameras at a time so that `raw` stays within kRawBudget (or one frame).  n frames
 // (n == b->n_cam), frame c at img + c * height * stride; stamps[c] (stamps may be null: no stamps).
 static constexpr size_t kRawBudget = (size_t)256 << 20;
+// frame z of a stack of dw x dh slots: every pixel outside the camera's fsize[4z + 2] x fsize[4z + 3] becomes 0
+__global__ void k_batch_zero_pads(uint8_t* __restrict__ frame, int dw, int dstride, int dh, const int* __restrict__ fsize) {
+  const int x = blockIdx.x * blockDim.x + threadIdx.x, y = blockIdx.y;
+  if (x >= dw) return;
+  const int* q = fsize + 4 * blockIdx.z;
+  if (x >= q[2] || y >= q[3]) frame[((size_t)blockIdx.z * dh + y) * dstride + x] = 0;
+}
 static int bcapture(ekf_batch* b, const uint8_t* img, int width, int height, int stride, int channels, const double* stamps, bool dev) {
   if (!b || !img || width < 8 || height < 8 || stride < width * channels) return EKF_ERR_ARG;
   const int scale = b->cfg.scale, n = b->n_cam;
   const int dw = width / scale, dh = height / scale;   // cv::Size(width / scale, height / scale), integer division
   if (dw < 8 || dh < 8) return bfail(b, EKF_ERR_ARG, "resized frame smaller than 8 x 8 pixels");
+  // frame sizes per camera: camera c is the top-left size_in[c] of its slot, resized to size_in[c] / scale
+  std::vector<int> fs;
+  bool pads = false;
+  if (!b->size_in.empty()) {
+    fs.resize((size_t)4 * n);
+    for (int c = 0; c < n; ++c) {
+      const int wc = b->size_in[2 * c], hc = b->size_in[2 * c + 1];
+      if (wc > width || hc > height)
+        return bfail(b, EKF_ERR_ARG, "camera " + std::to_string(c) + " is larger than the captured " + std::to_string(width) + " x " +
+                                         std::to_string(height) + " slot");
+      if (wc / scale < 8 || hc / scale < 8)
+        return bfail(b, EKF_ERR_ARG, "camera " + std::to_string(c) + ": resized frame smaller than 8 x 8 pixels");
+      fs[4 * c] = wc; fs[4 * c + 1] = hc; fs[4 * c + 2] = wc / scale; fs[4 * c + 3] = hc / scale;
+      pads = pads || fs[4 * c + 2] < dw || fs[4 * c + 3] < dh;
+    }
+  }
   BCHECK(cudaSetDevice(b->device));
   for (int c = 0; stamps && c < n; ++c) {
     if (stamps[c] >= 0) {
@@ -1831,6 +1886,12 @@ static int bcapture(ekf_batch* b, const uint8_t* img, int width, int height, int
   }
   const int dstride = (dw + 15) & ~15;
   const size_t fstep = (size_t)dstride * dh, need = fstep * n;
+  if (!fs.empty() && fs != b->fsize_host) {   // the table goes up when the sizes or the scale change, not per capture
+    if (!b->fsize_dev) BCHECK(balloc(&b->fsize_dev, 4 * b->n_cam));
+    b->fsize_host = fs;
+    BCHECK(cudaMemcpyAsync(b->fsize_dev, b->fsize_host.data(), sizeof(int) * fs.size(), cudaMemcpyHostToDevice, b->stream));
+  }
+  b->fsize_on = !fs.empty();
   if (need > b->frame_cap) {
     BCHECK(cudaStreamSynchronize(b->stream));
     cudaFree(b->frame);
@@ -1863,9 +1924,18 @@ static int bcapture(ekf_batch* b, const uint8_t* img, int width, int height, int
         src = b->raw; sstride = width * channels;
       }
       launch_capture_resize_gray(b->stream, src, width, height, sstride, channels, b->frame + (size_t)c0 * fstep, dw, dh, dstride,
-                                 &b->launches, k);
+                                 &b->launches, k, b->fsize_on ? b->fsize_dev + 4 * c0 : nullptr);
       BCHECK(cudaGetLastError());
     }
+  }
+  if (pads) {   // results must not depend on the bytes of a slot outside its camera's frame: zero them, one launch over the stack
+    for (int c0 = 0; c0 < n; c0 += 65535) {
+      const int k = std::min(65535, n - c0);
+      k_batch_zero_pads<<<dim3((dw + 255) / 256, dh, k), 256, 0, b->stream>>>(b->frame + (size_t)c0 * fstep, dw, dstride, dh,
+                                                                            b->fsize_dev + 4 * c0);
+      b->launches += 1;
+    }
+    BCHECK(cudaGetLastError());
   }
   if (b->fv.px != b->frame || b->fv.w != dw || b->fv.h != dh || b->fv.stride != dstride)
     match_make_tensor_map(&b->frame_map, b->frame, dw, dh, dstride, n, b->cfg.window_size, (int)b->cfg.search_clamp);
@@ -1904,20 +1974,63 @@ int ekf_batch_set_cameras(ekf_batch* b, int n_cameras, const int32_t* camera_of)
   }
   BCHECK(cudaSetDevice(b->device));
   BCHECK(cudaStreamSynchronize(b->stream));
-  cudaFree(b->cam_dev); cudaFree(b->det_slot); cudaFreeHost(b->h_det_slot);
-  b->cam_dev = nullptr; b->det_slot = nullptr; b->h_det_slot = nullptr;
+  cudaFree(b->cam_dev); cudaFree(b->det_slot); cudaFreeHost(b->h_det_slot); cudaFree(b->fsize_dev);
+  b->cam_dev = nullptr; b->det_slot = nullptr; b->h_det_slot = nullptr; b->fsize_dev = nullptr;
+  b->fsize_host.clear();
   if (n_cameras > 1) {
     BCHECK(balloc(&b->cam_dev, b->B));
     BCHECK(cudaMemcpy(b->cam_dev, cam.data(), sizeof(int) * b->B, cudaMemcpyHostToDevice));
   }
-  BCHECK(balloc(&b->det_slot, n_cameras));
-  BCHECK(cudaMallocHost((void**)&b->h_det_slot, sizeof(int) * n_cameras));
+  BCHECK(balloc(&b->det_slot, 2 * n_cameras));
+  BCHECK(cudaMallocHost((void**)&b->h_det_slot, sizeof(int) * 2 * n_cameras));
+  b->size_in.clear();   // sizes are per camera: back to the whole slot
+  b->fsize_on = false;
   b->cam_host = cam;
   b->n_cam = n_cameras;
   const double dT = b->cam_dT[0], ts = b->cam_ts[0];
   b->cam_dT.assign(n_cameras, dT); b->cam_ts.assign(n_cameras, ts);
   b->have_frame = false;
   b->fv = FrameView{nullptr, 0, 0, 0};   // the next capture encodes the stack's tensor map
+  return EKF_OK;
+}
+
+static_assert(sizeof(CamParams) == 9 * sizeof(double), "a row of ekf_batch_set_intrinsics is one CamParams");
+int ekf_batch_set_intrinsics(ekf_batch* b, const double* cam) {
+  if (!b) return EKF_ERR_ARG;
+  if (cam) {
+    for (int f = 0; f < b->B; ++f) {
+      const double* r = cam + 9 * (size_t)f;
+      bool ok = r[0] > 0 && r[1] > 0;
+      for (int c = 0; c < 9; ++c) ok = ok && std::isfinite(r[c]);
+      if (!ok) return bfail(b, EKF_ERR_ARG, "intrinsics of filter " + std::to_string(f) + ": non-finite, or fx / fy <= 0");
+    }
+  }
+  BCHECK(cudaSetDevice(b->device));
+  BCHECK(cudaStreamSynchronize(b->stream));   // work in flight may still read the table
+  if (!cam) {
+    cudaFree(b->intr_dev);
+    b->intr_dev = nullptr;
+    b->bv.cam = nullptr;
+    return EKF_OK;
+  }
+  if (!b->intr_dev) BCHECK(balloc(&b->intr_dev, b->B));
+  BCHECK(cudaMemcpyAsync(b->intr_dev, cam, sizeof(CamParams) * b->B, cudaMemcpyHostToDevice, b->stream));
+  BCHECK(cudaStreamSynchronize(b->stream));   // the caller's array is free once the call returns
+  b->bv.cam = b->intr_dev;
+  return EKF_OK;
+}
+
+int ekf_batch_set_frame_sizes(ekf_batch* b, const int32_t* wh) {
+  if (!b) return EKF_ERR_ARG;
+  if (wh) {
+    for (int c = 0; c < b->n_cam; ++c)
+      if (wh[2 * c] < 1 || wh[2 * c + 1] < 1) return bfail(b, EKF_ERR_ARG, "frame size of camera " + std::to_string(c) + " is not positive");
+    b->size_in.assign(wh, wh + 2 * (size_t)b->n_cam);
+  } else {
+    b->size_in.clear();
+  }
+  b->fsize_on = false;
+  b->have_frame = false;   // the sizes hold from the next capture on
   return EKF_OK;
 }
 
@@ -1930,10 +2043,11 @@ int ekf_batch_set_detect_budget(ekf_batch* b, int64_t bytes) {
 int ekf_batch_get_camera_frame(ekf_batch* b, int camera, uint8_t* out, int* width, int* height) {   // returnGrayImg (vslamRansac.cpp:1364)
   if (!b || !width || !height || camera < 0 || camera >= b->n_cam) return EKF_ERR_ARG;
   if (!b->have_frame) return bfail(b, EKF_ERR_STATE, "no frame captured");
-  *width = b->fv.w; *height = b->fv.h;
+  const int w = b->fsize_on ? b->fsize_host[4 * camera + 2] : b->fv.w, h = b->fsize_on ? b->fsize_host[4 * camera + 3] : b->fv.h;
+  *width = w; *height = h;
   if (out) {
     BCHECK(cudaSetDevice(b->device));
-    BCHECK(cudaMemcpy2DAsync(out, b->fv.w, b->frame + (size_t)camera * b->fv.h * b->fv.stride, b->fv.stride, b->fv.w, b->fv.h,
+    BCHECK(cudaMemcpy2DAsync(out, w, b->frame + (size_t)camera * b->fv.h * b->fv.stride, b->fv.stride, w, h,
                              cudaMemcpyDeviceToHost, b->stream));
     BCHECK(cudaStreamSynchronize(b->stream));
   }
@@ -2004,7 +2118,7 @@ static constexpr size_t kDetBytesPerPixel = 44;
 static int batch_detect(ekf_batch* b, const int* num, const int* hnum, int num_stride, int cap_mode) {
   cudaStream_t st = b->stream;
   const size_t npx = (size_t)b->fv.w * b->fv.h;
-  if (b->n_cam == 1) {
+  if (b->n_cam == 1 && !b->fsize_on) {
     BCHECK(batch_detect_reserve(b->det, npx, b->B, b->cstride));
     BCHECK(launch_batch_detect(st, b->det, b->fv, b->bv.ft.center, b->bv.N, b->Ncap, b->B, b->cfg.window_size, num, num_stride, cap_mode,
                                b->cstride, b->det_xy, b->det_n, &b->launches));
@@ -2019,11 +2133,14 @@ static int batch_detect(ekf_batch* b, const int* num, const int* hnum, int num_s
   const int n_req = (int)cams.size();
   const size_t fit = std::min<size_t>(b->det_budget / (kDetBytesPerPixel * npx), (size_t)INT_MAX / npx);
   const int chunk = (int)std::max<size_t>(1, std::min<size_t>(std::max(n_req, 1), fit));
-  BCHECK(cudaMemcpyAsync(b->det_slot, b->h_det_slot, sizeof(int) * b->n_cam, cudaMemcpyHostToDevice, st));
+  std::copy(cams.begin(), cams.end(), b->h_det_slot + b->n_cam);
+  BCHECK(cudaMemcpyAsync(b->det_slot, b->h_det_slot, sizeof(int) * (b->n_cam + n_req), cudaMemcpyHostToDevice, st));
   if (n_req > 0) BCHECK(batch_detect_reserve_cams(b->det, npx, chunk, b->B, b->cstride));
   else BCHECK(batch_detect_reserve(b->det, 0, b->B, b->cstride));   // the per-filter buffers only
   BCHECK(launch_batch_detect_cams(st, b->det, b->fv, cams.data(), n_req, chunk, b->cam_dev, b->det_slot, b->bv.ft.center, b->bv.N, b->Ncap,
-                                  b->B, b->cfg.window_size, num, num_stride, cap_mode, b->cstride, b->det_xy, b->det_n, &b->launches));
+                                  b->B, b->cfg.window_size, num, num_stride, cap_mode, b->cstride, b->det_xy, b->det_n, &b->launches,
+                                  b->fsize_on ? b->fsize_dev : nullptr, b->fsize_on ? b->fsize_host.data() : nullptr,
+                                  b->det_slot + b->n_cam));
   return EKF_OK;
 }
 
@@ -2033,8 +2150,9 @@ static int batch_topup(ekf_batch* b, const int* num, const int* hnum, int num_st
   cudaStream_t st = b->stream;
   const int rc = batch_detect(b, num, hnum, num_stride, 1);
   if (rc) return rc;
-  if (b->large) k_batch_add<true><<<b->B, BADD_THREADS, 0, st>>>(b->bv, b->fv, b->dcfg, b->det_xy, b->det_n, -1, 0.0f, 0.0f, decide, b->cam_dev);
-  else k_batch_add<false><<<b->B, BADD_THREADS, 0, st>>>(b->bv, b->fv, b->dcfg, b->det_xy, b->det_n, -1, 0.0f, 0.0f, decide, b->cam_dev);
+  auto* const add = b->large ? (b->bv.cam ? k_batch_add<true, true> : k_batch_add<true, false>)
+                             : (b->bv.cam ? k_batch_add<false, true> : k_batch_add<false, false>);
+  add<<<b->B, BADD_THREADS, 0, st>>>(b->bv, b->fv, b->dcfg, b->det_xy, b->det_n, -1, 0.0f, 0.0f, decide, b->cam_dev);
   b->launches += 1;
   BCHECK(cudaGetLastError());
   return EKF_OK;
@@ -2063,7 +2181,7 @@ static int batch_step(ekf_batch* b, const double* dv, const double* dw, int vcon
   BCHECK(cudaSetDevice(b->device));
   cudaStream_t st = b->stream;
   const size_t Bn = (size_t)b->B;
-  BatchStepIn in{b->cam_dev, nullptr, nullptr, nullptr};
+  BatchStepIn in{b->cam_dev, nullptr, nullptr, nullptr, b->fsize_on ? b->fsize_dev : nullptr};
   const uint32_t* picks_dev = b->picks_dev;
   const double z3[3] = {0, 0, 0};
   const double* a = (dv && !per_filter) ? dv : z3; const double* w = (dw && !per_filter) ? dw : z3;
@@ -2107,26 +2225,30 @@ static int batch_step(ekf_batch* b, const double* dv, const double* dw, int vcon
     picks_dev = reinterpret_cast<const uint32_t*>(reinterpret_cast<const int*>(dd + n_dT + n_ctl) + n_vc);
   }
   BCHECK(cudaEventRecord(b->ev[0], st));
-  k_batch_predict<<<b->B, BPRED_THREADS, 0, st>>>(b->bv, b->fv, b->dcfg, b->cam_dT[0], make_double3(a[0], a[1], a[2]),
-                                                   make_double3(w[0], w[1], w[2]), vcontrol, in);
+  auto* const predict = b->bv.cam ? k_batch_predict<true> : k_batch_predict<false>;
+  predict<<<b->B, BPRED_THREADS, 0, st>>>(b->bv, b->fv, b->dcfg, b->cam_dT[0], make_double3(a[0], a[1], a[2]),
+                                           make_double3(w[0], w[1], w[2]), vcontrol, in);
   b->launches += 1;
   if (b->blur) {   // matching_patch <- blurred patch where the prediction moves far enough (k_batch_predict copied patch)
-    if (b->large) k_batch_predict_blur<BNCAP_L><<<b->B, BBLUR_WARPS * 32, 0, st>>>(b->bv, b->dcfg, b->cam_dT[0], b->blur_out, in);
-    else k_batch_predict_blur<BNCAP><<<b->B, BBLUR_WARPS * 32, 0, st>>>(b->bv, b->dcfg, b->cam_dT[0], b->blur_out, in);
+    auto* const blur = b->large ? (b->bv.cam ? k_batch_predict_blur<BNCAP_L, true> : k_batch_predict_blur<BNCAP_L, false>)
+                                : (b->bv.cam ? k_batch_predict_blur<BNCAP, true> : k_batch_predict_blur<BNCAP, false>);
+    blur<<<b->B, BBLUR_WARPS * 32, 0, st>>>(b->bv, b->dcfg, b->cam_dT[0], b->blur_out, in);
     b->launches += 1;
   }
   BCHECK(cudaEventRecord(b->ev[1], st));
   launch_match_filter_batch(st, b->bv.ft, b->Ncap, b->bv.N, b->B, b->fv, b->dcfg, &b->frame_map, b->match_defer,
-                            b->match_defer + (size_t)b->B * b->Ncap, &b->launches, b->cam_dev);
+                            b->match_defer + (size_t)b->B * b->Ncap, &b->launches, b->cam_dev, b->fsize_on ? b->fsize_dev : nullptr);
   BCHECK(cudaEventRecord(b->ev[2], st));
   if (b->large) {   // one cluster of cl_ctas CTAs per filter
     cudaLaunchAttribute attr[1];
     const cudaLaunchConfig_t lc = cluster_config(b->B, b->cl_ctas, st, attr);
-    auto* const update = b->cfg.forsePlane ? k_batch_update_cluster<true> : k_batch_update_cluster<false>;
+    auto* const update = b->cfg.forsePlane ? (b->bv.cam ? k_batch_update_cluster<true, true> : k_batch_update_cluster<true, false>)
+                                           : (b->bv.cam ? k_batch_update_cluster<false, true> : k_batch_update_cluster<false, false>);
     BCHECK(cudaLaunchKernelEx(&lc, update, b->bv, b->dcfg, picks_dev, n_picks, b->out_mu14, b->out_S14,
                               b->out_stats, (int)b->cfg.min_features, (int)b->cfg.max_features, (int)b->cfg.xyz_conversion));
   } else {
-    auto* const update = b->cfg.forsePlane ? k_batch_update<true> : k_batch_update<false>;
+    auto* const update = b->cfg.forsePlane ? (b->bv.cam ? k_batch_update<true, true> : k_batch_update<true, false>)
+                                           : (b->bv.cam ? k_batch_update<false, true> : k_batch_update<false, false>);
     update<<<b->B, BUPD_THREADS, kUpdSmemBytes, st>>>(b->bv, b->dcfg, picks_dev, n_picks, b->out_mu14, b->out_S14,
                                                       b->out_stats, b->cfg.min_features, b->cfg.max_features,
                                                       b->cfg.xyz_conversion);
@@ -2289,10 +2411,12 @@ int ekf_batch_add_feature(ekf_batch* b, int f, float u, float v) {
   const int half = b->cfg.window_size / 2;
   // isInsideImage (vslamRansac.cpp:314,1644-1652), as ekf_add_feature
   const double x = (double)u, y = (double)v;
-  if (!(x > half && y > half && x < b->fv.w - half && y < b->fv.h - half)) return 0;
+  const int c = b->cam_host[f], fw = b->fsize_on ? b->fsize_host[4 * c + 2] : b->fv.w, fh = b->fsize_on ? b->fsize_host[4 * c + 3] : b->fv.h;
+  if (!(x > half && y > half && x < fw - half && y < fh - half)) return 0;
   if (b->h_N[f] >= b->Ncap || b->h_n[f] + 6 > b->ncap) return bfail(b, EKF_ERR_CAPACITY, "feature capacity exceeded");
-  if (b->large) k_batch_add<true><<<1, BADD_THREADS, 0, b->stream>>>(b->bv, b->fv, b->dcfg, nullptr, nullptr, f, u, v, 0, b->cam_dev);
-  else k_batch_add<false><<<1, BADD_THREADS, 0, b->stream>>>(b->bv, b->fv, b->dcfg, nullptr, nullptr, f, u, v, 0, b->cam_dev);
+  auto* const add = b->large ? (b->bv.cam ? k_batch_add<true, true> : k_batch_add<true, false>)
+                             : (b->bv.cam ? k_batch_add<false, true> : k_batch_add<false, false>);
+  add<<<1, BADD_THREADS, 0, b->stream>>>(b->bv, b->fv, b->dcfg, nullptr, nullptr, f, u, v, 0, b->cam_dev);
   b->launches += 1;
   BCHECK(cudaGetLastError());
   b->h_N[f] += 1;

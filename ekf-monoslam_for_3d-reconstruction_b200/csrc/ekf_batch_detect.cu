@@ -36,12 +36,19 @@
 
 // pixel keys (base mask, eig > 0) and candidate keys (those that are also raw 3x3 local maxima), one slot per pixel
 // (blockIdx.z: the camera's segment of a chunk)
+// fsize (ekf_batch_set_frame_sizes): segment z holds camera seg_cam[z] of fsize[4c + 2] x fsize[4c + 3] pixels, packed at the
+// segment's start with that width; the segment's other slots get no key.
 __global__ void k_bdet_keys(const float* __restrict__ eig, int W, int H, int estrem, unsigned long long* __restrict__ kp,
-                            unsigned long long* __restrict__ kc) {
-  const int x = blockIdx.x * blockDim.x + threadIdx.x, y = blockIdx.y;
+                            unsigned long long* __restrict__ kc, const int* __restrict__ fsize, const int* __restrict__ seg_cam) {
+  int x = blockIdx.x * blockDim.x + threadIdx.x, y = blockIdx.y;
   if (x >= W) return;
   const size_t seg = (size_t)blockIdx.z * W * H;
   eig += seg; kp += seg; kc += seg;
+  if (fsize) {
+    const int j = y * W + x, c = seg_cam[blockIdx.z], wc = fsize[4 * c + 2], hc = fsize[4 * c + 3];
+    if (j >= wc * hc) { kp[j] = 0ull; kc[j] = 0ull; return; }
+    W = wc; H = hc; x = j % wc; y = j / wc;
+  }
   const size_t i = (size_t)y * W + x;
   const float v = eig[i];
   unsigned long long p = 0ull, c = 0ull;
@@ -76,7 +83,8 @@ __global__ void __launch_bounds__(32 * BDET_WARPS) k_bdet_threshold(const unsign
                                                                      const int* __restrict__ num, int num_stride, int cap_mode,
                                                                      DetBox* __restrict__ boxes, unsigned* __restrict__ thr_bits,
                                                                      int* __restrict__ limit, const int* __restrict__ cam_of,
-                                                                     const int* __restrict__ slot_of_cam, int lo, int hi) {
+                                                                     const int* __restrict__ slot_of_cam, int lo, int hi,
+                                                                     const int* __restrict__ fsize) {
   __shared__ DetBox sb[BDET_WARPS][CS];
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int b = blockIdx.x * BDET_WARPS + warp;
@@ -84,6 +92,10 @@ __global__ void __launch_bounds__(32 * BDET_WARPS) k_bdet_threshold(const unsign
   const int seg = bdet_segment(cam_of, slot_of_cam, lo, hi, b);
   if (seg < 0) return;
   kp += (size_t)seg * npx;
+  if (fsize) {   // the camera's own size: its boxes clip and its keys decode with it
+    const int c = cam_of ? cam_of[b] : 0;
+    W = fsize[4 * c + 2]; H = fsize[4 * c + 3];
+  }
   const int nb = N[b];
   int lim = min(num[(size_t)b * num_stride], cap_mode ? Ncap - nb : EKF_BATCH_MAX_CORNERS);
   lim = max(0, min(lim, CS));
@@ -120,12 +132,13 @@ template <int CS>
 __global__ void k_bdet_select(const unsigned long long* __restrict__ kc, int nkeys, int W, const DetBox* __restrict__ boxes,
                               const int* __restrict__ N, const unsigned* __restrict__ thr_bits, const int* __restrict__ limit, int B,
                               float* __restrict__ out_xy, int* __restrict__ out_n, const int* __restrict__ cam_of,
-                              const int* __restrict__ slot_of_cam, int lo, int hi) {
+                              const int* __restrict__ slot_of_cam, int lo, int hi, const int* __restrict__ fsize) {
   const int b = blockIdx.x * blockDim.x + threadIdx.x;
   if (b >= B) return;
   const int seg = bdet_segment(cam_of, slot_of_cam, lo, hi, b);
   if (seg < 0) return;
   kc += (size_t)seg * nkeys;
+  if (fsize) W = fsize[4 * (cam_of ? cam_of[b] : 0) + 2];
   const int lim = limit[b];
   out_n[b] = lim > 0 ? det_select_walk(kc, nkeys, W, thr_bits[b], boxes + (size_t)b * CS, N[b], 144.0f, lim,
                                        out_xy + (size_t)b * 2 * CS)
@@ -191,7 +204,7 @@ cudaError_t launch_batch_detect(cudaStream_t st, BatchDetectBufs& d, FrameView f
   const int W = fr.w, H = fr.h, npx = W * H;
   unsigned long long *kp = d.keys, *kc = d.keys + d.cap, *kp_s = d.keys + 2 * d.cap, *kc_s = d.keys + 3 * d.cap;
   launch_det_eig(st, fr, d.eig, launches);
-  k_bdet_keys<<<dim3((W + 255) / 256, H), 256, 0, st>>>(d.eig, W, H, window, kp, kc);
+  k_bdet_keys<<<dim3((W + 255) / 256, H), 256, 0, st>>>(d.eig, W, H, window, kp, kc, nullptr, nullptr);
   size_t tmp = d.tmp_bytes;
   cudaError_t e = cub::DeviceRadixSort::SortKeysDescending(d.tmp, tmp, kp, kp_s, npx, 0, 64, st);
   if (e != cudaSuccess) return e;
@@ -202,15 +215,15 @@ cudaError_t launch_batch_detect(cudaStream_t st, BatchDetectBufs& d, FrameView f
   if (cstride == EKF_BATCH_MAX_CORNERS) {
     k_bdet_threshold<EKF_BATCH_MAX_CORNERS><<<gt, 32 * BDET_WARPS, 0, st>>>(kp_s, npx, W, H, window, centers, N, Ncap, B, num,
                                                                            num_stride, cap_mode, d.boxes, d.thr_bits, d.limit,
-                                                                           nullptr, nullptr, 0, 0);
+                                                                           nullptr, nullptr, 0, 0, nullptr);
     k_bdet_select<EKF_BATCH_MAX_CORNERS><<<gs, 128, 0, st>>>(kc_s, npx, W, d.boxes, N, d.thr_bits, d.limit, B, out_xy, out_n,
-                                                             nullptr, nullptr, 0, 0);
+                                                             nullptr, nullptr, 0, 0, nullptr);
   } else {
     k_bdet_threshold<EKF_BATCH_MAX_FEATURES><<<gt, 32 * BDET_WARPS, 0, st>>>(kp_s, npx, W, H, window, centers, N, Ncap, B, num,
                                                                             num_stride, cap_mode, d.boxes, d.thr_bits, d.limit,
-                                                                            nullptr, nullptr, 0, 0);
+                                                                            nullptr, nullptr, 0, 0, nullptr);
     k_bdet_select<EKF_BATCH_MAX_FEATURES><<<gs, 128, 0, st>>>(kc_s, npx, W, d.boxes, N, d.thr_bits, d.limit, B, out_xy, out_n,
-                                                              nullptr, nullptr, 0, 0);
+                                                              nullptr, nullptr, 0, 0, nullptr);
   }
   *launches += 5;   // keys, the two sorts (counted once each), threshold, select; the eig map counts itself
   return cudaGetLastError();
@@ -219,7 +232,7 @@ cudaError_t launch_batch_detect(cudaStream_t st, BatchDetectBufs& d, FrameView f
 cudaError_t launch_batch_detect_cams(cudaStream_t st, BatchDetectBufs& d, FrameView fr, const int* cams, int n_req, int chunk,
                                      const int* cam_of, const int* slot_of_cam, const float* centers, const int* N, int Ncap, int B,
                                      int window, const int* num, int num_stride, int cap_mode, int cstride, float* out_xy, int* out_n,
-                                     long long* launches) {
+                                     long long* launches, const int* fsize, const int* fsize_host, const int* seg_cam) {
   const int W = fr.w, H = fr.h, npx = W * H;
   const size_t fstep = (size_t)fr.h * fr.stride;
   cudaError_t e = cudaMemsetAsync(out_n, 0, sizeof(int) * (size_t)B, st);   // filters of cameras nobody asks from find nothing
@@ -228,9 +241,11 @@ cudaError_t launch_batch_detect_cams(cudaStream_t st, BatchDetectBufs& d, FrameV
   const unsigned gt = (B + BDET_WARPS - 1) / BDET_WARPS, gs = (B + 127) / 128;
   for (int lo = 0; lo < n_req; lo += chunk) {
     const int C = std::min(chunk, n_req - lo), hi = lo + C;
-    for (int s = 0; s < C; ++s)
-      launch_det_eig(st, FrameView{fr.px + (size_t)cams[lo + s] * fstep, W, H, fr.stride}, d.eig + (size_t)s * npx, launches);
-    k_bdet_keys<<<dim3((W + 255) / 256, H, C), 256, 0, st>>>(d.eig, W, H, window, kp, kc);
+    for (int s = 0; s < C; ++s) {   // with sizes, the eig map of the camera's own w x h (Sobel border at its own edge)
+      const int c = cams[lo + s], wc = fsize_host ? fsize_host[4 * c + 2] : W, hc = fsize_host ? fsize_host[4 * c + 3] : H;
+      launch_det_eig(st, FrameView{fr.px + (size_t)c * fstep, wc, hc, fr.stride}, d.eig + (size_t)s * npx, launches);
+    }
+    k_bdet_keys<<<dim3((W + 255) / 256, H, C), 256, 0, st>>>(d.eig, W, H, window, kp, kc, fsize, fsize ? seg_cam + lo : nullptr);
     size_t tmp = d.tmp_bytes;
     e = cub::DeviceSegmentedRadixSort::SortKeysDescending(d.tmp, tmp, kp, kp_s, C * npx, C, d.offs, d.offs + 1, 0, 64, st);
     if (e != cudaSuccess) return e;
@@ -240,15 +255,15 @@ cudaError_t launch_batch_detect_cams(cudaStream_t st, BatchDetectBufs& d, FrameV
     if (cstride == EKF_BATCH_MAX_CORNERS) {
       k_bdet_threshold<EKF_BATCH_MAX_CORNERS><<<gt, 32 * BDET_WARPS, 0, st>>>(kp_s, npx, W, H, window, centers, N, Ncap, B, num,
                                                                              num_stride, cap_mode, d.boxes, d.thr_bits, d.limit,
-                                                                             cam_of, slot_of_cam, lo, hi);
+                                                                             cam_of, slot_of_cam, lo, hi, fsize);
       k_bdet_select<EKF_BATCH_MAX_CORNERS><<<gs, 128, 0, st>>>(kc_s, npx, W, d.boxes, N, d.thr_bits, d.limit, B, out_xy, out_n,
-                                                               cam_of, slot_of_cam, lo, hi);
+                                                               cam_of, slot_of_cam, lo, hi, fsize);
     } else {
       k_bdet_threshold<EKF_BATCH_MAX_FEATURES><<<gt, 32 * BDET_WARPS, 0, st>>>(kp_s, npx, W, H, window, centers, N, Ncap, B, num,
                                                                               num_stride, cap_mode, d.boxes, d.thr_bits, d.limit,
-                                                                              cam_of, slot_of_cam, lo, hi);
+                                                                              cam_of, slot_of_cam, lo, hi, fsize);
       k_bdet_select<EKF_BATCH_MAX_FEATURES><<<gs, 128, 0, st>>>(kc_s, npx, W, d.boxes, N, d.thr_bits, d.limit, B, out_xy, out_n,
-                                                                cam_of, slot_of_cam, lo, hi);
+                                                                cam_of, slot_of_cam, lo, hi, fsize);
     }
     *launches += 5;
     if ((e = cudaGetLastError()) != cudaSuccess) return e;

@@ -201,11 +201,16 @@ __device__ __forceinline__ void resize_coeff(int d, double scale, int ssize, int
   *a1 = (short)__float2int_rn(f * 2048.f);
 }
 __global__ void k_capture_resize_gray(const uint8_t* __restrict__ src, int sw, int sh, int sstride, int cn, uint8_t* __restrict__ dst,
-                                      int dw, int dh, int dstride) {
+                                      int dw, int dh, int dstride, const int* __restrict__ fsize) {
   const int x = blockIdx.x * blockDim.x + threadIdx.x, y = blockIdx.y;
   if (x >= dw || y >= dh) return;
   src += (size_t)blockIdx.z * sh * sstride;   // frame z of a stack (batched cameras)
   dst += (size_t)blockIdx.z * dh * dstride;
+  if (fsize) {   // frame z is the top-left fsize[0] x fsize[1] of its slot, resized to fsize[2] x fsize[3] (cv::resize of the crop)
+    const int* q = fsize + 4 * blockIdx.z;
+    sw = q[0]; sh = q[1]; dw = q[2]; dh = q[3];
+    if (x >= dw || y >= dh) return;
+  }
   int ch[3] = {0, 0, 0};
   if (sw == dw && sh == dh) {
     for (int c = 0; c < cn; ++c) ch[c] = src[(size_t)y * sstride + x * cn + c];
@@ -234,7 +239,7 @@ __global__ void k_capture_resize_gray(const uint8_t* __restrict__ src, int sw, i
   dst[(size_t)y * dstride + x] = (uint8_t)min(max(g, 0), 255);
 }
 void launch_capture_resize_gray(cudaStream_t st, const uint8_t* src, int sw, int sh, int sstride, int cn, uint8_t* dst, int dw, int dh,
-                                int dstride, long long* launches, int n_frames) {
-  k_capture_resize_gray<<<dim3((dw + 255) / 256, dh, n_frames), 256, 0, st>>>(src, sw, sh, sstride, cn, dst, dw, dh, dstride);
+                                int dstride, long long* launches, int n_frames, const int* fsize) {
+  k_capture_resize_gray<<<dim3((dw + 255) / 256, dh, n_frames), 256, 0, st>>>(src, sw, sh, sstride, cn, dst, dw, dh, dstride, fsize);
   *launches += 1;
 }

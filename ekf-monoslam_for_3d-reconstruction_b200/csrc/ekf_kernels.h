@@ -34,7 +34,8 @@ void match_make_tensor_map(EkfTensorMap* out, const uint8_t* frames, int width, 
 void launch_match_filter(cudaStream_t st, FeatTab ft, int N, FrameView fr, const DevCfg& cfg, const EkfTensorMap* tmap, long long* launches);
 void launch_match_filter_batch(cudaStream_t st, FeatTab base, int Ncap, const int* Nper, int B, FrameView fr, const DevCfg& cfg,
                                const EkfTensorMap* tmap, int* defer_list, int* defer_cnt, long long* launches,
-                               const int* cam_of = nullptr);   // cam_of [B]: filter b searches frame cam_of[b] of the stack fr
+                               const int* cam_of = nullptr,    // cam_of [B]: filter b searches frame cam_of[b] of the stack fr
+                               const int* fsize = nullptr);    // [n_cameras][4] (in w, in h, w, h): camera c is the top-left w x h of its slot
 int launch_match_batch(cudaStream_t st, const uint8_t* frames, int n_frames, int width, int height, int stride,
                        const uint8_t* templates, int fpf, int w, const double* h, const double* S, float sigma_size,
                        float thr, float clampv, int32_t* out_uv, float* out_score);
@@ -122,7 +123,8 @@ int launch_detect_corners(cudaStream_t st, FrameView fr, FeatTab ft, int N, int 
 // the min-eigenvalue map of goodFeaturesToTrack for a whole frame (k_det_eig)
 void launch_det_eig(cudaStream_t st, FrameView fr, float* eig, long long* launches);
 void launch_capture_resize_gray(cudaStream_t st, const uint8_t* src, int sw, int sh, int sstride, int cn, uint8_t* dst, int dw, int dh,
-                                int dstride, long long* launches, int n_frames = 1);   // n_frames: a contiguous stack, frame z in blockIdx.z
+                                int dstride, long long* launches, int n_frames = 1,    // n_frames: a contiguous stack, frame z in blockIdx.z
+                                const int* fsize = nullptr);   // [n_frames][4]: frame z resizes its top-left fsize[0..1] to fsize[2..3]
 // ekf_batch_detect.cu: findNewFeatures' detection for every filter of a batch (one frame, per-filter masks)
 struct BatchDetectBufs {
   float* eig = nullptr;                 // [cap] min-eigenvalue map
@@ -151,4 +153,5 @@ cudaError_t batch_detect_reserve_cams(BatchDetectBufs& d, size_t npx, int chunk,
 cudaError_t launch_batch_detect_cams(cudaStream_t st, BatchDetectBufs& d, FrameView fr, const int* cams, int n_req, int chunk,
                                      const int* cam_of, const int* slot_of_cam, const float* centers, const int* N, int Ncap, int B,
                                      int window, const int* num, int num_stride, int cap_mode, int cstride, float* out_xy, int* out_n,
-                                     long long* launches);
+                                     long long* launches, const int* fsize = nullptr, const int* fsize_host = nullptr,
+                                     const int* seg_cam = nullptr);   // per-camera sizes (device / host [n_cameras][4]); seg_cam: cams on the device

@@ -1046,12 +1046,26 @@ __device__ __forceinline__ FrameView batch_frame(FrameView fr, int cam) {
   fr.px += (size_t)cam * fr.h * fr.stride;
   return fr;
 }
+// SIZES (ekf_batch_set_frame_sizes): camera c's frame is the top-left fsize[4c + 2] x fsize[4c + 3] of its slot, and the window
+// clipping uses that size.  cam_of may then be null (one camera).  Without sizes the kernels take SIZES = false, today's code.
+template <bool CAMS, bool SIZES>
+__device__ __forceinline__ FrameView batch_frame_of(FrameView fr, const int* __restrict__ cam_of, const int* __restrict__ fsize, int b) {
+  if constexpr (SIZES) {
+    const int c = cam_of ? cam_of[b] : 0;
+    fr = batch_frame(fr, c);
+    fr.w = fsize[4 * c + 2]; fr.h = fsize[4 * c + 3];
+  } else if constexpr (CAMS) {
+    fr = batch_frame(fr, cam_of[b]);
+  }
+  return fr;
+}
 
 // Batched filters, pass 1 with the full-window warp matcher (template side 11): one warp per (filter, feature)
-template <int MINB, bool TSMEM, bool SLIDE, bool CAMS>
+template <int MINB, bool TSMEM, bool SLIDE, bool CAMS, bool SIZES>
 __global__ void __launch_bounds__(MW2_WARPS * 32, MINB) k_match_filter_batch_warp2(FeatTab base, int Ncap, const int* __restrict__ Nper, int B,
                                                                                 FrameView fr, DevCfg cfg, int* __restrict__ defer_list,
-                                                                                int* __restrict__ defer_cnt, const int* __restrict__ cam_of) {
+                                                                                int* __restrict__ defer_cnt, const int* __restrict__ cam_of,
+                                                                                const int* __restrict__ fsize) {
   __shared__ MatchWarp2Smem<11> wsm[MW2_WARPS];
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const long long pair = (long long)blockIdx.x * MW2_WARPS + warp;
@@ -1060,7 +1074,7 @@ __global__ void __launch_bounds__(MW2_WARPS * 32, MINB) k_match_filter_batch_war
   const FeatTab ft = feattab_slice(base, b, Ncap, cfg.tstride);
   if (f >= Nper[b] || !ft.innov[f]) return;
   MatchJob jb;
-  if constexpr (CAMS) fr = batch_frame(fr, cam_of[b]);
+  fr = batch_frame_of<CAMS, SIZES>(fr, cam_of, fsize, b);
   jb.tmap = nullptr; jb.frame_index = 0;
   jb.frame = fr.px; jb.fw = fr.w; jb.fh = fr.h; jb.fstride = fr.stride;
   jb.tmpl = ft.mpatch + (size_t)f * cfg.tstride;
@@ -1078,11 +1092,11 @@ __global__ void __launch_bounds__(MW2_WARPS * 32, MINB) k_match_filter_batch_war
 }
 
 // Batched filters, pass 1: one warp per (filter, feature); features that do not fit go to defer_list.
-template <bool CAMS>
+template <bool CAMS, bool SIZES>
 __global__ void __launch_bounds__(MW_WARPS * 32) k_match_filter_batch_warp(FeatTab base, int Ncap, const int* __restrict__ Nper, int B,
                                                                            FrameView fr, DevCfg cfg, int* __restrict__ defer_list,
                                                                            int* __restrict__ defer_cnt, int warp_path,
-                                                                           const int* __restrict__ cam_of) {
+                                                                           const int* __restrict__ cam_of, const int* __restrict__ fsize) {
   __shared__ MatchWarpSmem wsm[MW_WARPS];
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const long long pair = (long long)blockIdx.x * MW_WARPS + warp;
@@ -1092,7 +1106,7 @@ __global__ void __launch_bounds__(MW_WARPS * 32) k_match_filter_batch_warp(FeatT
   if (f >= Nper[b] || !ft.innov[f]) return;
   const int w = cfg.window, w2 = w * w;
   MatchJob jb;
-  if constexpr (CAMS) fr = batch_frame(fr, cam_of[b]);
+  fr = batch_frame_of<CAMS, SIZES>(fr, cam_of, fsize, b);
   jb.tmap = nullptr; jb.frame_index = 0;
   jb.frame = fr.px; jb.fw = fr.w; jb.fh = fr.h; jb.fstride = fr.stride;
   jb.tmpl = ft.mpatch + (size_t)f * cfg.tstride;
@@ -1125,12 +1139,13 @@ __global__ void __launch_bounds__(MW_WARPS * 32) k_match_filter_batch_warp(FeatT
   }
 }
 // pass 2: a persistent grid of CTAs works off the deferred (filter, feature) pairs with match_one
-template <bool CAMS>
+template <bool CAMS, bool SIZES>
 __global__ void __launch_bounds__(MATCH_THREADS) k_match_filter_batch_deferred(FeatTab base, int Ncap, FrameView fr, DevCfg cfg,
                                                                                const __grid_constant__ CUtensorMap tmap, int use_tma,
                                                                                const int* __restrict__ defer_list,
                                                                                const int* __restrict__ defer_cnt,
-                                                                               const int* __restrict__ cam_of) {
+                                                                               const int* __restrict__ cam_of,
+                                                                               const int* __restrict__ fsize) {
   extern __shared__ __align__(128) unsigned char smem_raw[];
   const int n = *defer_cnt;
   unsigned phase = 0;
@@ -1139,8 +1154,9 @@ __global__ void __launch_bounds__(MATCH_THREADS) k_match_filter_batch_deferred(F
     const int pair = defer_list[i];
     const int b = pair / Ncap, f = pair - b * Ncap;
     const FeatTab ft = feattab_slice(base, b, Ncap, cfg.tstride);
-    const int cam = (CAMS && cam_of) ? cam_of[b] : 0;
-    match_filter_feature(ft, f, CAMS ? batch_frame(fr, cam) : fr, cfg, smem_raw, use_tma ? &tmap : nullptr, &phase, first, false, cam);
+    const int cam = ((CAMS || SIZES) && cam_of) ? cam_of[b] : 0;
+    match_filter_feature(ft, f, batch_frame_of<CAMS, SIZES>(fr, cam_of, fsize, b), cfg, smem_raw, use_tma ? &tmap : nullptr, &phase,
+                         first, false, cam);
     first = false;
     __syncthreads();
   }
@@ -1263,14 +1279,16 @@ void launch_match_filter(cudaStream_t st, FeatTab ft, int N, FrameView fr, const
 }
 
 void launch_match_filter_batch(cudaStream_t st, FeatTab base, int Ncap, const int* Nper, int B, FrameView fr, const DevCfg& cfg,
-                               const EkfTensorMap* tmap, int* defer_list, int* defer_cnt, long long* launches, const int* cam_of) {
+                               const EkfTensorMap* tmap, int* defer_list, int* defer_cnt, long long* launches, const int* cam_of,
+                               const int* fsize) {
   if (B <= 0 || Ncap <= 0) return;
   static PerDeviceOnce once;   // opt in to the largest supported window once per device
   const size_t smem = match_smem_bytes(cfg.window, cfg.search_clamp);
   if (once.ensure([] {
         const int bytes = (int)match_smem_bytes(MATCH_MAX_W, 20.0f);
-        const cudaError_t e = cudaFuncSetAttribute(k_match_filter_batch_deferred<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes);
-        return e != cudaSuccess ? e : cudaFuncSetAttribute(k_match_filter_batch_deferred<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes);
+        cudaError_t e = cudaFuncSetAttribute(k_match_filter_batch_deferred<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes);
+        if (e == cudaSuccess) e = cudaFuncSetAttribute(k_match_filter_batch_deferred<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes);
+        return e != cudaSuccess ? e : cudaFuncSetAttribute(k_match_filter_batch_deferred<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes);
       }) != cudaSuccess) return;   // the error stays in cudaGetLastError() for the caller
   static const EkfTensorMap none{};
   const EkfTensorMap& tm = (tmap && tmap->ok) ? *tmap : none;
@@ -1284,8 +1302,9 @@ void launch_match_filter_batch(cudaStream_t st, FeatTab base, int Ncap, const in
     const unsigned grid = (unsigned)((pairs + MW2_WARPS - 1) / MW2_WARPS);
     const int var = match_w2_variant();
 #define MW2_LAUNCH(MINB, TS, SL)                                                                                                        \
-  if (cam_of) k_match_filter_batch_warp2<MINB, TS, SL, true><<<grid, MW2_WARPS * 32, 0, st>>>(base, Ncap, Nper, B, fr, cfg, defer_list, defer_cnt, cam_of); \
-  else k_match_filter_batch_warp2<MINB, TS, SL, false><<<grid, MW2_WARPS * 32, 0, st>>>(base, Ncap, Nper, B, fr, cfg, defer_list, defer_cnt, cam_of)
+  if (fsize) k_match_filter_batch_warp2<MINB, TS, SL, true, true><<<grid, MW2_WARPS * 32, 0, st>>>(base, Ncap, Nper, B, fr, cfg, defer_list, defer_cnt, cam_of, fsize); \
+  else if (cam_of) k_match_filter_batch_warp2<MINB, TS, SL, true, false><<<grid, MW2_WARPS * 32, 0, st>>>(base, Ncap, Nper, B, fr, cfg, defer_list, defer_cnt, cam_of, fsize); \
+  else k_match_filter_batch_warp2<MINB, TS, SL, false, false><<<grid, MW2_WARPS * 32, 0, st>>>(base, Ncap, Nper, B, fr, cfg, defer_list, defer_cnt, cam_of, fsize)
     switch (var) {
       case 0: MW2_LAUNCH(2, false, false); break;
       case 2: MW2_LAUNCH(3, true, false); break;
@@ -1297,18 +1316,20 @@ void launch_match_filter_batch(cudaStream_t st, FeatTab base, int Ncap, const in
 #undef MW2_LAUNCH
   } else {
     const unsigned grid = (unsigned)((pairs + MW_WARPS - 1) / MW_WARPS);
-    if (cam_of) k_match_filter_batch_warp<true><<<grid, MW_WARPS * 32, 0, st>>>(base, Ncap, Nper, B, fr, cfg, defer_list, defer_cnt, warp_path, cam_of);
-    else k_match_filter_batch_warp<false><<<grid, MW_WARPS * 32, 0, st>>>(base, Ncap, Nper, B, fr, cfg, defer_list, defer_cnt, warp_path, cam_of);
+    if (fsize) k_match_filter_batch_warp<true, true><<<grid, MW_WARPS * 32, 0, st>>>(base, Ncap, Nper, B, fr, cfg, defer_list, defer_cnt, warp_path, cam_of, fsize);
+    else if (cam_of) k_match_filter_batch_warp<true, false><<<grid, MW_WARPS * 32, 0, st>>>(base, Ncap, Nper, B, fr, cfg, defer_list, defer_cnt, warp_path, cam_of, fsize);
+    else k_match_filter_batch_warp<false, false><<<grid, MW_WARPS * 32, 0, st>>>(base, Ncap, Nper, B, fr, cfg, defer_list, defer_cnt, warp_path, cam_of, fsize);
   }
   int dev = 0, sms = 148;
   if (cudaGetDevice(&dev) == cudaSuccess) cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
   int per_sm = 4;   // persistent grid: as many CTAs as are resident at this shared-memory footprint
-  auto* const deferred = cam_of ? k_match_filter_batch_deferred<true> : k_match_filter_batch_deferred<false>;   // the one launched
+  auto* const deferred = fsize ? k_match_filter_batch_deferred<true, true>
+                               : cam_of ? k_match_filter_batch_deferred<true, false> : k_match_filter_batch_deferred<false, false>;   // the one launched
   if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, deferred, MATCH_THREADS, smem) != cudaSuccess || per_sm < 1) {
     cudaGetLastError();
     per_sm = 4;
   }
-  deferred<<<sms * per_sm, MATCH_THREADS, smem, st>>>(base, Ncap, fr, cfg, as_cu(tm), tm.ok, defer_list, defer_cnt, cam_of);
+  deferred<<<sms * per_sm, MATCH_THREADS, smem, st>>>(base, Ncap, fr, cfg, as_cu(tm), tm.ok, defer_list, defer_cnt, cam_of, fsize);
   *launches += 2;
 }
 

@@ -298,6 +298,7 @@ class FilterBatch:
         self.h = h
         self.B = int(n_filters)
         self.n_cameras = 1
+        self.frame_sizes = None   # (n_cameras, 2) width, height of each camera's frame (set_frame_sizes), None: the whole frame
         self._cams = None   # (mu14, Sigma14) of every filter, read once per step for the views
 
     @classmethod
@@ -373,6 +374,7 @@ class FilterBatch:
             raise ValueError("camera_of expects (n_filters,)")
         self._ck(self.L.ekf_batch_set_cameras(self.h, int(n), _ptr(a) if a is not None else None))
         self.n_cameras = int(n)
+        self.frame_sizes = None
 
     def _stamps(self, stamps):
         if stamps is None:
@@ -380,9 +382,36 @@ class FilterBatch:
         s = np.ascontiguousarray(np.broadcast_to(np.asarray(stamps, dtype=np.float64), (self.n_cameras,)))
         return s
 
+    def set_frame_sizes(self, sizes):
+        """A frame size per camera: (n_cameras, 2) width, height in input pixels (before the resize by 1 / scale), or None for the
+        whole frame.  Camera c's frame is then the top-left of slot c of the stack captureNewFrames passes.  Forgets the
+        captured frames."""
+        if sizes is None:
+            self._ck(self.L.ekf_batch_set_frame_sizes(self.h, None))
+            self.frame_sizes = None
+            return
+        a = np.ascontiguousarray(sizes, dtype=np.int32)
+        if a.shape != (self.n_cameras, 2):
+            raise ValueError(f"set_frame_sizes expects ({self.n_cameras}, 2)")
+        self._ck(self.L.ekf_batch_set_frame_sizes(self.h, _ptr(a)))
+        self.frame_sizes = a.copy()
+
     def captureNewFrames(self, frames, stamps=None):
         """captureNewFrame for every camera: frames is (n_cameras, H, W) gray or (n_cameras, H, W, 3) BGR uint8 (host),
-        stamps one per camera or None.  A strided (n, H, W) view with padded rows is passed as it is."""
+        stamps one per camera or None.  A strided (n, H, W) view with padded rows is passed as it is.  With set_frame_sizes,
+        frames may also be a list of per-camera arrays of the declared sizes; they are packed into a zero-padded stack whose
+        slot is the largest width and height."""
+        if isinstance(frames, (list, tuple)):
+            if self.frame_sizes is None or len(frames) != self.n_cameras:
+                raise ValueError("a list of frames needs set_frame_sizes and one frame per camera")
+            fl = [np.asarray(x, dtype=np.uint8) for x in frames]
+            for c, x in enumerate(fl):
+                if x.shape[:2] != (int(self.frame_sizes[c, 1]), int(self.frame_sizes[c, 0])) or x.ndim != fl[0].ndim:
+                    raise ValueError(f"frame {c} has shape {x.shape}, camera {c} is {tuple(self.frame_sizes[c])} (width, height)")
+            H, W = int(self.frame_sizes[:, 1].max()), int(self.frame_sizes[:, 0].max())
+            frames = np.zeros((len(fl), H, W) + fl[0].shape[2:], np.uint8)
+            for c, x in enumerate(fl):
+                frames[c, :x.shape[0], :x.shape[1]] = x
         f = np.asarray(frames, dtype=np.uint8)
         if f.shape[0] != self.n_cameras or f.ndim not in (3, 4):
             raise ValueError(f"captureNewFrames expects ({self.n_cameras}, H, W) or ({self.n_cameras}, H, W, 3) uint8")
@@ -399,6 +428,20 @@ class FilterBatch:
         s = self._stamps(stamps)
         self._ck(self.L.ekf_batch_capture_frames_device(self.h, C.c_void_p(int(dev_ptr)), int(width), int(height), int(stride),
                                                         _ptr(s) if s is not None else None))
+
+    INTRINSICS = ("fx", "fy", "u0", "v0", "k1", "k2", "k3", "p1", "p2")
+
+    def set_intrinsics(self, params):
+        """Intrinsics per filter, columns in INTRINSICS order (EkfConfig's): a (9,) array for every filter, a (n_filters, 9)
+        array with filter f's row f, or None for the configuration's.  For intrinsics per camera, pass params[camera_of]."""
+        if params is None:
+            self._ck(self.L.ekf_batch_set_intrinsics(self.h, None))
+            return
+        a = np.asarray(params, dtype=np.float64)
+        if a.shape not in ((9,), (self.B, 9)):
+            raise ValueError(f"set_intrinsics expects (9,) or ({self.B}, 9)")
+        a = np.ascontiguousarray(np.broadcast_to(a, (self.B, 9)))
+        self._ck(self.L.ekf_batch_set_intrinsics(self.h, _ptr(a)))
 
     def set_detect_budget(self, nbytes):
         """Device scratch of one chunk of cameras in the per-camera detector (default 1 GiB)."""

@@ -99,10 +99,11 @@ class Scene:
     planar: bool = False      # a ground robot's camera: y = 0, q = (w, 0, q_y, 0) (identity at frame 0), moving in the x-z plane and
                               # turning about y only, so that forsePlane's pseudo-measurements (vslamRansac.cpp:1245-1272) hold;
                               # the filter's prior orientation is Q0, so set its camera state to (r[0], q[0]) before adding features
+    camera: Camera | None = None  # the calibration frames are rendered with (config_overrides reports it); None: Camera(u0=W/2, v0=H/2)
 
     def __post_init__(self):
         rng = np.random.default_rng(self.seed)
-        self.cam = Camera(u0=self.width / 2.0, v0=self.height / 2.0)
+        self.cam = self.camera if self.camera is not None else Camera(u0=self.width / 2.0, v0=self.height / 2.0)
         T = self.n_frames
         dT = 1.0 / self.fps
         # trajectory (world-frame v, body-frame w), integrated like Predict_State

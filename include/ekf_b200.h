@@ -279,12 +279,31 @@ int ekf_batch_capture_frame_bgr(ekf_batch* b, const uint8_t* bgr, int width, int
  * ekf_batch_get_frame return EKF_ERR_STATE: use the plural entries below. */
 int ekf_batch_get_frame(ekf_batch* b, uint8_t* out, int* width, int* height);
 /* Cameras: filter f follows camera camera_of[f] in [0, n_cameras) (HOST array of n_filters entries; NULL = identity, which
- * needs n_cameras == n_filters), 1 <= n_cameras <= n_filters, else EKF_ERR_ARG.  Cameras share the configuration (intrinsics,
- * window, scale) and one frame size.  The default is one camera followed by every filter.  The call forgets the captured
- * frames (a step then needs a capture first) and sets every camera's clock (dT, time stamp) to camera 0's;
+ * needs n_cameras == n_filters), 1 <= n_cameras <= n_filters, else EKF_ERR_ARG.  Cameras share the configuration (window,
+ * scale); intrinsics may differ per filter (ekf_batch_set_intrinsics) and frame sizes per camera (ekf_batch_set_frame_sizes).  The default is one camera
+ * followed by every filter.  The call forgets the captured frames (a step then needs a capture first) and sets every camera's clock (dT, time stamp) to camera 0's;
  * ekf_batch_seed_from sets every camera's clock from the source filter.  Memory: the gray frames, n_cameras x stride x
  * height bytes after resize (stride = width rounded up to 16), e.g. 1.26 GB for 4096 cameras of 640 x 480. */
 int ekf_batch_set_cameras(ekf_batch* b, int n_cameras, const int32_t* camera_of);
+/* Intrinsics per filter: cam is a HOST array of n_filters x 9 doubles in ekf_config order (fx fy u0 v0 k1 k2 k3 p1 p2), and
+ * filter f projects, linearises and unprojects with row f in predict, the blur prediction, RANSAC, the Hi rescue and
+ * addFeature.  NULL returns every filter to the configuration's intrinsics, which is the default.  A non-finite entry or
+ * fx <= 0 or fy <= 0 returns EKF_ERR_ARG and leaves the table as it was.  As for ekf_batch_set_scale, the intrinsics are
+ * those of the resized image.  The table goes to the device inside this call (no per-step copy); ekf_batch_seed_from and
+ * ekf_batch_set_cameras leave it alone.  For intrinsics per camera, pass row camera_of[f] for filter f.  Memory: 72 B per
+ * filter on the device while a table is set.  Window, sigmas and scale stay shared by the batch. */
+int ekf_batch_set_intrinsics(ekf_batch* b, const double* cam);
+/* A frame size per camera: wh is a HOST array of n_cameras x 2 int32 (width, height) in INPUT pixels, before the resize by
+ * 1 / scale; NULL (the default) means every camera uses the whole frame the capture calls pass.  The stack keeps one slot per
+ * camera: the capture calls' width / height / stride describe the slot, and camera c's frame is the top-left w_c x h_c of slot
+ * c, resized to w_c / scale x h_c / scale (integer division, like cv::Size) inside a slot of width / scale x height / scale.
+ * Prediction gate, matching and its window clipping, detection, addFeature's isInsideImage and ekf_batch_get_camera_frame use
+ * the camera's own size.  The bytes of a slot outside its camera's frame do not change any result: a capture zeroes them (one
+ * launch over the stack, none when every camera fills its slot).  Non-positive sizes return EKF_ERR_ARG; a capture with a
+ * camera larger than its slot or a resized side below 8 returns EKF_ERR_ARG.  The sizes hold from the next capture on (the
+ * call forgets the captured frames); ekf_batch_set_cameras returns to NULL.  Memory: 16 B per camera on the device; the stack
+ * stays n_cameras x slot. */
+int ekf_batch_set_frame_sizes(ekf_batch* b, const int32_t* wh);
 /* captureNewFrame for every camera: a stack of n_cameras frames, frame c at img + c * height * stride (the layout of
  * ekf_match_batch), gray from HOST / DEVICE memory or BGR from HOST memory.  stamps: n_cameras doubles or NULL; camera c
  * applies the single filter's rule to stamps[c] (>= 0: dT = stamp - old_ts once old_ts > 0).  Resize and colour conversion
