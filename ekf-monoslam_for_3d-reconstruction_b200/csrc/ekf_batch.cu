@@ -114,14 +114,23 @@ __device__ void cta_xyz_decide(const BatchView& bv, int b, const double* Sigma, 
 }
 
 // Per-filter inputs of a step, uploaded in one copy with the picks; a null field leaves the kernel's scalar argument in place
-// (one camera and ekf_batch_step: every field null).
+// (one camera and ekf_batch_step: every field null).  ctl / vcontrol are indexed by CTA: by filter without a list, in list
+// order with one.
 struct BatchStepIn {
   const int* cam_of;       // [B] camera of each filter (null: camera 0)
   const double* dT;        // [n_cameras] each camera's dT
   const double* ctl;       // [B][6] dv, dw of each filter (ekf_batch_step_controls)
   const int* vcontrol;     // [B]
   const int* fsize;        // [n_cameras][4] frame sizes (ekf_batch_set_frame_sizes): the gate uses [2], [3] of the filter's camera
+  const int* act;          // [n] the filters ekf_batch_step_filters steps, ascending; read by the ACT instantiations only
 };
+// The filter CTA i of a per-filter launch works on: i itself, or with a list (ACT, ekf_batch_step_filters) the list's entry i.
+// A template parameter, so that a step without a list runs the code it ran before.
+template <bool ACT>
+__device__ __forceinline__ int act_filter(const int* __restrict__ act, int i) {
+  if constexpr (ACT) return act[i];
+  else return i;
+}
 __device__ __forceinline__ double step_dT(const BatchStepIn& in, int b, double dT) {
   return in.dT ? in.dT[in.cam_of ? in.cam_of[b] : 0] : dT;
 }
@@ -130,17 +139,17 @@ __device__ __forceinline__ double step_dT(const BatchStepIn& in, int b, double d
 // predict for one filter per CTA: same arithmetic as k_predict_cov / k_predict_features / k_predict_S2
 // ------------------------------------------------------------------------------------------------
 #define BPRED_THREADS 128
-template <bool INTR>
+template <bool INTR, bool ACT>
 __global__ void __launch_bounds__(BPRED_THREADS, 4) k_batch_predict(BatchView bv, FrameView fr, DevCfg cfg, double dT, double3 dv,
                                                                  double3 dw, int vcontrol, BatchStepIn in) {
   __shared__ double F[169], C[169], T[169], Q[169], cam[13];
-  const int b = blockIdx.x, tid = threadIdx.x;
+  const int i0 = blockIdx.x, b = act_filter<ACT>(in.act, i0), tid = threadIdx.x;
   dT = step_dT(in, b, dT);
   if (in.ctl) {
-    const double* c = in.ctl + 6 * (size_t)b;
+    const double* c = in.ctl + 6 * (size_t)i0;
     dv = make_double3(c[0], c[1], c[2]); dw = make_double3(c[3], c[4], c[5]);
   }
-  if (in.vcontrol) vcontrol = in.vcontrol[b];
+  if (in.vcontrol) vcontrol = in.vcontrol[i0];
   const int n = bv.n[b], N = bv.N[b], ld = bv.ld;
   double* Sigma = bv.Sigma + (size_t)b * bv.sstride;
   double* mu = bv.mu + (size_t)b * ld;
@@ -270,19 +279,20 @@ __global__ void __launch_bounds__(BPRED_THREADS, 4) k_batch_predict(BatchView bv
 // k_batch_predict: same arithmetic as k_predict_blur (ekf_blur.cuh), another shape.  Warp 0 takes the blur decision with
 // lane = feature; then every blurred template goes to one warp, which stages it in shared memory, rasterises the line
 // with lane = point, keeps each distinct coefficient once, orders them by (row, column) and has every output pixel walk
-// that list: the terms and their order are the bit mask walk's, without the zeros.  out[b] = templates blurred,
-// out[B + b] = 1 when a kernel exceeded BLUR_MAXK (that template stays unblurred, as in k_predict_blur).
+// that list: the terms and their order are the bit mask walk's, without the zeros.  out[i] = templates blurred,
+// out[gridDim.x + i] = 1 when a kernel exceeded BLUR_MAXK (that template stays unblurred, as in k_predict_blur), i the CTA:
+// the filter, or its position in the list.
 // ------------------------------------------------------------------------------------------------
 #define BBLUR_WARPS 4
 // NC: feature capacity (BNCAP or BNCAP_L); warp 0 takes the decisions 32 features at a time, in ascending order.
-template <int NC, bool INTR>
+template <int NC, bool INTR, bool ACT>
 __global__ void __launch_bounds__(BBLUR_WARPS * 32) k_batch_predict_blur(BatchView bv, DevCfg cfg, double dT, int* __restrict__ out,
                                                                      BatchStepIn in) {
   __shared__ int s_feat[NC], s_rows[NC], s_cols[NC], s_nblur;
   __shared__ double s_dx[NC], s_dy[NC];
   __shared__ __align__(16) uint8_t s_tmpl[BBLUR_WARPS][1024];
   __shared__ int s_seq[BBLUR_WARPS][BLUR_MAXPTS], s_coef[BBLUR_WARPS][BLUR_MAXPTS];
-  const int b = blockIdx.x, lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  const int b = act_filter<ACT>(in.act, blockIdx.x), lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   dT = step_dT(in, b, dT);
   const int N = bv.N[b], ld = bv.ld;
   const double* mu = bv.mu + (size_t)b * ld;
@@ -315,8 +325,8 @@ __global__ void __launch_bounds__(BBLUR_WARPS * 32) k_batch_predict_blur(BatchVi
     }
     if (lane == 0) {
       s_nblur = nblur;
-      out[b] = nblur;
-      out[gridDim.x + b] = anybig != 0u;
+      out[blockIdx.x] = nblur;
+      out[gridDim.x + blockIdx.x] = anybig != 0u;
     }
   }
   __syncthreads();
@@ -612,11 +622,13 @@ __device__ void cta_stacked_update(const UpdSmem& sm, double* __restrict__ Sigma
 }
 
 // PLANE: forsePlane (ekf_batch_set_force_plane), a separate instantiation so that the plane-off kernel is the same code as without it.
-template <bool PLANE, bool INTR>
+// ACT: CTA i updates filter act[i] (ekf_batch_step_filters).
+template <bool PLANE, bool INTR, bool ACT>
 __global__ void __launch_bounds__(BUPD_THREADS, 1) k_batch_update(BatchView bv, DevCfg cfg, const uint32_t* __restrict__ picks,
                                                                   int n_picks, double* __restrict__ out_mu14,
                                                                   double* __restrict__ out_S14, int* __restrict__ out_stats,
-                                                                  int min_features, int max_features, int xyz_conversion) {
+                                                                  int min_features, int max_features, int xyz_conversion,
+                                                                  const int* __restrict__ act) {
   extern __shared__ __align__(16) double usm[];
   UpdSmem sm;
   sm.W = usm;
@@ -629,7 +641,7 @@ __global__ void __launch_bounds__(BUPD_THREADS, 1) k_batch_update(BatchView bv, 
   sm.Hs = sm.mu_i + BNMAX;
   sm.qj = sm.Hs + BNCAP * 27;
   sm.ibuf = reinterpret_cast<int*>(sm.qj + 48);
-  const int b = blockIdx.x, tid = threadIdx.x;
+  const int b = act_filter<ACT>(act, blockIdx.x), tid = threadIdx.x;
   const int n = bv.n[b], N = bv.N[b], ld = bv.ld;
   double* Sigma = bv.Sigma + (size_t)b * bv.sstride;
   double* mu = bv.mu + (size_t)b * ld;
@@ -1069,11 +1081,12 @@ static __device__ __noinline__ void cl_hi_rescue(double* Sigma, int ld, const do
   if (tid == 0) { ctl->n_hi = nh; ctl->k_rows = 2 * nh; }
 }
 
-template <bool PLANE, bool INTR>
+template <bool PLANE, bool INTR, bool ACT>
 __global__ void __launch_bounds__(BUPD_THREADS, 1) k_batch_update_cluster(BatchView bv, DevCfg cfg, const uint32_t* __restrict__ picks,
                                                                           int n_picks, double* __restrict__ out_mu14,
                                                                           double* __restrict__ out_S14, int* __restrict__ out_stats,
-                                                                          int min_features, int max_features, int xyz_conversion) {
+                                                                          int min_features, int max_features, int xyz_conversion,
+                                                                          const int* __restrict__ act) {
   extern __shared__ __align__(16) double usm[];
   UpdSmem sm;
   sm.W = usm;
@@ -1087,7 +1100,7 @@ __global__ void __launch_bounds__(BUPD_THREADS, 1) k_batch_update_cluster(BatchV
   sm.qj = sm.Hs + BNCAP * 27;
   sm.ibuf = reinterpret_cast<int*>(sm.qj + 48);
   const int C = (int)cg::this_cluster().num_blocks(), rank = (int)cg::this_cluster().block_rank();
-  const int b = blockIdx.x / C, tid = threadIdx.x;
+  const int b = act_filter<ACT>(act, blockIdx.x / C), tid = threadIdx.x;
   const int n = bv.n[b], N = bv.N[b], ld = bv.ld;
   double* Sigma = bv.Sigma + (size_t)b * bv.sstride;
   double* mu = bv.mu + (size_t)b * ld;
@@ -1186,22 +1199,22 @@ struct BatchArchive {
 // with the surviving records; the conversions follow its new features (ekf_batch_step).  NC: feature capacity (BNCAP or
 // BNCAP_L); one CTA covers every entry of n2 x n2 either way, and every record (N2 <= 128 <= BCMP_THREADS).
 // one >= 0 (grid of one CTA): removeFeature(one_idx) on filter `one` alone (ekf_batch_remove_feature): no other removal, no
-// max_features rule, no conversion; pending decisions move with the records as under hold.
+// max_features rule, no conversion; pending decisions move with the records as under hold.  ACT: CTA i works on filter act[i].
 // With the archive on, every removed feature that removeFeature archives (XYZ, n_find > 5) is appended to the filter's archive
 // in the single filter's order: the flagged features in ascending index (ekf_update_after_match's victims), then the
 // removeFeature(0) victim.  The records are read from Sigma and mu before the pass overwrites them.  A conversion fused into
 // the same pass never touches a removed feature's block: the reference removes before it converts, the decisions exclude the
 // removed features, and J is the identity on every row but the converted feature's.
-template <int NC>
+template <int NC, bool ACT>
 __global__ void __launch_bounds__(BCMP_THREADS, 1) k_batch_compact(BatchView bv, double* __restrict__ scratch, int min_features,
                                                                 int max_features, int remove, const int* __restrict__ hold_stats,
-                                                                BatchArchive ar, int one, int one_idx) {
+                                                                BatchArchive ar, int one, int one_idx, const int* __restrict__ act) {
   constexpr int MV = (EKF_CAM + 6 * NC + BCMP_THREADS - 1) / BCMP_THREADS;   // state entries a thread moves: 1 at NC = 32
   __shared__ int keep[NC], newpos[NC], conv[NC], arch[NC];
   __shared__ int2 rmap[EKF_CAM + 6 * NC + 2];
   __shared__ int s_N2, s_n2, s_narch, s_abase;
   const bool single = one >= 0;
-  const int b = single ? one : blockIdx.x, tid = threadIdx.x;
+  const int b = single ? one : act_filter<ACT>(act, blockIdx.x), tid = threadIdx.x;
   DevCtl* ctl = bv.ctl + b;
   const bool rem = single || (remove && ctl->n_remove > 0);
   const bool hold = single || (hold_stats && hold_stats[(size_t)b * EKF_BATCH_STAT_FIELDS + EKF_BSTAT_TOPUP] > 0);
@@ -1359,15 +1372,15 @@ __global__ void __launch_bounds__(BNCAP_L) k_batch_xyz_decide_large(BatchView bv
 // took for the filter's older features (adds change no entry their linearity test reads), for k_batch_compact to apply.
 // LARGE (capacity up to BNCAP_L): the corners sit at xy + 2 * BNCAP_L * b, the rows (n <= 776 before an add) are taken
 // BADD_THREADS at a time and the decisions one thread per feature.  Templates come from frame cam_of[b] of the stack fr
-// (cam_of null: frame 0).
+// (cam_of null: frame 0).  ACT: CTA i works on filter act[i] (ekf_batch_step_filters).
 #define BADD_THREADS 256
-template <bool LARGE, bool INTR>
+template <bool LARGE, bool INTR, bool ACT>
 __global__ void __launch_bounds__(BADD_THREADS) k_batch_add(BatchView bv, FrameView fr, DevCfg cfg, const float* __restrict__ xy,
                                                             const int* __restrict__ cnt, int one, float u, float v, int decide,
-                                                            const int* __restrict__ cam_of) {
+                                                            const int* __restrict__ cam_of, const int* __restrict__ act) {
   constexpr int CS = LARGE ? BNCAP_L : EKF_BATCH_MAX_CORNERS;   // corner stride of xy
   __shared__ double A[6 * 7], Ap[6 * 3], fnew[6], Tc[6 * 7];
-  const int b = one >= 0 ? one : blockIdx.x, tid = threadIdx.x;
+  const int b = one >= 0 ? one : (ACT ? act[blockIdx.x] : blockIdx.x), tid = threadIdx.x;
   const int k = one >= 0 ? 1 : cnt[b];
   if (k <= 0) return;
   if (cam_of) fr.px += (size_t)cam_of[b] * fr.h * fr.stride;
@@ -1510,6 +1523,28 @@ __global__ void k_batch_set_cam(BatchView bv, const double* __restrict__ mu14, i
   if (e < B * 14) bv.mu[(size_t)(e / 14) * bv.ld + (e % 14)] = mu14[e];
 }
 
+// The rows ekf_batch_get_camera_states reports, mu[0:14] and Sigma[0:14, 0:14], of every filter from its state as it stands: a
+// step with a list writes only its filters' rows, so the others' are gathered here after a call that changed them.
+__global__ void k_batch_camera_rows(BatchView bv, double* __restrict__ out_mu14, double* __restrict__ out_S14, int B) {
+  const int e = blockIdx.x * blockDim.x + threadIdx.x;
+  if (e >= B * 210) return;
+  const int b = e / 210, r = e - b * 210;
+  if (r < 14) out_mu14[(size_t)b * 14 + r] = bv.mu[(size_t)b * bv.ld + r];
+  else out_S14[(size_t)b * 196 + r - 14] = bv.Sigma[(size_t)b * bv.sstride + (size_t)((r - 14) / 14) * bv.ld + (r - 14) % 14];
+}
+
+// frame z of a stack of dw x dh slots: every pixel outside the camera's fsize[4z + 2] x fsize[4z + 3] becomes 0.  SLOTS: frame z is
+// slot slot[z].
+template <bool SLOTS>
+__global__ void k_batch_zero_pads(uint8_t* __restrict__ frame, int dw, int dstride, int dh, const int* __restrict__ fsize,
+                                  const int* __restrict__ slot) {
+  const int x = blockIdx.x * blockDim.x + threadIdx.x, y = blockIdx.y;
+  if (x >= dw) return;
+  const int z = SLOTS ? slot[blockIdx.z] : blockIdx.z;
+  const int* q = fsize + 4 * z;
+  if (x >= q[2] || y >= q[3]) frame[((size_t)z * dh + y) * dstride + x] = 0;
+}
+
 // ================================================================================================
 // host side
 // ================================================================================================
@@ -1559,7 +1594,10 @@ struct ekf_batch {
   int* h_added = nullptr;                       // pinned: features each filter added in the last step / top-up call
   int* blur_out = nullptr;                      // [2][B] k_batch_predict_blur: templates blurred, kernel too large
   int* h_blur = nullptr;                        // pinned mirror of blur_out
-  bool have_frame = false, seeded = false, results_valid = false, topup = false, blur = false;
+  std::vector<char> cam_frame;                  // [n_cam] the camera holds a frame (a capture that listed it since the frames were forgotten)
+  int* slot_dev = nullptr;                      // [n_cam] destination slots of a capture of listed cameras
+  bool rows_stale = true;                       // out_mu14 / out_S14 may differ from some filter's state (seed, set_camera_states, set_full)
+  bool seeded = false, results_valid = false, topup = false, blur = false;
   bool large = false;                           // ekf_batch_create_large with capacity > 32: the cluster update, BNCAP_L kernels
   int cl_ctas = 1, cl_resident = 0;             // CTAs per filter in the update; clusters resident at once (large only)
   int cstride = EKF_BATCH_MAX_CORNERS;          // corners per filter in det_xy (BNCAP_L when large)
@@ -1607,7 +1645,7 @@ int ekf_batch_destroy(ekf_batch* b) {
   cudaFree(b->match_defer);
   cudaFree(b->scratch); cudaFree(b->frame); cudaFree(b->raw); cudaFree(b->picks_dev); cudaFree(b->out_mu14); cudaFree(b->out_S14);
   cudaFree(b->out_stats); cudaFree(b->stage_mu14); cudaFree(b->bv.patchnumbre);
-  cudaFree(b->cam_dev); cudaFree(b->det_slot); cudaFree(b->step_dev); cudaFree(b->intr_dev); cudaFree(b->fsize_dev);
+  cudaFree(b->cam_dev); cudaFree(b->det_slot); cudaFree(b->step_dev); cudaFree(b->intr_dev); cudaFree(b->fsize_dev); cudaFree(b->slot_dev);
   if (b->h_det_slot) cudaFreeHost(b->h_det_slot);
   if (b->step_host) cudaFreeHost(b->step_host);
   batch_detect_free(b->det);
@@ -1672,15 +1710,19 @@ static int batch_create(const ekf_config* cfg, int n_filters, int feature_capaci
   TRY(cudaSetDevice(device))
   TRY(cudaStreamCreateWithFlags(&b->own_stream, cudaStreamNonBlocking))
   b->stream = b->own_stream;
-  for (void* k : {(void*)k_batch_update<false, false>, (void*)k_batch_update<true, false>, (void*)k_batch_update<false, true>,
-                  (void*)k_batch_update<true, true>})
+  for (void* k : {(void*)k_batch_update<false, false, false>, (void*)k_batch_update<true, false, false>,
+                  (void*)k_batch_update<false, true, false>, (void*)k_batch_update<true, true, false>,
+                  (void*)k_batch_update<false, false, true>, (void*)k_batch_update<true, false, true>,
+                  (void*)k_batch_update<false, true, true>, (void*)k_batch_update<true, true, true>})
     TRY(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kUpdSmemBytes))
   if (large) {
-    void* const cl[4] = {(void*)k_batch_update_cluster<false, false>, (void*)k_batch_update_cluster<true, false>,
-                         (void*)k_batch_update_cluster<false, true>, (void*)k_batch_update_cluster<true, true>};
+    void* const cl[8] = {(void*)k_batch_update_cluster<false, false, false>, (void*)k_batch_update_cluster<true, false, false>,
+                         (void*)k_batch_update_cluster<false, true, false>, (void*)k_batch_update_cluster<true, true, false>,
+                         (void*)k_batch_update_cluster<false, false, true>, (void*)k_batch_update_cluster<true, false, true>,
+                         (void*)k_batch_update_cluster<false, true, true>, (void*)k_batch_update_cluster<true, true, true>};
     for (void* k : cl) TRY(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kUpdSmemBytes))
     cudaLaunchAttribute attr[1];
-    for (int i = 0; i < 4; ++i) {   // forsePlane x intrinsics table
+    for (int i = 0; i < 8; ++i) {   // forsePlane x intrinsics table x filter list
       const cudaLaunchConfig_t lc = cluster_config(1, b->cl_ctas, nullptr, attr);
       int ncl = 0;
       TRY(cudaOccupancyMaxActiveClusters(&ncl, cl[i], &lc))
@@ -1729,6 +1771,7 @@ static int batch_create(const ekf_config* cfg, int n_filters, int feature_capaci
   for (size_t i = 0; i < Bn; ++i) { b->h_n[i] = 0; b->h_N[i] = 0; b->h_added[i] = 0; }
   b->cam_host.assign(Bn, 0);
   b->cam_dT.assign(1, 1.0); b->cam_ts.assign(1, -1.0);
+  b->cam_frame.assign(1, 0);
   std::fill(b->h_blur, b->h_blur + 2 * Bn, 0);
   DevCfg& d = b->dcfg;
   d.cam = CamParams{cfg->fx, cfg->fy, cfg->u0, cfg->v0, cfg->k1, cfg->k2, cfg->k3, cfg->p1, cfg->p2};
@@ -1829,6 +1872,7 @@ int ekf_batch_seed_from(ekf_batch* b, ekf_handle* src) {
   b->cam_dT.assign(b->n_cam, src->dT); b->cam_ts.assign(b->n_cam, src->old_ts);
   b->seeded = true;
   b->results_valid = false;
+  b->rows_stale = true;
   return EKF_OK;
 }
 
@@ -1840,6 +1884,7 @@ int ekf_batch_set_camera_states(ekf_batch* b, const double* mu14) {
   b->launches += 1;
   BCHECK(cudaGetLastError());
   BCHECK(cudaStreamSynchronize(b->stream));
+  b->rows_stale = true;
   return EKF_OK;
 }
 
@@ -1848,25 +1893,32 @@ int ekf_batch_set_camera_states(ekf_batch* b, const double* mu14) {
 // BGR -> gray in k_capture_resize_gray with the camera in blockIdx.z, from device frames directly and from host frames through
 // the staging buffer `raw`, a chunk of cameras at a time so that `raw` stays within kRawBudget (or one frame).  n frames
 // (n == b->n_cam), frame c at img + c * height * stride; stamps[c] (stamps may be null: no stamps).
+// list (n_list cameras, ekf_batch_capture_camera_frames*): frame k of the stack and stamps[k] are camera list[k]'s, and the
+// frames go through k_capture_resize_gray at every scale, which writes frame k to slot list[k] of the existing stack.
 static constexpr size_t kRawBudget = (size_t)256 << 20;
-// frame z of a stack of dw x dh slots: every pixel outside the camera's fsize[4z + 2] x fsize[4z + 3] becomes 0
-__global__ void k_batch_zero_pads(uint8_t* __restrict__ frame, int dw, int dstride, int dh, const int* __restrict__ fsize) {
-  const int x = blockIdx.x * blockDim.x + threadIdx.x, y = blockIdx.y;
-  if (x >= dw) return;
-  const int* q = fsize + 4 * blockIdx.z;
-  if (x >= q[2] || y >= q[3]) frame[((size_t)blockIdx.z * dh + y) * dstride + x] = 0;
-}
-static int bcapture(ekf_batch* b, const uint8_t* img, int width, int height, int stride, int channels, const double* stamps, bool dev) {
+static int bcapture(ekf_batch* b, const uint8_t* img, int width, int height, int stride, int channels, const double* stamps, bool dev,
+                    int n_list = 0, const int32_t* list = nullptr) {
   if (!b || !img || width < 8 || height < 8 || stride < width * channels) return EKF_ERR_ARG;
-  const int scale = b->cfg.scale, n = b->n_cam;
+  const bool sub = list != nullptr;
+  if (sub) {
+    if (n_list < 1 || n_list > b->n_cam) return bfail(b, EKF_ERR_ARG, "n must lie in [1, n_cameras]");
+    std::vector<char> seen(b->n_cam, 0);
+    for (int k = 0; k < n_list; ++k) {
+      const int c = list[k];
+      if (c < 0 || c >= b->n_cam || seen[c])
+        return bfail(b, EKF_ERR_ARG, "cameras[" + std::to_string(k) + "] = " + std::to_string(c) + " is not a camera, or listed twice");
+      seen[c] = 1;
+    }
+  }
+  const int scale = b->cfg.scale, n_all = b->n_cam, n = sub ? n_list : n_all;
   const int dw = width / scale, dh = height / scale;   // cv::Size(width / scale, height / scale), integer division
   if (dw < 8 || dh < 8) return bfail(b, EKF_ERR_ARG, "resized frame smaller than 8 x 8 pixels");
   // frame sizes per camera: camera c is the top-left size_in[c] of its slot, resized to size_in[c] / scale
   std::vector<int> fs;
   bool pads = false;
   if (!b->size_in.empty()) {
-    fs.resize((size_t)4 * n);
-    for (int c = 0; c < n; ++c) {
+    fs.resize((size_t)4 * n_all);
+    for (int c = 0; c < n_all; ++c) {
       const int wc = b->size_in[2 * c], hc = b->size_in[2 * c + 1];
       if (wc > width || hc > height)
         return bfail(b, EKF_ERR_ARG, "camera " + std::to_string(c) + " is larger than the captured " + std::to_string(width) + " x " +
@@ -1874,18 +1926,30 @@ static int bcapture(ekf_batch* b, const uint8_t* img, int width, int height, int
       if (wc / scale < 8 || hc / scale < 8)
         return bfail(b, EKF_ERR_ARG, "camera " + std::to_string(c) + ": resized frame smaller than 8 x 8 pixels");
       fs[4 * c] = wc; fs[4 * c + 1] = hc; fs[4 * c + 2] = wc / scale; fs[4 * c + 3] = hc / scale;
+    }
+    for (int k = 0; k < n; ++k) {
+      const int c = sub ? list[k] : k;
       pads = pads || fs[4 * c + 2] < dw || fs[4 * c + 3] < dh;
     }
   }
+  if (sub && std::find(b->cam_frame.begin(), b->cam_frame.end(), 1) != b->cam_frame.end()) {
+    // other cameras hold frames in the stack: the slot and every camera's resized size stay as they are
+    static const std::vector<int> none;
+    if (dw != b->fv.w || dh != b->fv.h || fs != (b->fsize_on ? b->fsize_host : none))
+      return bfail(b, EKF_ERR_ARG, "the resized slot " + std::to_string(dw) + " x " + std::to_string(dh) + " differs from the stack's " +
+                                       std::to_string(b->fv.w) + " x " + std::to_string(b->fv.h) +
+                                       " (or the frame sizes changed): only a capture of every camera may change it");
+  }
   BCHECK(cudaSetDevice(b->device));
-  for (int c = 0; stamps && c < n; ++c) {
-    if (stamps[c] >= 0) {
-      if (b->cam_ts[c] > 0) b->cam_dT[c] = (stamps[c] - b->cam_ts[c]);
-      b->cam_ts[c] = stamps[c];
+  for (int k = 0; stamps && k < n; ++k) {
+    const int c = sub ? list[k] : k;
+    if (stamps[k] >= 0) {
+      if (b->cam_ts[c] > 0) b->cam_dT[c] = (stamps[k] - b->cam_ts[c]);
+      b->cam_ts[c] = stamps[k];
     }
   }
   const int dstride = (dw + 15) & ~15;
-  const size_t fstep = (size_t)dstride * dh, need = fstep * n;
+  const size_t fstep = (size_t)dstride * dh, need = fstep * n_all;
   if (!fs.empty() && fs != b->fsize_host) {   // the table goes up when the sizes or the scale change, not per capture
     if (!b->fsize_dev) BCHECK(balloc(&b->fsize_dev, 4 * b->n_cam));
     b->fsize_host = fs;
@@ -1900,7 +1964,12 @@ static int bcapture(ekf_batch* b, const uint8_t* img, int width, int height, int
     BCHECK(cudaMalloc((void**)&b->frame, need));
     b->frame_cap = need;
   }
-  if (scale == 1 && channels == 1) {
+  if (sub) {   // the slot of each listed frame, from a pageable copy: the driver has staged it when the call returns
+    if (!b->slot_dev) BCHECK(balloc(&b->slot_dev, b->n_cam));
+    const std::vector<int> slots(list, list + n);
+    BCHECK(cudaMemcpyAsync(b->slot_dev, slots.data(), sizeof(int) * n, cudaMemcpyHostToDevice, b->stream));
+  }
+  if (scale == 1 && channels == 1 && !sub) {
     BCHECK(cudaMemcpy2DAsync(b->frame, dstride, img, stride, width, (size_t)height * n, dev ? cudaMemcpyDeviceToDevice : cudaMemcpyHostToDevice,
                              b->stream));
   } else {
@@ -1923,24 +1992,29 @@ static int bcapture(ekf_batch* b, const uint8_t* img, int width, int height, int
                                  cudaMemcpyHostToDevice, b->stream));
         src = b->raw; sstride = width * channels;
       }
-      launch_capture_resize_gray(b->stream, src, width, height, sstride, channels, b->frame + (size_t)c0 * fstep, dw, dh, dstride,
-                                 &b->launches, k, b->fsize_on ? b->fsize_dev + 4 * c0 : nullptr);
+      if (sub)
+        launch_capture_resize_gray(b->stream, src, width, height, sstride, channels, b->frame, dw, dh, dstride, &b->launches, k,
+                                   b->fsize_on ? b->fsize_dev : nullptr, b->slot_dev + c0);
+      else
+        launch_capture_resize_gray(b->stream, src, width, height, sstride, channels, b->frame + (size_t)c0 * fstep, dw, dh, dstride,
+                                   &b->launches, k, b->fsize_on ? b->fsize_dev + 4 * c0 : nullptr);
       BCHECK(cudaGetLastError());
     }
   }
   if (pads) {   // results must not depend on the bytes of a slot outside its camera's frame: zero them, one launch over the stack
     for (int c0 = 0; c0 < n; c0 += 65535) {
       const int k = std::min(65535, n - c0);
-      k_batch_zero_pads<<<dim3((dw + 255) / 256, dh, k), 256, 0, b->stream>>>(b->frame + (size_t)c0 * fstep, dw, dstride, dh,
-                                                                            b->fsize_dev + 4 * c0);
+      const dim3 grid((dw + 255) / 256, dh, k);
+      if (sub) k_batch_zero_pads<true><<<grid, 256, 0, b->stream>>>(b->frame, dw, dstride, dh, b->fsize_dev, b->slot_dev + c0);
+      else k_batch_zero_pads<false><<<grid, 256, 0, b->stream>>>(b->frame + (size_t)c0 * fstep, dw, dstride, dh, b->fsize_dev + 4 * c0, nullptr);
       b->launches += 1;
     }
     BCHECK(cudaGetLastError());
   }
   if (b->fv.px != b->frame || b->fv.w != dw || b->fv.h != dh || b->fv.stride != dstride)
-    match_make_tensor_map(&b->frame_map, b->frame, dw, dh, dstride, n, b->cfg.window_size, (int)b->cfg.search_clamp);
+    match_make_tensor_map(&b->frame_map, b->frame, dw, dh, dstride, n_all, b->cfg.window_size, (int)b->cfg.search_clamp);
   b->fv = FrameView{b->frame, dw, dh, dstride};
-  b->have_frame = true;
+  for (int k = 0; k < n; ++k) b->cam_frame[sub ? list[k] : k] = 1;
   return EKF_OK;
 }
 static int bcapture1(ekf_batch* b, const uint8_t* img, int width, int height, int stride, int channels, double stamp, bool dev) {
@@ -1961,6 +2035,20 @@ int ekf_batch_capture_frames_device(ekf_batch* b, const uint8_t* g, int w, int h
 int ekf_batch_capture_frames_bgr(ekf_batch* b, const uint8_t* bgr, int w, int h, int s, const double* stamps) {
   return bcapture(b, bgr, w, h, s, 3, stamps, false);
 }
+int ekf_batch_capture_camera_frames(ekf_batch* b, int n, const int32_t* cameras, const uint8_t* g, int w, int h, int s, const double* stamps) {
+  if (b && !cameras) return bfail(b, EKF_ERR_ARG, "cameras is NULL");
+  return bcapture(b, g, w, h, s, 1, stamps, false, n, cameras);
+}
+int ekf_batch_capture_camera_frames_device(ekf_batch* b, int n, const int32_t* cameras, const uint8_t* g, int w, int h, int s,
+                                           const double* stamps) {
+  if (b && !cameras) return bfail(b, EKF_ERR_ARG, "cameras is NULL");
+  return bcapture(b, g, w, h, s, 1, stamps, true, n, cameras);
+}
+int ekf_batch_capture_camera_frames_bgr(ekf_batch* b, int n, const int32_t* cameras, const uint8_t* bgr, int w, int h, int s,
+                                        const double* stamps) {
+  if (b && !cameras) return bfail(b, EKF_ERR_ARG, "cameras is NULL");
+  return bcapture(b, bgr, w, h, s, 3, stamps, false, n, cameras);
+}
 
 int ekf_batch_set_cameras(ekf_batch* b, int n_cameras, const int32_t* camera_of) {
   if (!b) return EKF_ERR_ARG;
@@ -1974,8 +2062,8 @@ int ekf_batch_set_cameras(ekf_batch* b, int n_cameras, const int32_t* camera_of)
   }
   BCHECK(cudaSetDevice(b->device));
   BCHECK(cudaStreamSynchronize(b->stream));
-  cudaFree(b->cam_dev); cudaFree(b->det_slot); cudaFreeHost(b->h_det_slot); cudaFree(b->fsize_dev);
-  b->cam_dev = nullptr; b->det_slot = nullptr; b->h_det_slot = nullptr; b->fsize_dev = nullptr;
+  cudaFree(b->cam_dev); cudaFree(b->det_slot); cudaFreeHost(b->h_det_slot); cudaFree(b->fsize_dev); cudaFree(b->slot_dev);
+  b->cam_dev = nullptr; b->det_slot = nullptr; b->h_det_slot = nullptr; b->fsize_dev = nullptr; b->slot_dev = nullptr;
   b->fsize_host.clear();
   if (n_cameras > 1) {
     BCHECK(balloc(&b->cam_dev, b->B));
@@ -1989,7 +2077,7 @@ int ekf_batch_set_cameras(ekf_batch* b, int n_cameras, const int32_t* camera_of)
   b->n_cam = n_cameras;
   const double dT = b->cam_dT[0], ts = b->cam_ts[0];
   b->cam_dT.assign(n_cameras, dT); b->cam_ts.assign(n_cameras, ts);
-  b->have_frame = false;
+  b->cam_frame.assign(n_cameras, 0);
   b->fv = FrameView{nullptr, 0, 0, 0};   // the next capture encodes the stack's tensor map
   return EKF_OK;
 }
@@ -2030,7 +2118,7 @@ int ekf_batch_set_frame_sizes(ekf_batch* b, const int32_t* wh) {
     b->size_in.clear();
   }
   b->fsize_on = false;
-  b->have_frame = false;   // the sizes hold from the next capture on
+  std::fill(b->cam_frame.begin(), b->cam_frame.end(), 0);   // the sizes hold from the next capture on
   return EKF_OK;
 }
 
@@ -2042,7 +2130,7 @@ int ekf_batch_set_detect_budget(ekf_batch* b, int64_t bytes) {
 
 int ekf_batch_get_camera_frame(ekf_batch* b, int camera, uint8_t* out, int* width, int* height) {   // returnGrayImg (vslamRansac.cpp:1364)
   if (!b || !width || !height || camera < 0 || camera >= b->n_cam) return EKF_ERR_ARG;
-  if (!b->have_frame) return bfail(b, EKF_ERR_STATE, "no frame captured");
+  if (!b->cam_frame[camera]) return bfail(b, EKF_ERR_STATE, "no frame captured for camera " + std::to_string(camera));
   const int w = b->fsize_on ? b->fsize_host[4 * camera + 2] : b->fv.w, h = b->fsize_on ? b->fsize_host[4 * camera + 3] : b->fv.h;
   *width = w; *height = h;
   if (out) {
@@ -2078,15 +2166,20 @@ int ekf_batch_set_force_plane(ekf_batch* b, int on) {
   return EKF_OK;
 }
 
-// k_batch_compact at the batch's capacity; one >= 0: removeFeature(one_idx) on filter `one` alone (one CTA)
-static void launch_compact(ekf_batch* b, int remove, const int* hold_stats, int one = -1, int one_idx = -1) {
-  const unsigned grid = one >= 0 ? 1u : (unsigned)b->B;
-  if (b->large)
-    k_batch_compact<BNCAP_L><<<grid, BCMP_THREADS, 0, b->stream>>>(b->bv, b->scratch, b->cfg.min_features, b->cfg.max_features, remove,
-                                                                   hold_stats, b->ar, one, one_idx);
-  else
-    k_batch_compact<BNCAP><<<grid, BCMP_THREADS, 0, b->stream>>>(b->bv, b->scratch, b->cfg.min_features, b->cfg.max_features, remove,
-                                                                 hold_stats, b->ar, one, one_idx);
+// The filters a step works on: n_act of them listed at act (device) by ekf_batch_step_filters, or every filter (act null).
+struct StepList {
+  const int* act = nullptr;
+  int n_act = 0;
+};
+static unsigned step_grid(const ekf_batch* b, const StepList& sl) { return (unsigned)(sl.act ? sl.n_act : b->B); }
+
+// k_batch_compact at the batch's capacity on the step's filters; one >= 0: removeFeature(one_idx) on filter `one` alone (one CTA)
+static void launch_compact(ekf_batch* b, int remove, const int* hold_stats, int one = -1, int one_idx = -1, const StepList& sl = {}) {
+  const unsigned grid = one >= 0 ? 1u : step_grid(b, sl);
+  auto* const compact = b->large ? (sl.act ? k_batch_compact<BNCAP_L, true> : k_batch_compact<BNCAP_L, false>)
+                                 : (sl.act ? k_batch_compact<BNCAP, true> : k_batch_compact<BNCAP, false>);
+  compact<<<grid, BCMP_THREADS, 0, b->stream>>>(b->bv, b->scratch, b->cfg.min_features, b->cfg.max_features, remove, hold_stats, b->ar,
+                                                one, one_idx, sl.act);
   b->launches += 1;
 }
 
@@ -2144,15 +2237,25 @@ static int batch_detect(ekf_batch* b, const int* num, const int* hnum, int num_s
   return EKF_OK;
 }
 
+// k_batch_add at the batch's capacity and intrinsics, with or without a list of filters
+static void (*add_kernel(const ekf_batch* b, bool act))(BatchView, FrameView, DevCfg, const float*, const int*, int, float, float, int,
+                                                        const int*, const int*) {
+  const bool intr = b->bv.cam != nullptr;
+  if (b->large) return act ? (intr ? k_batch_add<true, true, true> : k_batch_add<true, false, true>)
+                           : (intr ? k_batch_add<true, true, false> : k_batch_add<true, false, false>);
+  return act ? (intr ? k_batch_add<false, true, true> : k_batch_add<false, false, true>)
+             : (intr ? k_batch_add<false, true, false> : k_batch_add<false, false, false>);
+}
+
 // detection + adds for every filter, as batch_detect; decide: also take the new features' XYZ decisions (in-step top-up).
+// The detector runs on every filter (one that asks for nothing costs next to nothing), the adds on the step's filters.
 // Enqueued only.
-static int batch_topup(ekf_batch* b, const int* num, const int* hnum, int num_stride, int decide) {
+static int batch_topup(ekf_batch* b, const int* num, const int* hnum, int num_stride, int decide, const StepList& sl = {}) {
   cudaStream_t st = b->stream;
   const int rc = batch_detect(b, num, hnum, num_stride, 1);
   if (rc) return rc;
-  auto* const add = b->large ? (b->bv.cam ? k_batch_add<true, true> : k_batch_add<true, false>)
-                             : (b->bv.cam ? k_batch_add<false, true> : k_batch_add<false, false>);
-  add<<<b->B, BADD_THREADS, 0, st>>>(b->bv, b->fv, b->dcfg, b->det_xy, b->det_n, -1, 0.0f, 0.0f, decide, b->cam_dev);
+  add_kernel(b, sl.act)<<<step_grid(b, sl), BADD_THREADS, 0, st>>>(b->bv, b->fv, b->dcfg, b->det_xy, b->det_n, -1, 0.0f, 0.0f, decide,
+                                                                   b->cam_dev, sl.act);
   b->launches += 1;
   BCHECK(cudaGetLastError());
   return EKF_OK;
@@ -2170,22 +2273,46 @@ static int batch_readback(ekf_batch* b, bool added) {
   return EKF_OK;
 }
 
-// ekf_batch_step (per_filter false: dv / dw / vcontrol for every filter) and ekf_batch_step_controls (per_filter: dv / dw
-// n_filters x 3, vcontrol n_filters; null = zeros).  With one camera and shared controls the picks go up alone; otherwise the
-// cameras' dT, the filters' controls and the picks are staged together and go up in one copy (BatchStepIn).
+// EKF_ERR_STATE unless filter f's camera holds a frame
+static int need_frame(ekf_batch* b, int f, const char* what) {
+  const int c = b->cam_host[f];
+  if (b->cam_frame[c]) return EKF_OK;
+  return bfail(b, EKF_ERR_STATE, std::string(what) + " before captureNewFrame: camera " + std::to_string(c) + " of filter " +
+                                     std::to_string(f) + " holds no frame");
+}
+
+// ekf_batch_step (per_filter false: dv / dw / vcontrol for every filter), ekf_batch_step_controls (per_filter: dv / dw
+// n_filters x 3, vcontrol n_filters; null = zeros) and ekf_batch_step_filters (filters: the n_act listed filters, strictly
+// ascending, with per_filter controls in list order).  With one camera, shared controls and no list the picks go up alone;
+// otherwise the cameras' dT, the filters' controls, the list and the picks are staged together and go up in one copy (BatchStepIn).
+// With a list every per-filter kernel runs on the listed filters only; the counters of the others are zeroed on the device and
+// their camera rows gathered when they may be stale, so that ekf_batch_get_camera_states reports every filter as it stands.
 static int batch_step(ekf_batch* b, const double* dv, const double* dw, int vcontrol, const int32_t* vcontrols, bool per_filter,
-                      const uint32_t* picks, int n_picks) {
+                      const uint32_t* picks, int n_picks, const int32_t* filters = nullptr, int n_act = 0) {
   if (!b || n_picks < 0 || (n_picks > 0 && !picks)) return EKF_ERR_ARG;
+  if (filters) {
+    if (n_act < 1 || n_act > b->B) return bfail(b, EKF_ERR_ARG, "n must lie in [1, n_filters]");
+    for (int i = 0; i < n_act; ++i)
+      if (filters[i] < 0 || filters[i] >= b->B || (i > 0 && filters[i] <= filters[i - 1]))
+        return bfail(b, EKF_ERR_ARG, "filters must be strictly ascending in [0, n_filters): filters[" + std::to_string(i) + "] = " +
+                                         std::to_string(filters[i]));
+  }
   if (!b->seeded) return bfail(b, EKF_ERR_STATE, "batch step before ekf_batch_seed_from");
-  if (!b->have_frame) return bfail(b, EKF_ERR_STATE, "batch step before captureNewFrame");
+  const int n_rows = filters ? n_act : b->B;   // filters the step works on
+  const bool every_frame = std::find(b->cam_frame.begin(), b->cam_frame.end(), 0) == b->cam_frame.end();
+  for (int i = 0; !every_frame && i < n_rows; ++i) {
+    const int rc = need_frame(b, filters ? filters[i] : i, "batch step");
+    if (rc) return rc;
+  }
   BCHECK(cudaSetDevice(b->device));
   cudaStream_t st = b->stream;
   const size_t Bn = (size_t)b->B;
-  BatchStepIn in{b->cam_dev, nullptr, nullptr, nullptr, b->fsize_on ? b->fsize_dev : nullptr};
+  BatchStepIn in{b->cam_dev, nullptr, nullptr, nullptr, b->fsize_on ? b->fsize_dev : nullptr, nullptr};
+  StepList sl;
   const uint32_t* picks_dev = b->picks_dev;
   const double z3[3] = {0, 0, 0};
   const double* a = (dv && !per_filter) ? dv : z3; const double* w = (dw && !per_filter) ? dw : z3;
-  if (b->n_cam == 1 && !per_filter) {
+  if (b->n_cam == 1 && !per_filter && !filters) {
     if (n_picks > b->picks_cap) {
       BCHECK(cudaStreamSynchronize(st));
       cudaFree(b->picks_dev);
@@ -2196,9 +2323,11 @@ static int batch_step(ekf_batch* b, const double* dv, const double* dw, int vcon
     if (n_picks > 0) BCHECK(cudaMemcpyAsync(b->picks_dev, picks, sizeof(uint32_t) * n_picks, cudaMemcpyHostToDevice, st));
     picks_dev = b->picks_dev;
   } else {
-    // [dT: n_cam doubles, n_cam > 1][ctl: B x 6 doubles, vcontrol: B int32, per_filter][picks]
-    const size_t n_dT = b->n_cam > 1 ? (size_t)b->n_cam : 0, n_ctl = per_filter ? 6 * Bn : 0, n_vc = per_filter ? Bn : 0;
-    const size_t bytes = sizeof(double) * (n_dT + n_ctl) + sizeof(int) * n_vc + sizeof(uint32_t) * (size_t)n_picks;
+    // [dT: n_cam doubles, n_cam > 1][ctl: rows x 6 doubles, vcontrol: rows int32, per_filter][act: n_act int32, a list][picks]
+    const size_t rows = (size_t)n_rows;
+    const size_t n_dT = b->n_cam > 1 ? (size_t)b->n_cam : 0, n_ctl = per_filter ? 6 * rows : 0, n_vc = per_filter ? rows : 0;
+    const size_t n_al = filters ? rows : 0;
+    const size_t bytes = sizeof(double) * (n_dT + n_ctl) + sizeof(int) * (n_vc + n_al) + sizeof(uint32_t) * (size_t)n_picks;
     if (bytes > b->step_cap) {
       BCHECK(cudaStreamSynchronize(st));
       cudaFree(b->step_dev); cudaFreeHost(b->step_host);
@@ -2216,42 +2345,65 @@ static int batch_step(ekf_batch* b, const double* dv, const double* dw, int vcon
       }
     int* hi = reinterpret_cast<int*>(hd + n_dT + n_ctl);
     for (size_t f = 0; f < n_vc; ++f) hi[f] = vcontrols ? (vcontrols[f] != 0) : 0;
-    uint32_t* hp = reinterpret_cast<uint32_t*>(hi + n_vc);
+    if (n_al) std::copy(filters, filters + n_al, hi + n_vc);
+    uint32_t* hp = reinterpret_cast<uint32_t*>(hi + n_vc + n_al);
     if (n_picks > 0) std::copy(picks, picks + n_picks, hp);
     BCHECK(cudaMemcpyAsync(b->step_dev, b->step_host, bytes, cudaMemcpyHostToDevice, st));
     const double* dd = static_cast<const double*>(b->step_dev);
+    const int* di = reinterpret_cast<const int*>(dd + n_dT + n_ctl);
     if (n_dT) in.dT = dd;
-    if (per_filter) { in.ctl = dd + n_dT; in.vcontrol = reinterpret_cast<const int*>(dd + n_dT + n_ctl); }
-    picks_dev = reinterpret_cast<const uint32_t*>(reinterpret_cast<const int*>(dd + n_dT + n_ctl) + n_vc);
+    if (per_filter) { in.ctl = dd + n_dT; in.vcontrol = di; }
+    if (filters) { in.act = di + n_vc; sl.act = in.act; sl.n_act = n_act; }
+    picks_dev = reinterpret_cast<const uint32_t*>(di + n_vc + n_al);
+  }
+  const bool act = sl.act != nullptr, intr = b->bv.cam != nullptr;
+  const unsigned grid = step_grid(b, sl);
+  if (act) {   // the others' counters read zero; their camera rows are gathered once a call changed some filter's
+    BCHECK(cudaMemsetAsync(b->out_stats, 0, sizeof(int) * Bn * EKF_BATCH_STAT_FIELDS, st));
+    if (b->rows_stale) {
+      k_batch_camera_rows<<<(unsigned)((Bn * 210 + 255) / 256), 256, 0, st>>>(b->bv, b->out_mu14, b->out_S14, b->B);
+      b->launches += 1;
+    }
   }
   BCHECK(cudaEventRecord(b->ev[0], st));
-  auto* const predict = b->bv.cam ? k_batch_predict<true> : k_batch_predict<false>;
-  predict<<<b->B, BPRED_THREADS, 0, st>>>(b->bv, b->fv, b->dcfg, b->cam_dT[0], make_double3(a[0], a[1], a[2]),
-                                           make_double3(w[0], w[1], w[2]), vcontrol, in);
+  auto* const predict = act ? (intr ? k_batch_predict<true, true> : k_batch_predict<false, true>)
+                            : (intr ? k_batch_predict<true, false> : k_batch_predict<false, false>);
+  predict<<<grid, BPRED_THREADS, 0, st>>>(b->bv, b->fv, b->dcfg, b->cam_dT[0], make_double3(a[0], a[1], a[2]),
+                                          make_double3(w[0], w[1], w[2]), vcontrol, in);
   b->launches += 1;
   if (b->blur) {   // matching_patch <- blurred patch where the prediction moves far enough (k_batch_predict copied patch)
-    auto* const blur = b->large ? (b->bv.cam ? k_batch_predict_blur<BNCAP_L, true> : k_batch_predict_blur<BNCAP_L, false>)
-                                : (b->bv.cam ? k_batch_predict_blur<BNCAP, true> : k_batch_predict_blur<BNCAP, false>);
-    blur<<<b->B, BBLUR_WARPS * 32, 0, st>>>(b->bv, b->dcfg, b->cam_dT[0], b->blur_out, in);
+    void (*blur)(BatchView, DevCfg, double, int*, BatchStepIn);
+    if (b->large) blur = act ? (intr ? k_batch_predict_blur<BNCAP_L, true, true> : k_batch_predict_blur<BNCAP_L, false, true>)
+                             : (intr ? k_batch_predict_blur<BNCAP_L, true, false> : k_batch_predict_blur<BNCAP_L, false, false>);
+    else blur = act ? (intr ? k_batch_predict_blur<BNCAP, true, true> : k_batch_predict_blur<BNCAP, false, true>)
+                    : (intr ? k_batch_predict_blur<BNCAP, true, false> : k_batch_predict_blur<BNCAP, false, false>);
+    blur<<<grid, BBLUR_WARPS * 32, 0, st>>>(b->bv, b->dcfg, b->cam_dT[0], b->blur_out, in);
     b->launches += 1;
   }
   BCHECK(cudaEventRecord(b->ev[1], st));
-  launch_match_filter_batch(st, b->bv.ft, b->Ncap, b->bv.N, b->B, b->fv, b->dcfg, &b->frame_map, b->match_defer,
-                            b->match_defer + (size_t)b->B * b->Ncap, &b->launches, b->cam_dev, b->fsize_on ? b->fsize_dev : nullptr);
+  launch_match_filter_batch(st, b->bv.ft, b->Ncap, b->bv.N, (int)grid, b->fv, b->dcfg, &b->frame_map, b->match_defer,
+                            b->match_defer + (size_t)b->B * b->Ncap, &b->launches, b->cam_dev, b->fsize_on ? b->fsize_dev : nullptr, sl.act);
   BCHECK(cudaEventRecord(b->ev[2], st));
+  const bool plane = b->cfg.forsePlane != 0;
   if (b->large) {   // one cluster of cl_ctas CTAs per filter
     cudaLaunchAttribute attr[1];
-    const cudaLaunchConfig_t lc = cluster_config(b->B, b->cl_ctas, st, attr);
-    auto* const update = b->cfg.forsePlane ? (b->bv.cam ? k_batch_update_cluster<true, true> : k_batch_update_cluster<true, false>)
-                                           : (b->bv.cam ? k_batch_update_cluster<false, true> : k_batch_update_cluster<false, false>);
+    const cudaLaunchConfig_t lc = cluster_config((int)grid, b->cl_ctas, st, attr);
+    void (*update)(BatchView, DevCfg, const uint32_t*, int, double*, double*, int*, int, int, int, const int*);
+    if (act) update = plane ? (intr ? k_batch_update_cluster<true, true, true> : k_batch_update_cluster<true, false, true>)
+                            : (intr ? k_batch_update_cluster<false, true, true> : k_batch_update_cluster<false, false, true>);
+    else update = plane ? (intr ? k_batch_update_cluster<true, true, false> : k_batch_update_cluster<true, false, false>)
+                        : (intr ? k_batch_update_cluster<false, true, false> : k_batch_update_cluster<false, false, false>);
     BCHECK(cudaLaunchKernelEx(&lc, update, b->bv, b->dcfg, picks_dev, n_picks, b->out_mu14, b->out_S14,
-                              b->out_stats, (int)b->cfg.min_features, (int)b->cfg.max_features, (int)b->cfg.xyz_conversion));
+                              b->out_stats, (int)b->cfg.min_features, (int)b->cfg.max_features, (int)b->cfg.xyz_conversion, sl.act));
   } else {
-    auto* const update = b->cfg.forsePlane ? (b->bv.cam ? k_batch_update<true, true> : k_batch_update<true, false>)
-                                           : (b->bv.cam ? k_batch_update<false, true> : k_batch_update<false, false>);
-    update<<<b->B, BUPD_THREADS, kUpdSmemBytes, st>>>(b->bv, b->dcfg, picks_dev, n_picks, b->out_mu14, b->out_S14,
+    void (*update)(BatchView, DevCfg, const uint32_t*, int, double*, double*, int*, int, int, int, const int*);
+    if (act) update = plane ? (intr ? k_batch_update<true, true, true> : k_batch_update<true, false, true>)
+                            : (intr ? k_batch_update<false, true, true> : k_batch_update<false, false, true>);
+    else update = plane ? (intr ? k_batch_update<true, true, false> : k_batch_update<true, false, false>)
+                        : (intr ? k_batch_update<false, true, false> : k_batch_update<false, false, false>);
+    update<<<grid, BUPD_THREADS, kUpdSmemBytes, st>>>(b->bv, b->dcfg, picks_dev, n_picks, b->out_mu14, b->out_S14,
                                                       b->out_stats, b->cfg.min_features, b->cfg.max_features,
-                                                      b->cfg.xyz_conversion);
+                                                      b->cfg.xyz_conversion, sl.act);
   }
   b->launches += 1;
   BCHECK(cudaEventRecord(b->ev[3], st));
@@ -2259,11 +2411,18 @@ static int batch_step(ekf_batch* b, const double* dv, const double* dw, int vcon
   BCHECK(cudaMemcpyAsync(b->h_stats, b->out_stats, sizeof(int) * Bn * EKF_BATCH_STAT_FIELDS, cudaMemcpyDeviceToHost, st));
   BCHECK(cudaMemcpyAsync(b->h_mu14, b->out_mu14, sizeof(double) * Bn * 14, cudaMemcpyDeviceToHost, st));
   if (b->cfg.xyz_conversion) BCHECK(cudaMemcpyAsync(b->h_xyz_count, b->bv.xyz_count, sizeof(int) * Bn, cudaMemcpyDeviceToHost, st));
-  if (b->blur) BCHECK(cudaMemcpyAsync(b->h_blur, b->blur_out, sizeof(int) * 2 * Bn, cudaMemcpyDeviceToHost, st));
+  if (b->blur) BCHECK(cudaMemcpyAsync(b->h_blur, b->blur_out, sizeof(int) * 2 * grid, cudaMemcpyDeviceToHost, st));
   BCHECK(cudaStreamSynchronize(st));
   b->results_valid = true;
+  b->rows_stale = false;
+  if (b->blur && act) {   // the kernel wrote list positions: scatter them to filters, zeros for the others
+    const std::vector<int> got(b->h_blur, b->h_blur + 2 * (size_t)n_act);
+    std::fill(b->h_blur, b->h_blur + 2 * Bn, 0);
+    for (int i = 0; i < n_act; ++i) { b->h_blur[filters[i]] = got[i]; b->h_blur[Bn + filters[i]] = got[n_act + i]; }
+  }
   long long removed = 0, converted = 0, fails = 0, topups = 0;
-  for (size_t i = 0; i < Bn; ++i) {
+  for (int k = 0; k < n_rows; ++k) {   // the step's filters: the others have zero counters and nothing pending
+    const size_t i = filters ? (size_t)filters[k] : (size_t)k;
     removed += b->h_stats[i * EKF_BATCH_STAT_FIELDS + EKF_BSTAT_REMOVED];
     fails += b->h_stats[i * EKF_BATCH_STAT_FIELDS + EKF_BSTAT_CHOL_FAIL];
     topups += b->h_stats[i * EKF_BATCH_STAT_FIELDS + EKF_BSTAT_TOPUP] > 0;
@@ -2272,7 +2431,7 @@ static int batch_step(ekf_batch* b, const double* dv, const double* dw, int vcon
   std::fill(b->h_added, b->h_added + Bn, 0);
   if (!b->topup || topups == 0) {
     if (removed > 0 || converted > 0) {   // removals, then convert2XYZ_ifLinearAll (V:1312-1317), in one pass
-      launch_compact(b, 1, nullptr);
+      launch_compact(b, 1, nullptr, -1, -1, sl);
       BCHECK(cudaGetLastError());
       const int rc = batch_readback(b, false);
       if (rc) return rc;
@@ -2283,12 +2442,12 @@ static int batch_step(ekf_batch* b, const double* dv, const double* dw, int vcon
     // and converting first would give A (J Sigma[cam, f]), equal only up to rounding.  So its compaction removes only;
     // every other filter keeps the fused pass.
     if (removed > 0 || converted > 0) {
-      launch_compact(b, 1, b->out_stats);
+      launch_compact(b, 1, b->out_stats, -1, -1, sl);
     }
-    int rc = batch_topup(b, b->out_stats + EKF_BSTAT_TOPUP, b->h_stats + EKF_BSTAT_TOPUP, EKF_BATCH_STAT_FIELDS, b->cfg.xyz_conversion);
+    int rc = batch_topup(b, b->out_stats + EKF_BSTAT_TOPUP, b->h_stats + EKF_BSTAT_TOPUP, EKF_BATCH_STAT_FIELDS, b->cfg.xyz_conversion, sl);
     if (rc) return rc;
     if (b->cfg.xyz_conversion) {   // the held conversions and the new features' (filters with none return at once)
-      launch_compact(b, 0, nullptr);
+      launch_compact(b, 0, nullptr, -1, -1, sl);
     }
     BCHECK(cudaGetLastError());
     rc = batch_readback(b, true);
@@ -2305,6 +2464,11 @@ int ekf_batch_step(ekf_batch* b, const double dv[3], const double dw[3], int vco
 }
 int ekf_batch_step_controls(ekf_batch* b, const double* dv, const double* dw, const int32_t* vcontrol, const uint32_t* picks, int n_picks) {
   return batch_step(b, dv, dw, 0, vcontrol, true, picks, n_picks);
+}
+int ekf_batch_step_filters(ekf_batch* b, int n, const int32_t* filters, const double* dv, const double* dw, const int32_t* vcontrol,
+                           const uint32_t* picks, int n_picks) {
+  if (b && !filters) return bfail(b, EKF_ERR_ARG, "filters is NULL");
+  return batch_step(b, dv, dw, 0, vcontrol, true, picks, n_picks, filters, n);
 }
 
 int ekf_batch_convert2xyz_if_linear_all(ekf_batch* b) {
@@ -2369,6 +2533,7 @@ int ekf_batch_set_full(ekf_batch* b, int f, const double* mu, const double* sigm
   BCHECK(cudaMemcpy2DAsync(b->bv.Sigma + (size_t)f * b->bv.sstride, sizeof(double) * b->ld, sigma, sizeof(double) * ld,
                            sizeof(double) * n, n, cudaMemcpyHostToDevice, b->stream));
   BCHECK(cudaStreamSynchronize(b->stream));
+  b->rows_stale = true;
   return EKF_OK;
 }
 
@@ -2406,7 +2571,8 @@ int ekf_batch_get_feature(ekf_batch* b, int f, int idx, ekf_feature_info* o) {
 int ekf_batch_add_feature(ekf_batch* b, int f, float u, float v) {
   if (!b || f < 0 || f >= b->B) return EKF_ERR_ARG;
   if (!b->seeded) return bfail(b, EKF_ERR_STATE, "addFeature before ekf_batch_seed_from");
-  if (!b->have_frame) return bfail(b, EKF_ERR_STATE, "addFeature before captureNewFrame");
+  const int rc = need_frame(b, f, "addFeature");
+  if (rc) return rc;
   BCHECK(cudaSetDevice(b->device));
   const int half = b->cfg.window_size / 2;
   // isInsideImage (vslamRansac.cpp:314,1644-1652), as ekf_add_feature
@@ -2414,14 +2580,22 @@ int ekf_batch_add_feature(ekf_batch* b, int f, float u, float v) {
   const int c = b->cam_host[f], fw = b->fsize_on ? b->fsize_host[4 * c + 2] : b->fv.w, fh = b->fsize_on ? b->fsize_host[4 * c + 3] : b->fv.h;
   if (!(x > half && y > half && x < fw - half && y < fh - half)) return 0;
   if (b->h_N[f] >= b->Ncap || b->h_n[f] + 6 > b->ncap) return bfail(b, EKF_ERR_CAPACITY, "feature capacity exceeded");
-  auto* const add = b->large ? (b->bv.cam ? k_batch_add<true, true> : k_batch_add<true, false>)
-                             : (b->bv.cam ? k_batch_add<false, true> : k_batch_add<false, false>);
-  add<<<1, BADD_THREADS, 0, b->stream>>>(b->bv, b->fv, b->dcfg, nullptr, nullptr, f, u, v, 0, b->cam_dev);
+  add_kernel(b, false)<<<1, BADD_THREADS, 0, b->stream>>>(b->bv, b->fv, b->dcfg, nullptr, nullptr, f, u, v, 0, b->cam_dev, nullptr);
   b->launches += 1;
   BCHECK(cudaGetLastError());
   b->h_N[f] += 1;
   b->h_n[f] += 6;
   return 1;
+}
+
+// EKF_ERR_STATE unless the camera of every filter that asks for corners (num[f * stride] > 0) holds a frame
+static int need_frames_asked(ekf_batch* b, const int* num, int stride) {
+  for (int f = 0; f < b->B; ++f) {
+    if (num[(size_t)f * stride] <= 0) continue;
+    const int rc = need_frame(b, f, "findNewFeatures");
+    if (rc) return rc;
+  }
+  return EKF_OK;
 }
 
 static int batch_stage_num(ekf_batch* b, const int32_t* num) {
@@ -2433,11 +2607,12 @@ static int batch_stage_num(ekf_batch* b, const int32_t* num) {
 int ekf_batch_detect_corners(ekf_batch* b, const int32_t* num, float* out_xy, int32_t* out_n) {
   if (!b || !num || !out_xy || !out_n) return EKF_ERR_ARG;
   if (!b->seeded) return bfail(b, EKF_ERR_STATE, "findNewFeatures before ekf_batch_seed_from");
-  if (!b->have_frame) return bfail(b, EKF_ERR_STATE, "findNewFeatures before captureNewFrame");
+  int rc = need_frames_asked(b, num, 1);
+  if (rc) return rc;
   BCHECK(cudaSetDevice(b->device));
   cudaStream_t st = b->stream;
   const size_t Bn = (size_t)b->B;
-  int rc = batch_stage_num(b, num);
+  rc = batch_stage_num(b, num);
   if (rc) return rc;
   rc = batch_detect(b, b->det_num, b->h_num, 1, 0);
   if (rc) return rc;
@@ -2456,10 +2631,11 @@ int ekf_batch_detect_corners(ekf_batch* b, const int32_t* num, float* out_xy, in
 int ekf_batch_find_new_features(ekf_batch* b, const int32_t* num, int32_t* added) {
   if (!b) return EKF_ERR_ARG;
   if (!b->seeded) return bfail(b, EKF_ERR_STATE, "findNewFeatures before ekf_batch_seed_from");
-  if (!b->have_frame) return bfail(b, EKF_ERR_STATE, "findNewFeatures before captureNewFrame");
   if (!num && !b->results_valid) return bfail(b, EKF_ERR_STATE, "findNewFeatures(EKF_BSTAT_TOPUP) without a completed step");
+  int rc = num ? need_frames_asked(b, num, 1) : need_frames_asked(b, b->h_stats + EKF_BSTAT_TOPUP, EKF_BATCH_STAT_FIELDS);
+  if (rc) return rc;
   BCHECK(cudaSetDevice(b->device));
-  int rc = num ? batch_stage_num(b, num) : EKF_OK;
+  rc = num ? batch_stage_num(b, num) : EKF_OK;
   if (rc) return rc;
   rc = num ? batch_topup(b, b->det_num, b->h_num, 1, 0)
            : batch_topup(b, b->out_stats + EKF_BSTAT_TOPUP, b->h_stats + EKF_BSTAT_TOPUP, EKF_BATCH_STAT_FIELDS, 0);

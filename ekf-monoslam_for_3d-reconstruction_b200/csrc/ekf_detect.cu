@@ -200,14 +200,18 @@ __device__ __forceinline__ void resize_coeff(int d, double scale, int ssize, int
   *a0 = (short)__float2int_rn((1.f - f) * 2048.f);
   *a1 = (short)__float2int_rn(f * 2048.f);
 }
+// SLOTS: frame z of the source stack goes to slot slot[z] of the destination stack (a capture of some cameras of a batch).
+template <bool SLOTS>
 __global__ void k_capture_resize_gray(const uint8_t* __restrict__ src, int sw, int sh, int sstride, int cn, uint8_t* __restrict__ dst,
-                                      int dw, int dh, int dstride, const int* __restrict__ fsize) {
+                                      int dw, int dh, int dstride, const int* __restrict__ fsize, const int* __restrict__ slot) {
   const int x = blockIdx.x * blockDim.x + threadIdx.x, y = blockIdx.y;
   if (x >= dw || y >= dh) return;
-  src += (size_t)blockIdx.z * sh * sstride;   // frame z of a stack (batched cameras)
-  dst += (size_t)blockIdx.z * dh * dstride;
+  int z = blockIdx.z;
+  src += (size_t)z * sh * sstride;   // frame z of a stack (batched cameras)
+  if constexpr (SLOTS) z = slot[z];
+  dst += (size_t)z * dh * dstride;
   if (fsize) {   // frame z is the top-left fsize[0] x fsize[1] of its slot, resized to fsize[2] x fsize[3] (cv::resize of the crop)
-    const int* q = fsize + 4 * blockIdx.z;
+    const int* q = fsize + 4 * z;
     sw = q[0]; sh = q[1]; dw = q[2]; dh = q[3];
     if (x >= dw || y >= dh) return;
   }
@@ -239,7 +243,9 @@ __global__ void k_capture_resize_gray(const uint8_t* __restrict__ src, int sw, i
   dst[(size_t)y * dstride + x] = (uint8_t)min(max(g, 0), 255);
 }
 void launch_capture_resize_gray(cudaStream_t st, const uint8_t* src, int sw, int sh, int sstride, int cn, uint8_t* dst, int dw, int dh,
-                                int dstride, long long* launches, int n_frames, const int* fsize) {
-  k_capture_resize_gray<<<dim3((dw + 255) / 256, dh, n_frames), 256, 0, st>>>(src, sw, sh, sstride, cn, dst, dw, dh, dstride, fsize);
+                                int dstride, long long* launches, int n_frames, const int* fsize, const int* slot) {
+  const dim3 grid((dw + 255) / 256, dh, n_frames);
+  if (slot) k_capture_resize_gray<true><<<grid, 256, 0, st>>>(src, sw, sh, sstride, cn, dst, dw, dh, dstride, fsize, slot);
+  else k_capture_resize_gray<false><<<grid, 256, 0, st>>>(src, sw, sh, sstride, cn, dst, dw, dh, dstride, fsize, slot);
   *launches += 1;
 }

@@ -35,7 +35,8 @@ void launch_match_filter(cudaStream_t st, FeatTab ft, int N, FrameView fr, const
 void launch_match_filter_batch(cudaStream_t st, FeatTab base, int Ncap, const int* Nper, int B, FrameView fr, const DevCfg& cfg,
                                const EkfTensorMap* tmap, int* defer_list, int* defer_cnt, long long* launches,
                                const int* cam_of = nullptr,    // cam_of [B]: filter b searches frame cam_of[b] of the stack fr
-                               const int* fsize = nullptr);    // [n_cameras][4] (in w, in h, w, h): camera c is the top-left w x h of its slot
+                               const int* fsize = nullptr,     // [n_cameras][4] (in w, in h, w, h): camera c is the top-left w x h of its slot
+                               const int* act = nullptr);      // [B]: the pairs' filter i is filter act[i] (a list of B filters)
 int launch_match_batch(cudaStream_t st, const uint8_t* frames, int n_frames, int width, int height, int stride,
                        const uint8_t* templates, int fpf, int w, const double* h, const double* S, float sigma_size,
                        float thr, float clampv, int32_t* out_uv, float* out_score);
@@ -124,7 +125,8 @@ int launch_detect_corners(cudaStream_t st, FrameView fr, FeatTab ft, int N, int 
 void launch_det_eig(cudaStream_t st, FrameView fr, float* eig, long long* launches);
 void launch_capture_resize_gray(cudaStream_t st, const uint8_t* src, int sw, int sh, int sstride, int cn, uint8_t* dst, int dw, int dh,
                                 int dstride, long long* launches, int n_frames = 1,    // n_frames: a contiguous stack, frame z in blockIdx.z
-                                const int* fsize = nullptr);   // [n_frames][4]: frame z resizes its top-left fsize[0..1] to fsize[2..3]
+                                const int* fsize = nullptr,    // [n_frames][4]: frame z resizes its top-left fsize[0..1] to fsize[2..3]
+                                const int* slot = nullptr);    // [n_frames]: frame z goes to slot slot[z] of dst (and reads fsize row slot[z])
 // ekf_batch_detect.cu: findNewFeatures' detection for every filter of a batch (one frame, per-filter masks)
 struct BatchDetectBufs {
   float* eig = nullptr;                 // [cap] min-eigenvalue map

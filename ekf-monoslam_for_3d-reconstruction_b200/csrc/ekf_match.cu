@@ -1060,17 +1060,26 @@ __device__ __forceinline__ FrameView batch_frame_of(FrameView fr, const int* __r
   return fr;
 }
 
+// ACT (ekf_batch_step_filters): the pairs run over the B = n listed filters, the list's entry i being filter act[i]; the deferred
+// list keeps the pair of the filter itself, b * Ncap + f.  Without a list the kernels are the code they were before.
+template <bool ACT>
+__device__ __forceinline__ int batch_pair_filter(const int* __restrict__ act, int i) {
+  if constexpr (ACT) return act[i];
+  else return i;
+}
+
 // Batched filters, pass 1 with the full-window warp matcher (template side 11): one warp per (filter, feature)
-template <int MINB, bool TSMEM, bool SLIDE, bool CAMS, bool SIZES>
+template <int MINB, bool TSMEM, bool SLIDE, bool CAMS, bool SIZES, bool ACT>
 __global__ void __launch_bounds__(MW2_WARPS * 32, MINB) k_match_filter_batch_warp2(FeatTab base, int Ncap, const int* __restrict__ Nper, int B,
                                                                                 FrameView fr, DevCfg cfg, int* __restrict__ defer_list,
                                                                                 int* __restrict__ defer_cnt, const int* __restrict__ cam_of,
-                                                                                const int* __restrict__ fsize) {
+                                                                                const int* __restrict__ fsize, const int* __restrict__ act) {
   __shared__ MatchWarp2Smem<11> wsm[MW2_WARPS];
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const long long pair = (long long)blockIdx.x * MW2_WARPS + warp;
-  if (pair >= (long long)B * Ncap) return;
-  const int b = (int)(pair / Ncap), f = (int)(pair - (long long)b * Ncap);
+  const long long pair_i = (long long)blockIdx.x * MW2_WARPS + warp;
+  if (pair_i >= (long long)B * Ncap) return;
+  const int i = (int)(pair_i / Ncap), f = (int)(pair_i - (long long)i * Ncap), b = batch_pair_filter<ACT>(act, i);
+  const long long pair = ACT ? (long long)b * Ncap + f : pair_i;
   const FeatTab ft = feattab_slice(base, b, Ncap, cfg.tstride);
   if (f >= Nper[b] || !ft.innov[f]) return;
   MatchJob jb;
@@ -1092,16 +1101,18 @@ __global__ void __launch_bounds__(MW2_WARPS * 32, MINB) k_match_filter_batch_war
 }
 
 // Batched filters, pass 1: one warp per (filter, feature); features that do not fit go to defer_list.
-template <bool CAMS, bool SIZES>
+template <bool CAMS, bool SIZES, bool ACT>
 __global__ void __launch_bounds__(MW_WARPS * 32) k_match_filter_batch_warp(FeatTab base, int Ncap, const int* __restrict__ Nper, int B,
                                                                            FrameView fr, DevCfg cfg, int* __restrict__ defer_list,
                                                                            int* __restrict__ defer_cnt, int warp_path,
-                                                                           const int* __restrict__ cam_of, const int* __restrict__ fsize) {
+                                                                           const int* __restrict__ cam_of, const int* __restrict__ fsize,
+                                                                           const int* __restrict__ act) {
   __shared__ MatchWarpSmem wsm[MW_WARPS];
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const long long pair = (long long)blockIdx.x * MW_WARPS + warp;
-  if (pair >= (long long)B * Ncap) return;
-  const int b = (int)(pair / Ncap), f = (int)(pair - (long long)b * Ncap);
+  const long long pair_i = (long long)blockIdx.x * MW_WARPS + warp;
+  if (pair_i >= (long long)B * Ncap) return;
+  const int i = (int)(pair_i / Ncap), f = (int)(pair_i - (long long)i * Ncap), b = batch_pair_filter<ACT>(act, i);
+  const long long pair = ACT ? (long long)b * Ncap + f : pair_i;
   const FeatTab ft = feattab_slice(base, b, Ncap, cfg.tstride);
   if (f >= Nper[b] || !ft.innov[f]) return;
   const int w = cfg.window, w2 = w * w;
@@ -1280,7 +1291,7 @@ void launch_match_filter(cudaStream_t st, FeatTab ft, int N, FrameView fr, const
 
 void launch_match_filter_batch(cudaStream_t st, FeatTab base, int Ncap, const int* Nper, int B, FrameView fr, const DevCfg& cfg,
                                const EkfTensorMap* tmap, int* defer_list, int* defer_cnt, long long* launches, const int* cam_of,
-                               const int* fsize) {
+                               const int* fsize, const int* act) {
   if (B <= 0 || Ncap <= 0) return;
   static PerDeviceOnce once;   // opt in to the largest supported window once per device
   const size_t smem = match_smem_bytes(cfg.window, cfg.search_clamp);
@@ -1301,10 +1312,13 @@ void launch_match_filter_batch(cudaStream_t st, FeatTab base, int Ncap, const in
   if (warp_path >= 2 && cfg.window == 11 && cfg.search_clamp <= 20.0f) {
     const unsigned grid = (unsigned)((pairs + MW2_WARPS - 1) / MW2_WARPS);
     const int var = match_w2_variant();
-#define MW2_LAUNCH(MINB, TS, SL)                                                                                                        \
-  if (fsize) k_match_filter_batch_warp2<MINB, TS, SL, true, true><<<grid, MW2_WARPS * 32, 0, st>>>(base, Ncap, Nper, B, fr, cfg, defer_list, defer_cnt, cam_of, fsize); \
-  else if (cam_of) k_match_filter_batch_warp2<MINB, TS, SL, true, false><<<grid, MW2_WARPS * 32, 0, st>>>(base, Ncap, Nper, B, fr, cfg, defer_list, defer_cnt, cam_of, fsize); \
-  else k_match_filter_batch_warp2<MINB, TS, SL, false, false><<<grid, MW2_WARPS * 32, 0, st>>>(base, Ncap, Nper, B, fr, cfg, defer_list, defer_cnt, cam_of, fsize)
+#define MW2_LAUNCH_ACT(MINB, TS, SL, ACT)                                                                                               \
+  if (fsize) k_match_filter_batch_warp2<MINB, TS, SL, true, true, ACT><<<grid, MW2_WARPS * 32, 0, st>>>(base, Ncap, Nper, B, fr, cfg, defer_list, defer_cnt, cam_of, fsize, act); \
+  else if (cam_of) k_match_filter_batch_warp2<MINB, TS, SL, true, false, ACT><<<grid, MW2_WARPS * 32, 0, st>>>(base, Ncap, Nper, B, fr, cfg, defer_list, defer_cnt, cam_of, fsize, act); \
+  else k_match_filter_batch_warp2<MINB, TS, SL, false, false, ACT><<<grid, MW2_WARPS * 32, 0, st>>>(base, Ncap, Nper, B, fr, cfg, defer_list, defer_cnt, cam_of, fsize, act)
+#define MW2_LAUNCH(MINB, TS, SL)                   \
+  if (act) { MW2_LAUNCH_ACT(MINB, TS, SL, true); } \
+  else { MW2_LAUNCH_ACT(MINB, TS, SL, false); }
     switch (var) {
       case 0: MW2_LAUNCH(2, false, false); break;
       case 2: MW2_LAUNCH(3, true, false); break;
@@ -1314,11 +1328,16 @@ void launch_match_filter_batch(cudaStream_t st, FeatTab base, int Ncap, const in
       default: MW2_LAUNCH(2, true, false); break;   // 1
     }
 #undef MW2_LAUNCH
+#undef MW2_LAUNCH_ACT
   } else {
     const unsigned grid = (unsigned)((pairs + MW_WARPS - 1) / MW_WARPS);
-    if (fsize) k_match_filter_batch_warp<true, true><<<grid, MW_WARPS * 32, 0, st>>>(base, Ncap, Nper, B, fr, cfg, defer_list, defer_cnt, warp_path, cam_of, fsize);
-    else if (cam_of) k_match_filter_batch_warp<true, false><<<grid, MW_WARPS * 32, 0, st>>>(base, Ncap, Nper, B, fr, cfg, defer_list, defer_cnt, warp_path, cam_of, fsize);
-    else k_match_filter_batch_warp<false, false><<<grid, MW_WARPS * 32, 0, st>>>(base, Ncap, Nper, B, fr, cfg, defer_list, defer_cnt, warp_path, cam_of, fsize);
+#define MW_LAUNCH(ACT)                                                                                                                \
+  if (fsize) k_match_filter_batch_warp<true, true, ACT><<<grid, MW_WARPS * 32, 0, st>>>(base, Ncap, Nper, B, fr, cfg, defer_list, defer_cnt, warp_path, cam_of, fsize, act); \
+  else if (cam_of) k_match_filter_batch_warp<true, false, ACT><<<grid, MW_WARPS * 32, 0, st>>>(base, Ncap, Nper, B, fr, cfg, defer_list, defer_cnt, warp_path, cam_of, fsize, act); \
+  else k_match_filter_batch_warp<false, false, ACT><<<grid, MW_WARPS * 32, 0, st>>>(base, Ncap, Nper, B, fr, cfg, defer_list, defer_cnt, warp_path, cam_of, fsize, act)
+    if (act) { MW_LAUNCH(true); }
+    else { MW_LAUNCH(false); }
+#undef MW_LAUNCH
   }
   int dev = 0, sms = 148;
   if (cudaGetDevice(&dev) == cudaSuccess) cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);

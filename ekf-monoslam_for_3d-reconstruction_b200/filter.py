@@ -376,11 +376,18 @@ class FilterBatch:
         self.n_cameras = int(n)
         self.frame_sizes = None
 
-    def _stamps(self, stamps):
+    def _stamps(self, stamps, n=None):
         if stamps is None:
             return None
-        s = np.ascontiguousarray(np.broadcast_to(np.asarray(stamps, dtype=np.float64), (self.n_cameras,)))
+        s = np.ascontiguousarray(np.broadcast_to(np.asarray(stamps, dtype=np.float64), (self.n_cameras if n is None else n,)))
         return s
+
+    @staticmethod
+    def _list(ids, what):
+        a = np.ascontiguousarray(ids, dtype=np.int32).reshape(-1)
+        if a.size < 1:
+            raise ValueError(f"{what} must list at least one entry")
+        return a
 
     def set_frame_sizes(self, sizes):
         """A frame size per camera: (n_cameras, 2) width, height in input pixels (before the resize by 1 / scale), or None for the
@@ -396,38 +403,56 @@ class FilterBatch:
         self._ck(self.L.ekf_batch_set_frame_sizes(self.h, _ptr(a)))
         self.frame_sizes = a.copy()
 
-    def captureNewFrames(self, frames, stamps=None):
+    def captureNewFrames(self, frames, stamps=None, cameras=None):
         """captureNewFrame for every camera: frames is (n_cameras, H, W) gray or (n_cameras, H, W, 3) BGR uint8 (host),
         stamps one per camera or None.  A strided (n, H, W) view with padded rows is passed as it is.  With set_frame_sizes,
         frames may also be a list of per-camera arrays of the declared sizes; they are packed into a zero-padded stack whose
-        slot is the largest width and height."""
+        slot is the largest width and height.
+        cameras: capture these cameras only (ekf_batch_capture_camera_frames): frames is then (len(cameras), H, W[, 3]) or a
+        list of per-camera arrays of the declared sizes, in list order, and stamps one per listed camera.  The other cameras
+        keep their frames and clocks."""
+        cams = None if cameras is None else self._list(cameras, "cameras")
+        n = self.n_cameras if cams is None else cams.size
         if isinstance(frames, (list, tuple)):
-            if self.frame_sizes is None or len(frames) != self.n_cameras:
-                raise ValueError("a list of frames needs set_frame_sizes and one frame per camera")
+            if self.frame_sizes is None or len(frames) != n:
+                raise ValueError("a list of frames needs set_frame_sizes and one frame per (listed) camera")
+            ids = range(n) if cams is None else [int(c) for c in cams]
             fl = [np.asarray(x, dtype=np.uint8) for x in frames]
-            for c, x in enumerate(fl):
+            for c, x in zip(ids, fl):
                 if x.shape[:2] != (int(self.frame_sizes[c, 1]), int(self.frame_sizes[c, 0])) or x.ndim != fl[0].ndim:
-                    raise ValueError(f"frame {c} has shape {x.shape}, camera {c} is {tuple(self.frame_sizes[c])} (width, height)")
+                    raise ValueError(f"frame of camera {c} has shape {x.shape}, camera {c} is {tuple(self.frame_sizes[c])} (width, height)")
             H, W = int(self.frame_sizes[:, 1].max()), int(self.frame_sizes[:, 0].max())
             frames = np.zeros((len(fl), H, W) + fl[0].shape[2:], np.uint8)
-            for c, x in enumerate(fl):
-                frames[c, :x.shape[0], :x.shape[1]] = x
+            for k, x in enumerate(fl):
+                frames[k, :x.shape[0], :x.shape[1]] = x
         f = np.asarray(frames, dtype=np.uint8)
-        if f.shape[0] != self.n_cameras or f.ndim not in (3, 4):
-            raise ValueError(f"captureNewFrames expects ({self.n_cameras}, H, W) or ({self.n_cameras}, H, W, 3) uint8")
+        if f.ndim not in (3, 4) or f.shape[0] != n:
+            raise ValueError(f"captureNewFrames expects ({n}, H, W) or ({n}, H, W, 3) uint8")
         rowb = f.shape[2] * (3 if f.ndim == 4 else 1)
         if not (f.strides[-1] == 1 and (f.ndim == 3 or f.strides[2] == 3) and f.strides[1] >= rowb
                 and f.strides[0] == f.strides[1] * f.shape[1]):
             f = np.ascontiguousarray(f)
-        s = self._stamps(stamps)
-        fn = self.L.ekf_batch_capture_frames_bgr if f.ndim == 4 else self.L.ekf_batch_capture_frames
-        self._ck(fn(self.h, _ptr(f), f.shape[2], f.shape[1], f.strides[1], _ptr(s) if s is not None else None))
+        s = self._stamps(stamps, n)
+        sp = _ptr(s) if s is not None else None
+        if cams is None:
+            fn = self.L.ekf_batch_capture_frames_bgr if f.ndim == 4 else self.L.ekf_batch_capture_frames
+            self._ck(fn(self.h, _ptr(f), f.shape[2], f.shape[1], f.strides[1], sp))
+        else:
+            fn = self.L.ekf_batch_capture_camera_frames_bgr if f.ndim == 4 else self.L.ekf_batch_capture_camera_frames
+            self._ck(fn(self.h, int(n), _ptr(cams), _ptr(f), f.shape[2], f.shape[1], f.strides[1], sp))
 
-    def captureNewFrames_device(self, dev_ptr, width, height, stride, stamps=None):
-        """captureNewFrames from a gray stack in device memory: frame c at dev_ptr + c * height * stride."""
-        s = self._stamps(stamps)
-        self._ck(self.L.ekf_batch_capture_frames_device(self.h, C.c_void_p(int(dev_ptr)), int(width), int(height), int(stride),
-                                                        _ptr(s) if s is not None else None))
+    def captureNewFrames_device(self, dev_ptr, width, height, stride, stamps=None, cameras=None):
+        """captureNewFrames from a gray stack in device memory: frame c at dev_ptr + c * height * stride.  cameras: the
+        stack holds len(cameras) frames, frame k camera cameras[k]'s (ekf_batch_capture_camera_frames_device)."""
+        if cameras is None:
+            s = self._stamps(stamps)
+            self._ck(self.L.ekf_batch_capture_frames_device(self.h, C.c_void_p(int(dev_ptr)), int(width), int(height), int(stride),
+                                                            _ptr(s) if s is not None else None))
+            return
+        cams = self._list(cameras, "cameras")
+        s = self._stamps(stamps, cams.size)
+        self._ck(self.L.ekf_batch_capture_camera_frames_device(self.h, int(cams.size), _ptr(cams), C.c_void_p(int(dev_ptr)), int(width),
+                                                               int(height), int(stride), _ptr(s) if s is not None else None))
 
     INTRINSICS = ("fx", "fy", "u0", "v0", "k1", "k2", "k3", "p1", "p2")
 
@@ -469,13 +494,22 @@ class FilterBatch:
         """EkfConfig.forsePlane for every filter (vslamRansac.cpp:1245-1272; default off)."""
         self._ck(self.L.ekf_batch_set_force_plane(self.h, int(bool(on))))
 
-    def step(self, picks=None, dv=(0.0, 0.0, 0.0), dw=(0.0, 0.0, 0.0), vcontrol=False):
+    def step(self, picks=None, dv=(0.0, 0.0, 0.0), dw=(0.0, 0.0, 0.0), vcontrol=False, filters=None):
         """predict + update of every filter.  dv / dw are 3-vectors for every filter, or (n_filters, 3) arrays with vcontrol
-        a bool or an (n_filters,) array: controls per filter (ekf_batch_step_controls)."""
+        a bool or an (n_filters,) array: controls per filter (ekf_batch_step_controls).
+        filters: step these filters only (strictly ascending; ekf_batch_step_filters), the others stay as they are; dv / dw
+        are then (3,) or (len(filters), 3) and vcontrol a bool or a (len(filters),) array."""
         p = np.ascontiguousarray(picks if picks is not None else np.zeros(0), dtype=np.uint32)
         a = np.ascontiguousarray(dv, dtype=np.float64); b = np.ascontiguousarray(dw, dtype=np.float64)
         vc = np.asarray(vcontrol)
         self._cams = None
+        if filters is not None:
+            fl = self._list(filters, "filters")
+            n = fl.size
+            a = np.ascontiguousarray(np.broadcast_to(a, (n, 3))); b = np.ascontiguousarray(np.broadcast_to(b, (n, 3)))
+            v = np.ascontiguousarray(np.broadcast_to(vc, (n,)), dtype=np.int32)
+            self._ck(self.L.ekf_batch_step_filters(self.h, int(n), _ptr(fl), _ptr(a), _ptr(b), _ptr(v), _ptr(p), int(p.size)))
+            return
         if a.shape == (3,) and b.shape == (3,) and vc.ndim == 0:
             self._ck(self.L.ekf_batch_step(self.h, _ptr(a), _ptr(b), int(bool(vc)), _ptr(p), int(p.size)))
             return

@@ -311,7 +311,26 @@ int ekf_batch_set_frame_sizes(ekf_batch* b, const int32_t* wh);
 int ekf_batch_capture_frames(ekf_batch* b, const uint8_t* gray, int width, int height, int stride, const double* stamps);
 int ekf_batch_capture_frames_device(ekf_batch* b, const uint8_t* gray_dev, int width, int height, int stride, const double* stamps);
 int ekf_batch_capture_frames_bgr(ekf_batch* b, const uint8_t* bgr, int width, int height, int stride, const double* stamps);
-/* returnGrayImg for one camera (out may be NULL to query the size); EKF_ERR_ARG for a bad camera, EKF_ERR_STATE before a frame. */
+/* captureNewFrame for the listed cameras only: frame k of the stack (img + k * height * stride) is camera cameras[k]'s, and
+ * stamps (n entries or NULL) follow the same order.  Cameras that are not listed keep their frame, time stamp and dT.
+ * cameras holds 1 <= n distinct cameras in [0, n_cameras), in any order; else EKF_ERR_ARG and nothing changes.
+ * Each camera has a frame from the capture that last listed it (a capture of every camera lists all); ekf_batch_set_cameras
+ * and ekf_batch_set_frame_sizes forget every frame.  The frames go into the stack's slots: the first capture after the
+ * frames were forgotten defines the slot (width / scale x height / scale), and the other cameras stay without a frame; while
+ * some camera holds a frame, a call whose resized slot (or frame sizes) differs returns EKF_ERR_ARG, and only a capture of
+ * every camera may change it.  Scale, BGR input and frame sizes act camera by camera as in a capture of every camera, and
+ * a listed camera's frame is bit-identical to the one such a capture of the same image produces (its pads zeroed).  Each
+ * listed camera applies the single filter's stamp rule, so a camera captured twice between steps of its filters has the
+ * last interval.  Host frames go up in one copy per staging chunk, device frames are read in place, and one launch places
+ * (and resizes) the listed frames. */
+int ekf_batch_capture_camera_frames(ekf_batch* b, int n, const int32_t* cameras, const uint8_t* gray, int width, int height,
+                                    int stride, const double* stamps);
+int ekf_batch_capture_camera_frames_device(ekf_batch* b, int n, const int32_t* cameras, const uint8_t* gray_dev, int width,
+                                           int height, int stride, const double* stamps);
+int ekf_batch_capture_camera_frames_bgr(ekf_batch* b, int n, const int32_t* cameras, const uint8_t* bgr, int width, int height,
+                                        int stride, const double* stamps);
+/* returnGrayImg for one camera (out may be NULL to query the size); EKF_ERR_ARG for a bad camera, EKF_ERR_STATE while the
+ * camera holds no frame. */
 int ekf_batch_get_camera_frame(ekf_batch* b, int camera, uint8_t* out, int* width, int* height);
 /* getDt for every filter (HOST array of n_filters): its camera's dT. */
 int ekf_batch_get_dt(ekf_batch* b, double* out);
@@ -333,6 +352,18 @@ int ekf_batch_step(ekf_batch* b, const double dv[3], const double dw[3], int vco
  * NULL, meaning zeros).  picks stay shared. */
 int ekf_batch_step_controls(ekf_batch* b, const double* dv, const double* dw, const int32_t* vcontrol, const uint32_t* picks,
                             int n_picks);
+/* ekf_batch_step_controls for the listed filters only.  filters: 1 <= n filters, strictly ascending in [0, n_filters), else
+ * EKF_ERR_ARG and nothing changes.  dv / dw are n x 3 and vcontrol is n, in list order (any may be NULL, meaning zeros).  The
+ * picks are shared, as in ekf_batch_step.  Each listed filter runs exactly what ekf_batch_step_controls runs for it: predict
+ * (with blur if on), match, both updates, removals and archive, top-up if on, and XYZ conversion.  Every other filter stays
+ * bit-identical: state, covariance, feature table, both templates, archive and its overflow count, real_index counter.
+ * After the call ekf_batch_get_camera_states reports every filter's camera state and block as it stands; the counters
+ * (EKF_BSTAT_*), ekf_batch_last_added and ekf_batch_last_blur_counts are zero for the filters not listed, so
+ * ekf_batch_find_new_features(NULL) adds nothing to them.  EKF_ERR_STATE when a listed filter's camera holds no frame (as
+ * ekf_batch_step / ekf_batch_step_controls for any filter's).  The per-filter kernels run on the listed filters only, so the
+ * step's cost follows the list. */
+int ekf_batch_step_filters(ekf_batch* b, int n, const int32_t* filters, const double* dv, const double* dw,
+                           const int32_t* vcontrol, const uint32_t* picks, int n_picks);
 /* convert2XYZ_ifLinearAll (vslamRansac.cpp:776-780) on every filter of the batch. */
 int ekf_batch_convert2xyz_if_linear_all(ekf_batch* b);
 /* Results of the last step, HOST output arrays: camera state (n_filters x 14), 14 x 14 covariance
@@ -345,13 +376,16 @@ int ekf_batch_get_full(ekf_batch* b, int filter, double* mu, double* sigma, int 
 int ekf_batch_set_full(ekf_batch* b, int filter, const double* mu, const double* sigma, int ld);
 int ekf_batch_get_feature(ekf_batch* b, int filter, int idx, ekf_feature_info* out);
 /* VSlamFilter::addFeature (vslamRansac.cpp:309-371) on one filter of the batch: returns 1 added, 0 rejected by
- * isInsideImage, EKF_ERR_CAPACITY when the filter is full, EKF_ERR_STATE before a frame or before seeding.  The new
+ * isInsideImage, EKF_ERR_CAPACITY when the filter is full, EKF_ERR_STATE while the filter's camera holds no frame or before
+ * seeding.  The new
  * feature's real_index comes from the filter's own counter (seeded from the source filter's), as in ekf_add_feature. */
 int ekf_batch_add_feature(ekf_batch* b, int filter, float u, float v);
 /* findNewFeatures' detection alone (vslamRansac.cpp:783-831) for every filter: its own mask around its own patches, its
  * camera's frame.  num: HOST array of n_filters entries; filter b gets up to min(num[b], EKF_BATCH_MAX_CORNERS) corners
  * (none when num[b] <= 0), as (x, y) pairs in out_xy (n_filters x EKF_BATCH_MAX_CORNERS x 2 floats), their count in
- * out_n (n_filters).  Each filter's list equals ekf_detect_corners on a single filter holding the same patch centres. */
+ * out_n (n_filters).  Each filter's list equals ekf_detect_corners on a single filter holding the same patch centres.
+ * EKF_ERR_STATE when a filter that asks for corners follows a camera that holds no frame (here and in
+ * ekf_batch_find_new_features). */
 #define EKF_BATCH_MAX_CORNERS 32
 int ekf_batch_detect_corners(ekf_batch* b, const int32_t* num, float* out_xy, int32_t* out_n);
 /* VSlamFilter::findNewFeatures(num[b]) (vslamRansac.cpp:783-839) on every filter in one call: detection as above, then
