@@ -11,7 +11,7 @@ from .build import build  # noqa: F401
 
 
 def __getattr__(name):  # lazy: importing the package must not require the built library
-    if name in ("VSlamFilter", "EkfError", "match_batch", "FilterBatch", "nccl_unique_id", "load_nccl"):
+    if name in ("VSlamFilter", "EkfError", "match_batch", "FilterBatch", "systematic_ancestors", "nccl_unique_id", "load_nccl"):
         from . import filter as _f
         return getattr(_f, name)
     if name == "lib":

@@ -112,6 +112,7 @@ SIGNATURES = {
     "ekf_batch_capture_camera_frames_device": (_i, [_vp, _i, _vp, _vp, _i, _i, _i, _vp]),
     "ekf_batch_capture_camera_frames_bgr": (_i, [_vp, _i, _vp, _vp, _i, _i, _i, _vp]),
     "ekf_batch_step_filters": (_i, [_vp, _i, _vp, _vp, _vp, _vp, _vp, _i]),
+    "ekf_batch_resample": (_i, [_vp, _vp]),
     "ekf_dist_load_nccl": (_i, [C.c_char_p]),
     "ekf_dist_unique_id": (_i, [_vp]),
     "ekf_dist_attach": (_i, [_vp, _vp, _i, _i]),

@@ -29,6 +29,7 @@
 #include <cmath>
 #include <cstdio>
 #include <string>
+#include <type_traits>
 #include <vector>
 
 #include <cooperative_groups.h>
@@ -1533,6 +1534,80 @@ __global__ void k_batch_camera_rows(BatchView bv, double* __restrict__ out_mu14,
   else out_S14[(size_t)b * 196 + r - 14] = bv.Sigma[(size_t)b * bv.sstride + (size_t)((r - 14) / 14) * bv.ld + (r - 14) % 14];
 }
 
+// Everything of a filter that a later call reads (ekf_batch_resample), in a set of slots: the batch's own, or the staging slots of
+// filters that are both copied from and overwritten (Sigma in the compaction scratch, the rest in a temporary buffer).  All sets
+// share the batch's ld, sstride, Ncap, tstride and archive capacity.
+struct BatchSlots {
+  BatchView v;        // Sigma, mu, ft, ctl, n, N, patchnumbre, xyz_*; v.cam is not used (cam below)
+  BatchArchive ar;    // records, count, overflow; cap 0: no archive
+  CamParams* cam;     // intrinsics row; null: the batch has no table
+  double* mu14;       // [14] the camera rows ekf_batch_get_camera_states reports
+  double* S14;        // [196]
+  int* stats;         // [EKF_BATCH_STAT_FIELDS] the last step's counters (findNewFeatures(NULL) reads EKF_BSTAT_TOPUP)
+};
+
+// dst slot pairs[p].x <- src slot pairs[p].y, for p = blockIdx.x.  Sigma rows [0, n) are n * ld contiguous doubles: gridDim.y CTAs
+// share them in 16-byte vectors (sstride and ld are multiples of 8 doubles), four loads in flight a thread.  CTA y = 0 also copies
+// the rest: mu[0, n), the N table entries and templates, the pending XYZ decisions, the archive's held records, the rows.
+#define BRS_THREADS 256
+__global__ void __launch_bounds__(BRS_THREADS, 4) k_batch_resample(BatchSlots dst, BatchSlots src, const int2* __restrict__ pairs) {
+  const int2 pr = pairs[blockIdx.x];
+  const int d = pr.x, s = pr.y, tid = threadIdx.x;
+  const int n = src.v.n[s], N = src.v.N[s];
+  const double2* __restrict__ S = reinterpret_cast<const double2*>(src.v.Sigma + (size_t)s * src.v.sstride);
+  double2* __restrict__ D = reinterpret_cast<double2*>(dst.v.Sigma + (size_t)d * dst.v.sstride);
+  const size_t nv = (size_t)n * src.v.ld / 2, stride = (size_t)gridDim.y * BRS_THREADS;
+  size_t i = (size_t)blockIdx.y * BRS_THREADS + tid;
+  for (; i + 3 * stride < nv; i += 4 * stride) {
+    const double2 a = S[i], b = S[i + stride], c = S[i + 2 * stride], e = S[i + 3 * stride];
+    D[i] = a; D[i + stride] = b; D[i + 2 * stride] = c; D[i + 3 * stride] = e;
+  }
+  for (; i < nv; i += stride) D[i] = S[i];
+  if (blockIdx.y != 0) return;
+
+  const double* smu = src.v.mu + (size_t)s * src.v.ld;
+  double* dmu = dst.v.mu + (size_t)d * dst.v.ld;
+  for (int e = tid; e < n; e += BRS_THREADS) dmu[e] = smu[e];
+  const int Ncap = src.v.Ncap, ts = src.v.tstride;
+  const FeatTab a = feattab_slice(src.v.ft, s, Ncap, ts), o = feattab_slice(dst.v.ft, d, Ncap, ts);
+  const size_t ks = (size_t)s * Ncap, kd = (size_t)d * Ncap;
+  for (int f = tid; f < N; f += BRS_THREADS) {
+    o.pos[f] = a.pos[f]; o.coding[f] = a.coding[f]; o.innov[f] = a.innov[f]; o.li[f] = a.li[f]; o.hi[f] = a.hi[f];
+    o.removef[f] = a.removef[f]; o.n_tot[f] = a.n_tot[f]; o.n_find[f] = a.n_find[f]; o.real_index[f] = a.real_index[f];
+    o.pos_in_z[f] = a.pos_in_z[f]; o.sel[f] = a.sel[f]; o.quality[f] = a.quality[f]; o.last_ncc[f] = a.last_ncc[f];
+    dst.v.xyz_flag[kd + f] = src.v.xyz_flag[ks + f];
+  }
+  for (int e = tid; e < 2 * N; e += BRS_THREADS) { o.center[e] = a.center[e]; o.z[e] = a.z[e]; o.h[e] = a.h[e]; }
+  for (int e = tid; e < 4 * N; e += BRS_THREADS) o.S2[e] = a.S2[e];
+  for (int e = tid; e < 26 * N; e += BRS_THREADS) o.Hc[e] = a.Hc[e];
+  for (int e = tid; e < 18 * N; e += BRS_THREADS) dst.v.xyz_J[18 * kd + e] = src.v.xyz_J[18 * ks + e];
+  for (int e = tid; e < 3 * N; e += BRS_THREADS) dst.v.xyz_y[3 * kd + e] = src.v.xyz_y[3 * ks + e];
+  {   // both templates, tstride a multiple of 16 bytes
+    const uint4* __restrict__ p = reinterpret_cast<const uint4*>(a.patch);
+    const uint4* __restrict__ m = reinterpret_cast<const uint4*>(a.mpatch);
+    uint4* __restrict__ po = reinterpret_cast<uint4*>(o.patch);
+    uint4* __restrict__ mo = reinterpret_cast<uint4*>(o.mpatch);
+    for (int e = tid; e < N * ts / 16; e += BRS_THREADS) { po[e] = p[e]; mo[e] = m[e]; }
+  }
+  if (src.ar.cap > 0) {
+    const int held = src.ar.count[s];
+    const double* r = src.ar.rec + (size_t)s * src.ar.cap * PTS_COLS;
+    double* ro = dst.ar.rec + (size_t)d * dst.ar.cap * PTS_COLS;
+    for (int e = tid; e < held * PTS_COLS; e += BRS_THREADS) ro[e] = r[e];
+    for (int e = tid; e < held; e += BRS_THREADS) dst.ar.real_index[(size_t)d * dst.ar.cap + e] = src.ar.real_index[(size_t)s * src.ar.cap + e];
+    if (tid == 0) { dst.ar.count[d] = held; dst.ar.overflow[d] = src.ar.overflow[s]; }
+  }
+  if (tid < 14) dst.mu14[(size_t)d * 14 + tid] = src.mu14[(size_t)s * 14 + tid];
+  if (tid < 196) dst.S14[(size_t)d * 196 + tid] = src.S14[(size_t)s * 196 + tid];
+  if (tid < EKF_BATCH_STAT_FIELDS)
+    dst.stats[(size_t)d * EKF_BATCH_STAT_FIELDS + tid] = src.stats[(size_t)s * EKF_BATCH_STAT_FIELDS + tid];
+  if (tid == 0) {
+    dst.v.n[d] = n; dst.v.N[d] = N; dst.v.patchnumbre[d] = src.v.patchnumbre[s]; dst.v.xyz_count[d] = src.v.xyz_count[s];
+    dst.v.ctl[d] = src.v.ctl[s];
+    if (src.cam) dst.cam[d] = src.cam[s];
+  }
+}
+
 // frame z of a stack of dw x dh slots: every pixel outside the camera's fsize[4z + 2] x fsize[4z + 3] becomes 0.  SLOTS: frame z is
 // slot slot[z].
 template <bool SLOTS>
@@ -1606,6 +1681,7 @@ struct ekf_batch {
   int* h_over = nullptr;                        // pinned mirror of ar.overflow, read back with the step's n / N
   std::vector<int> over_seen;                   // ar.overflow at the last check
   int *pts_dev = nullptr, *h_pts = nullptr;     // [2][B] row counts and archive sizes of ekf_batch_get_points_features; pinned mirror
+  int2* rs_pairs = nullptr;                     // [2 * B] (destination, source) slot pairs of ekf_batch_resample's launches
   cudaEvent_t ev[4] = {nullptr, nullptr, nullptr, nullptr};
   std::string err;
 };
@@ -1663,6 +1739,7 @@ int ekf_batch_destroy(ekf_batch* b) {
   if (b->h_n) cudaFreeHost(b->h_n);
   if (b->h_N) cudaFreeHost(b->h_N);
   cudaFree(b->ar.rec); cudaFree(b->ar.real_index); cudaFree(b->ar.count); cudaFree(b->ar.overflow); cudaFree(b->pts_dev);
+  cudaFree(b->rs_pairs);
   if (b->h_over) cudaFreeHost(b->h_over);
   if (b->h_pts) cudaFreeHost(b->h_pts);
   for (auto& e : b->ev) if (e) cudaEventDestroy(e);
@@ -2794,6 +2871,111 @@ int ekf_batch_get_points_features(ekf_batch* b, int first, int count, double* ou
   for (int k = 0; k < count; ++k)   // the clear rule (R:395-403), on the device's archive of every exported filter
     if (pts_clears(b->h_pts[count + k])) BCHECK(cudaMemsetAsync(b->ar.count + first + k, 0, sizeof(int), st));
   BCHECK(cudaStreamSynchronize(st));
+  return EKF_OK;
+}
+
+// Filter f <- filter ancestors[f], both as they stood before the call.  Pairs with ancestors[f] != f move; a source that is itself
+// overwritten (ancestors[s] != s) is first staged, once however many destinations read it: its Sigma rows into its scratch slot
+// (the compaction scratch is idle between calls), everything else into a temporary buffer of one slot per staged filter.  Then
+// one launch copies the pairs whose source is not overwritten, and one the pairs whose source was staged.  The moved filters'
+// host mirrors (n, N, counters, camera rows, added and blur counts, archive overflow) follow on the host.
+static constexpr size_t kResampleBytesPerCta = (size_t)64 << 10;   // Sigma bytes one CTA of k_batch_resample copies, about
+int ekf_batch_resample(ekf_batch* b, const int32_t* ancestors) {
+  if (!b) return EKF_ERR_ARG;
+  if (!ancestors) return bfail(b, EKF_ERR_ARG, "ancestors is NULL");
+  for (int f = 0; f < b->B; ++f) {
+    const int a = ancestors[f];
+    if (a < 0 || a >= b->B)
+      return bfail(b, EKF_ERR_ARG, "ancestors[" + std::to_string(f) + "] = " + std::to_string(a) + " lies outside [0, n_filters)");
+    if (b->cam_host[a] != b->cam_host[f])
+      return bfail(b, EKF_ERR_ARG, "ancestors[" + std::to_string(f) + "] = " + std::to_string(a) + " follows camera " +
+                                       std::to_string(b->cam_host[a]) + ", filter " + std::to_string(f) + " camera " +
+                                       std::to_string(b->cam_host[f]));
+  }
+  if (!b->seeded) return bfail(b, EKF_ERR_STATE, "resample before ekf_batch_seed_from");
+  const int B = b->B;
+  std::vector<int> slot(B, -1);
+  std::vector<int2> stage, direct, staged;   // (staging slot, filter), (filter, filter), (filter, staging slot)
+  int most = 0;
+  for (int f = 0; f < B; ++f) {
+    const int a = ancestors[f];
+    if (a == f) continue;
+    most = std::max(most, b->h_n[a]);
+    if (ancestors[a] == a) { direct.push_back(make_int2(f, a)); continue; }
+    if (slot[a] < 0) { slot[a] = (int)stage.size(); stage.push_back(make_int2(slot[a], a)); }
+    staged.push_back(make_int2(f, slot[a]));
+  }
+  if (direct.empty() && staged.empty()) return EKF_OK;
+  BCHECK(cudaSetDevice(b->device));
+  cudaStream_t st = b->stream;
+  if (!b->rs_pairs) BCHECK(balloc(&b->rs_pairs, 2 * (size_t)B));
+  std::vector<int2> pairs(stage);
+  pairs.insert(pairs.end(), direct.begin(), direct.end());
+  pairs.insert(pairs.end(), staged.begin(), staged.end());
+  BCHECK(cudaMemcpyAsync(b->rs_pairs, pairs.data(), sizeof(int2) * pairs.size(), cudaMemcpyHostToDevice, st));
+  const BatchSlots live{b->bv, b->ar, b->intr_dev, b->out_mu14, b->out_S14, b->out_stats};
+  const unsigned ctas = (unsigned)std::max<size_t>(1, (sizeof(double) * most * b->ld + kResampleBytesPerCta - 1) / kResampleBytesPerCta);
+  const int2* pd = b->rs_pairs;
+  void* tmp = nullptr;
+  if (!stage.empty()) {
+    // the staging slots: Sigma in the scratch, the rest carved from one allocation (256-byte aligned arrays)
+    const size_t ns = stage.size(), nf = ns * b->Ncap, tsb = (size_t)b->bv.tstride;
+    BatchSlots sg = live;
+    sg.v.Sigma = b->scratch;
+    auto layout = [&](char* base) {
+      size_t off = 0;
+      auto take = [&](auto*& p, size_t count) {
+        using T = std::remove_reference_t<decltype(*p)>;
+        off = (off + 255) & ~(size_t)255;
+        p = reinterpret_cast<T*>(base + off);
+        off += sizeof(T) * count;
+      };
+      FeatTab& t = sg.v.ft;
+      take(sg.v.mu, ns * b->ld);
+      for (int** p : {&t.pos, &t.coding, &t.innov, &t.li, &t.hi, &t.removef, &t.n_tot, &t.n_find, &t.real_index, &t.pos_in_z, &t.sel})
+        take(*p, nf);
+      take(t.center, 2 * nf); take(t.quality, nf); take(t.last_ncc, nf);
+      take(t.z, 2 * nf); take(t.h, 2 * nf); take(t.Hc, 26 * nf); take(t.S2, 4 * nf);
+      take(t.patch, nf * tsb); take(t.mpatch, nf * tsb);
+      take(sg.v.ctl, ns); take(sg.v.n, ns); take(sg.v.N, ns); take(sg.v.patchnumbre, ns);
+      take(sg.v.xyz_flag, nf); take(sg.v.xyz_J, 18 * nf); take(sg.v.xyz_y, 3 * nf); take(sg.v.xyz_count, ns);
+      if (live.cam) take(sg.cam, ns);
+      if (b->ar.cap > 0) {
+        take(sg.ar.rec, ns * b->ar.cap * PTS_COLS); take(sg.ar.real_index, ns * b->ar.cap);
+        take(sg.ar.count, ns); take(sg.ar.overflow, ns);
+      }
+      take(sg.mu14, 14 * ns); take(sg.S14, 196 * ns); take(sg.stats, EKF_BATCH_STAT_FIELDS * ns);
+      return off;
+    };
+    const size_t bytes = layout(nullptr);
+    BCHECK(cudaMallocAsync(&tmp, bytes, st));
+    layout(static_cast<char*>(tmp));
+    k_batch_resample<<<dim3((unsigned)ns, ctas), BRS_THREADS, 0, st>>>(sg, live, pd);
+    b->launches += 1;
+    BCHECK(cudaGetLastError());
+    if (!direct.empty()) {
+      k_batch_resample<<<dim3((unsigned)direct.size(), ctas), BRS_THREADS, 0, st>>>(live, live, pd + ns);
+      b->launches += 1;
+    }
+    k_batch_resample<<<dim3((unsigned)staged.size(), ctas), BRS_THREADS, 0, st>>>(live, sg, pd + ns + direct.size());
+    b->launches += 1;
+    BCHECK(cudaGetLastError());
+    BCHECK(cudaFreeAsync(tmp, st));
+  } else {
+    k_batch_resample<<<dim3((unsigned)direct.size(), ctas), BRS_THREADS, 0, st>>>(live, live, pd);
+    b->launches += 1;
+    BCHECK(cudaGetLastError());
+  }
+  BCHECK(cudaStreamSynchronize(st));
+  auto follow = [&](auto* p, size_t width) {   // row f of a host mirror <- row ancestors[f]
+    using T = std::remove_reference_t<decltype(*p)>;
+    const std::vector<T> old(p, p + (size_t)B * width);
+    for (int f = 0; f < B; ++f) std::copy_n(old.begin() + (size_t)ancestors[f] * width, width, p + (size_t)f * width);
+  };
+  follow(b->h_n, 1); follow(b->h_N, 1); follow(b->h_added, 1); follow(b->h_xyz_count, 1);
+  follow(b->h_mu14, 14); follow(b->h_stats, EKF_BATCH_STAT_FIELDS);
+  follow(b->h_blur, 1); follow(b->h_blur + B, 1);   // [2][B]: blurred templates, then kernel too large
+  if (b->ar.cap > 0) { follow(b->h_over, 1); follow(b->over_seen.data(), 1); }
   return EKF_OK;
 }
 

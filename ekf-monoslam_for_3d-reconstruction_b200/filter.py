@@ -595,6 +595,16 @@ class FilterBatch:
         """Filter f's (rows, 12) matrix, as VSlamFilter.getPointsFeatures()."""
         return self.points_features(f, 1)[0]
 
+    def resample(self, ancestors):
+        """Filter f becomes an exact copy of filter ancestors[f] ((n_filters,) ints), both as they stood before the call
+        (ekf_batch_resample): state, covariance, feature table, templates, archive, intrinsics row, counters.  Every
+        ancestors[f] follows f's camera.  systematic_ancestors builds such a vector from weights."""
+        a = np.ascontiguousarray(ancestors, dtype=np.int32)
+        if a.shape != (self.B,):
+            raise ValueError(f"resample expects ({self.B},) ancestors")
+        self._cams = None
+        self._ck(self.L.ekf_batch_resample(self.h, _ptr(a)))
+
     def view(self, f):
         """Filter f as the object keyframes.KeyframeRecorder drives (getState, getSigma, Covariance_Parameter,
         getPointsFeatures, Point4sba).  Every view of the batch reads its camera state from one cached read-back per step."""
@@ -670,6 +680,40 @@ class FilterBatch:
         out = np.zeros(3, dtype=np.float32)
         self._ck(self.L.ekf_batch_last_step_ms(self.h, _ptr(out)))
         return dict(predict=float(out[0]), match=float(out[1]), update=float(out[2]))
+
+
+def systematic_ancestors(weights, u, camera_of=None):
+    """Ancestors for FilterBatch.resample from one weight per filter: systematic resampling with offset u in [0, 1), separately
+    within each camera's filters (camera_of: (n_filters,) ints, None: one group).  A group of M filters draws M times at
+    (u + k) / M of its cumulative normalised weight.  Every filter drawn at least once keeps its own slot; the extra copies
+    fill the slots of the filters not drawn, in ascending order, so no filter is both read and overwritten.  Equal weights
+    give the identity.  ValueError for negative or non-finite weights and for a group whose weights sum to 0."""
+    w = np.asarray(weights, dtype=np.float64)
+    if w.ndim != 1:
+        raise ValueError("weights must be one per filter")
+    if not np.all(np.isfinite(w)) or np.any(w < 0):
+        raise ValueError("weights must be finite and non-negative")
+    if not 0.0 <= float(u) < 1.0:
+        raise ValueError("u must lie in [0, 1)")
+    B = w.size
+    cam = np.zeros(B, dtype=np.int64) if camera_of is None else np.asarray(camera_of, dtype=np.int64)
+    if cam.shape != (B,):
+        raise ValueError("camera_of must be one camera per filter")
+    anc = np.arange(B, dtype=np.int32)
+    for c in np.unique(cam):
+        idx = np.flatnonzero(cam == c)
+        M = idx.size
+        top = w[idx].max()
+        if top <= 0:
+            raise ValueError(f"the weights of camera {int(c)} sum to 0")
+        cum = np.cumsum(w[idx] / top)   # scaled so that equal weights give exact integer steps
+        pos = (float(u) + np.arange(M)) * (cum[-1] / M)
+        draws = np.minimum(np.searchsorted(cum, pos, side="right"), M - 1)
+        count = np.bincount(draws, minlength=M)
+        extra = np.repeat(np.arange(M), np.maximum(count - 1, 0))
+        free = np.flatnonzero(count == 0)
+        anc[idx[free]] = idx[extra]
+    return anc
 
 
 class BatchFilterView:

@@ -435,6 +435,21 @@ int ekf_batch_get_deleted(ekf_batch* b, int filter, ekf_deleted_info* out, int c
  * records overwrite theirs in archive order (position * the filter's current map_scale = mu[13]; records past the last live
  * real_index are dropped).  After the export every exported filter whose archive holds more than 7000 records has it cleared. */
 int ekf_batch_get_points_features(ekf_batch* b, int first, int count, double* out, int rows_cap, int32_t* rows);
+/* Resampling of a multi-hypothesis ensemble: filter f becomes an exact copy of filter ancestors[f] (HOST array of n_filters
+ * entries), both as they stood before the call, so duplicates, swaps and cycles are all fine; ancestors[f] == f leaves f
+ * untouched, and the identity launches nothing.  What moves is everything of the filter that a later call reads: state and
+ * covariance, feature table, both templates, real_index counter, pending XYZ decisions, archive (with its overflow count,
+ * so the next step reports only new drops), intrinsics row (ekf_batch_set_intrinsics), counters, added and blur counts.
+ * Afterwards every per-filter accessor reports for f what it reported for ancestors[f] before the call: ekf_batch_get_full,
+ * _get_feature, _get_template, _num_features, _state_dim, _get_camera_states (camera rows and counters), _last_added,
+ * _last_blur_counts, _num_deleted, _get_deleted and _get_points_features; and every later call treats f as it treats its
+ * ancestor (a step that gives f its ancestor's controls produces its ancestor's bits).  ancestors[f] must lie in
+ * [0, n_filters) and follow f's camera (a hypothesis maps one camera's scene); otherwise EKF_ERR_ARG, ekf_batch_last_error
+ * names the first bad entry and nothing changes.  EKF_ERR_ARG for NULL, EKF_ERR_STATE before seeding; no frame is needed.
+ * A source that is itself overwritten is staged first (its covariance in the compaction scratch, the rest in a temporary
+ * buffer), which costs one more read and write of it; a vector from systematic resampling that keeps every drawn filter in
+ * its own slot never needs that.  Returns once the copy is done. */
+int ekf_batch_resample(ekf_batch* b, const int32_t* ancestors);
 /* which: 0 = Patch::patch, 1 = Patch::matching_patch of feature idx of one filter; out holds window_size^2 bytes */
 int ekf_batch_get_template(ekf_batch* b, int filter, int idx, int which, uint8_t* out);
 /* Kernels of this library launched on the batch so far. */
