@@ -1,6 +1,8 @@
 """ctypes mirrors of the structs in include/ekf_b200.h (kept field-for-field in sync)."""
 import ctypes as C
 
+import numpy as np
+
 STATE_DIM = 14  # vslamRansac.cpp:22
 
 EKF_OK, EKF_ERR_ARG, EKF_ERR_CUDA, EKF_ERR_CAPACITY, EKF_ERR_UNSUPPORTED, EKF_ERR_STATE = 0, -1, -2, -3, -4, -5
@@ -16,6 +18,70 @@ class EkfConfig(C.Structure):
         "window_size", "sigma_pixel", "kernel_size", "sigma_size", "scale",
         "nInitFeatures", "min_features", "max_features", "forsePlane",
         "ransac_nhyp0", "xyz_conversion", "abs_int_quirk")]
+
+
+class EkfFilterParams(C.Structure):
+    """ekf_filter_params: the ekf_config fields a filter of a batch may take on its own (ekf_batch_set_filter_params)."""
+    _fields_ = [(n, C.c_double) for n in (
+        "sigma_vx", "sigma_vy", "sigma_vz", "sigma_wx", "sigma_wy", "sigma_wz",
+        "rho_0", "sigma_rho_0", "T_camera", "ncc_threshold", "ransac_p", "li_threshold_factor", "hi_chi2_threshold",
+        "quality_ratio", "linearity_threshold")] + [(n, C.c_int32) for n in (
+        "sigma_pixel", "sigma_size", "min_features", "max_features", "ransac_nhyp0", "_pad")]
+
+
+# ekf_config fields every filter of a batch shares (buffer sizes, launch structure, emulation mode); intrinsics have their own
+# table (ekf_batch_set_intrinsics), nInitFeatures is never read by a batch.
+BATCH_SHARED_FIELDS = ("window_size", "search_clamp", "scale", "kernel_size", "forsePlane", "xyz_conversion", "abs_int_quirk")
+INTRINSICS = ("fx", "fy", "u0", "v0", "k1", "k2", "k3", "p1", "p2")
+
+
+def batch_rows(base, cfgs):
+    """The per-filter tables of a batch built from `base` whose filter f runs configuration cfgs[f]: an (n, 9) float64 array
+    of intrinsics (INTRINSICS order) and an array of n EkfFilterParams.  ValueError, naming the field and the filter, when a
+    field of BATCH_SHARED_FIELDS differs from base's or a row is one the C calls refuse."""
+    cfgs = list(cfgs)
+    cam = np.zeros((len(cfgs), 9), dtype=np.float64)
+    rows = (EkfFilterParams * len(cfgs))()
+    for f, c in enumerate(cfgs):
+        for name in BATCH_SHARED_FIELDS:
+            if getattr(c, name) != getattr(base, name):
+                raise ValueError(f"filter {f}: {name} = {getattr(c, name)} differs from the batch's {getattr(base, name)}; "
+                                 f"it is shared by every filter of a batch")
+        cam[f] = [getattr(c, n) for n in INTRINSICS]
+        for name, _ in EkfFilterParams._fields_:
+            if name != "_pad":
+                setattr(rows[f], name, getattr(c, name))
+        bad = _row_error(cam[f], rows[f])
+        if bad:
+            raise ValueError(f"filter {f}: {bad}")
+    return cam, rows
+
+
+def _row_error(cam, p):
+    """What ekf_batch_set_intrinsics / ekf_batch_set_filter_params refuse in one filter's rows (None when both are valid), so
+    that FilterBatch.set_configs can check every row before it changes either table."""
+    for n, v in zip(INTRINSICS, cam):
+        if not np.isfinite(v):
+            return f"{n} is not finite"
+    if not (cam[0] > 0 and cam[1] > 0):
+        return "fx / fy <= 0"
+    for name, t in EkfFilterParams._fields_:
+        if t is C.c_double and not np.isfinite(getattr(p, name)):
+            return f"{name} is not finite"
+    for name in ("sigma_vx", "sigma_vy", "sigma_vz", "sigma_wx", "sigma_wy", "sigma_wz", "sigma_rho_0"):
+        if getattr(p, name) < 0:
+            return f"{name} is negative"
+    if p.sigma_pixel < 1:
+        return "sigma_pixel < 1"
+    if p.sigma_size < 1:
+        return "sigma_size < 1"
+    if not 0 < p.ransac_p < 1:
+        return "ransac_p outside (0, 1)"
+    if p.ransac_nhyp0 < 1:
+        return "ransac_nhyp0 < 1"
+    if p.min_features < 0 or p.max_features < 0:
+        return "min_features / max_features negative"
+    return None
 
 
 def default_config(**over) -> EkfConfig:

@@ -67,16 +67,28 @@ struct BatchView {
   double* xyz_y;        // [B][Ncap][3] its XYZ point
   int* xyz_count;       // [B] conversions pending (k_batch_compact resets it)
   int* patchnumbre;     // [B] real_index of the filter's next new feature (VSlamFilter::patchnumbre)
-  const CamParams* cam; // [B] intrinsics of each filter (ekf_batch_set_intrinsics); null: every filter uses cfg.cam
+  const FilterRow* row; // [B] each filter's row (ekf_batch_set_intrinsics, ekf_batch_set_filter_params); null: every filter uses cfg
 };
 
-// The intrinsics filter b projects, linearises and unprojects with.  INTR: the batch has a table (kernels that project take it
-// as a template parameter, so that a batch without one runs the code it ran before).  A reference, so that the fields load
-// where they are used.
-template <bool INTR>
+// The configuration filter b runs: its intrinsics and tuning.  ROWS: the batch has per-filter rows (kernels that read the
+// row take it as a template parameter, so that a batch without rows runs the code it ran before).  A reference, so that the
+// fields load where they are used.  A row is the whole configuration: upload_rows rebuilds every row from dcfg whenever dcfg
+// or a table changes, so a row's shared fields (window, search clamp, blur switch, forsePlane) always equal cfg's; the kernels
+// still read those from cfg, so that they load from the parameter bank.
+template <bool ROWS>
+__device__ __forceinline__ const DevCfg& filter_cfg(const BatchView& bv, const DevCfg& cfg, int b) {
+  if constexpr (ROWS) return bv.row[b].cfg;
+  else return cfg;
+}
+template <bool ROWS>
 __device__ __forceinline__ const CamParams& filter_cam(const BatchView& bv, const DevCfg& cfg, int b) {
-  if constexpr (INTR) return bv.cam[b];
-  else return cfg.cam;
+  return filter_cfg<ROWS>(bv, cfg, b).cam;
+}
+// min_features / max_features of filter b (kernel arguments without rows)
+template <bool ROWS>
+__device__ __forceinline__ int2 filter_minmax(const BatchView& bv, int b, int min_features, int max_features) {
+  if constexpr (ROWS) return make_int2(bv.row[b].min_features, bv.row[b].max_features);
+  else return make_int2(min_features, max_features);
 }
 
 // convert2XYZ_ifLinear's decision (V:741-772, xyz_linear_decide) for feature i = lane of filter b, if `eligible` and still
@@ -140,7 +152,7 @@ __device__ __forceinline__ double step_dT(const BatchStepIn& in, int b, double d
 // predict for one filter per CTA: same arithmetic as k_predict_cov / k_predict_features / k_predict_S2
 // ------------------------------------------------------------------------------------------------
 #define BPRED_THREADS 128
-template <bool INTR, bool ACT>
+template <bool ROWS, bool ACT>
 __global__ void __launch_bounds__(BPRED_THREADS, 4) k_batch_predict(BatchView bv, FrameView fr, DevCfg cfg, double dT, double3 dv,
                                                                  double3 dw, int vcontrol, BatchStepIn in) {
   __shared__ double F[169], C[169], T[169], Q[169], cam[13];
@@ -151,6 +163,7 @@ __global__ void __launch_bounds__(BPRED_THREADS, 4) k_batch_predict(BatchView bv
     dv = make_double3(c[0], c[1], c[2]); dw = make_double3(c[3], c[4], c[5]);
   }
   if (in.vcontrol) vcontrol = in.vcontrol[i0];
+  const DevCfg& fc = filter_cfg<ROWS>(bv, cfg, b);
   const int n = bv.n[b], N = bv.N[b], ld = bv.ld;
   double* Sigma = bv.Sigma + (size_t)b * bv.sstride;
   double* mu = bv.mu + (size_t)b * ld;
@@ -171,7 +184,7 @@ __global__ void __launch_bounds__(BPRED_THREADS, 4) k_batch_predict(BatchView bv
     const int a = e / 13, c = e % 13;
     double s = 0;
     for (int k = 0; k < 6; ++k) {
-      const double vmax = vcontrol ? cfg.Vmax[k] : cfg.Vmax[k] * 2.0;
+      const double vmax = vcontrol ? fc.Vmax[k] : fc.Vmax[k] * 2.0;
       const double vs = (vmax / dT) / dT;
       s += (F[a * 13 + 7 + k] * vs) * F[c * 13 + 7 + k];
     }
@@ -220,7 +233,7 @@ __global__ void __launch_bounds__(BPRED_THREADS, 4) k_batch_predict(BatchView bv
       for (int c = 0; c < 13; ++c) cm[c] = cam[c];
       double qc[4] = {cm[3], -cm[4], -cm[5], -cm[6]}, Rcw[9], hi[2], Hc[26], hcz;
       d_quat2rot(qc, Rcw);
-      d_feature_hH(filter_cam<INTR>(bv, cfg, b), fs, coding, cm, qc, Rcw, hi, Hc, &hcz);
+      d_feature_hH(fc.cam, fs, coding, cm, qc, Rcw, hi, Hc, &hcz);
       const int half = cfg.window / 2;
       int fw = fr.w, fh = fr.h;
       if (in.fsize) {
@@ -269,8 +282,8 @@ __global__ void __launch_bounds__(BPRED_THREADS, 4) k_batch_predict(BatchView bv
       s10 += __shfl_down_sync(0xffffffffu, s10, o, 16); s11 += __shfl_down_sync(0xffffffffu, s11, o, 16);
     }
     if (lane == 0) {
-      ft.S2[4 * f + 0] = s00 + cfg.sigma_pixel_2; ft.S2[4 * f + 1] = s01;
-      ft.S2[4 * f + 2] = s10; ft.S2[4 * f + 3] = s11 + cfg.sigma_pixel_2;
+      ft.S2[4 * f + 0] = s00 + fc.sigma_pixel_2; ft.S2[4 * f + 1] = s01;
+      ft.S2[4 * f + 2] = s10; ft.S2[4 * f + 3] = s11 + fc.sigma_pixel_2;
     }
   }
 }
@@ -286,7 +299,7 @@ __global__ void __launch_bounds__(BPRED_THREADS, 4) k_batch_predict(BatchView bv
 // ------------------------------------------------------------------------------------------------
 #define BBLUR_WARPS 4
 // NC: feature capacity (BNCAP or BNCAP_L); warp 0 takes the decisions 32 features at a time, in ascending order.
-template <int NC, bool INTR, bool ACT>
+template <int NC, bool ROWS, bool ACT>
 __global__ void __launch_bounds__(BBLUR_WARPS * 32) k_batch_predict_blur(BatchView bv, DevCfg cfg, double dT, int* __restrict__ out,
                                                                      BatchStepIn in) {
   __shared__ int s_feat[NC], s_rows[NC], s_cols[NC], s_nblur;
@@ -309,11 +322,11 @@ __global__ void __launch_bounds__(BBLUR_WARPS * 32) k_batch_predict_blur(BatchVi
       if (f < N && ft.innov[f]) {
         double cam[13], rb[3], Rb[9];
         for (int c = 0; c < 13; ++c) cam[c] = mu[c];   // predicted camera state, committed by k_batch_predict
-        blur_pose(cam, cfg.T_camera, dT, rb, Rb);
+        blur_pose(cam, filter_cfg<ROWS>(bv, cfg, b).T_camera, dT, rb, Rb);
         const int pos = ft.pos[f], coding = ft.coding[f];
         double fs[6];
         for (int c = 0; c < (coding ? 3 : 6); ++c) fs[c] = mu[pos + c];
-        blur_displacement(filter_cam<INTR>(bv, cfg, b), fs, coding, rb, Rb, ft.h[2 * f], ft.h[2 * f + 1], &ddx, &ddy);
+        blur_displacement(filter_cam<ROWS>(bv, cfg, b), fs, coding, rb, Rb, ft.h[2 * f], ft.h[2 * f + 1], &ddx, &ddy);
         d = blur_decide(ddx, ddy, cfg.kernel_min_size, &krows, &kcols);
       }
       const unsigned blur = __ballot_sync(0xffffffffu, d > 0), big = __ballot_sync(0xffffffffu, d < 0);
@@ -624,7 +637,7 @@ __device__ void cta_stacked_update(const UpdSmem& sm, double* __restrict__ Sigma
 
 // PLANE: forsePlane (ekf_batch_set_force_plane), a separate instantiation so that the plane-off kernel is the same code as without it.
 // ACT: CTA i updates filter act[i] (ekf_batch_step_filters).
-template <bool PLANE, bool INTR, bool ACT>
+template <bool PLANE, bool ROWS, bool ACT>
 __global__ void __launch_bounds__(BUPD_THREADS, 1) k_batch_update(BatchView bv, DevCfg cfg, const uint32_t* __restrict__ picks,
                                                                   int n_picks, double* __restrict__ out_mu14,
                                                                   double* __restrict__ out_S14, int* __restrict__ out_stats,
@@ -649,17 +662,19 @@ __global__ void __launch_bounds__(BUPD_THREADS, 1) k_batch_update(BatchView bv, 
   const FeatTab ft = feattab_slice(bv.ft, b, bv.Ncap, bv.tstride);
   DevCtl* ctl = bv.ctl + b;
   if (tid == 0) ctl->chol_fail = 0;
-  // 1-point RANSAC, low-innovation update
-  if constexpr (INTR) {   // a configuration with the filter's intrinsics for cta_ransac; the Hi rescue below reads the row itself
-    DevCfg rcfg = cfg;
-    rcfg.cam = bv.cam[b];
+  const DevCfg& fc = filter_cfg<ROWS>(bv, cfg, b);   // the filter's intrinsics and tuning
+  // 1-point RANSAC, low-innovation update.  With rows cta_ransac takes a local copy of the filter's configuration, as it took
+  // the intrinsics-patched copy before rows held the tuning: handing it the row itself changes the code of the kernels
+  // without rows too (cta_ransac is one function for every instantiation).
+  if constexpr (ROWS) {
+    const DevCfg rcfg = fc;
     cta_ransac(Sigma, ld, n, mu, ft, N, ctl, rcfg, picks, n_picks, sm.mu_i, sm.ibuf);
   } else {
     cta_ransac(Sigma, ld, n, mu, ft, N, ctl, cfg, picks, n_picks, sm.mu_i, sm.ibuf);
   }
   __syncthreads();
   const int n_li = ctl->n_li;
-  if (n_li > 0) cta_stacked_update(sm, Sigma, ld, n, mu, ft, n_li, cfg, ctl);
+  if (n_li > 0) cta_stacked_update(sm, Sigma, ld, n, mu, ft, n_li, fc, ctl);
   // high-innovation rescue (k_hi_rescue): pose from the old mu, feature parameters from mu_tmp
   for (int i = tid; i < N; i += BUPD_THREADS) {
     int flag = 0;
@@ -671,7 +686,7 @@ __global__ void __launch_bounds__(BUPD_THREADS, 1) k_batch_update(BatchView bv, 
       for (int c = 0; c < 3; ++c) r[c] = ctl->cam_old[c];
       qc[0] = ctl->cam_old[3]; qc[1] = -ctl->cam_old[4]; qc[2] = -ctl->cam_old[5]; qc[3] = -ctl->cam_old[6];
       d_quat2rot(qc, Rcw);
-      d_feature_hH(filter_cam<INTR>(bv, cfg, b), fs, coding, r, qc, Rcw, hi, Hc, &hcz);
+      d_feature_hH(fc.cam, fs, coding, r, qc, Rcw, hi, Hc, &hcz);
       ft.h[2 * i] = hi[0]; ft.h[2 * i + 1] = hi[1];
       for (int c = 0; c < 26; ++c) ft.Hc[26 * i + c] = Hc[c];
       double Tm[26];
@@ -698,7 +713,7 @@ __global__ void __launch_bounds__(BUPD_THREADS, 1) k_batch_update(BatchView bv, 
       const double t0 = e0 * i00 + e1 * i10;
       const double t1 = e0 * i01 + e1 * i11;
       const double chi = t0 * e0 + t1 * e1;
-      flag = (chi <= cfg.th_hi) ? 1 : 0;
+      flag = (chi <= fc.th_hi) ? 1 : 0;
     }
     ft.hi[i] = flag;
   }
@@ -708,14 +723,14 @@ __global__ void __launch_bounds__(BUPD_THREADS, 1) k_batch_update(BatchView bv, 
   __syncthreads();
   if constexpr (PLANE) {   // the second update runs with or without Hi rows (z_hi.rows() > 0 with the plane rows, V:1245-1272)
     if (n_hi > 0) {
-      cta_gather_features(sm, Sigma, ld, n, ft, n_hi, cfg);
+      cta_gather_features(sm, Sigma, ld, n, ft, n_hi, fc);
       cta_block_gain_downdate(sm, Sigma, ld, n, mu, 2 * n_hi, ctl);
     }
     cta_gather_plane(sm, Sigma, ld, n, mu, ctl);
     cta_block_gain_downdate(sm, Sigma, ld, n, mu, 3, ctl);
     cta_normalize_quaternion(sm, Sigma, ld, n, mu);
   } else {
-    if (n_hi > 0) cta_stacked_update(sm, Sigma, ld, n, mu, ft, n_hi, cfg, ctl);
+    if (n_hi > 0) cta_stacked_update(sm, Sigma, ld, n, mu, ft, n_hi, fc, ctl);
   }
   // book-keeping (k_bookkeeping) + visibility count (V:1296-1315)
   int my_remove = 0, my_vis = 0;
@@ -726,12 +741,15 @@ __global__ void __launch_bounds__(BUPD_THREADS, 1) k_batch_update(BatchView bv, 
     ft.n_find[i] = nfind;
     const float qi = (float)(ntot - nfind) / ((float)nfind);
     ft.quality[i] = qi;
-    if (qi > cfg.quality_ratio) ft.removef[i] = 1;
+    if (qi > fc.quality_ratio) ft.removef[i] = 1;
     if (ft.removef[i]) my_remove++;
     else if (ft.innov[i]) my_vis++;
   }
   const int n_rem = __syncthreads_count(my_remove);   // N <= 32 <= blockDim: one feature per thread
   const int n_vis = __syncthreads_count(my_vis);
+  if constexpr (ROWS) {   // the filter's min / max_features; without rows the kernel arguments, as before
+    min_features = bv.row[b].min_features; max_features = bv.row[b].max_features;
+  }
   for (int e = tid; e < 14; e += BUPD_THREADS) out_mu14[(size_t)b * 14 + e] = mu[e];
   if (out_S14)
     for (int e = tid; e < 196; e += BUPD_THREADS) out_S14[(size_t)b * 196 + e] = Sigma[(size_t)(e / 14) * ld + (e % 14)];
@@ -758,7 +776,7 @@ __global__ void __launch_bounds__(BUPD_THREADS, 1) k_batch_update(BatchView bv, 
     const unsigned alive_mask = __ballot_sync(0xffffffffu, alive);
     const bool drop_first = (n_vis < min_features) && (N - n_rem > max_features);
     const int victim = drop_first ? __ffs(alive_mask) - 1 : -1;
-    warp_xyz_decide(bv, b, Sigma, mu, ft, N, alive && tid != victim, cfg);
+    warp_xyz_decide(bv, b, Sigma, mu, ft, N, alive && tid != victim, fc);
   }
 }
 
@@ -1082,7 +1100,7 @@ static __device__ __noinline__ void cl_hi_rescue(double* Sigma, int ld, const do
   if (tid == 0) { ctl->n_hi = nh; ctl->k_rows = 2 * nh; }
 }
 
-template <bool PLANE, bool INTR, bool ACT>
+template <bool PLANE, bool ROWS, bool ACT>
 __global__ void __launch_bounds__(BUPD_THREADS, 1) k_batch_update_cluster(BatchView bv, DevCfg cfg, const uint32_t* __restrict__ picks,
                                                                           int n_picks, double* __restrict__ out_mu14,
                                                                           double* __restrict__ out_S14, int* __restrict__ out_stats,
@@ -1107,7 +1125,7 @@ __global__ void __launch_bounds__(BUPD_THREADS, 1) k_batch_update_cluster(BatchV
   double* mu = bv.mu + (size_t)b * ld;
   const FeatTab ft = feattab_slice(bv.ft, b, bv.Ncap, bv.tstride);
   DevCtl* ctl = bv.ctl + b;
-  if constexpr (INTR) cfg.cam = bv.cam[b];   // every device function below projects with the filter's intrinsics
+  if constexpr (ROWS) cfg = bv.row[b].cfg;   // every device function below runs with the filter's intrinsics and tuning
   for (int i = tid; i < BSTRIP; i += BUPD_THREADS) sm.mu_i[i] = 0.0;
   if (rank == 0) {   // 1-point RANSAC: mu_i (n <= 782) in the Cholesky workspace, the candidates (N <= 128) in ibuf
     if (tid == 0) ctl->chol_fail = 0;
@@ -1151,6 +1169,9 @@ __global__ void __launch_bounds__(BUPD_THREADS, 1) k_batch_update_cluster(BatchV
   }
   const int n_rem = __syncthreads_count(my_remove);   // N <= 128 <= blockDim: one feature per thread
   const int n_vis = __syncthreads_count(my_vis);
+  if constexpr (ROWS) {   // the filter's min / max_features; without rows the kernel arguments, as before
+    min_features = bv.row[b].min_features; max_features = bv.row[b].max_features;
+  }
   for (int e = tid; e < 14; e += BUPD_THREADS) out_mu14[(size_t)b * 14 + e] = mu[e];
   if (out_S14)
     for (int e = tid; e < 196; e += BUPD_THREADS) out_S14[(size_t)b * 196 + e] = Sigma[(size_t)(e / 14) * ld + (e % 14)];
@@ -1201,12 +1222,13 @@ struct BatchArchive {
 // BNCAP_L); one CTA covers every entry of n2 x n2 either way, and every record (N2 <= 128 <= BCMP_THREADS).
 // one >= 0 (grid of one CTA): removeFeature(one_idx) on filter `one` alone (ekf_batch_remove_feature): no other removal, no
 // max_features rule, no conversion; pending decisions move with the records as under hold.  ACT: CTA i works on filter act[i].
+// ROWS: the max_features rule takes the filter's min / max_features from its row.
 // With the archive on, every removed feature that removeFeature archives (XYZ, n_find > 5) is appended to the filter's archive
 // in the single filter's order: the flagged features in ascending index (ekf_update_after_match's victims), then the
 // removeFeature(0) victim.  The records are read from Sigma and mu before the pass overwrites them.  A conversion fused into
 // the same pass never touches a removed feature's block: the reference removes before it converts, the decisions exclude the
 // removed features, and J is the identity on every row but the converted feature's.
-template <int NC, bool ACT>
+template <int NC, bool ROWS, bool ACT>
 __global__ void __launch_bounds__(BCMP_THREADS, 1) k_batch_compact(BatchView bv, double* __restrict__ scratch, int min_features,
                                                                 int max_features, int remove, const int* __restrict__ hold_stats,
                                                                 BatchArchive ar, int one, int one_idx, const int* __restrict__ act) {
@@ -1234,7 +1256,8 @@ __global__ void __launch_bounds__(BCMP_THREADS, 1) k_batch_compact(BatchView bv,
     int flagged = 0;
     for (int f = 0; f < N; ++f) flagged += DEAD(f) ? 1 : 0;
     // removeFeature(0) after the flagged ones are gone (V:1312-1313): first survivor
-    const bool drop_first = !single && rem && (ctl->n_visible < min_features) && (N - flagged > max_features);
+    const int2 mm = filter_minmax<ROWS>(bv, b, min_features, max_features);
+    const bool drop_first = !single && rem && (ctl->n_visible < mm.x) && (N - flagged > mm.y);
     int victim = -1;
     for (int f = 0; drop_first && f < N && victim < 0; ++f)
       if (!DEAD(f)) victim = f;
@@ -1352,17 +1375,19 @@ __global__ void __launch_bounds__(BCMP_THREADS, 1) k_batch_compact(BatchView bv,
 }
 
 // convert2XYZ_ifLinearAll (V:776-780) outside a step: the decisions of every filter, one CTA per filter, one thread per
-// feature; k_batch_compact (remove = 0) applies them.
+// feature; k_batch_compact (remove = 0) applies them.  ROWS: each filter's linearity threshold from its row.
+template <bool ROWS>
 __global__ void __launch_bounds__(BNCAP) k_batch_xyz_decide(BatchView bv, DevCfg cfg) {
   const int b = blockIdx.x;
   const FeatTab ft = feattab_slice(bv.ft, b, bv.Ncap, bv.tstride);
-  warp_xyz_decide(bv, b, bv.Sigma + (size_t)b * bv.sstride, bv.mu + (size_t)b * bv.ld, ft, bv.N[b], true, cfg);
+  warp_xyz_decide(bv, b, bv.Sigma + (size_t)b * bv.sstride, bv.mu + (size_t)b * bv.ld, ft, bv.N[b], true, filter_cfg<ROWS>(bv, cfg, b));
 }
 // The same for a large batch (capacity up to BNCAP_L): one thread per feature, BNCAP_L threads.
+template <bool ROWS>
 __global__ void __launch_bounds__(BNCAP_L) k_batch_xyz_decide_large(BatchView bv, DevCfg cfg) {
   const int b = blockIdx.x;
   const FeatTab ft = feattab_slice(bv.ft, b, bv.Ncap, bv.tstride);
-  cta_xyz_decide(bv, b, bv.Sigma + (size_t)b * bv.sstride, bv.mu + (size_t)b * bv.ld, ft, bv.N[b], false, -1, cfg);
+  cta_xyz_decide(bv, b, bv.Sigma + (size_t)b * bv.sstride, bv.mu + (size_t)b * bv.ld, ft, bv.N[b], false, -1, filter_cfg<ROWS>(bv, cfg, b));
 }
 
 // addFeature (V:309-371) for the corners of every filter that has some (cnt[b] of them at xy + 2 * EKF_BATCH_MAX_CORNERS * b),
@@ -1375,7 +1400,7 @@ __global__ void __launch_bounds__(BNCAP_L) k_batch_xyz_decide_large(BatchView bv
 // BADD_THREADS at a time and the decisions one thread per feature.  Templates come from frame cam_of[b] of the stack fr
 // (cam_of null: frame 0).  ACT: CTA i works on filter act[i] (ekf_batch_step_filters).
 #define BADD_THREADS 256
-template <bool LARGE, bool INTR, bool ACT>
+template <bool LARGE, bool ROWS, bool ACT>
 __global__ void __launch_bounds__(BADD_THREADS) k_batch_add(BatchView bv, FrameView fr, DevCfg cfg, const float* __restrict__ xy,
                                                             const int* __restrict__ cnt, int one, float u, float v, int decide,
                                                             const int* __restrict__ cam_of, const int* __restrict__ act) {
@@ -1385,6 +1410,7 @@ __global__ void __launch_bounds__(BADD_THREADS) k_batch_add(BatchView bv, FrameV
   const int k = one >= 0 ? 1 : cnt[b];
   if (k <= 0) return;
   if (cam_of) fr.px += (size_t)cam_of[b] * fr.h * fr.stride;
+  const DevCfg& fc = filter_cfg<ROWS>(bv, cfg, b);
   const int ld = bv.ld, w = cfg.window, w2 = w * w;
   double* Sigma = bv.Sigma + (size_t)b * bv.sstride;
   double* mu = bv.mu + (size_t)b * ld;
@@ -1394,7 +1420,7 @@ __global__ void __launch_bounds__(BADD_THREADS) k_batch_add(BatchView bv, FrameV
   for (int j = 0; j < k; ++j) {
     const float px = one >= 0 ? u : xy[(size_t)b * 2 * CS + 2 * j];
     const float py = one >= 0 ? v : xy[(size_t)b * 2 * CS + 2 * j + 1];
-    if (tid == 0) add_feature_jacobians(filter_cam<INTR>(bv, cfg, b), mu, px, py, cfg.rho_0, A, Ap, fnew);
+    if (tid == 0) add_feature_jacobians(fc.cam, mu, px, py, fc.rho_0, A, Ap, fnew);
     __syncthreads();
     if constexpr (LARGE) {
       for (int r = tid; r < n; r += BADD_THREADS) add_feature_cross(Sigma, ld, n, r, A);
@@ -1404,7 +1430,7 @@ __global__ void __launch_bounds__(BADD_THREADS) k_batch_add(BatchView bv, FrameV
     for (int e = tid; e < 42; e += BADD_THREADS) Tc[e] = add_feature_corner_T(Sigma, ld, A, e);   // rows / columns < 7: not written above
     __syncthreads();
     for (int e = tid; e < 36; e += BADD_THREADS)
-      Sigma[(size_t)(n + e / 6) * ld + n + e % 6] = add_feature_corner(Tc, A, Ap, e, cfg.sigma_pixel_2, cfg.sigma_rho_0);
+      Sigma[(size_t)(n + e / 6) * ld + n + e % 6] = add_feature_corner(Tc, A, Ap, e, fc.sigma_pixel_2, fc.sigma_rho_0);
     if (tid < 6) mu[n + tid] = fnew[tid];
     for (int e = tid; e < w2; e += BADD_THREADS) ft.patch[(size_t)N * cfg.tstride + e] = add_feature_template_px(fr, w, px, py, e);
     if (tid == 0) add_feature_record(ft, N, n, px, py, real);
@@ -1419,7 +1445,7 @@ __global__ void __launch_bounds__(BADD_THREADS) k_batch_add(BatchView bv, FrameV
       int conv = 0;
       if (i >= N0 && i < N) {
         const int pos = ft.pos[i];
-        conv = xyz_linear_decide(mu + pos, mu, Sigma[(size_t)(pos + 5) * ld + pos + 5], cfg.linearity_threshold, cfg.abs_int_quirk,
+        conv = xyz_linear_decide(mu + pos, mu, Sigma[(size_t)(pos + 5) * ld + pos + 5], fc.linearity_threshold, cfg.abs_int_quirk,
                                  bv.xyz_y + 3 * kk, bv.xyz_J + 18 * kk);
         bv.xyz_flag[kk] = conv;
       }
@@ -1434,7 +1460,7 @@ __global__ void __launch_bounds__(BADD_THREADS) k_batch_add(BatchView bv, FrameV
     int conv = 0;
     if (i >= N0 && i < N) {
       const int pos = ft.pos[i];
-      conv = xyz_linear_decide(mu + pos, mu, Sigma[(size_t)(pos + 5) * ld + pos + 5], cfg.linearity_threshold, cfg.abs_int_quirk,
+      conv = xyz_linear_decide(mu + pos, mu, Sigma[(size_t)(pos + 5) * ld + pos + 5], fc.linearity_threshold, cfg.abs_int_quirk,
                                bv.xyz_y + 3 * kk, bv.xyz_J + 18 * kk);
       bv.xyz_flag[kk] = conv;
     }
@@ -1538,9 +1564,9 @@ __global__ void k_batch_camera_rows(BatchView bv, double* __restrict__ out_mu14,
 // filters that are both copied from and overwritten (Sigma in the compaction scratch, the rest in a temporary buffer).  All sets
 // share the batch's ld, sstride, Ncap, tstride and archive capacity.
 struct BatchSlots {
-  BatchView v;        // Sigma, mu, ft, ctl, n, N, patchnumbre, xyz_*; v.cam is not used (cam below)
+  BatchView v;        // Sigma, mu, ft, ctl, n, N, patchnumbre, xyz_*; v.row is not used (row below)
   BatchArchive ar;    // records, count, overflow; cap 0: no archive
-  CamParams* cam;     // intrinsics row; null: the batch has no table
+  FilterRow* row;     // intrinsics and tuning row; null: the batch has no rows
   double* mu14;       // [14] the camera rows ekf_batch_get_camera_states reports
   double* S14;        // [196]
   int* stats;         // [EKF_BATCH_STAT_FIELDS] the last step's counters (findNewFeatures(NULL) reads EKF_BSTAT_TOPUP)
@@ -1604,7 +1630,7 @@ __global__ void __launch_bounds__(BRS_THREADS, 4) k_batch_resample(BatchSlots ds
   if (tid == 0) {
     dst.v.n[d] = n; dst.v.N[d] = N; dst.v.patchnumbre[d] = src.v.patchnumbre[s]; dst.v.xyz_count[d] = src.v.xyz_count[s];
     dst.v.ctl[d] = src.v.ctl[s];
-    if (src.cam) dst.cam[d] = src.cam[s];
+    if (src.row) dst.row[d] = src.row[s];
   }
 }
 
@@ -1642,7 +1668,9 @@ struct ekf_batch {
   std::vector<int> fsize_host;                  // [n_cam][4] in w, in h, resized w, h of the last capture with sizes (fsize_dev)
   int* fsize_dev = nullptr;
   bool fsize_on = false;                        // the captured stack has per-camera sizes
-  CamParams* intr_dev = nullptr;                // [B] intrinsics of each filter (ekf_batch_set_intrinsics); bv.cam, null without
+  std::vector<CamParams> intr_host;             // [B] intrinsics of each filter (ekf_batch_set_intrinsics); empty: the configuration's
+  std::vector<ekf_filter_params> tune_host;     // [B] tuning of each filter (ekf_batch_set_filter_params); empty: the configuration's
+  FilterRow* rows_dev = nullptr;                // [B] rows built from dcfg and both tables; bv.row, null while neither is set
   int* det_slot = nullptr;                      // [n_cam] position of each camera among those a detection asks from, or -1
   int* h_det_slot = nullptr;                    // pinned
   size_t det_budget = (size_t)1 << 30;          // scratch of one chunk of cameras of the per-camera detector
@@ -1721,7 +1749,7 @@ int ekf_batch_destroy(ekf_batch* b) {
   cudaFree(b->match_defer);
   cudaFree(b->scratch); cudaFree(b->frame); cudaFree(b->raw); cudaFree(b->picks_dev); cudaFree(b->out_mu14); cudaFree(b->out_S14);
   cudaFree(b->out_stats); cudaFree(b->stage_mu14); cudaFree(b->bv.patchnumbre);
-  cudaFree(b->cam_dev); cudaFree(b->det_slot); cudaFree(b->step_dev); cudaFree(b->intr_dev); cudaFree(b->fsize_dev); cudaFree(b->slot_dev);
+  cudaFree(b->cam_dev); cudaFree(b->det_slot); cudaFree(b->step_dev); cudaFree(b->rows_dev); cudaFree(b->fsize_dev); cudaFree(b->slot_dev);
   if (b->h_det_slot) cudaFreeHost(b->h_det_slot);
   if (b->step_host) cudaFreeHost(b->step_host);
   batch_detect_free(b->det);
@@ -1762,6 +1790,34 @@ static cudaLaunchConfig_t cluster_config(int B, int C, cudaStream_t st, cudaLaun
   return lc;
 }
 
+// The tuning fields of a configuration (ekf_filter_params), and their device form.  batch_create derives the configuration's
+// DevCfg through set_tuning too, so a row equal to the configuration gives the configuration's bits.
+static ekf_filter_params params_of(const ekf_config& c) {
+  ekf_filter_params p{};
+  p.sigma_vx = c.sigma_vx; p.sigma_vy = c.sigma_vy; p.sigma_vz = c.sigma_vz;
+  p.sigma_wx = c.sigma_wx; p.sigma_wy = c.sigma_wy; p.sigma_wz = c.sigma_wz;
+  p.rho_0 = c.rho_0; p.sigma_rho_0 = c.sigma_rho_0; p.T_camera = c.T_camera;
+  p.ncc_threshold = c.ncc_threshold; p.ransac_p = c.ransac_p; p.li_threshold_factor = c.li_threshold_factor;
+  p.hi_chi2_threshold = c.hi_chi2_threshold; p.quality_ratio = c.quality_ratio; p.linearity_threshold = c.linearity_threshold;
+  p.sigma_pixel = c.sigma_pixel; p.sigma_size = c.sigma_size; p.min_features = c.min_features; p.max_features = c.max_features;
+  p.ransac_nhyp0 = c.ransac_nhyp0;
+  return p;
+}
+static void set_tuning(DevCfg& d, const ekf_filter_params& p) {
+  d.Vmax[0] = p.sigma_vx * p.sigma_vx; d.Vmax[1] = p.sigma_vy * p.sigma_vy; d.Vmax[2] = p.sigma_vz * p.sigma_vz;
+  d.Vmax[3] = p.sigma_wx * p.sigma_wx; d.Vmax[4] = p.sigma_wy * p.sigma_wy; d.Vmax[5] = p.sigma_wz * p.sigma_wz;
+  d.sigma_pixel_2 = (double)(p.sigma_pixel * p.sigma_pixel);
+  d.th_low = p.li_threshold_factor * p.sigma_pixel;
+  d.th_hi = p.hi_chi2_threshold;
+  d.ransac_p = p.ransac_p;
+  d.linearity_threshold = p.linearity_threshold;
+  d.rho_0 = p.rho_0; d.sigma_rho_0 = p.sigma_rho_0;
+  d.T_camera = p.T_camera;
+  d.ncc_threshold = (float)p.ncc_threshold;
+  d.sigma_size_f = (float)p.sigma_size; d.quality_ratio = (float)p.quality_ratio;
+  d.sigma_pixel = p.sigma_pixel; d.nhyp0 = p.ransac_nhyp0;
+}
+
 static int batch_create(const ekf_config* cfg, int n_filters, int feature_capacity, int device, bool large, ekf_batch** out) {
   if (cfg->kernel_size < 100000 || cfg->scale != 1 || cfg->forsePlane != 0) return EKF_ERR_UNSUPPORTED;
   if (cfg->window_size < 3 || cfg->window_size > 31 || cfg->search_clamp > 20 || cfg->search_clamp < 0) return EKF_ERR_UNSUPPORTED;
@@ -1799,7 +1855,7 @@ static int batch_create(const ekf_config* cfg, int n_filters, int feature_capaci
                          (void*)k_batch_update_cluster<false, true, true>, (void*)k_batch_update_cluster<true, true, true>};
     for (void* k : cl) TRY(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kUpdSmemBytes))
     cudaLaunchAttribute attr[1];
-    for (int i = 0; i < 8; ++i) {   // forsePlane x intrinsics table x filter list
+    for (int i = 0; i < 8; ++i) {   // forsePlane x per-filter rows x filter list
       const cudaLaunchConfig_t lc = cluster_config(1, b->cl_ctas, nullptr, attr);
       int ncl = 0;
       TRY(cudaOccupancyMaxActiveClusters(&ncl, cl[i], &lc))
@@ -1852,18 +1908,10 @@ static int batch_create(const ekf_config* cfg, int n_filters, int feature_capaci
   std::fill(b->h_blur, b->h_blur + 2 * Bn, 0);
   DevCfg& d = b->dcfg;
   d.cam = CamParams{cfg->fx, cfg->fy, cfg->u0, cfg->v0, cfg->k1, cfg->k2, cfg->k3, cfg->p1, cfg->p2};
-  d.Vmax[0] = cfg->sigma_vx * cfg->sigma_vx; d.Vmax[1] = cfg->sigma_vy * cfg->sigma_vy; d.Vmax[2] = cfg->sigma_vz * cfg->sigma_vz;
-  d.Vmax[3] = cfg->sigma_wx * cfg->sigma_wx; d.Vmax[4] = cfg->sigma_wy * cfg->sigma_wy; d.Vmax[5] = cfg->sigma_wz * cfg->sigma_wz;
-  d.sigma_pixel_2 = (double)(cfg->sigma_pixel * cfg->sigma_pixel);
-  d.th_low = cfg->li_threshold_factor * cfg->sigma_pixel;
-  d.th_hi = cfg->hi_chi2_threshold;
-  d.ransac_p = cfg->ransac_p;
-  d.linearity_threshold = cfg->linearity_threshold;
-  d.rho_0 = cfg->rho_0; d.sigma_rho_0 = cfg->sigma_rho_0;
-  d.T_camera = cfg->T_camera; d.kernel_min_size = cfg->kernel_size;
-  d.ncc_threshold = (float)cfg->ncc_threshold; d.search_clamp = (float)cfg->search_clamp;
-  d.sigma_size_f = (float)cfg->sigma_size; d.quality_ratio = (float)cfg->quality_ratio;
-  d.window = cfg->window_size; d.sigma_pixel = cfg->sigma_pixel; d.nhyp0 = cfg->ransac_nhyp0;
+  set_tuning(d, params_of(*cfg));
+  d.kernel_min_size = cfg->kernel_size;
+  d.search_clamp = (float)cfg->search_clamp;
+  d.window = cfg->window_size;
   d.forsePlane = cfg->forsePlane; d.abs_int_quirk = cfg->abs_int_quirk;
   d.tstride = w2;
   *out = b;
@@ -2160,6 +2208,32 @@ int ekf_batch_set_cameras(ekf_batch* b, int n_cameras, const int32_t* camera_of)
 }
 
 static_assert(sizeof(CamParams) == 9 * sizeof(double), "a row of ekf_batch_set_intrinsics is one CamParams");
+// The device rows from the configuration and both tables (ekf_batch_set_intrinsics, ekf_batch_set_filter_params), in one copy;
+// no rows while neither table is set.
+static int upload_rows(ekf_batch* b) {
+  BCHECK(cudaSetDevice(b->device));
+  BCHECK(cudaStreamSynchronize(b->stream));   // work in flight may still read the rows
+  if (b->intr_host.empty() && b->tune_host.empty()) {
+    cudaFree(b->rows_dev);
+    b->rows_dev = nullptr;
+    b->bv.row = nullptr;
+    return EKF_OK;
+  }
+  std::vector<FilterRow> rows((size_t)b->B, FilterRow{b->dcfg, b->cfg.min_features, b->cfg.max_features});
+  for (int f = 0; f < b->B; ++f) {
+    FilterRow& r = rows[f];
+    if (!b->intr_host.empty()) r.cfg.cam = b->intr_host[f];
+    if (!b->tune_host.empty()) {
+      set_tuning(r.cfg, b->tune_host[f]);
+      r.min_features = b->tune_host[f].min_features; r.max_features = b->tune_host[f].max_features;
+    }
+  }
+  if (!b->rows_dev) BCHECK(balloc(&b->rows_dev, b->B));
+  BCHECK(cudaMemcpyAsync(b->rows_dev, rows.data(), sizeof(FilterRow) * b->B, cudaMemcpyHostToDevice, b->stream));
+  BCHECK(cudaStreamSynchronize(b->stream));   // the host rows are freed when the call returns
+  b->bv.row = b->rows_dev;
+  return EKF_OK;
+}
 int ekf_batch_set_intrinsics(ekf_batch* b, const double* cam) {
   if (!b) return EKF_ERR_ARG;
   if (cam) {
@@ -2170,19 +2244,35 @@ int ekf_batch_set_intrinsics(ekf_batch* b, const double* cam) {
       if (!ok) return bfail(b, EKF_ERR_ARG, "intrinsics of filter " + std::to_string(f) + ": non-finite, or fx / fy <= 0");
     }
   }
-  BCHECK(cudaSetDevice(b->device));
-  BCHECK(cudaStreamSynchronize(b->stream));   // work in flight may still read the table
-  if (!cam) {
-    cudaFree(b->intr_dev);
-    b->intr_dev = nullptr;
-    b->bv.cam = nullptr;
-    return EKF_OK;
+  if (cam) b->intr_host.assign(reinterpret_cast<const CamParams*>(cam), reinterpret_cast<const CamParams*>(cam) + b->B);
+  else b->intr_host.clear();
+  return upload_rows(b);
+}
+
+static_assert(sizeof(ekf_filter_params) == 15 * sizeof(double) + 6 * sizeof(int32_t), "ekf_filter_params has no hidden padding");
+int ekf_batch_set_filter_params(ekf_batch* b, const ekf_filter_params* rows) {
+  if (!b) return EKF_ERR_ARG;
+  for (int f = 0; rows && f < b->B; ++f) {
+    const ekf_filter_params& p = rows[f];
+    const std::string at = "filter params of filter " + std::to_string(f) + ": ";
+    const double* d = &p.sigma_vx;
+    static const char* const dnames[15] = {"sigma_vx", "sigma_vy", "sigma_vz", "sigma_wx", "sigma_wy", "sigma_wz", "rho_0", "sigma_rho_0",
+                                           "T_camera", "ncc_threshold", "ransac_p", "li_threshold_factor", "hi_chi2_threshold",
+                                           "quality_ratio", "linearity_threshold"};
+    for (int c = 0; c < 15; ++c)
+      if (!std::isfinite(d[c])) return bfail(b, EKF_ERR_ARG, at + dnames[c] + " is not finite");
+    for (int c : {0, 1, 2, 3, 4, 5, 7})   // the standard deviations
+      if (d[c] < 0) return bfail(b, EKF_ERR_ARG, at + dnames[c] + " is negative");
+    if (p.sigma_pixel < 1) return bfail(b, EKF_ERR_ARG, at + "sigma_pixel < 1");
+    if (p.sigma_size < 1) return bfail(b, EKF_ERR_ARG, at + "sigma_size < 1");
+    if (!(p.ransac_p > 0 && p.ransac_p < 1)) return bfail(b, EKF_ERR_ARG, at + "ransac_p outside (0, 1)");
+    if (p.ransac_nhyp0 < 1) return bfail(b, EKF_ERR_ARG, at + "ransac_nhyp0 < 1");
+    if (p.min_features < 0) return bfail(b, EKF_ERR_ARG, at + "min_features is negative");
+    if (p.max_features < 0) return bfail(b, EKF_ERR_ARG, at + "max_features is negative");
   }
-  if (!b->intr_dev) BCHECK(balloc(&b->intr_dev, b->B));
-  BCHECK(cudaMemcpyAsync(b->intr_dev, cam, sizeof(CamParams) * b->B, cudaMemcpyHostToDevice, b->stream));
-  BCHECK(cudaStreamSynchronize(b->stream));   // the caller's array is free once the call returns
-  b->bv.cam = b->intr_dev;
-  return EKF_OK;
+  if (rows) b->tune_host.assign(rows, rows + b->B);
+  else b->tune_host.clear();
+  return upload_rows(b);
 }
 
 int ekf_batch_set_frame_sizes(ekf_batch* b, const int32_t* wh) {
@@ -2240,7 +2330,7 @@ int ekf_batch_set_force_plane(ekf_batch* b, int on) {
   if (!b) return EKF_ERR_ARG;
   b->cfg.forsePlane = on != 0;
   b->dcfg.forsePlane = on != 0;
-  return EKF_OK;
+  return b->bv.row ? upload_rows(b) : EKF_OK;   // the rows are whole configurations: they follow dcfg
 }
 
 // The filters a step works on: n_act of them listed at act (device) by ekf_batch_step_filters, or every filter (act null).
@@ -2253,8 +2343,11 @@ static unsigned step_grid(const ekf_batch* b, const StepList& sl) { return (unsi
 // k_batch_compact at the batch's capacity on the step's filters; one >= 0: removeFeature(one_idx) on filter `one` alone (one CTA)
 static void launch_compact(ekf_batch* b, int remove, const int* hold_stats, int one = -1, int one_idx = -1, const StepList& sl = {}) {
   const unsigned grid = one >= 0 ? 1u : step_grid(b, sl);
-  auto* const compact = b->large ? (sl.act ? k_batch_compact<BNCAP_L, true> : k_batch_compact<BNCAP_L, false>)
-                                 : (sl.act ? k_batch_compact<BNCAP, true> : k_batch_compact<BNCAP, false>);
+  const bool rows = b->bv.row != nullptr;
+  auto* const compact = b->large ? (sl.act ? (rows ? k_batch_compact<BNCAP_L, true, true> : k_batch_compact<BNCAP_L, false, true>)
+                                           : (rows ? k_batch_compact<BNCAP_L, true, false> : k_batch_compact<BNCAP_L, false, false>))
+                                 : (sl.act ? (rows ? k_batch_compact<BNCAP, true, true> : k_batch_compact<BNCAP, false, true>)
+                                           : (rows ? k_batch_compact<BNCAP, true, false> : k_batch_compact<BNCAP, false, false>));
   compact<<<grid, BCMP_THREADS, 0, b->stream>>>(b->bv, b->scratch, b->cfg.min_features, b->cfg.max_features, remove, hold_stats, b->ar,
                                                 one, one_idx, sl.act);
   b->launches += 1;
@@ -2317,11 +2410,11 @@ static int batch_detect(ekf_batch* b, const int* num, const int* hnum, int num_s
 // k_batch_add at the batch's capacity and intrinsics, with or without a list of filters
 static void (*add_kernel(const ekf_batch* b, bool act))(BatchView, FrameView, DevCfg, const float*, const int*, int, float, float, int,
                                                         const int*, const int*) {
-  const bool intr = b->bv.cam != nullptr;
-  if (b->large) return act ? (intr ? k_batch_add<true, true, true> : k_batch_add<true, false, true>)
-                           : (intr ? k_batch_add<true, true, false> : k_batch_add<true, false, false>);
-  return act ? (intr ? k_batch_add<false, true, true> : k_batch_add<false, false, true>)
-             : (intr ? k_batch_add<false, true, false> : k_batch_add<false, false, false>);
+  const bool rows = b->bv.row != nullptr;
+  if (b->large) return act ? (rows ? k_batch_add<true, true, true> : k_batch_add<true, false, true>)
+                           : (rows ? k_batch_add<true, true, false> : k_batch_add<true, false, false>);
+  return act ? (rows ? k_batch_add<false, true, true> : k_batch_add<false, false, true>)
+             : (rows ? k_batch_add<false, true, false> : k_batch_add<false, false, false>);
 }
 
 // detection + adds for every filter, as batch_detect; decide: also take the new features' XYZ decisions (in-step top-up).
@@ -2433,7 +2526,7 @@ static int batch_step(ekf_batch* b, const double* dv, const double* dw, int vcon
     if (filters) { in.act = di + n_vc; sl.act = in.act; sl.n_act = n_act; }
     picks_dev = reinterpret_cast<const uint32_t*>(di + n_vc + n_al);
   }
-  const bool act = sl.act != nullptr, intr = b->bv.cam != nullptr;
+  const bool act = sl.act != nullptr, rows = b->bv.row != nullptr;
   const unsigned grid = step_grid(b, sl);
   if (act) {   // the others' counters read zero; their camera rows are gathered once a call changed some filter's
     BCHECK(cudaMemsetAsync(b->out_stats, 0, sizeof(int) * Bn * EKF_BATCH_STAT_FIELDS, st));
@@ -2443,41 +2536,42 @@ static int batch_step(ekf_batch* b, const double* dv, const double* dw, int vcon
     }
   }
   BCHECK(cudaEventRecord(b->ev[0], st));
-  auto* const predict = act ? (intr ? k_batch_predict<true, true> : k_batch_predict<false, true>)
-                            : (intr ? k_batch_predict<true, false> : k_batch_predict<false, false>);
+  auto* const predict = act ? (rows ? k_batch_predict<true, true> : k_batch_predict<false, true>)
+                            : (rows ? k_batch_predict<true, false> : k_batch_predict<false, false>);
   predict<<<grid, BPRED_THREADS, 0, st>>>(b->bv, b->fv, b->dcfg, b->cam_dT[0], make_double3(a[0], a[1], a[2]),
                                           make_double3(w[0], w[1], w[2]), vcontrol, in);
   b->launches += 1;
   if (b->blur) {   // matching_patch <- blurred patch where the prediction moves far enough (k_batch_predict copied patch)
     void (*blur)(BatchView, DevCfg, double, int*, BatchStepIn);
-    if (b->large) blur = act ? (intr ? k_batch_predict_blur<BNCAP_L, true, true> : k_batch_predict_blur<BNCAP_L, false, true>)
-                             : (intr ? k_batch_predict_blur<BNCAP_L, true, false> : k_batch_predict_blur<BNCAP_L, false, false>);
-    else blur = act ? (intr ? k_batch_predict_blur<BNCAP, true, true> : k_batch_predict_blur<BNCAP, false, true>)
-                    : (intr ? k_batch_predict_blur<BNCAP, true, false> : k_batch_predict_blur<BNCAP, false, false>);
+    if (b->large) blur = act ? (rows ? k_batch_predict_blur<BNCAP_L, true, true> : k_batch_predict_blur<BNCAP_L, false, true>)
+                             : (rows ? k_batch_predict_blur<BNCAP_L, true, false> : k_batch_predict_blur<BNCAP_L, false, false>);
+    else blur = act ? (rows ? k_batch_predict_blur<BNCAP, true, true> : k_batch_predict_blur<BNCAP, false, true>)
+                    : (rows ? k_batch_predict_blur<BNCAP, true, false> : k_batch_predict_blur<BNCAP, false, false>);
     blur<<<grid, BBLUR_WARPS * 32, 0, st>>>(b->bv, b->dcfg, b->cam_dT[0], b->blur_out, in);
     b->launches += 1;
   }
   BCHECK(cudaEventRecord(b->ev[1], st));
   launch_match_filter_batch(st, b->bv.ft, b->Ncap, b->bv.N, (int)grid, b->fv, b->dcfg, &b->frame_map, b->match_defer,
-                            b->match_defer + (size_t)b->B * b->Ncap, &b->launches, b->cam_dev, b->fsize_on ? b->fsize_dev : nullptr, sl.act);
+                            b->match_defer + (size_t)b->B * b->Ncap, &b->launches, b->cam_dev, b->fsize_on ? b->fsize_dev : nullptr, sl.act,
+                            b->bv.row);
   BCHECK(cudaEventRecord(b->ev[2], st));
   const bool plane = b->cfg.forsePlane != 0;
   if (b->large) {   // one cluster of cl_ctas CTAs per filter
     cudaLaunchAttribute attr[1];
     const cudaLaunchConfig_t lc = cluster_config((int)grid, b->cl_ctas, st, attr);
     void (*update)(BatchView, DevCfg, const uint32_t*, int, double*, double*, int*, int, int, int, const int*);
-    if (act) update = plane ? (intr ? k_batch_update_cluster<true, true, true> : k_batch_update_cluster<true, false, true>)
-                            : (intr ? k_batch_update_cluster<false, true, true> : k_batch_update_cluster<false, false, true>);
-    else update = plane ? (intr ? k_batch_update_cluster<true, true, false> : k_batch_update_cluster<true, false, false>)
-                        : (intr ? k_batch_update_cluster<false, true, false> : k_batch_update_cluster<false, false, false>);
+    if (act) update = plane ? (rows ? k_batch_update_cluster<true, true, true> : k_batch_update_cluster<true, false, true>)
+                            : (rows ? k_batch_update_cluster<false, true, true> : k_batch_update_cluster<false, false, true>);
+    else update = plane ? (rows ? k_batch_update_cluster<true, true, false> : k_batch_update_cluster<true, false, false>)
+                        : (rows ? k_batch_update_cluster<false, true, false> : k_batch_update_cluster<false, false, false>);
     BCHECK(cudaLaunchKernelEx(&lc, update, b->bv, b->dcfg, picks_dev, n_picks, b->out_mu14, b->out_S14,
                               b->out_stats, (int)b->cfg.min_features, (int)b->cfg.max_features, (int)b->cfg.xyz_conversion, sl.act));
   } else {
     void (*update)(BatchView, DevCfg, const uint32_t*, int, double*, double*, int*, int, int, int, const int*);
-    if (act) update = plane ? (intr ? k_batch_update<true, true, true> : k_batch_update<true, false, true>)
-                            : (intr ? k_batch_update<false, true, true> : k_batch_update<false, false, true>);
-    else update = plane ? (intr ? k_batch_update<true, true, false> : k_batch_update<true, false, false>)
-                        : (intr ? k_batch_update<false, true, false> : k_batch_update<false, false, false>);
+    if (act) update = plane ? (rows ? k_batch_update<true, true, true> : k_batch_update<true, false, true>)
+                            : (rows ? k_batch_update<false, true, true> : k_batch_update<false, false, true>);
+    else update = plane ? (rows ? k_batch_update<true, true, false> : k_batch_update<true, false, false>)
+                        : (rows ? k_batch_update<false, true, false> : k_batch_update<false, false, false>);
     update<<<grid, BUPD_THREADS, kUpdSmemBytes, st>>>(b->bv, b->dcfg, picks_dev, n_picks, b->out_mu14, b->out_S14,
                                                       b->out_stats, b->cfg.min_features, b->cfg.max_features,
                                                       b->cfg.xyz_conversion, sl.act);
@@ -2554,8 +2648,9 @@ int ekf_batch_convert2xyz_if_linear_all(ekf_batch* b) {
   BCHECK(cudaSetDevice(b->device));
   cudaStream_t st = b->stream;
   const size_t Bn = (size_t)b->B;
-  if (b->large) k_batch_xyz_decide_large<<<b->B, BNCAP_L, 0, st>>>(b->bv, b->dcfg);
-  else k_batch_xyz_decide<<<b->B, BNCAP, 0, st>>>(b->bv, b->dcfg);
+  const bool rows = b->bv.row != nullptr;
+  if (b->large) (rows ? k_batch_xyz_decide_large<true> : k_batch_xyz_decide_large<false>)<<<b->B, BNCAP_L, 0, st>>>(b->bv, b->dcfg);
+  else (rows ? k_batch_xyz_decide<true> : k_batch_xyz_decide<false>)<<<b->B, BNCAP, 0, st>>>(b->bv, b->dcfg);
   b->launches += 1;
   BCHECK(cudaGetLastError());
   BCHECK(cudaMemcpyAsync(b->h_xyz_count, b->bv.xyz_count, sizeof(int) * Bn, cudaMemcpyDeviceToHost, st));
@@ -2736,7 +2831,7 @@ int ekf_batch_set_motion_blur(ekf_batch* b, int32_t kernel_size) {
   b->dcfg.kernel_min_size = kernel_size;
   b->blur = kernel_size < 100000;
   if (!b->blur) std::fill(b->h_blur, b->h_blur + 2 * (size_t)b->B, 0);   // steps without blur leave the counts at zero
-  return EKF_OK;
+  return b->bv.row ? upload_rows(b) : EKF_OK;   // the rows are whole configurations: they follow dcfg
 }
 
 int ekf_batch_last_blur_counts(ekf_batch* b, int32_t* out) {
@@ -2913,7 +3008,7 @@ int ekf_batch_resample(ekf_batch* b, const int32_t* ancestors) {
   pairs.insert(pairs.end(), direct.begin(), direct.end());
   pairs.insert(pairs.end(), staged.begin(), staged.end());
   BCHECK(cudaMemcpyAsync(b->rs_pairs, pairs.data(), sizeof(int2) * pairs.size(), cudaMemcpyHostToDevice, st));
-  const BatchSlots live{b->bv, b->ar, b->intr_dev, b->out_mu14, b->out_S14, b->out_stats};
+  const BatchSlots live{b->bv, b->ar, b->rows_dev, b->out_mu14, b->out_S14, b->out_stats};
   const unsigned ctas = (unsigned)std::max<size_t>(1, (sizeof(double) * most * b->ld + kResampleBytesPerCta - 1) / kResampleBytesPerCta);
   const int2* pd = b->rs_pairs;
   void* tmp = nullptr;
@@ -2939,7 +3034,7 @@ int ekf_batch_resample(ekf_batch* b, const int32_t* ancestors) {
       take(t.patch, nf * tsb); take(t.mpatch, nf * tsb);
       take(sg.v.ctl, ns); take(sg.v.n, ns); take(sg.v.N, ns); take(sg.v.patchnumbre, ns);
       take(sg.v.xyz_flag, nf); take(sg.v.xyz_J, 18 * nf); take(sg.v.xyz_y, 3 * nf); take(sg.v.xyz_count, ns);
-      if (live.cam) take(sg.cam, ns);
+      if (live.row) take(sg.row, ns);
       if (b->ar.cap > 0) {
         take(sg.ar.rec, ns * b->ar.cap * PTS_COLS); take(sg.ar.real_index, ns * b->ar.cap);
         take(sg.ar.count, ns); take(sg.ar.overflow, ns);
@@ -2976,6 +3071,8 @@ int ekf_batch_resample(ekf_batch* b, const int32_t* ancestors) {
   follow(b->h_mu14, 14); follow(b->h_stats, EKF_BATCH_STAT_FIELDS);
   follow(b->h_blur, 1); follow(b->h_blur + B, 1);   // [2][B]: blurred templates, then kernel too large
   if (b->ar.cap > 0) { follow(b->h_over, 1); follow(b->over_seen.data(), 1); }
+  if (!b->intr_host.empty()) follow(b->intr_host.data(), 1);   // the tables the rows are rebuilt from
+  if (!b->tune_host.empty()) follow(b->tune_host.data(), 1);
   return EKF_OK;
 }
 

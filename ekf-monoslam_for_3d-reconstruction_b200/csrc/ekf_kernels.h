@@ -32,11 +32,18 @@ struct alignas(64) EkfTensorMap {
 };
 void match_make_tensor_map(EkfTensorMap* out, const uint8_t* frames, int width, int height, int stride, int n_frames, int w, int clamp);
 void launch_match_filter(cudaStream_t st, FeatTab ft, int N, FrameView fr, const DevCfg& cfg, const EkfTensorMap* tmap, long long* launches);
+// One filter's row of a batch with per-filter rows (ekf_batch.cu): the batch's configuration with the filter's intrinsics
+// (ekf_batch_set_intrinsics) and tuning (ekf_batch_set_filter_params) in place, and its min / max_features.
+struct FilterRow {
+  DevCfg cfg;
+  int min_features, max_features;
+};
 void launch_match_filter_batch(cudaStream_t st, FeatTab base, int Ncap, const int* Nper, int B, FrameView fr, const DevCfg& cfg,
                                const EkfTensorMap* tmap, int* defer_list, int* defer_cnt, long long* launches,
                                const int* cam_of = nullptr,    // cam_of [B]: filter b searches frame cam_of[b] of the stack fr
                                const int* fsize = nullptr,     // [n_cameras][4] (in w, in h, w, h): camera c is the top-left w x h of its slot
-                               const int* act = nullptr);      // [B]: the pairs' filter i is filter act[i] (a list of B filters)
+                               const int* act = nullptr,       // [B]: the pairs' filter i is filter act[i] (a list of B filters)
+                               const FilterRow* rows = nullptr);   // [B]: filter b matches with rows[b].cfg's sigma_size and ncc_threshold
 int launch_match_batch(cudaStream_t st, const uint8_t* frames, int n_frames, int width, int height, int stride,
                        const uint8_t* templates, int fpf, int w, const double* h, const double* S, float sigma_size,
                        float thr, float clampv, int32_t* out_uv, float* out_score);

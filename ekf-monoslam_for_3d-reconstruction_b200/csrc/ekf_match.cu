@@ -1068,12 +1068,21 @@ __device__ __forceinline__ int batch_pair_filter(const int* __restrict__ act, in
   else return i;
 }
 
+// ROWS (a batch with per-filter rows, ekf_batch_set_filter_params / ekf_batch_set_intrinsics): filter b searches and accepts with
+// its row's sigma_size and ncc_threshold.  Without rows the kernels are the code they were before.
+template <bool ROWS>
+__device__ __forceinline__ const DevCfg& batch_filter_cfg(const DevCfg& cfg, const FilterRow* __restrict__ rows, int b) {
+  if constexpr (ROWS) return rows[b].cfg;
+  else return cfg;
+}
+
 // Batched filters, pass 1 with the full-window warp matcher (template side 11): one warp per (filter, feature)
-template <int MINB, bool TSMEM, bool SLIDE, bool CAMS, bool SIZES, bool ACT>
+template <int MINB, bool TSMEM, bool SLIDE, bool CAMS, bool SIZES, bool ACT, bool ROWS>
 __global__ void __launch_bounds__(MW2_WARPS * 32, MINB) k_match_filter_batch_warp2(FeatTab base, int Ncap, const int* __restrict__ Nper, int B,
                                                                                 FrameView fr, DevCfg cfg, int* __restrict__ defer_list,
                                                                                 int* __restrict__ defer_cnt, const int* __restrict__ cam_of,
-                                                                                const int* __restrict__ fsize, const int* __restrict__ act) {
+                                                                                const int* __restrict__ fsize, const int* __restrict__ act,
+                                                                                const FilterRow* __restrict__ rows) {
   __shared__ MatchWarp2Smem<11> wsm[MW2_WARPS];
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const long long pair_i = (long long)blockIdx.x * MW2_WARPS + warp;
@@ -1092,21 +1101,22 @@ __global__ void __launch_bounds__(MW2_WARPS * 32, MINB) k_match_filter_batch_war
   if (lane == 0) wsm[warp].cnt = 0;
   __syncwarp();
   MatchResult r;
-  if (!match_one_warp2<11, TSMEM, SLIDE>(jb, cfg.sigma_size_f, cfg.search_clamp, wsm[warp], r)) {
+  const DevCfg& fc = batch_filter_cfg<ROWS>(cfg, rows, b);
+  if (!match_one_warp2<11, TSMEM, SLIDE>(jb, fc.sigma_size_f, cfg.search_clamp, wsm[warp], r)) {
     if (lane == 0) defer_list[atomicAdd(defer_cnt, 1)] = (int)pair;
     return;
   }
   __syncwarp();
-  match_warp_commit(ft, f, fr, cfg, r);
+  match_warp_commit(ft, f, fr, fc, r);
 }
 
 // Batched filters, pass 1: one warp per (filter, feature); features that do not fit go to defer_list.
-template <bool CAMS, bool SIZES, bool ACT>
+template <bool CAMS, bool SIZES, bool ACT, bool ROWS>
 __global__ void __launch_bounds__(MW_WARPS * 32) k_match_filter_batch_warp(FeatTab base, int Ncap, const int* __restrict__ Nper, int B,
                                                                            FrameView fr, DevCfg cfg, int* __restrict__ defer_list,
                                                                            int* __restrict__ defer_cnt, int warp_path,
                                                                            const int* __restrict__ cam_of, const int* __restrict__ fsize,
-                                                                           const int* __restrict__ act) {
+                                                                           const int* __restrict__ act, const FilterRow* __restrict__ rows) {
   __shared__ MatchWarpSmem wsm[MW_WARPS];
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const long long pair_i = (long long)blockIdx.x * MW_WARPS + warp;
@@ -1126,12 +1136,13 @@ __global__ void __launch_bounds__(MW_WARPS * 32) k_match_filter_batch_warp(FeatT
   if (lane == 0) wsm[warp].cnt = 0;
   __syncwarp();
   MatchResult r;
-  if (!warp_path || !match_one_warp(jb, w, cfg.sigma_size_f, cfg.search_clamp, wsm[warp], r)) {
+  const DevCfg& fc = batch_filter_cfg<ROWS>(cfg, rows, b);
+  if (!warp_path || !match_one_warp(jb, w, fc.sigma_size_f, cfg.search_clamp, wsm[warp], r)) {
     if (lane == 0) defer_list[atomicAdd(defer_cnt, 1)] = (int)pair;
     return;
   }
   __syncwarp();
-  const bool accept = !(r.best < cfg.ncc_threshold);  // Patch.cpp:278
+  const bool accept = !(r.best < fc.ncc_threshold);  // Patch.cpp:278
   if (accept) {   // matching_patch <- matched ROI (Patch.cpp:285)
     const int x0 = r.bi - w / 2, y0 = r.bj - w / 2;
     for (int e = lane; e < w2; e += 32)
@@ -1150,13 +1161,14 @@ __global__ void __launch_bounds__(MW_WARPS * 32) k_match_filter_batch_warp(FeatT
   }
 }
 // pass 2: a persistent grid of CTAs works off the deferred (filter, feature) pairs with match_one
-template <bool CAMS, bool SIZES>
+template <bool CAMS, bool SIZES, bool ROWS>
 __global__ void __launch_bounds__(MATCH_THREADS) k_match_filter_batch_deferred(FeatTab base, int Ncap, FrameView fr, DevCfg cfg,
                                                                                const __grid_constant__ CUtensorMap tmap, int use_tma,
                                                                                const int* __restrict__ defer_list,
                                                                                const int* __restrict__ defer_cnt,
                                                                                const int* __restrict__ cam_of,
-                                                                               const int* __restrict__ fsize) {
+                                                                               const int* __restrict__ fsize,
+                                                                               const FilterRow* __restrict__ rows) {
   extern __shared__ __align__(128) unsigned char smem_raw[];
   const int n = *defer_cnt;
   unsigned phase = 0;
@@ -1166,8 +1178,8 @@ __global__ void __launch_bounds__(MATCH_THREADS) k_match_filter_batch_deferred(F
     const int b = pair / Ncap, f = pair - b * Ncap;
     const FeatTab ft = feattab_slice(base, b, Ncap, cfg.tstride);
     const int cam = ((CAMS || SIZES) && cam_of) ? cam_of[b] : 0;
-    match_filter_feature(ft, f, batch_frame_of<CAMS, SIZES>(fr, cam_of, fsize, b), cfg, smem_raw, use_tma ? &tmap : nullptr, &phase,
-                         first, false, cam);
+    match_filter_feature(ft, f, batch_frame_of<CAMS, SIZES>(fr, cam_of, fsize, b), batch_filter_cfg<ROWS>(cfg, rows, b), smem_raw,
+                         use_tma ? &tmap : nullptr, &phase, first, false, cam);
     first = false;
     __syncthreads();
   }
@@ -1291,15 +1303,18 @@ void launch_match_filter(cudaStream_t st, FeatTab ft, int N, FrameView fr, const
 
 void launch_match_filter_batch(cudaStream_t st, FeatTab base, int Ncap, const int* Nper, int B, FrameView fr, const DevCfg& cfg,
                                const EkfTensorMap* tmap, int* defer_list, int* defer_cnt, long long* launches, const int* cam_of,
-                               const int* fsize, const int* act) {
+                               const int* fsize, const int* act, const FilterRow* rows) {
   if (B <= 0 || Ncap <= 0) return;
   static PerDeviceOnce once;   // opt in to the largest supported window once per device
   const size_t smem = match_smem_bytes(cfg.window, cfg.search_clamp);
   if (once.ensure([] {
         const int bytes = (int)match_smem_bytes(MATCH_MAX_W, 20.0f);
-        cudaError_t e = cudaFuncSetAttribute(k_match_filter_batch_deferred<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes);
-        if (e == cudaSuccess) e = cudaFuncSetAttribute(k_match_filter_batch_deferred<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes);
-        return e != cudaSuccess ? e : cudaFuncSetAttribute(k_match_filter_batch_deferred<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes);
+        cudaError_t e = cudaSuccess;
+        for (void* k : {(void*)k_match_filter_batch_deferred<false, false, false>, (void*)k_match_filter_batch_deferred<true, false, false>,
+                        (void*)k_match_filter_batch_deferred<true, true, false>, (void*)k_match_filter_batch_deferred<false, false, true>,
+                        (void*)k_match_filter_batch_deferred<true, false, true>, (void*)k_match_filter_batch_deferred<true, true, true>})
+          if (e == cudaSuccess) e = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes);
+        return e;
       }) != cudaSuccess) return;   // the error stays in cudaGetLastError() for the caller
   static const EkfTensorMap none{};
   const EkfTensorMap& tm = (tmap && tmap->ok) ? *tmap : none;
@@ -1312,13 +1327,15 @@ void launch_match_filter_batch(cudaStream_t st, FeatTab base, int Ncap, const in
   if (warp_path >= 2 && cfg.window == 11 && cfg.search_clamp <= 20.0f) {
     const unsigned grid = (unsigned)((pairs + MW2_WARPS - 1) / MW2_WARPS);
     const int var = match_w2_variant();
-#define MW2_LAUNCH_ACT(MINB, TS, SL, ACT)                                                                                               \
-  if (fsize) k_match_filter_batch_warp2<MINB, TS, SL, true, true, ACT><<<grid, MW2_WARPS * 32, 0, st>>>(base, Ncap, Nper, B, fr, cfg, defer_list, defer_cnt, cam_of, fsize, act); \
-  else if (cam_of) k_match_filter_batch_warp2<MINB, TS, SL, true, false, ACT><<<grid, MW2_WARPS * 32, 0, st>>>(base, Ncap, Nper, B, fr, cfg, defer_list, defer_cnt, cam_of, fsize, act); \
-  else k_match_filter_batch_warp2<MINB, TS, SL, false, false, ACT><<<grid, MW2_WARPS * 32, 0, st>>>(base, Ncap, Nper, B, fr, cfg, defer_list, defer_cnt, cam_of, fsize, act)
-#define MW2_LAUNCH(MINB, TS, SL)                   \
-  if (act) { MW2_LAUNCH_ACT(MINB, TS, SL, true); } \
-  else { MW2_LAUNCH_ACT(MINB, TS, SL, false); }
+#define MW2_LAUNCH_ACT(MINB, TS, SL, ACT, RW)                                                                                           \
+  if (fsize) k_match_filter_batch_warp2<MINB, TS, SL, true, true, ACT, RW><<<grid, MW2_WARPS * 32, 0, st>>>(base, Ncap, Nper, B, fr, cfg, defer_list, defer_cnt, cam_of, fsize, act, rows); \
+  else if (cam_of) k_match_filter_batch_warp2<MINB, TS, SL, true, false, ACT, RW><<<grid, MW2_WARPS * 32, 0, st>>>(base, Ncap, Nper, B, fr, cfg, defer_list, defer_cnt, cam_of, fsize, act, rows); \
+  else k_match_filter_batch_warp2<MINB, TS, SL, false, false, ACT, RW><<<grid, MW2_WARPS * 32, 0, st>>>(base, Ncap, Nper, B, fr, cfg, defer_list, defer_cnt, cam_of, fsize, act, rows)
+#define MW2_LAUNCH(MINB, TS, SL)                                        \
+  if (act && rows) { MW2_LAUNCH_ACT(MINB, TS, SL, true, true); }        \
+  else if (act) { MW2_LAUNCH_ACT(MINB, TS, SL, true, false); }          \
+  else if (rows) { MW2_LAUNCH_ACT(MINB, TS, SL, false, true); }         \
+  else { MW2_LAUNCH_ACT(MINB, TS, SL, false, false); }
     switch (var) {
       case 0: MW2_LAUNCH(2, false, false); break;
       case 2: MW2_LAUNCH(3, true, false); break;
@@ -1331,24 +1348,28 @@ void launch_match_filter_batch(cudaStream_t st, FeatTab base, int Ncap, const in
 #undef MW2_LAUNCH_ACT
   } else {
     const unsigned grid = (unsigned)((pairs + MW_WARPS - 1) / MW_WARPS);
-#define MW_LAUNCH(ACT)                                                                                                                \
-  if (fsize) k_match_filter_batch_warp<true, true, ACT><<<grid, MW_WARPS * 32, 0, st>>>(base, Ncap, Nper, B, fr, cfg, defer_list, defer_cnt, warp_path, cam_of, fsize, act); \
-  else if (cam_of) k_match_filter_batch_warp<true, false, ACT><<<grid, MW_WARPS * 32, 0, st>>>(base, Ncap, Nper, B, fr, cfg, defer_list, defer_cnt, warp_path, cam_of, fsize, act); \
-  else k_match_filter_batch_warp<false, false, ACT><<<grid, MW_WARPS * 32, 0, st>>>(base, Ncap, Nper, B, fr, cfg, defer_list, defer_cnt, warp_path, cam_of, fsize, act)
-    if (act) { MW_LAUNCH(true); }
-    else { MW_LAUNCH(false); }
+#define MW_LAUNCH(ACT, RW)                                                                                                            \
+  if (fsize) k_match_filter_batch_warp<true, true, ACT, RW><<<grid, MW_WARPS * 32, 0, st>>>(base, Ncap, Nper, B, fr, cfg, defer_list, defer_cnt, warp_path, cam_of, fsize, act, rows); \
+  else if (cam_of) k_match_filter_batch_warp<true, false, ACT, RW><<<grid, MW_WARPS * 32, 0, st>>>(base, Ncap, Nper, B, fr, cfg, defer_list, defer_cnt, warp_path, cam_of, fsize, act, rows); \
+  else k_match_filter_batch_warp<false, false, ACT, RW><<<grid, MW_WARPS * 32, 0, st>>>(base, Ncap, Nper, B, fr, cfg, defer_list, defer_cnt, warp_path, cam_of, fsize, act, rows)
+    if (act && rows) { MW_LAUNCH(true, true); }
+    else if (act) { MW_LAUNCH(true, false); }
+    else if (rows) { MW_LAUNCH(false, true); }
+    else { MW_LAUNCH(false, false); }
 #undef MW_LAUNCH
   }
   int dev = 0, sms = 148;
   if (cudaGetDevice(&dev) == cudaSuccess) cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
   int per_sm = 4;   // persistent grid: as many CTAs as are resident at this shared-memory footprint
-  auto* const deferred = fsize ? k_match_filter_batch_deferred<true, true>
-                               : cam_of ? k_match_filter_batch_deferred<true, false> : k_match_filter_batch_deferred<false, false>;   // the one launched
+  auto* const deferred = rows ? (fsize ? k_match_filter_batch_deferred<true, true, true>
+                                       : cam_of ? k_match_filter_batch_deferred<true, false, true> : k_match_filter_batch_deferred<false, false, true>)
+                              : (fsize ? k_match_filter_batch_deferred<true, true, false>
+                                       : cam_of ? k_match_filter_batch_deferred<true, false, false> : k_match_filter_batch_deferred<false, false, false>);   // the one launched
   if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, deferred, MATCH_THREADS, smem) != cudaSuccess || per_sm < 1) {
     cudaGetLastError();
     per_sm = 4;
   }
-  deferred<<<sms * per_sm, MATCH_THREADS, smem, st>>>(base, Ncap, fr, cfg, as_cu(tm), tm.ok, defer_list, defer_cnt, cam_of, fsize);
+  deferred<<<sms * per_sm, MATCH_THREADS, smem, st>>>(base, Ncap, fr, cfg, as_cu(tm), tm.ok, defer_list, defer_cnt, cam_of, fsize, rows);
   *launches += 2;
 }
 

@@ -334,6 +334,13 @@ class FilterBatch:
             raise EkfError(f"ekf batch error {rc}: {self.L.ekf_batch_last_error(self.h).decode()}")
         return rc
 
+    def _set_cfg(self, **fields):
+        """self.cfg follows what the batch runs (set_configs checks the shared fields against it); a copy, so that the
+        caller's configuration stays as it was."""
+        self.cfg = _abi.EkfConfig.from_buffer_copy(self.cfg)
+        for k, v in fields.items():
+            setattr(self.cfg, k, v)
+
     def describe(self):
         d = _abi.EkfBatchDesc()
         self._ck(self.L.ekf_batch_describe(self.h, C.byref(d)))
@@ -454,7 +461,7 @@ class FilterBatch:
         self._ck(self.L.ekf_batch_capture_camera_frames_device(self.h, int(cams.size), _ptr(cams), C.c_void_p(int(dev_ptr)), int(width),
                                                                int(height), int(stride), _ptr(s) if s is not None else None))
 
-    INTRINSICS = ("fx", "fy", "u0", "v0", "k1", "k2", "k3", "p1", "p2")
+    INTRINSICS = _abi.INTRINSICS
 
     def set_intrinsics(self, params):
         """Intrinsics per filter, columns in INTRINSICS order (EkfConfig's): a (9,) array for every filter, a (n_filters, 9)
@@ -467,6 +474,35 @@ class FilterBatch:
             raise ValueError(f"set_intrinsics expects (9,) or ({self.B}, 9)")
         a = np.ascontiguousarray(np.broadcast_to(a, (self.B, 9)))
         self._ck(self.L.ekf_batch_set_intrinsics(self.h, _ptr(a)))
+
+    def set_filter_params(self, rows):
+        """Tuning per filter (ekf_batch_set_filter_params): a sequence of n_filters _abi.EkfFilterParams, or None for the
+        configuration's values."""
+        if rows is None:
+            self._ck(self.L.ekf_batch_set_filter_params(self.h, None))
+            return
+        if len(rows) != self.B:
+            raise ValueError(f"set_filter_params expects {self.B} rows")
+        arr = rows if isinstance(rows, C.Array) else (_abi.EkfFilterParams * self.B)(*rows)
+        self._ck(self.L.ekf_batch_set_filter_params(self.h, arr))
+
+    def set_configs(self, cfgs):
+        """Filter f runs configuration cfgs[f], as a VSlamFilter given it would: its intrinsics and its tuning (both tables).
+        cfgs holds n_filters EkfConfig (one per camera: [cfgs[c] for c in camera_of]); None returns every filter to the
+        batch's configuration.  ValueError, naming the field and the filter, when a field every filter shares
+        (_abi.BATCH_SHARED_FIELDS) differs from the batch's configuration as it stands (set_motion_blur, set_scale and
+        set_force_plane included), or when a row is invalid; every row is checked before either table changes.
+        nInitFeatures is not read."""
+        if cfgs is None:
+            self.set_intrinsics(None)
+            self.set_filter_params(None)
+            return
+        cfgs = list(cfgs)
+        if len(cfgs) != self.B:
+            raise ValueError(f"set_configs expects {self.B} configurations")
+        cam, rows = _abi.batch_rows(self.cfg, cfgs)
+        self.set_intrinsics(cam)
+        self.set_filter_params(rows)
 
     def set_detect_budget(self, nbytes):
         """Device scratch of one chunk of cameras in the per-camera detector (default 1 GiB)."""
@@ -489,10 +525,12 @@ class FilterBatch:
     def set_scale(self, scale):
         """EkfConfig.scale for the batch's captures (default 1); the configuration's intrinsics are the resized image's."""
         self._ck(self.L.ekf_batch_set_scale(self.h, int(scale)))
+        self._set_cfg(scale=int(scale))
 
     def set_force_plane(self, on=True):
         """EkfConfig.forsePlane for every filter (vslamRansac.cpp:1245-1272; default off)."""
         self._ck(self.L.ekf_batch_set_force_plane(self.h, int(bool(on))))
+        self._set_cfg(forsePlane=int(bool(on)))
 
     def step(self, picks=None, dv=(0.0, 0.0, 0.0), dw=(0.0, 0.0, 0.0), vcontrol=False, filters=None):
         """predict + update of every filter.  dv / dw are 3-vectors for every filter, or (n_filters, 3) arrays with vcontrol
@@ -650,6 +688,7 @@ class FilterBatch:
         """Patch::blur (Patch.cpp:50-57) in every filter's predict: kernel_size as EkfConfig.kernel_size (>= 100000: off,
         the default); T_camera is the batch configuration's."""
         self._ck(self.L.ekf_batch_set_motion_blur(self.h, int(kernel_size)))
+        self._set_cfg(kernel_size=int(kernel_size))
 
     def last_blur_counts(self):
         """Templates each filter blurred in the last step (int32, zeros with blur off)."""

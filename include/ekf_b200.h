@@ -217,7 +217,7 @@ int ekf_match_batch(const uint8_t* frames, int n_frames, int width, int height, 
                     float search_clamp, int32_t* out_uv, float* out_score, void* stream);
 
 /* ---- batch of independent filters (BASELINE config 3: multi-hypothesis / Monte-Carlo) ----------- */
-/* B filters with the same configuration, stepped together on one device: one fused CTA per filter
+/* B filters built from one configuration, stepped together on one device: one fused CTA per filter
  * for predict (vslamRansac.cpp:451-603) and for update (:964-1341), one CTA per (filter, feature)
  * for the active search (:870-880).  Filter b follows camera camera_of[b] (ekf_batch_set_cameras): each camera has its
  * own frame and time stamp, and every filter of a camera searches that camera's frame.  By default one camera is followed
@@ -233,7 +233,10 @@ int ekf_match_batch(const uint8_t* frames, int n_frames, int width, int height, 
  * ekf_batch_create_large takes up to 128 (the update of one filter on a cluster of CTAs).  ekf_batch_create
  * refuses motion blur (kernel_size < 100000), scale != 1 and forsePlane (EKF_ERR_UNSUPPORTED); each of them is
  * switched on after creation instead, with ekf_batch_set_motion_blur, ekf_batch_set_scale and
- * ekf_batch_set_force_plane, so that a batch honours every ConfigVSLAM switch a single filter honours. */
+ * ekf_batch_set_force_plane, so that a batch honours every ConfigVSLAM switch a single filter honours.
+ * The configuration is every filter's by default; ekf_batch_set_intrinsics and ekf_batch_set_filter_params give each filter
+ * intrinsics and tuning of its own, while window_size, search_clamp, scale, kernel_size, forsePlane, xyz_conversion and
+ * abs_int_quirk stay shared by the batch. */
 typedef struct ekf_batch ekf_batch;
 typedef struct ekf_batch_desc {
   int32_t n_filters, feature_capacity, state_capacity /* 14 + 6 * feature_capacity */, ld /* Sigma row stride */;
@@ -290,9 +293,41 @@ int ekf_batch_set_cameras(ekf_batch* b, int n_cameras, const int32_t* camera_of)
  * addFeature.  NULL returns every filter to the configuration's intrinsics, which is the default.  A non-finite entry or
  * fx <= 0 or fy <= 0 returns EKF_ERR_ARG and leaves the table as it was.  As for ekf_batch_set_scale, the intrinsics are
  * those of the resized image.  The table goes to the device inside this call (no per-step copy); ekf_batch_seed_from and
- * ekf_batch_set_cameras leave it alone.  For intrinsics per camera, pass row camera_of[f] for filter f.  Memory: 72 B per
- * filter on the device while a table is set.  Window, sigmas and scale stay shared by the batch. */
+ * ekf_batch_set_cameras leave it alone.  For intrinsics per camera, pass row camera_of[f] for filter f.  Memory: one device
+ * row of 240 B per filter (intrinsics and tuning together) while this table or the tuning table is set.  The tuning (ekf_batch_set_filter_params) is a table of its own: setting or
+ * clearing one leaves the other alone.  Window, search clamp and scale stay shared by the batch. */
 int ekf_batch_set_intrinsics(ekf_batch* b, const double* cam);
+/* The ekf_config fields a filter of a batch may take on its own (its tuning), under their ekf_config names and types. */
+typedef struct ekf_filter_params {
+  double sigma_vx, sigma_vy, sigma_vz; /* process noise: Vmax of predict (vslamRansac.cpp:194-200) */
+  double sigma_wx, sigma_wy, sigma_wz;
+  double rho_0, sigma_rho_0;           /* addFeature's inverse-depth prior */
+  double T_camera;                     /* blur pose (with ekf_batch_set_motion_blur) */
+  double ncc_threshold;                /* matcher acceptance */
+  double ransac_p;                     /* 1-point RANSAC */
+  double li_threshold_factor;          /* Li threshold = li_threshold_factor * sigma_pixel */
+  double hi_chi2_threshold;            /* Hi rescue */
+  double quality_ratio;                /* quality deletion */
+  double linearity_threshold;          /* XYZ conversion decisions */
+  int32_t sigma_pixel;                 /* R, the S blocks and addFeature's covariance */
+  int32_t sigma_size;                  /* matcher search box */
+  int32_t min_features, max_features;  /* top-up request (EKF_BSTAT_TOPUP) and the removeFeature(0) rule */
+  int32_t ransac_nhyp0;
+  int32_t _pad;
+} ekf_filter_params;
+/* Tuning per filter: rows is a HOST array of n_filters ekf_filter_params, and filter f predicts, matches, updates, deletes,
+ * asks for features and adds them with row f (predict and its blur pose, the three matcher kernels, RANSAC, the Hi rescue,
+ * both updates, the book-keeping, the XYZ decisions and addFeature), exactly as a single filter whose ekf_config carries
+ * row f.  NULL returns every filter to the configuration's values, which is the default.  A non-finite entry, a negative
+ * standard deviation (sigma_v*, sigma_w*, sigma_rho_0), sigma_pixel < 1, sigma_size < 1, ransac_p outside (0, 1),
+ * ransac_nhyp0 < 1 or a negative min_features / max_features returns EKF_ERR_ARG, ekf_batch_last_error names the first bad
+ * filter and field, and the table stays as it was; EKF_ERR_ARG for a NULL batch.  The table goes to the device inside this
+ * call (no per-step copy).  It is independent of ekf_batch_set_intrinsics (setting or clearing one leaves the other alone);
+ * ekf_batch_seed_from and ekf_batch_set_cameras leave it alone, ekf_batch_resample moves the row with the filter,
+ * ekf_batch_step_filters steps each listed filter with its row, and ekf_batch_find_new_features(NULL) serves each filter's
+ * request from its own min_features.  For a tuning per camera, pass row camera_of[f] for filter f.  Memory: one row of
+ * 240 B per filter on the device (the row it shares with the intrinsics) while either table is set. */
+int ekf_batch_set_filter_params(ekf_batch* b, const ekf_filter_params* rows);
 /* A frame size per camera: wh is a HOST array of n_cameras x 2 int32 (width, height) in INPUT pixels, before the resize by
  * 1 / scale; NULL (the default) means every camera uses the whole frame the capture calls pass.  The stack keeps one slot per
  * camera: the capture calls' width / height / stride describe the slot, and camera c's frame is the top-left w_c x h_c of slot
@@ -402,7 +437,7 @@ int ekf_batch_last_added(ekf_batch* b, int32_t* added);
 /* Patch::blur (Patch.cpp:50-57, libblur.cpp:17-81) in every filter's predict: kernel_size has the meaning of
  * ekf_config.kernel_size for a single filter (a template is blurred when the prediction moves by more than kernel_size px
  * over T_camera * dT; >= 100000 = off, the default).  ekf_batch_create still refuses a configuration with blur on.
- * T_camera is the batch configuration's.  A kernel above 256 x 256 px leaves that template unblurred; the step then runs
+ * T_camera is the filter's (ekf_batch_set_filter_params; the configuration's by default).  A kernel above 256 x 256 px leaves that template unblurred; the step then runs
  * to its end and returns EKF_ERR_UNSUPPORTED, and ekf_batch_last_error names the first such filter. */
 int ekf_batch_set_motion_blur(ekf_batch* b, int32_t kernel_size);
 /* Templates each filter blurred in the last step (n_filters entries; zeros with blur off). */
@@ -439,7 +474,8 @@ int ekf_batch_get_points_features(ekf_batch* b, int first, int count, double* ou
  * entries), both as they stood before the call, so duplicates, swaps and cycles are all fine; ancestors[f] == f leaves f
  * untouched, and the identity launches nothing.  What moves is everything of the filter that a later call reads: state and
  * covariance, feature table, both templates, real_index counter, pending XYZ decisions, archive (with its overflow count,
- * so the next step reports only new drops), intrinsics row (ekf_batch_set_intrinsics), counters, added and blur counts.
+ * so the next step reports only new drops), intrinsics row (ekf_batch_set_intrinsics), tuning row
+ * (ekf_batch_set_filter_params), counters, added and blur counts.
  * Afterwards every per-filter accessor reports for f what it reported for ancestors[f] before the call: ekf_batch_get_full,
  * _get_feature, _get_template, _num_features, _state_dim, _get_camera_states (camera rows and counters), _last_added,
  * _last_blur_counts, _num_deleted, _get_deleted and _get_points_features; and every later call treats f as it treats its
