@@ -29,9 +29,17 @@ class EkfFilterParams(C.Structure):
         "sigma_pixel", "sigma_size", "min_features", "max_features", "ransac_nhyp0", "_pad")]
 
 
+class EkfCameraSettings(C.Structure):
+    """ekf_camera_settings: the ekf_config fields a camera of a batch may take on its own (ekf_batch_set_camera_settings)."""
+    _fields_ = [(n, C.c_int32) for n in ("window_size", "scale", "kernel_size", "_pad")]
+
+
 # ekf_config fields every filter of a batch shares (buffer sizes, launch structure, emulation mode); intrinsics have their own
-# table (ekf_batch_set_intrinsics), nInitFeatures is never read by a batch.
+# table (ekf_batch_set_intrinsics), nInitFeatures is never read by a batch.  With a camera table (ekf_batch_set_camera_settings)
+# the CAMERA_FIELDS among them are shared by the filters of a camera only, and BATCH_WIDE_FIELDS stay shared by the batch.
 BATCH_SHARED_FIELDS = ("window_size", "search_clamp", "scale", "kernel_size", "forsePlane", "xyz_conversion", "abs_int_quirk")
+CAMERA_FIELDS = ("window_size", "scale", "kernel_size")
+BATCH_WIDE_FIELDS = ("search_clamp", "forsePlane", "xyz_conversion", "abs_int_quirk")
 INTRINSICS = ("fx", "fy", "u0", "v0", "k1", "k2", "k3", "p1", "p2")
 
 
@@ -39,14 +47,62 @@ def batch_rows(base, cfgs):
     """The per-filter tables of a batch built from `base` whose filter f runs configuration cfgs[f]: an (n, 9) float64 array
     of intrinsics (INTRINSICS order) and an array of n EkfFilterParams.  ValueError, naming the field and the filter, when a
     field of BATCH_SHARED_FIELDS differs from base's or a row is one the C calls refuse."""
+    def want(f, name):
+        return getattr(base, name), "the batch's", "every filter of a batch"
+    return _rows(cfgs, want)
+
+
+def batch_rows_per_camera(base, cfgs, settings, camera_of):
+    """batch_rows for a batch with a camera table: filter f's CAMERA_FIELDS are checked against row camera_of[f] of settings
+    (an (n_cameras, 3) array of window_size, scale, kernel_size), its BATCH_WIDE_FIELDS against base's."""
+    settings = np.asarray(settings).reshape(-1, 3)
+    camera_of = np.asarray(camera_of).reshape(-1)
+
+    def want(f, name):
+        if name in CAMERA_FIELDS:
+            k = int(camera_of[f])
+            return int(settings[k, CAMERA_FIELDS.index(name)]), f"camera {k}'s", "every filter of a camera"
+        return getattr(base, name), "the batch's", "every filter of a batch"
+    return _rows(cfgs, want)
+
+
+def camera_settings_of(cfgs, camera_of):
+    """The camera table of a batch whose filter f runs cfgs[f] and follows camera camera_of[f]: an (n_cameras, 3) int array of
+    (window_size, scale, kernel_size), n_cameras = max(camera_of) + 1.  ValueError, naming the filter and field, when filters
+    of one camera disagree on a CAMERA_FIELDS entry or any filters on a BATCH_WIDE_FIELDS entry, or a camera has no filter."""
+    cfgs = list(cfgs)
+    cam = np.asarray(camera_of, dtype=np.int64).reshape(-1)
+    if cam.shape != (len(cfgs),) or len(cfgs) < 1 or cam.min() < 0:
+        raise ValueError("camera_of needs one camera >= 0 per configuration")
+    n_cam = int(cam.max()) + 1
+    first = np.full(n_cam, -1)
+    for f in range(len(cfgs)):
+        if first[cam[f]] < 0:
+            first[cam[f]] = f
+    if (first < 0).any():
+        raise ValueError(f"camera {int(np.argmax(first < 0))} has no filter")
+    for f, c in enumerate(cfgs):
+        for name in CAMERA_FIELDS:
+            g = cfgs[first[cam[f]]]
+            if getattr(c, name) != getattr(g, name):
+                raise ValueError(f"filter {f}: {name} = {getattr(c, name)} differs from {getattr(g, name)} of filter "
+                                 f"{first[cam[f]]}, which follows the same camera {cam[f]}; it is shared by every filter of a camera")
+        for name in BATCH_WIDE_FIELDS:
+            if getattr(c, name) != getattr(cfgs[0], name):
+                raise ValueError(f"filter {f}: {name} = {getattr(c, name)} differs from filter 0's {getattr(cfgs[0], name)}; "
+                                 f"it is shared by every filter of a batch")
+    return np.array([[getattr(cfgs[first[k]], n) for n in CAMERA_FIELDS] for k in range(n_cam)], dtype=np.int64)
+
+
+def _rows(cfgs, want):
     cfgs = list(cfgs)
     cam = np.zeros((len(cfgs), 9), dtype=np.float64)
     rows = (EkfFilterParams * len(cfgs))()
     for f, c in enumerate(cfgs):
         for name in BATCH_SHARED_FIELDS:
-            if getattr(c, name) != getattr(base, name):
-                raise ValueError(f"filter {f}: {name} = {getattr(c, name)} differs from the batch's {getattr(base, name)}; "
-                                 f"it is shared by every filter of a batch")
+            v, whose, shared = want(f, name)
+            if getattr(c, name) != v:
+                raise ValueError(f"filter {f}: {name} = {getattr(c, name)} differs from {whose} {v}; it is shared by {shared}")
         cam[f] = [getattr(c, n) for n in INTRINSICS]
         for name, _ in EkfFilterParams._fields_:
             if name != "_pad":

@@ -107,6 +107,7 @@ SIGNATURES = {
     "ekf_batch_set_detect_budget": (_i, [_vp, C.c_int64]),
     "ekf_batch_set_intrinsics": (_i, [_vp, _vp]),
     "ekf_batch_set_filter_params": (_i, [_vp, _vp]),
+    "ekf_batch_set_camera_settings": (_i, [_vp, _vp]),
     "ekf_batch_set_frame_sizes": (_i, [_vp, _vp]),
     "ekf_batch_step_controls": (_i, [_vp, _vp, _vp, _vp, _vp, _i]),
     "ekf_batch_capture_camera_frames": (_i, [_vp, _i, _vp, _vp, _i, _i, _i, _vp]),

@@ -73,12 +73,18 @@ struct BatchView {
 // The configuration filter b runs: its intrinsics and tuning.  ROWS: the batch has per-filter rows (kernels that read the
 // row take it as a template parameter, so that a batch without rows runs the code it ran before).  A reference, so that the
 // fields load where they are used.  A row is the whole configuration: upload_rows rebuilds every row from dcfg whenever dcfg
-// or a table changes, so a row's shared fields (window, search clamp, blur switch, forsePlane) always equal cfg's; the kernels
-// still read those from cfg, so that they load from the parameter bank.
+// or a table changes, so a row's batch-wide fields (search clamp, template stride, forsePlane) always equal cfg's, and the
+// kernels read those from cfg, so that they load from the parameter bank.  The window and the blur threshold are the filter's
+// camera's (ekf_batch_set_camera_settings): with rows the kernels read them from the row (filter_window, filter_blur_min).
 template <bool ROWS>
 __device__ __forceinline__ const DevCfg& filter_cfg(const BatchView& bv, const DevCfg& cfg, int b) {
   if constexpr (ROWS) return bv.row[b].cfg;
   else return cfg;
+}
+template <bool ROWS>
+__device__ __forceinline__ int filter_window(const BatchView& bv, const DevCfg& cfg, int b) {
+  if constexpr (ROWS) return bv.row[b].cfg.window;
+  else return cfg.window;
 }
 template <bool ROWS>
 __device__ __forceinline__ const CamParams& filter_cam(const BatchView& bv, const DevCfg& cfg, int b) {
@@ -234,7 +240,7 @@ __global__ void __launch_bounds__(BPRED_THREADS, 4) k_batch_predict(BatchView bv
       double qc[4] = {cm[3], -cm[4], -cm[5], -cm[6]}, Rcw[9], hi[2], Hc[26], hcz;
       d_quat2rot(qc, Rcw);
       d_feature_hH(fc.cam, fs, coding, cm, qc, Rcw, hi, Hc, &hcz);
-      const int half = cfg.window / 2;
+      const int half = filter_window<ROWS>(bv, cfg, b) / 2;
       int fw = fr.w, fh = fr.h;
       if (in.fsize) {
         const int c = in.cam_of ? in.cam_of[b] : 0;
@@ -311,6 +317,9 @@ __global__ void __launch_bounds__(BBLUR_WARPS * 32) k_batch_predict_blur(BatchVi
   const int N = bv.N[b], ld = bv.ld;
   const double* mu = bv.mu + (size_t)b * ld;
   const FeatTab ft = feattab_slice(bv.ft, b, bv.Ncap, bv.tstride);
+  // with rows, the threshold of the filter's camera; a camera with blur off (>= 100000) blurs nothing, as a single filter
+  // without blur runs no blur prediction
+  const int kmin = ROWS ? filter_cfg<ROWS>(bv, cfg, b).kernel_min_size : 0;
   if (warp == 0) {   // one feature per lane, NC / 32 rounds
     int nblur = 0;
     unsigned anybig = 0u;
@@ -319,7 +328,7 @@ __global__ void __launch_bounds__(BBLUR_WARPS * 32) k_batch_predict_blur(BatchVi
       const int f = f0 + lane;
       int d = 0, krows = 0, kcols = 0;
       double ddx = 0.0, ddy = 0.0;
-      if (f < N && ft.innov[f]) {
+      if (f < N && ft.innov[f] && (!ROWS || kmin < 100000)) {
         double cam[13], rb[3], Rb[9];
         for (int c = 0; c < 13; ++c) cam[c] = mu[c];   // predicted camera state, committed by k_batch_predict
         blur_pose(cam, filter_cfg<ROWS>(bv, cfg, b).T_camera, dT, rb, Rb);
@@ -327,7 +336,7 @@ __global__ void __launch_bounds__(BBLUR_WARPS * 32) k_batch_predict_blur(BatchVi
         double fs[6];
         for (int c = 0; c < (coding ? 3 : 6); ++c) fs[c] = mu[pos + c];
         blur_displacement(filter_cam<ROWS>(bv, cfg, b), fs, coding, rb, Rb, ft.h[2 * f], ft.h[2 * f + 1], &ddx, &ddy);
-        d = blur_decide(ddx, ddy, cfg.kernel_min_size, &krows, &kcols);
+        d = blur_decide(ddx, ddy, ROWS ? kmin : cfg.kernel_min_size, &krows, &kcols);
       }
       const unsigned blur = __ballot_sync(0xffffffffu, d > 0), big = __ballot_sync(0xffffffffu, d < 0);
       if (d > 0) {
@@ -344,7 +353,7 @@ __global__ void __launch_bounds__(BBLUR_WARPS * 32) k_batch_predict_blur(BatchVi
     }
   }
   __syncthreads();
-  const int w = cfg.window, w2 = w * w;
+  const int w = filter_window<ROWS>(bv, cfg, b), w2 = w * w;
   uint8_t* tm = s_tmpl[warp];
   int* seq = s_seq[warp];
   int* coef = s_coef[warp];
@@ -1411,7 +1420,7 @@ __global__ void __launch_bounds__(BADD_THREADS) k_batch_add(BatchView bv, FrameV
   if (k <= 0) return;
   if (cam_of) fr.px += (size_t)cam_of[b] * fr.h * fr.stride;
   const DevCfg& fc = filter_cfg<ROWS>(bv, cfg, b);
-  const int ld = bv.ld, w = cfg.window, w2 = w * w;
+  const int ld = bv.ld, w = filter_window<ROWS>(bv, cfg, b), w2 = w * w;
   double* Sigma = bv.Sigma + (size_t)b * bv.sstride;
   double* mu = bv.mu + (size_t)b * ld;
   const FeatTab ft = feattab_slice(bv.ft, b, bv.Ncap, bv.tstride);
@@ -1670,7 +1679,11 @@ struct ekf_batch {
   bool fsize_on = false;                        // the captured stack has per-camera sizes
   std::vector<CamParams> intr_host;             // [B] intrinsics of each filter (ekf_batch_set_intrinsics); empty: the configuration's
   std::vector<ekf_filter_params> tune_host;     // [B] tuning of each filter (ekf_batch_set_filter_params); empty: the configuration's
-  FilterRow* rows_dev = nullptr;                // [B] rows built from dcfg and both tables; bv.row, null while neither is set
+  FilterRow* rows_dev = nullptr;                // [B] rows built from dcfg and the three tables; bv.row, null while none is set
+  std::vector<ekf_camera_settings> camset;      // [n_cam] window, scale, blur threshold of each camera (ekf_batch_set_camera_settings); empty: the batch's
+  int* cwin_dev = nullptr;                      // [n_cam] each camera's window for the detector, while camset is set
+  std::vector<int> map_win;                     // the distinct windows of camset and a tensor map of the stack for each (build_window_maps)
+  std::vector<EkfTensorMap> win_maps;
   int* det_slot = nullptr;                      // [n_cam] position of each camera among those a detection asks from, or -1
   int* h_det_slot = nullptr;                    // pinned
   size_t det_budget = (size_t)1 << 30;          // scratch of one chunk of cameras of the per-camera detector
@@ -1731,6 +1744,42 @@ static int bfail(ekf_batch* b, int code, const std::string& msg) {
 template <class T>
 static cudaError_t balloc(T** p, size_t count) { return cudaMalloc((void**)p, sizeof(T) * std::max<size_t>(count, 1)); }
 
+// Camera c's window, scale and blur threshold: its row of ekf_batch_set_camera_settings, or the batch's values without a table.
+static int cam_window(const ekf_batch* b, int c) { return b->camset.empty() ? b->cfg.window_size : b->camset[c].window_size; }
+static int cam_scale(const ekf_batch* b, int c) { return b->camset.empty() ? b->cfg.scale : b->camset[c].scale; }
+// A step blurs when some camera's threshold switches blur on; steps without blur leave the counts at zero.
+static void update_blur(ekf_batch* b) {
+  b->blur = b->dcfg.kernel_min_size < 100000;
+  if (!b->camset.empty()) {
+    b->blur = false;
+    for (const ekf_camera_settings& r : b->camset) b->blur = b->blur || r.kernel_size < 100000;
+  }
+  if (!b->blur) std::fill(b->h_blur, b->h_blur + 2 * (size_t)b->B, 0);
+}
+// MATCH_WIN_* of the windows the filters match with (launch_match_filter_batch); 0 without a table: every filter at cfg.window.
+static int match_windows(const ekf_batch* b) {
+  int m = 0;
+  for (int c = 0; c < (int)b->camset.size(); ++c) {
+    const int w = b->camset[c].window_size;
+    m |= w == 11 ? MATCH_WIN_11 : MATCH_WIN_NOT_11;
+  }
+  return m;
+}
+// With a table: the distinct camera windows and a tensor map of the frame stack for each, whose box is that window's (the CTA
+// matcher runs once per window with its map).  Rebuilt whenever the stack or the table changes; empty without a table.
+static void build_window_maps(ekf_batch* b) {
+  b->map_win.clear(); b->win_maps.clear();
+  if (b->camset.empty() || !b->fv.px) return;
+  for (const ekf_camera_settings& r : b->camset) {
+    if (std::find(b->map_win.begin(), b->map_win.end(), r.window_size) != b->map_win.end()) continue;
+    b->map_win.push_back(r.window_size);
+    EkfTensorMap m{};
+    if (r.window_size == b->cfg.window_size) m = b->frame_map;
+    else match_make_tensor_map(&m, b->fv.px, b->fv.w, b->fv.h, b->fv.stride, b->n_cam, r.window_size, (int)b->cfg.search_clamp);
+    b->win_maps.push_back(m);
+  }
+}
+
 extern "C" {
 
 const char* ekf_batch_last_error(const ekf_batch* b) { return b ? b->err.c_str() : "null batch"; }
@@ -1750,6 +1799,7 @@ int ekf_batch_destroy(ekf_batch* b) {
   cudaFree(b->scratch); cudaFree(b->frame); cudaFree(b->raw); cudaFree(b->picks_dev); cudaFree(b->out_mu14); cudaFree(b->out_S14);
   cudaFree(b->out_stats); cudaFree(b->stage_mu14); cudaFree(b->bv.patchnumbre);
   cudaFree(b->cam_dev); cudaFree(b->det_slot); cudaFree(b->step_dev); cudaFree(b->rows_dev); cudaFree(b->fsize_dev); cudaFree(b->slot_dev);
+  cudaFree(b->cwin_dev);
   if (b->h_det_slot) cudaFreeHost(b->h_det_slot);
   if (b->step_host) cudaFreeHost(b->step_host);
   batch_detect_free(b->det);
@@ -1962,15 +2012,33 @@ int ekf_batch_seed_from(ekf_batch* b, ekf_handle* src) {
   if (!b || !src) return EKF_ERR_ARG;
   if (src->device != b->device) return bfail(b, EKF_ERR_ARG, "seed filter lives on another device");
   if (src->N > b->Ncap || src->n > b->ncap) return bfail(b, EKF_ERR_CAPACITY, "seed filter holds more features than the batch capacity");
-  if (src->cfg.window_size != b->cfg.window_size) return bfail(b, EKF_ERR_ARG, "window_size differs");
+  if (b->camset.empty()) {
+    if (src->cfg.window_size != b->cfg.window_size) return bfail(b, EKF_ERR_ARG, "window_size differs");
+  } else if (src->N > 0) {   // its templates have its window: every camera must run it
+    for (int c = 0; c < b->n_cam; ++c)
+      if (b->camset[c].window_size != src->cfg.window_size)
+        return bfail(b, EKF_ERR_ARG, "seed filter holds features of window_size " + std::to_string(src->cfg.window_size) + ", camera " +
+                                         std::to_string(c) + " runs window_size " + std::to_string(b->camset[c].window_size));
+  }
   const int nd = (int)src->deleted.size();
   if (b->ar.cap > 0 && nd > b->ar.cap)
     return bfail(b, EKF_ERR_CAPACITY, "seed filter's feature archive holds more records than the batch's archive capacity");
   BCHECK(cudaSetDevice(b->device));
   BCHECK(cudaStreamSynchronize(src->stream));
-  k_batch_seed<<<b->B, 256, 0, b->stream>>>(b->bv, src->Sigma, src->ld, src->mu, src->ft, src->n, src->N, src->patchnumbre);
+  FeatTab sft = src->ft;
+  uint8_t* restride = nullptr;
+  if (src->N > 0 && src->dcfg.tstride != b->bv.tstride) {   // a smaller window than the batch's: templates to the batch's stride
+    const size_t tb = (size_t)b->bv.tstride, wb = (size_t)src->cfg.window_size * src->cfg.window_size;
+    BCHECK(cudaMallocAsync((void**)&restride, 2 * tb * src->N, b->stream));
+    BCHECK(cudaMemsetAsync(restride, 0, 2 * tb * src->N, b->stream));
+    sft.patch = restride; sft.mpatch = restride + tb * src->N;
+    BCHECK(cudaMemcpy2DAsync(sft.patch, tb, src->ft.patch, src->dcfg.tstride, wb, src->N, cudaMemcpyDeviceToDevice, b->stream));
+    BCHECK(cudaMemcpy2DAsync(sft.mpatch, tb, src->ft.mpatch, src->dcfg.tstride, wb, src->N, cudaMemcpyDeviceToDevice, b->stream));
+  }
+  k_batch_seed<<<b->B, 256, 0, b->stream>>>(b->bv, src->Sigma, src->ld, src->mu, sft, src->n, src->N, src->patchnumbre);
   b->launches += 1;
   BCHECK(cudaGetLastError());
+  if (restride) BCHECK(cudaFreeAsync(restride, b->stream));
   if (b->ar.cap > 0) {   // deleted_patches travels with the filter: every filter starts from the source's archive
     std::vector<double> rec((size_t)std::max(nd, 1) * PTS_COLS);
     std::vector<int> ri((size_t)std::max(nd, 1));
@@ -2035,22 +2103,28 @@ static int bcapture(ekf_batch* b, const uint8_t* img, int width, int height, int
       seen[c] = 1;
     }
   }
-  const int scale = b->cfg.scale, n_all = b->n_cam, n = sub ? n_list : n_all;
+  const int n_all = b->n_cam, n = sub ? n_list : n_all;
+  // the slot is sized by the smallest scale (ekf_batch_set_camera_settings); a camera of another scale fills part of it
+  int scale = cam_scale(b, 0);
+  bool one_scale = true;
+  for (int c = 1; c < n_all; ++c) { scale = std::min(scale, cam_scale(b, c)); one_scale = one_scale && cam_scale(b, c) == cam_scale(b, 0); }
   const int dw = width / scale, dh = height / scale;   // cv::Size(width / scale, height / scale), integer division
   if (dw < 8 || dh < 8) return bfail(b, EKF_ERR_ARG, "resized frame smaller than 8 x 8 pixels");
-  // frame sizes per camera: camera c is the top-left size_in[c] of its slot, resized to size_in[c] / scale
+  // frame sizes per camera: camera c is the top-left size_in[c] of its slot (the whole slot without sizes), resized to
+  // size_in[c] / scale_c
   std::vector<int> fs;
   bool pads = false;
-  if (!b->size_in.empty()) {
+  if (!b->size_in.empty() || !one_scale) {
     fs.resize((size_t)4 * n_all);
     for (int c = 0; c < n_all; ++c) {
-      const int wc = b->size_in[2 * c], hc = b->size_in[2 * c + 1];
+      const int wc = b->size_in.empty() ? width : b->size_in[2 * c], hc = b->size_in.empty() ? height : b->size_in[2 * c + 1];
+      const int sc = cam_scale(b, c);
       if (wc > width || hc > height)
         return bfail(b, EKF_ERR_ARG, "camera " + std::to_string(c) + " is larger than the captured " + std::to_string(width) + " x " +
                                          std::to_string(height) + " slot");
-      if (wc / scale < 8 || hc / scale < 8)
+      if (wc / sc < 8 || hc / sc < 8)
         return bfail(b, EKF_ERR_ARG, "camera " + std::to_string(c) + ": resized frame smaller than 8 x 8 pixels");
-      fs[4 * c] = wc; fs[4 * c + 1] = hc; fs[4 * c + 2] = wc / scale; fs[4 * c + 3] = hc / scale;
+      fs[4 * c] = wc; fs[4 * c + 1] = hc; fs[4 * c + 2] = wc / sc; fs[4 * c + 3] = hc / sc;
     }
     for (int k = 0; k < n; ++k) {
       const int c = sub ? list[k] : k;
@@ -2094,7 +2168,7 @@ static int bcapture(ekf_batch* b, const uint8_t* img, int width, int height, int
     const std::vector<int> slots(list, list + n);
     BCHECK(cudaMemcpyAsync(b->slot_dev, slots.data(), sizeof(int) * n, cudaMemcpyHostToDevice, b->stream));
   }
-  if (scale == 1 && channels == 1 && !sub) {
+  if (scale == 1 && one_scale && channels == 1 && !sub) {
     BCHECK(cudaMemcpy2DAsync(b->frame, dstride, img, stride, width, (size_t)height * n, dev ? cudaMemcpyDeviceToDevice : cudaMemcpyHostToDevice,
                              b->stream));
   } else {
@@ -2138,7 +2212,10 @@ static int bcapture(ekf_batch* b, const uint8_t* img, int width, int height, int
   }
   if (b->fv.px != b->frame || b->fv.w != dw || b->fv.h != dh || b->fv.stride != dstride)
     match_make_tensor_map(&b->frame_map, b->frame, dw, dh, dstride, n_all, b->cfg.window_size, (int)b->cfg.search_clamp);
-  b->fv = FrameView{b->frame, dw, dh, dstride};
+  if (b->fv.px != b->frame || b->fv.w != dw || b->fv.h != dh || b->fv.stride != dstride) {
+    b->fv = FrameView{b->frame, dw, dh, dstride};
+    build_window_maps(b);
+  }
   for (int k = 0; k < n; ++k) b->cam_frame[sub ? list[k] : k] = 1;
   return EKF_OK;
 }
@@ -2175,6 +2252,7 @@ int ekf_batch_capture_camera_frames_bgr(ekf_batch* b, int n, const int32_t* came
   return bcapture(b, bgr, w, h, s, 3, stamps, false, n, cameras);
 }
 
+static int upload_rows(ekf_batch* b);
 int ekf_batch_set_cameras(ekf_batch* b, int n_cameras, const int32_t* camera_of) {
   if (!b) return EKF_ERR_ARG;
   if (n_cameras < 1 || n_cameras > b->B) return bfail(b, EKF_ERR_ARG, "n_cameras must lie in [1, n_filters]");
@@ -2185,6 +2263,11 @@ int ekf_batch_set_cameras(ekf_batch* b, int n_cameras, const int32_t* camera_of)
     if (cam[f] < 0 || cam[f] >= n_cameras)
       return bfail(b, EKF_ERR_ARG, "camera_of[" + std::to_string(f) + "] = " + std::to_string(cam[f]) + " is not a camera");
   }
+  const bool had_table = !b->camset.empty();   // cleared below: every camera returns to the batch's window
+  for (int f = 0; had_table && f < b->B; ++f)
+    if (b->h_N[f] > 0 && cam_window(b, b->cam_host[f]) != b->cfg.window_size)
+      return bfail(b, EKF_ERR_STATE, "filter " + std::to_string(f) + " holds features of window_size " +
+                                         std::to_string(cam_window(b, b->cam_host[f])) + ": clearing the camera settings would change it");
   BCHECK(cudaSetDevice(b->device));
   BCHECK(cudaStreamSynchronize(b->stream));
   cudaFree(b->cam_dev); cudaFree(b->det_slot); cudaFreeHost(b->h_det_slot); cudaFree(b->fsize_dev); cudaFree(b->slot_dev);
@@ -2204,16 +2287,22 @@ int ekf_batch_set_cameras(ekf_batch* b, int n_cameras, const int32_t* camera_of)
   b->cam_dT.assign(n_cameras, dT); b->cam_ts.assign(n_cameras, ts);
   b->cam_frame.assign(n_cameras, 0);
   b->fv = FrameView{nullptr, 0, 0, 0};   // the next capture encodes the stack's tensor map
-  return EKF_OK;
+  if (!had_table) return EKF_OK;
+  b->camset.clear();
+  cudaFree(b->cwin_dev);
+  b->cwin_dev = nullptr;
+  build_window_maps(b);
+  update_blur(b);
+  return upload_rows(b);
 }
 
 static_assert(sizeof(CamParams) == 9 * sizeof(double), "a row of ekf_batch_set_intrinsics is one CamParams");
-// The device rows from the configuration and both tables (ekf_batch_set_intrinsics, ekf_batch_set_filter_params), in one copy;
-// no rows while neither table is set.
+// The device rows from the configuration and the three tables (ekf_batch_set_intrinsics, ekf_batch_set_filter_params and, by
+// the filter's camera, ekf_batch_set_camera_settings), in one copy; no rows while no table is set.
 static int upload_rows(ekf_batch* b) {
   BCHECK(cudaSetDevice(b->device));
   BCHECK(cudaStreamSynchronize(b->stream));   // work in flight may still read the rows
-  if (b->intr_host.empty() && b->tune_host.empty()) {
+  if (b->intr_host.empty() && b->tune_host.empty() && b->camset.empty()) {
     cudaFree(b->rows_dev);
     b->rows_dev = nullptr;
     b->bv.row = nullptr;
@@ -2226,6 +2315,10 @@ static int upload_rows(ekf_batch* b) {
     if (!b->tune_host.empty()) {
       set_tuning(r.cfg, b->tune_host[f]);
       r.min_features = b->tune_host[f].min_features; r.max_features = b->tune_host[f].max_features;
+    }
+    if (!b->camset.empty()) {
+      const ekf_camera_settings& c = b->camset[b->cam_host[f]];
+      r.cfg.window = c.window_size; r.cfg.kernel_min_size = c.kernel_size;
     }
   }
   if (!b->rows_dev) BCHECK(balloc(&b->rows_dev, b->B));
@@ -2272,6 +2365,48 @@ int ekf_batch_set_filter_params(ekf_batch* b, const ekf_filter_params* rows) {
   }
   if (rows) b->tune_host.assign(rows, rows + b->B);
   else b->tune_host.clear();
+  return upload_rows(b);
+}
+
+static_assert(sizeof(ekf_camera_settings) == 4 * sizeof(int32_t), "ekf_camera_settings has no hidden padding");
+int ekf_batch_set_camera_settings(ekf_batch* b, const ekf_camera_settings* rows) {
+  if (!b) return EKF_ERR_ARG;
+  for (int c = 0; rows && c < b->n_cam; ++c) {
+    const std::string at = "camera settings of camera " + std::to_string(c) + ": ";
+    if (rows[c].window_size < 3 || rows[c].window_size > b->cfg.window_size)
+      return bfail(b, EKF_ERR_ARG, at + "window_size = " + std::to_string(rows[c].window_size) + " outside [3, " +
+                                       std::to_string(b->cfg.window_size) + "] (the batch's window_size is the largest)");
+    if (rows[c].scale < 1 || rows[c].scale > 64)
+      return bfail(b, EKF_ERR_ARG, at + "scale = " + std::to_string(rows[c].scale) + " outside [1, 64]");
+  }
+  bool rescale = false;
+  for (int c = 0; c < b->n_cam; ++c) rescale = rescale || (rows ? rows[c].scale : b->cfg.scale) != cam_scale(b, c);
+  for (int f = 0; f < b->B; ++f) {   // templates keep the size they were cut with
+    const int c = b->cam_host[f], w = rows ? rows[c].window_size : b->cfg.window_size;
+    if (b->h_N[f] > 0 && w != cam_window(b, c))
+      return bfail(b, EKF_ERR_STATE, "filter " + std::to_string(f) + " holds features of window_size " + std::to_string(cam_window(b, c)) +
+                                         ": camera " + std::to_string(c) + " cannot change it to " + std::to_string(w));
+  }
+  BCHECK(cudaSetDevice(b->device));
+  BCHECK(cudaStreamSynchronize(b->stream));   // work in flight may still read the windows
+  if (rows) {
+    std::vector<int> win(b->n_cam);
+    for (int c = 0; c < b->n_cam; ++c) win[c] = rows[c].window_size;
+    if (!b->cwin_dev) BCHECK(balloc(&b->cwin_dev, b->n_cam));
+    BCHECK(cudaMemcpyAsync(b->cwin_dev, win.data(), sizeof(int) * b->n_cam, cudaMemcpyHostToDevice, b->stream));
+    BCHECK(cudaStreamSynchronize(b->stream));   // win is freed when the call returns
+    b->camset.assign(rows, rows + b->n_cam);
+  } else {
+    cudaFree(b->cwin_dev);
+    b->cwin_dev = nullptr;
+    b->camset.clear();
+  }
+  if (rescale) {   // the slot and the cameras' resized sizes change from the next capture on
+    b->fsize_on = false;
+    std::fill(b->cam_frame.begin(), b->cam_frame.end(), 0);
+  }
+  update_blur(b);
+  build_window_maps(b);
   return upload_rows(b);
 }
 
@@ -2322,6 +2457,7 @@ int ekf_batch_get_dt(ekf_batch* b, double* out) {   // getDt for every filter
 
 int ekf_batch_set_scale(ekf_batch* b, int32_t scale) {
   if (!b || scale < 1 || scale > 64) return EKF_ERR_ARG;   // the range ekf_create accepts
+  if (!b->camset.empty()) return bfail(b, EKF_ERR_STATE, "the batch has camera settings: set each camera's scale there");
   b->cfg.scale = scale;
   return EKF_OK;
 }
@@ -2383,7 +2519,7 @@ static int batch_detect(ekf_batch* b, const int* num, const int* hnum, int num_s
   const size_t npx = (size_t)b->fv.w * b->fv.h;
   if (b->n_cam == 1 && !b->fsize_on) {
     BCHECK(batch_detect_reserve(b->det, npx, b->B, b->cstride));
-    BCHECK(launch_batch_detect(st, b->det, b->fv, b->bv.ft.center, b->bv.N, b->Ncap, b->B, b->cfg.window_size, num, num_stride, cap_mode,
+    BCHECK(launch_batch_detect(st, b->det, b->fv, b->bv.ft.center, b->bv.N, b->Ncap, b->B, cam_window(b, 0), num, num_stride, cap_mode,
                                b->cstride, b->det_xy, b->det_n, &b->launches));
     return EKF_OK;
   }
@@ -2403,7 +2539,7 @@ static int batch_detect(ekf_batch* b, const int* num, const int* hnum, int num_s
   BCHECK(launch_batch_detect_cams(st, b->det, b->fv, cams.data(), n_req, chunk, b->cam_dev, b->det_slot, b->bv.ft.center, b->bv.N, b->Ncap,
                                   b->B, b->cfg.window_size, num, num_stride, cap_mode, b->cstride, b->det_xy, b->det_n, &b->launches,
                                   b->fsize_on ? b->fsize_dev : nullptr, b->fsize_on ? b->fsize_host.data() : nullptr,
-                                  b->det_slot + b->n_cam));
+                                  b->det_slot + b->n_cam, b->cwin_dev));
   return EKF_OK;
 }
 
@@ -2553,7 +2689,7 @@ static int batch_step(ekf_batch* b, const double* dv, const double* dw, int vcon
   BCHECK(cudaEventRecord(b->ev[1], st));
   launch_match_filter_batch(st, b->bv.ft, b->Ncap, b->bv.N, (int)grid, b->fv, b->dcfg, &b->frame_map, b->match_defer,
                             b->match_defer + (size_t)b->B * b->Ncap, &b->launches, b->cam_dev, b->fsize_on ? b->fsize_dev : nullptr, sl.act,
-                            b->bv.row);
+                            b->bv.row, match_windows(b), b->win_maps.data(), b->map_win.data(), (int)b->win_maps.size());
   BCHECK(cudaEventRecord(b->ev[2], st));
   const bool plane = b->cfg.forsePlane != 0;
   if (b->large) {   // one cluster of cl_ctas CTAs per filter
@@ -2746,10 +2882,10 @@ int ekf_batch_add_feature(ekf_batch* b, int f, float u, float v) {
   const int rc = need_frame(b, f, "addFeature");
   if (rc) return rc;
   BCHECK(cudaSetDevice(b->device));
-  const int half = b->cfg.window_size / 2;
+  const int c = b->cam_host[f], half = cam_window(b, c) / 2;
   // isInsideImage (vslamRansac.cpp:314,1644-1652), as ekf_add_feature
   const double x = (double)u, y = (double)v;
-  const int c = b->cam_host[f], fw = b->fsize_on ? b->fsize_host[4 * c + 2] : b->fv.w, fh = b->fsize_on ? b->fsize_host[4 * c + 3] : b->fv.h;
+  const int fw = b->fsize_on ? b->fsize_host[4 * c + 2] : b->fv.w, fh = b->fsize_on ? b->fsize_host[4 * c + 3] : b->fv.h;
   if (!(x > half && y > half && x < fw - half && y < fh - half)) return 0;
   if (b->h_N[f] >= b->Ncap || b->h_n[f] + 6 > b->ncap) return bfail(b, EKF_ERR_CAPACITY, "feature capacity exceeded");
   add_kernel(b, false)<<<1, BADD_THREADS, 0, b->stream>>>(b->bv, b->fv, b->dcfg, nullptr, nullptr, f, u, v, 0, b->cam_dev, nullptr);
@@ -2828,9 +2964,9 @@ int ekf_batch_set_topup(ekf_batch* b, int on) {
 
 int ekf_batch_set_motion_blur(ekf_batch* b, int32_t kernel_size) {
   if (!b) return EKF_ERR_ARG;
+  if (!b->camset.empty()) return bfail(b, EKF_ERR_STATE, "the batch has camera settings: set each camera's kernel_size there");
   b->dcfg.kernel_min_size = kernel_size;
-  b->blur = kernel_size < 100000;
-  if (!b->blur) std::fill(b->h_blur, b->h_blur + 2 * (size_t)b->B, 0);   // steps without blur leave the counts at zero
+  update_blur(b);
   return b->bv.row ? upload_rows(b) : EKF_OK;   // the rows are whole configurations: they follow dcfg
 }
 
@@ -2851,7 +2987,8 @@ int ekf_batch_get_template(ekf_batch* b, int f, int idx, int which, uint8_t* out
   BCHECK(cudaSetDevice(b->device));
   const FeatTab t = feattab_slice(b->bv.ft, f, b->Ncap, b->bv.tstride);
   const uint8_t* src = (which ? t.mpatch : t.patch) + (size_t)idx * b->bv.tstride;
-  BCHECK(cudaMemcpyAsync(out, src, (size_t)b->cfg.window_size * b->cfg.window_size, cudaMemcpyDeviceToHost, b->stream));
+  const size_t w = (size_t)cam_window(b, b->cam_host[f]);
+  BCHECK(cudaMemcpyAsync(out, src, w * w, cudaMemcpyDeviceToHost, b->stream));
   BCHECK(cudaStreamSynchronize(b->stream));
   return EKF_OK;
 }

@@ -37,11 +37,15 @@
 // pixel keys (base mask, eig > 0) and candidate keys (those that are also raw 3x3 local maxima), one slot per pixel
 // (blockIdx.z: the camera's segment of a chunk)
 // fsize (ekf_batch_set_frame_sizes): segment z holds camera seg_cam[z] of fsize[4c + 2] x fsize[4c + 3] pixels, packed at the
-// segment's start with that width; the segment's other slots get no key.
+// segment's start with that width; the segment's other slots get no key.  WIN (ekf_batch_set_camera_settings): the mask border
+// of segment z is its camera's window cwin[seg_cam[z]] instead of estrem.
+template <bool WIN>
 __global__ void k_bdet_keys(const float* __restrict__ eig, int W, int H, int estrem, unsigned long long* __restrict__ kp,
-                            unsigned long long* __restrict__ kc, const int* __restrict__ fsize, const int* __restrict__ seg_cam) {
+                            unsigned long long* __restrict__ kc, const int* __restrict__ fsize, const int* __restrict__ seg_cam,
+                            const int* __restrict__ cwin) {
   int x = blockIdx.x * blockDim.x + threadIdx.x, y = blockIdx.y;
   if (x >= W) return;
+  if constexpr (WIN) estrem = cwin[seg_cam[blockIdx.z]];
   const size_t seg = (size_t)blockIdx.z * W * H;
   eig += seg; kp += seg; kc += seg;
   if (fsize) {
@@ -74,9 +78,10 @@ __device__ __forceinline__ int bdet_segment(const int* __restrict__ cam_of, cons
 }
 
 // One warp per filter: its boxes, its corner limit and thr_b from the first sorted pixel outside its boxes.  CS: boxes and
-// corners a filter has room for (EKF_BATCH_MAX_CORNERS, or EKF_BATCH_MAX_FEATURES in a large batch).
+// corners a filter has room for (EKF_BATCH_MAX_CORNERS, or EKF_BATCH_MAX_FEATURES in a large batch).  WIN: the boxes of filter b
+// have its camera's window cwin[cam_of[b]].
 #define BDET_WARPS 8
-template <int CS>
+template <int CS, bool WIN>
 __global__ void __launch_bounds__(32 * BDET_WARPS) k_bdet_threshold(const unsigned long long* __restrict__ kp, int npx, int W, int H,
                                                                      int window, const float* __restrict__ centers,
                                                                      const int* __restrict__ N, int Ncap, int B,
@@ -84,7 +89,7 @@ __global__ void __launch_bounds__(32 * BDET_WARPS) k_bdet_threshold(const unsign
                                                                      DetBox* __restrict__ boxes, unsigned* __restrict__ thr_bits,
                                                                      int* __restrict__ limit, const int* __restrict__ cam_of,
                                                                      const int* __restrict__ slot_of_cam, int lo, int hi,
-                                                                     const int* __restrict__ fsize) {
+                                                                     const int* __restrict__ fsize, const int* __restrict__ cwin) {
   __shared__ DetBox sb[BDET_WARPS][CS];
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int b = blockIdx.x * BDET_WARPS + warp;
@@ -96,6 +101,7 @@ __global__ void __launch_bounds__(32 * BDET_WARPS) k_bdet_threshold(const unsign
     const int c = cam_of ? cam_of[b] : 0;
     W = fsize[4 * c + 2]; H = fsize[4 * c + 3];
   }
+  if constexpr (WIN) window = cwin[cam_of ? cam_of[b] : 0];
   const int nb = N[b];
   int lim = min(num[(size_t)b * num_stride], cap_mode ? Ncap - nb : EKF_BATCH_MAX_CORNERS);
   lim = max(0, min(lim, CS));
@@ -204,7 +210,7 @@ cudaError_t launch_batch_detect(cudaStream_t st, BatchDetectBufs& d, FrameView f
   const int W = fr.w, H = fr.h, npx = W * H;
   unsigned long long *kp = d.keys, *kc = d.keys + d.cap, *kp_s = d.keys + 2 * d.cap, *kc_s = d.keys + 3 * d.cap;
   launch_det_eig(st, fr, d.eig, launches);
-  k_bdet_keys<<<dim3((W + 255) / 256, H), 256, 0, st>>>(d.eig, W, H, window, kp, kc, nullptr, nullptr);
+  k_bdet_keys<false><<<dim3((W + 255) / 256, H), 256, 0, st>>>(d.eig, W, H, window, kp, kc, nullptr, nullptr, nullptr);
   size_t tmp = d.tmp_bytes;
   cudaError_t e = cub::DeviceRadixSort::SortKeysDescending(d.tmp, tmp, kp, kp_s, npx, 0, 64, st);
   if (e != cudaSuccess) return e;
@@ -213,15 +219,15 @@ cudaError_t launch_batch_detect(cudaStream_t st, BatchDetectBufs& d, FrameView f
   if (e != cudaSuccess) return e;
   const unsigned gt = (B + BDET_WARPS - 1) / BDET_WARPS, gs = (B + 127) / 128;
   if (cstride == EKF_BATCH_MAX_CORNERS) {
-    k_bdet_threshold<EKF_BATCH_MAX_CORNERS><<<gt, 32 * BDET_WARPS, 0, st>>>(kp_s, npx, W, H, window, centers, N, Ncap, B, num,
-                                                                           num_stride, cap_mode, d.boxes, d.thr_bits, d.limit,
-                                                                           nullptr, nullptr, 0, 0, nullptr);
+    k_bdet_threshold<EKF_BATCH_MAX_CORNERS, false><<<gt, 32 * BDET_WARPS, 0, st>>>(kp_s, npx, W, H, window, centers, N, Ncap, B, num,
+                                                                                  num_stride, cap_mode, d.boxes, d.thr_bits, d.limit,
+                                                                                  nullptr, nullptr, 0, 0, nullptr, nullptr);
     k_bdet_select<EKF_BATCH_MAX_CORNERS><<<gs, 128, 0, st>>>(kc_s, npx, W, d.boxes, N, d.thr_bits, d.limit, B, out_xy, out_n,
                                                              nullptr, nullptr, 0, 0, nullptr);
   } else {
-    k_bdet_threshold<EKF_BATCH_MAX_FEATURES><<<gt, 32 * BDET_WARPS, 0, st>>>(kp_s, npx, W, H, window, centers, N, Ncap, B, num,
-                                                                            num_stride, cap_mode, d.boxes, d.thr_bits, d.limit,
-                                                                            nullptr, nullptr, 0, 0, nullptr);
+    k_bdet_threshold<EKF_BATCH_MAX_FEATURES, false><<<gt, 32 * BDET_WARPS, 0, st>>>(kp_s, npx, W, H, window, centers, N, Ncap, B, num,
+                                                                                   num_stride, cap_mode, d.boxes, d.thr_bits, d.limit,
+                                                                                   nullptr, nullptr, 0, 0, nullptr, nullptr);
     k_bdet_select<EKF_BATCH_MAX_FEATURES><<<gs, 128, 0, st>>>(kc_s, npx, W, d.boxes, N, d.thr_bits, d.limit, B, out_xy, out_n,
                                                               nullptr, nullptr, 0, 0, nullptr);
   }
@@ -232,7 +238,7 @@ cudaError_t launch_batch_detect(cudaStream_t st, BatchDetectBufs& d, FrameView f
 cudaError_t launch_batch_detect_cams(cudaStream_t st, BatchDetectBufs& d, FrameView fr, const int* cams, int n_req, int chunk,
                                      const int* cam_of, const int* slot_of_cam, const float* centers, const int* N, int Ncap, int B,
                                      int window, const int* num, int num_stride, int cap_mode, int cstride, float* out_xy, int* out_n,
-                                     long long* launches, const int* fsize, const int* fsize_host, const int* seg_cam) {
+                                     long long* launches, const int* fsize, const int* fsize_host, const int* seg_cam, const int* cwin) {
   const int W = fr.w, H = fr.h, npx = W * H;
   const size_t fstep = (size_t)fr.h * fr.stride;
   cudaError_t e = cudaMemsetAsync(out_n, 0, sizeof(int) * (size_t)B, st);   // filters of cameras nobody asks from find nothing
@@ -245,7 +251,9 @@ cudaError_t launch_batch_detect_cams(cudaStream_t st, BatchDetectBufs& d, FrameV
       const int c = cams[lo + s], wc = fsize_host ? fsize_host[4 * c + 2] : W, hc = fsize_host ? fsize_host[4 * c + 3] : H;
       launch_det_eig(st, FrameView{fr.px + (size_t)c * fstep, wc, hc, fr.stride}, d.eig + (size_t)s * npx, launches);
     }
-    k_bdet_keys<<<dim3((W + 255) / 256, H, C), 256, 0, st>>>(d.eig, W, H, window, kp, kc, fsize, fsize ? seg_cam + lo : nullptr);
+    if (cwin) k_bdet_keys<true><<<dim3((W + 255) / 256, H, C), 256, 0, st>>>(d.eig, W, H, window, kp, kc, fsize, seg_cam + lo, cwin);
+    else k_bdet_keys<false><<<dim3((W + 255) / 256, H, C), 256, 0, st>>>(d.eig, W, H, window, kp, kc, fsize, fsize ? seg_cam + lo : nullptr,
+                                                                       nullptr);
     size_t tmp = d.tmp_bytes;
     e = cub::DeviceSegmentedRadixSort::SortKeysDescending(d.tmp, tmp, kp, kp_s, C * npx, C, d.offs, d.offs + 1, 0, 64, st);
     if (e != cudaSuccess) return e;
@@ -253,15 +261,15 @@ cudaError_t launch_batch_detect_cams(cudaStream_t st, BatchDetectBufs& d, FrameV
     e = cub::DeviceSegmentedRadixSort::SortKeysDescending(d.tmp, tmp, kc, kc_s, C * npx, C, d.offs, d.offs + 1, 0, 64, st);
     if (e != cudaSuccess) return e;
     if (cstride == EKF_BATCH_MAX_CORNERS) {
-      k_bdet_threshold<EKF_BATCH_MAX_CORNERS><<<gt, 32 * BDET_WARPS, 0, st>>>(kp_s, npx, W, H, window, centers, N, Ncap, B, num,
-                                                                             num_stride, cap_mode, d.boxes, d.thr_bits, d.limit,
-                                                                             cam_of, slot_of_cam, lo, hi, fsize);
+      (cwin ? k_bdet_threshold<EKF_BATCH_MAX_CORNERS, true> : k_bdet_threshold<EKF_BATCH_MAX_CORNERS, false>)<<<gt, 32 * BDET_WARPS, 0, st>>>(
+          kp_s, npx, W, H, window, centers, N, Ncap, B, num, num_stride, cap_mode, d.boxes, d.thr_bits, d.limit, cam_of, slot_of_cam, lo, hi,
+          fsize, cwin);
       k_bdet_select<EKF_BATCH_MAX_CORNERS><<<gs, 128, 0, st>>>(kc_s, npx, W, d.boxes, N, d.thr_bits, d.limit, B, out_xy, out_n,
                                                                cam_of, slot_of_cam, lo, hi, fsize);
     } else {
-      k_bdet_threshold<EKF_BATCH_MAX_FEATURES><<<gt, 32 * BDET_WARPS, 0, st>>>(kp_s, npx, W, H, window, centers, N, Ncap, B, num,
-                                                                              num_stride, cap_mode, d.boxes, d.thr_bits, d.limit,
-                                                                              cam_of, slot_of_cam, lo, hi, fsize);
+      (cwin ? k_bdet_threshold<EKF_BATCH_MAX_FEATURES, true> : k_bdet_threshold<EKF_BATCH_MAX_FEATURES, false>)<<<gt, 32 * BDET_WARPS, 0, st>>>(
+          kp_s, npx, W, H, window, centers, N, Ncap, B, num, num_stride, cap_mode, d.boxes, d.thr_bits, d.limit, cam_of, slot_of_cam, lo, hi,
+          fsize, cwin);
       k_bdet_select<EKF_BATCH_MAX_FEATURES><<<gs, 128, 0, st>>>(kc_s, npx, W, d.boxes, N, d.thr_bits, d.limit, B, out_xy, out_n,
                                                                 cam_of, slot_of_cam, lo, hi, fsize);
     }

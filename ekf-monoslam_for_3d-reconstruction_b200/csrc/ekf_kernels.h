@@ -43,7 +43,13 @@ void launch_match_filter_batch(cudaStream_t st, FeatTab base, int Ncap, const in
                                const int* cam_of = nullptr,    // cam_of [B]: filter b searches frame cam_of[b] of the stack fr
                                const int* fsize = nullptr,     // [n_cameras][4] (in w, in h, w, h): camera c is the top-left w x h of its slot
                                const int* act = nullptr,       // [B]: the pairs' filter i is filter act[i] (a list of B filters)
-                               const FilterRow* rows = nullptr);   // [B]: filter b matches with rows[b].cfg's sigma_size and ncc_threshold
+                               const FilterRow* rows = nullptr,    // [B]: filter b matches with rows[b].cfg's sigma_size, ncc_threshold and window
+                               int windows = 0,    // MATCH_WIN_* of the rows' windows (rows only); 0: every filter at cfg.window
+                               // rows only: the n_wmaps distinct windows of the filters and a tensor map of the stack for each (its box
+                               // is that window's); the CTA matcher then runs once per window with its map.  0: one run with tmap
+                               const EkfTensorMap* wmaps = nullptr, const int* wmap_window = nullptr, int n_wmaps = 0);
+// The windows a batch's filters match with (ekf_batch_set_camera_settings): some filter at 11, some at another.
+enum { MATCH_WIN_11 = 1, MATCH_WIN_NOT_11 = 2 };
 int launch_match_batch(cudaStream_t st, const uint8_t* frames, int n_frames, int width, int height, int stride,
                        const uint8_t* templates, int fpf, int w, const double* h, const double* S, float sigma_size,
                        float thr, float clampv, int32_t* out_uv, float* out_score);
@@ -163,4 +169,5 @@ cudaError_t launch_batch_detect_cams(cudaStream_t st, BatchDetectBufs& d, FrameV
                                      const int* cam_of, const int* slot_of_cam, const float* centers, const int* N, int Ncap, int B,
                                      int window, const int* num, int num_stride, int cap_mode, int cstride, float* out_xy, int* out_n,
                                      long long* launches, const int* fsize = nullptr, const int* fsize_host = nullptr,
-                                     const int* seg_cam = nullptr);   // per-camera sizes (device / host [n_cameras][4]); seg_cam: cams on the device
+                                     const int* seg_cam = nullptr,   // per-camera sizes (device / host [n_cameras][4]); seg_cam: cams on the device
+                                     const int* cwin = nullptr);   // [n_cameras] each camera's window (mask border, boxes); null: `window`

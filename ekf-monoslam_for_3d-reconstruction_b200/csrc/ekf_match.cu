@@ -550,6 +550,7 @@ __global__ void __launch_bounds__(MATCH_THREADS, 4) k_match_filter(FeatTab ft, i
 #define MW_GRID 16
 #define MW_MAXW 15
 #define MW_WARPS 8
+#define MATCH_WARP_SKIP11 3   // warp_path of k_match_filter_batch_warp beside k_match_filter_batch_warp2 (a batch of mixed windows)
 #define MW_ROWS (MW_GRID + MW_MAXW - 1)   // 30 window rows
 #define MW_WS 40                          // window row stride in bytes (30 columns + slack for whole-word reads)
 #define MW_LIST 16
@@ -1068,8 +1069,9 @@ __device__ __forceinline__ int batch_pair_filter(const int* __restrict__ act, in
   else return i;
 }
 
-// ROWS (a batch with per-filter rows, ekf_batch_set_filter_params / ekf_batch_set_intrinsics): filter b searches and accepts with
-// its row's sigma_size and ncc_threshold.  Without rows the kernels are the code they were before.
+// ROWS (a batch with per-filter rows, ekf_batch_set_filter_params / ekf_batch_set_intrinsics / ekf_batch_set_camera_settings):
+// filter b searches and accepts with its row's sigma_size and ncc_threshold, and with its row's window, its camera's.  Without
+// rows the kernels are the code they were before.
 template <bool ROWS>
 __device__ __forceinline__ const DevCfg& batch_filter_cfg(const DevCfg& cfg, const FilterRow* __restrict__ rows, int b) {
   if constexpr (ROWS) return rows[b].cfg;
@@ -1102,6 +1104,9 @@ __global__ void __launch_bounds__(MW2_WARPS * 32, MINB) k_match_filter_batch_war
   __syncwarp();
   MatchResult r;
   const DevCfg& fc = batch_filter_cfg<ROWS>(cfg, rows, b);
+  if constexpr (ROWS) {
+    if (fc.window != 11) return;   // a filter whose camera has another window takes k_match_filter_batch_warp
+  }
   if (!match_one_warp2<11, TSMEM, SLIDE>(jb, fc.sigma_size_f, cfg.search_clamp, wsm[warp], r)) {
     if (lane == 0) defer_list[atomicAdd(defer_cnt, 1)] = (int)pair;
     return;
@@ -1110,7 +1115,8 @@ __global__ void __launch_bounds__(MW2_WARPS * 32, MINB) k_match_filter_batch_war
   match_warp_commit(ft, f, fr, fc, r);
 }
 
-// Batched filters, pass 1: one warp per (filter, feature); features that do not fit go to defer_list.
+// Batched filters, pass 1: one warp per (filter, feature); features that do not fit go to defer_list.  warp_path ==
+// MATCH_WARP_SKIP11 (rows only): the window-11 filters were matched by k_match_filter_batch_warp2 and are skipped here.
 template <bool CAMS, bool SIZES, bool ACT, bool ROWS>
 __global__ void __launch_bounds__(MW_WARPS * 32) k_match_filter_batch_warp(FeatTab base, int Ncap, const int* __restrict__ Nper, int B,
                                                                            FrameView fr, DevCfg cfg, int* __restrict__ defer_list,
@@ -1125,7 +1131,11 @@ __global__ void __launch_bounds__(MW_WARPS * 32) k_match_filter_batch_warp(FeatT
   const long long pair = ACT ? (long long)b * Ncap + f : pair_i;
   const FeatTab ft = feattab_slice(base, b, Ncap, cfg.tstride);
   if (f >= Nper[b] || !ft.innov[f]) return;
-  const int w = cfg.window, w2 = w * w;
+  const DevCfg& fc = batch_filter_cfg<ROWS>(cfg, rows, b);
+  if constexpr (ROWS) {
+    if (warp_path == MATCH_WARP_SKIP11 && fc.window == 11) return;   // k_match_filter_batch_warp2 took this filter
+  }
+  const int w = ROWS ? fc.window : cfg.window, w2 = w * w;
   MatchJob jb;
   fr = batch_frame_of<CAMS, SIZES>(fr, cam_of, fsize, b);
   jb.tmap = nullptr; jb.frame_index = 0;
@@ -1136,7 +1146,6 @@ __global__ void __launch_bounds__(MW_WARPS * 32) k_match_filter_batch_warp(FeatT
   if (lane == 0) wsm[warp].cnt = 0;
   __syncwarp();
   MatchResult r;
-  const DevCfg& fc = batch_filter_cfg<ROWS>(cfg, rows, b);
   if (!warp_path || !match_one_warp(jb, w, fc.sigma_size_f, cfg.search_clamp, wsm[warp], r)) {
     if (lane == 0) defer_list[atomicAdd(defer_cnt, 1)] = (int)pair;
     return;
@@ -1160,7 +1169,9 @@ __global__ void __launch_bounds__(MW_WARPS * 32) k_match_filter_batch_warp(FeatT
     }
   }
 }
-// pass 2: a persistent grid of CTAs works off the deferred (filter, feature) pairs with match_one
+// pass 2: a persistent grid of CTAs works off the deferred (filter, feature) pairs with match_one.  only_window > 0 (rows only):
+// the pairs of the filters at that window alone, the ones the tensor map tmap has the box of.  One window per launch keeps the
+// shared-memory plan, and with it the TMA mbarrier's place, the same for every pair a CTA takes.
 template <bool CAMS, bool SIZES, bool ROWS>
 __global__ void __launch_bounds__(MATCH_THREADS) k_match_filter_batch_deferred(FeatTab base, int Ncap, FrameView fr, DevCfg cfg,
                                                                                const __grid_constant__ CUtensorMap tmap, int use_tma,
@@ -1168,7 +1179,7 @@ __global__ void __launch_bounds__(MATCH_THREADS) k_match_filter_batch_deferred(F
                                                                                const int* __restrict__ defer_cnt,
                                                                                const int* __restrict__ cam_of,
                                                                                const int* __restrict__ fsize,
-                                                                               const FilterRow* __restrict__ rows) {
+                                                                               const FilterRow* __restrict__ rows, int only_window) {
   extern __shared__ __align__(128) unsigned char smem_raw[];
   const int n = *defer_cnt;
   unsigned phase = 0;
@@ -1176,6 +1187,9 @@ __global__ void __launch_bounds__(MATCH_THREADS) k_match_filter_batch_deferred(F
   for (int i = blockIdx.x; i < n; i += gridDim.x) {
     const int pair = defer_list[i];
     const int b = pair / Ncap, f = pair - b * Ncap;
+    if constexpr (ROWS) {
+      if (only_window > 0 && rows[b].cfg.window != only_window) continue;   // uniform over the CTA
+    }
     const FeatTab ft = feattab_slice(base, b, Ncap, cfg.tstride);
     const int cam = ((CAMS || SIZES) && cam_of) ? cam_of[b] : 0;
     match_filter_feature(ft, f, batch_frame_of<CAMS, SIZES>(fr, cam_of, fsize, b), batch_filter_cfg<ROWS>(cfg, rows, b), smem_raw,
@@ -1303,7 +1317,8 @@ void launch_match_filter(cudaStream_t st, FeatTab ft, int N, FrameView fr, const
 
 void launch_match_filter_batch(cudaStream_t st, FeatTab base, int Ncap, const int* Nper, int B, FrameView fr, const DevCfg& cfg,
                                const EkfTensorMap* tmap, int* defer_list, int* defer_cnt, long long* launches, const int* cam_of,
-                               const int* fsize, const int* act, const FilterRow* rows) {
+                               const int* fsize, const int* act, const FilterRow* rows, int windows, const EkfTensorMap* wmaps,
+                               const int* wmap_window, int n_wmaps) {
   if (B <= 0 || Ncap <= 0) return;
   static PerDeviceOnce once;   // opt in to the largest supported window once per device
   const size_t smem = match_smem_bytes(cfg.window, cfg.search_clamp);
@@ -1318,13 +1333,18 @@ void launch_match_filter_batch(cudaStream_t st, FeatTab base, int Ncap, const in
       }) != cudaSuccess) return;   // the error stays in cudaGetLastError() for the caller
   static const EkfTensorMap none{};
   const EkfTensorMap& tm = (tmap && tmap->ok) ? *tmap : none;
+  const bool has11 = windows ? (windows & MATCH_WIN_11) != 0 : cfg.window == 11;
+  const bool has_other = windows ? (windows & MATCH_WIN_NOT_11) != 0 : cfg.window != 11;
   // pass 1: a warp per (filter, feature) for small windows; pass 2: a persistent grid of CTAs for the deferred rest
   cudaMemsetAsync(defer_cnt, 0, sizeof(int), st);
   const long long pairs = (long long)B * Ncap;
   // EKF_MATCH_WARP: 2 (default) full-window warp matcher where the template side allows it, 1 the small-window warp matcher only,
   // 0 every feature takes the CTA matcher (A/B timing, tests)
   static const int warp_path = [] { const char* e = getenv("EKF_MATCH_WARP"); return e ? atoi(e) : 2; }();
-  if (warp_path >= 2 && cfg.window == 11 && cfg.search_clamp <= 20.0f) {
+  // window-11 filters take the full-window warp matcher, the others the small-window one; with both in the batch (rows only),
+  // each launch skips the other's filters
+  const bool full = warp_path >= 2 && cfg.search_clamp <= 20.0f;
+  if (full && has11) {
     const unsigned grid = (unsigned)((pairs + MW2_WARPS - 1) / MW2_WARPS);
     const int var = match_w2_variant();
 #define MW2_LAUNCH_ACT(MINB, TS, SL, ACT, RW)                                                                                           \
@@ -1346,12 +1366,14 @@ void launch_match_filter_batch(cudaStream_t st, FeatTab base, int Ncap, const in
     }
 #undef MW2_LAUNCH
 #undef MW2_LAUNCH_ACT
-  } else {
+  }
+  if (!full || has_other) {
     const unsigned grid = (unsigned)((pairs + MW_WARPS - 1) / MW_WARPS);
+    const int wp = (full && has11) ? MATCH_WARP_SKIP11 : warp_path;
 #define MW_LAUNCH(ACT, RW)                                                                                                            \
-  if (fsize) k_match_filter_batch_warp<true, true, ACT, RW><<<grid, MW_WARPS * 32, 0, st>>>(base, Ncap, Nper, B, fr, cfg, defer_list, defer_cnt, warp_path, cam_of, fsize, act, rows); \
-  else if (cam_of) k_match_filter_batch_warp<true, false, ACT, RW><<<grid, MW_WARPS * 32, 0, st>>>(base, Ncap, Nper, B, fr, cfg, defer_list, defer_cnt, warp_path, cam_of, fsize, act, rows); \
-  else k_match_filter_batch_warp<false, false, ACT, RW><<<grid, MW_WARPS * 32, 0, st>>>(base, Ncap, Nper, B, fr, cfg, defer_list, defer_cnt, warp_path, cam_of, fsize, act, rows)
+  if (fsize) k_match_filter_batch_warp<true, true, ACT, RW><<<grid, MW_WARPS * 32, 0, st>>>(base, Ncap, Nper, B, fr, cfg, defer_list, defer_cnt, wp, cam_of, fsize, act, rows); \
+  else if (cam_of) k_match_filter_batch_warp<true, false, ACT, RW><<<grid, MW_WARPS * 32, 0, st>>>(base, Ncap, Nper, B, fr, cfg, defer_list, defer_cnt, wp, cam_of, fsize, act, rows); \
+  else k_match_filter_batch_warp<false, false, ACT, RW><<<grid, MW_WARPS * 32, 0, st>>>(base, Ncap, Nper, B, fr, cfg, defer_list, defer_cnt, wp, cam_of, fsize, act, rows)
     if (act && rows) { MW_LAUNCH(true, true); }
     else if (act) { MW_LAUNCH(true, false); }
     else if (rows) { MW_LAUNCH(false, true); }
@@ -1369,8 +1391,24 @@ void launch_match_filter_batch(cudaStream_t st, FeatTab base, int Ncap, const in
     cudaGetLastError();
     per_sm = 4;
   }
-  deferred<<<sms * per_sm, MATCH_THREADS, smem, st>>>(base, Ncap, fr, cfg, as_cu(tm), tm.ok, defer_list, defer_cnt, cam_of, fsize, rows);
-  *launches += 2;
+  if (n_wmaps > 0) {
+    // one run per window, each with the map whose box is that window's and the shared memory and persistent grid a batch of that
+    // window has (a smaller window than cfg.window fits more CTAs on an SM)
+    for (int k = 0; k < n_wmaps; ++k) {
+      const EkfTensorMap& mk = wmaps[k].ok ? wmaps[k] : none;
+      const size_t smem_k = match_smem_bytes(wmap_window[k], cfg.search_clamp);
+      int per_sm_k = 4;
+      if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm_k, deferred, MATCH_THREADS, smem_k) != cudaSuccess || per_sm_k < 1) {
+        cudaGetLastError();
+        per_sm_k = 4;
+      }
+      deferred<<<sms * per_sm_k, MATCH_THREADS, smem_k, st>>>(base, Ncap, fr, cfg, as_cu(mk), mk.ok, defer_list, defer_cnt, cam_of, fsize,
+                                                              rows, wmap_window[k]);
+    }
+  } else {
+    deferred<<<sms * per_sm, MATCH_THREADS, smem, st>>>(base, Ncap, fr, cfg, as_cu(tm), tm.ok, defer_list, defer_cnt, cam_of, fsize, rows, 0);
+  }
+  *launches += (n_wmaps > 0 ? n_wmaps : 1) + (full && has11) + (!full || has_other);
 }
 
 int launch_match_batch(cudaStream_t st, const uint8_t* frames, int n_frames, int width, int height, int stride,

@@ -298,7 +298,9 @@ class FilterBatch:
         self.h = h
         self.B = int(n_filters)
         self.n_cameras = 1
+        self.camera_of = np.zeros(self.B, dtype=np.int32)
         self.frame_sizes = None   # (n_cameras, 2) width, height of each camera's frame (set_frame_sizes), None: the whole frame
+        self.camera_settings = None   # (n_cameras, 3) window_size, scale, kernel_size (set_camera_settings), None: the batch's
         self._cams = None   # (mu14, Sigma14) of every filter, read once per step for the views
 
     @classmethod
@@ -314,6 +316,28 @@ class FilterBatch:
             batch.set_motion_blur(cfg.kernel_size)
         batch.set_scale(cfg.scale)
         batch.set_force_plane(cfg.forsePlane)
+        if archive:
+            batch.set_archive(archive)
+        return batch
+
+    @classmethod
+    def from_configs(cls, cfgs, camera_of, feature_capacity=32, large=False, archive=0, device=0):
+        """A batch whose filter f runs configuration cfgs[f] (one EkfConfig per filter) and follows camera camera_of[f]: the
+        rigs of several configuration files in one batch.  Filters of one camera must agree on window_size, scale and
+        kernel_size, and every filter on search_clamp, forsePlane, xyz_conversion and abs_int_quirk (ValueError naming the
+        filter and field otherwise).  The batch is created with the largest window, then set_cameras, set_camera_settings,
+        set_force_plane, set_configs and, when archive > 0, set_archive."""
+        cfgs = list(cfgs)
+        cam = np.ascontiguousarray(camera_of, dtype=np.int32).reshape(-1)
+        settings = _abi.camera_settings_of(cfgs, cam)
+        base = _abi.EkfConfig.from_buffer_copy(cfgs[0])
+        base.window_size = int(settings[:, 0].max())
+        base.kernel_size, base.scale, base.forsePlane = _abi.default_config().kernel_size, 1, 0
+        batch = cls(base, len(cfgs), feature_capacity=feature_capacity, device=device, large=large)
+        batch.set_cameras(settings.shape[0], cam)
+        batch.set_camera_settings(settings)
+        batch.set_force_plane(cfgs[0].forsePlane)
+        batch.set_configs(cfgs)
         if archive:
             batch.set_archive(archive)
         return batch
@@ -381,7 +405,37 @@ class FilterBatch:
             raise ValueError("camera_of expects (n_filters,)")
         self._ck(self.L.ekf_batch_set_cameras(self.h, int(n), _ptr(a) if a is not None else None))
         self.n_cameras = int(n)
+        self.camera_of = a.copy() if a is not None else np.arange(self.B, dtype=np.int32)
         self.frame_sizes = None
+        self.camera_settings = None   # set_cameras clears the camera table
+
+    def set_camera_settings(self, settings):
+        """Window, scale and blur threshold per camera (ekf_batch_set_camera_settings): an (n_cameras, 3) int array of
+        (window_size, scale, kernel_size), filter f running with row camera_of[f] as a batch of that window, scale and
+        kernel_size would; None returns every camera to the batch's values.  A window above the batch's window_size, a window
+        change under features and set_scale / set_motion_blur while a table is set raise EkfError.  A scale change forgets
+        the captured frames."""
+        if settings is None:
+            self._ck(self.L.ekf_batch_set_camera_settings(self.h, None))
+            self.camera_settings = None
+            return
+        a = np.asarray(settings, dtype=np.int64)
+        if a.shape != (self.n_cameras, 3):
+            raise ValueError(f"set_camera_settings expects ({self.n_cameras}, 3)")
+        i32 = np.iinfo(np.int32)
+        bad = np.argwhere((a < i32.min) | (a > i32.max))
+        if bad.size:   # the C rows are int32: a wider value would wrap (a huge kernel_size could turn blur on)
+            c, k = bad[0]
+            raise ValueError(f"camera {c}: {_abi.CAMERA_FIELDS[k]} = {a[c, k]} does not fit an int32")
+        rows = (_abi.EkfCameraSettings * self.n_cameras)(*[_abi.EkfCameraSettings(int(w), int(s), int(k), 0) for w, s, k in a])
+        self._ck(self.L.ekf_batch_set_camera_settings(self.h, rows))
+        self.camera_settings = a.copy()
+
+    def window_of(self, f):
+        """The template side filter f runs with: its camera's window (set_camera_settings), or the batch's."""
+        if self.camera_settings is None:
+            return int(self.cfg.window_size)
+        return int(self.camera_settings[self.camera_of[int(f)], 0])
 
     def _stamps(self, stamps, n=None):
         if stamps is None:
@@ -491,8 +545,9 @@ class FilterBatch:
         cfgs holds n_filters EkfConfig (one per camera: [cfgs[c] for c in camera_of]); None returns every filter to the
         batch's configuration.  ValueError, naming the field and the filter, when a field every filter shares
         (_abi.BATCH_SHARED_FIELDS) differs from the batch's configuration as it stands (set_motion_blur, set_scale and
-        set_force_plane included), or when a row is invalid; every row is checked before either table changes.
-        nInitFeatures is not read."""
+        set_force_plane included), or when a row is invalid; every row is checked before either table changes.  With a camera
+        table (set_camera_settings), window_size, scale and kernel_size of cfgs[f] are checked against row camera_of[f] of it
+        instead.  nInitFeatures is not read."""
         if cfgs is None:
             self.set_intrinsics(None)
             self.set_filter_params(None)
@@ -500,7 +555,10 @@ class FilterBatch:
         cfgs = list(cfgs)
         if len(cfgs) != self.B:
             raise ValueError(f"set_configs expects {self.B} configurations")
-        cam, rows = _abi.batch_rows(self.cfg, cfgs)
+        if self.camera_settings is None:
+            cam, rows = _abi.batch_rows(self.cfg, cfgs)
+        else:
+            cam, rows = _abi.batch_rows_per_camera(self.cfg, cfgs, self.camera_settings, self.camera_of)
         self.set_intrinsics(cam)
         self.set_filter_params(rows)
 
@@ -697,7 +755,8 @@ class FilterBatch:
         return out
 
     def template(self, f, i, which=0):
-        w = self.cfg.window_size
+        """Patch::patch (which 0) or Patch::matching_patch (1) of feature i of filter f: window_of(f) x window_of(f)."""
+        w = self.window_of(f)
         out = np.zeros((w, w), dtype=np.uint8)
         self._ck(self.L.ekf_batch_get_template(self.h, int(f), int(i), int(which), _ptr(out)))
         return out

@@ -235,8 +235,8 @@ int ekf_match_batch(const uint8_t* frames, int n_frames, int width, int height, 
  * switched on after creation instead, with ekf_batch_set_motion_blur, ekf_batch_set_scale and
  * ekf_batch_set_force_plane, so that a batch honours every ConfigVSLAM switch a single filter honours.
  * The configuration is every filter's by default; ekf_batch_set_intrinsics and ekf_batch_set_filter_params give each filter
- * intrinsics and tuning of its own, while window_size, search_clamp, scale, kernel_size, forsePlane, xyz_conversion and
- * abs_int_quirk stay shared by the batch. */
+ * intrinsics and tuning of its own, ekf_batch_set_camera_settings each camera a window_size, scale and kernel_size of its own,
+ * while search_clamp, forsePlane, xyz_conversion and abs_int_quirk stay shared by the batch. */
 typedef struct ekf_batch ekf_batch;
 typedef struct ekf_batch_desc {
   int32_t n_filters, feature_capacity, state_capacity /* 14 + 6 * feature_capacity */, ld /* Sigma row stride */;
@@ -328,6 +328,36 @@ typedef struct ekf_filter_params {
  * request from its own min_features.  For a tuning per camera, pass row camera_of[f] for filter f.  Memory: one row of
  * 240 B per filter on the device (the row it shares with the intrinsics) while either table is set. */
 int ekf_batch_set_filter_params(ekf_batch* b, const ekf_filter_params* rows);
+/* Settings per camera: the three ekf_config fields a camera's filters may take on their own (ekf_batch_set_camera_settings). */
+typedef struct ekf_camera_settings {
+  int32_t window_size;   /* template side, 3 .. the window_size the batch was created with */
+  int32_t scale;         /* capture resizes by 1 / scale, 1 .. 64 */
+  int32_t kernel_size;   /* Patch::blur threshold; >= 100000: no motion blur on this camera */
+  int32_t _pad;
+} ekf_camera_settings;
+/* Window, scale and blur threshold per camera: rows is a HOST array of n_cameras ekf_camera_settings, and filter f runs with
+ * row camera_of[f] exactly as it would in a batch created with that row's window, scale and blur threshold: the same matches,
+ * NCC scores, templates, feature tables, counters, state and covariance, bit for bit.  NULL returns every camera to the
+ * batch's values (window_size of the configuration, ekf_batch_set_scale, ekf_batch_set_motion_blur), which is the default.
+ *  - Templates stay stored at the create-time stride, so the configuration's window_size is the largest window a camera may take.
+ *  - A window outside [3, create-time window_size] or a scale outside [1, 64] returns EKF_ERR_ARG, ekf_batch_last_error names the
+ *    camera and the field, and the table stays as it was.  kernel_size takes any value, as in ekf_batch_set_motion_blur.
+ *  - A call that changes the window of a camera whose filters hold features returns EKF_ERR_STATE and names the filter (its
+ *    templates have the old size); the table stays as it was.
+ *  - Frames: camera c's frame is resized to w_c / s_c x h_c / s_c, w_c x h_c its ekf_batch_set_frame_sizes size or the whole slot.
+ *    The stack's slot is sized by the smallest scale s_min: n_cameras x (width / s_min rounded up to 16) x height / s_min bytes,
+ *    however large the other cameras' scales are.  A call that changes some camera's scale forgets the captured frames, as
+ *    ekf_batch_set_frame_sizes does.  Gray frames at scale 1 on every camera, captured for every camera, still go up in one copy.
+ *  - While a table is set, ekf_batch_set_scale and ekf_batch_set_motion_blur return EKF_ERR_STATE; ekf_batch_set_cameras clears
+ *    the table (EKF_ERR_STATE, changing nothing, when that would change the window of a filter that holds features);
+ *    ekf_batch_seed_from with a source that holds features returns EKF_ERR_ARG unless the source's window equals every camera's
+ *    (an empty source seeds any table); ekf_batch_resample moves filters within a camera, so their settings stay.
+ *  - Motion blur runs in a step when some camera's kernel_size is below 100000; each filter uses its camera's threshold and its
+ *    own T_camera, and the filters of a camera with blur off blur nothing.
+ *  - ekf_batch_get_template writes window_c^2 bytes for a filter of camera c; findNewFeatures' mask border and patch boxes,
+ *    addFeature's isInsideImage, the prediction gate and the matcher use the camera's window.
+ * Memory: one device row of 240 B per filter (the row of ekf_batch_set_filter_params) and 4 B per camera while the table is set. */
+int ekf_batch_set_camera_settings(ekf_batch* b, const ekf_camera_settings* rows);
 /* A frame size per camera: wh is a HOST array of n_cameras x 2 int32 (width, height) in INPUT pixels, before the resize by
  * 1 / scale; NULL (the default) means every camera uses the whole frame the capture calls pass.  The stack keeps one slot per
  * camera: the capture calls' width / height / stride describe the slot, and camera c's frame is the top-left w_c x h_c of slot
@@ -486,7 +516,8 @@ int ekf_batch_get_points_features(ekf_batch* b, int first, int count, double* ou
  * buffer), which costs one more read and write of it; a vector from systematic resampling that keeps every drawn filter in
  * its own slot never needs that.  Returns once the copy is done. */
 int ekf_batch_resample(ekf_batch* b, const int32_t* ancestors);
-/* which: 0 = Patch::patch, 1 = Patch::matching_patch of feature idx of one filter; out holds window_size^2 bytes */
+/* which: 0 = Patch::patch, 1 = Patch::matching_patch of feature idx of one filter; out holds window_size^2 bytes (the window of
+ * the filter's camera, ekf_batch_set_camera_settings) */
 int ekf_batch_get_template(ekf_batch* b, int filter, int idx, int which, uint8_t* out);
 /* Kernels of this library launched on the batch so far. */
 int64_t ekf_batch_kernel_launches(const ekf_batch* b);
