@@ -23,6 +23,8 @@
 // ekf_batch_create_large: up to BNCAP_L = 128 features (n <= 782); the update then runs on a cluster of 2 to 4 CTAs per filter
 // (k_batch_update_cluster) and the other kernels take their BNCAP_L instantiations.  Sigma and the compaction scratch are
 // B x ncap x ld doubles each: 4.9 MB per filter each at capacity 128, 40 GB in total for 4096 filters.
+// Every per-filter launch reads a device list of the filters it works on, CTA i on filter act[i]: ekf_batch_step_filters' list,
+// or the identity list iota (0 ... B - 1) for a full step and the calls outside a step.
 // Every stage evaluates the same expressions as the single-filter kernels (same device functions).
 #include <algorithm>
 #include <climits>
@@ -141,15 +143,8 @@ struct BatchStepIn {
   const double* ctl;       // [B][6] dv, dw of each filter (ekf_batch_step_controls)
   const int* vcontrol;     // [B]
   const int* fsize;        // [n_cameras][4] frame sizes (ekf_batch_set_frame_sizes): the gate uses [2], [3] of the filter's camera
-  const int* act;          // [n] the filters ekf_batch_step_filters steps, ascending; read by the ACT instantiations only
+  const int* act;          // [n] the filters the step works on, ascending: CTA i works on filter act[i]
 };
-// The filter CTA i of a per-filter launch works on: i itself, or with a list (ACT, ekf_batch_step_filters) the list's entry i.
-// A template parameter, so that a step without a list runs the code it ran before.
-template <bool ACT>
-__device__ __forceinline__ int act_filter(const int* __restrict__ act, int i) {
-  if constexpr (ACT) return act[i];
-  else return i;
-}
 __device__ __forceinline__ double step_dT(const BatchStepIn& in, int b, double dT) {
   return in.dT ? in.dT[in.cam_of ? in.cam_of[b] : 0] : dT;
 }
@@ -158,11 +153,11 @@ __device__ __forceinline__ double step_dT(const BatchStepIn& in, int b, double d
 // predict for one filter per CTA: same arithmetic as k_predict_cov / k_predict_features / k_predict_S2
 // ------------------------------------------------------------------------------------------------
 #define BPRED_THREADS 128
-template <bool ROWS, bool ACT>
+template <bool ROWS>
 __global__ void __launch_bounds__(BPRED_THREADS, 4) k_batch_predict(BatchView bv, FrameView fr, DevCfg cfg, double dT, double3 dv,
                                                                  double3 dw, int vcontrol, BatchStepIn in) {
   __shared__ double F[169], C[169], T[169], Q[169], cam[13];
-  const int i0 = blockIdx.x, b = act_filter<ACT>(in.act, i0), tid = threadIdx.x;
+  const int i0 = blockIdx.x, b = in.act[i0], tid = threadIdx.x;
   dT = step_dT(in, b, dT);
   if (in.ctl) {
     const double* c = in.ctl + 6 * (size_t)i0;
@@ -301,18 +296,18 @@ __global__ void __launch_bounds__(BPRED_THREADS, 4) k_batch_predict(BatchView bv
 // with lane = point, keeps each distinct coefficient once, orders them by (row, column) and has every output pixel walk
 // that list: the terms and their order are the bit mask walk's, without the zeros.  out[i] = templates blurred,
 // out[gridDim.x + i] = 1 when a kernel exceeded BLUR_MAXK (that template stays unblurred, as in k_predict_blur), i the CTA:
-// the filter, or its position in the list.
+// the filter's position in the step's list.
 // ------------------------------------------------------------------------------------------------
 #define BBLUR_WARPS 4
 // NC: feature capacity (BNCAP or BNCAP_L); warp 0 takes the decisions 32 features at a time, in ascending order.
-template <int NC, bool ROWS, bool ACT>
+template <int NC, bool ROWS>
 __global__ void __launch_bounds__(BBLUR_WARPS * 32) k_batch_predict_blur(BatchView bv, DevCfg cfg, double dT, int* __restrict__ out,
                                                                      BatchStepIn in) {
   __shared__ int s_feat[NC], s_rows[NC], s_cols[NC], s_nblur;
   __shared__ double s_dx[NC], s_dy[NC];
   __shared__ __align__(16) uint8_t s_tmpl[BBLUR_WARPS][1024];
   __shared__ int s_seq[BBLUR_WARPS][BLUR_MAXPTS], s_coef[BBLUR_WARPS][BLUR_MAXPTS];
-  const int b = act_filter<ACT>(in.act, blockIdx.x), lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  const int b = in.act[blockIdx.x], lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   dT = step_dT(in, b, dT);
   const int N = bv.N[b], ld = bv.ld;
   const double* mu = bv.mu + (size_t)b * ld;
@@ -645,8 +640,8 @@ __device__ void cta_stacked_update(const UpdSmem& sm, double* __restrict__ Sigma
 }
 
 // PLANE: forsePlane (ekf_batch_set_force_plane), a separate instantiation so that the plane-off kernel is the same code as without it.
-// ACT: CTA i updates filter act[i] (ekf_batch_step_filters).
-template <bool PLANE, bool ROWS, bool ACT>
+// CTA i updates filter act[i].
+template <bool PLANE, bool ROWS>
 __global__ void __launch_bounds__(BUPD_THREADS, 1) k_batch_update(BatchView bv, DevCfg cfg, const uint32_t* __restrict__ picks,
                                                                   int n_picks, double* __restrict__ out_mu14,
                                                                   double* __restrict__ out_S14, int* __restrict__ out_stats,
@@ -664,7 +659,7 @@ __global__ void __launch_bounds__(BUPD_THREADS, 1) k_batch_update(BatchView bv, 
   sm.Hs = sm.mu_i + BNMAX;
   sm.qj = sm.Hs + BNCAP * 27;
   sm.ibuf = reinterpret_cast<int*>(sm.qj + 48);
-  const int b = act_filter<ACT>(act, blockIdx.x), tid = threadIdx.x;
+  const int b = act[blockIdx.x], tid = threadIdx.x;
   const int n = bv.n[b], N = bv.N[b], ld = bv.ld;
   double* Sigma = bv.Sigma + (size_t)b * bv.sstride;
   double* mu = bv.mu + (size_t)b * ld;
@@ -1109,7 +1104,7 @@ static __device__ __noinline__ void cl_hi_rescue(double* Sigma, int ld, const do
   if (tid == 0) { ctl->n_hi = nh; ctl->k_rows = 2 * nh; }
 }
 
-template <bool PLANE, bool ROWS, bool ACT>
+template <bool PLANE, bool ROWS>
 __global__ void __launch_bounds__(BUPD_THREADS, 1) k_batch_update_cluster(BatchView bv, DevCfg cfg, const uint32_t* __restrict__ picks,
                                                                           int n_picks, double* __restrict__ out_mu14,
                                                                           double* __restrict__ out_S14, int* __restrict__ out_stats,
@@ -1128,7 +1123,7 @@ __global__ void __launch_bounds__(BUPD_THREADS, 1) k_batch_update_cluster(BatchV
   sm.qj = sm.Hs + BNCAP * 27;
   sm.ibuf = reinterpret_cast<int*>(sm.qj + 48);
   const int C = (int)cg::this_cluster().num_blocks(), rank = (int)cg::this_cluster().block_rank();
-  const int b = act_filter<ACT>(act, blockIdx.x / C), tid = threadIdx.x;
+  const int b = act[blockIdx.x / C], tid = threadIdx.x;
   const int n = bv.n[b], N = bv.N[b], ld = bv.ld;
   double* Sigma = bv.Sigma + (size_t)b * bv.sstride;
   double* mu = bv.mu + (size_t)b * ld;
@@ -1230,14 +1225,14 @@ struct BatchArchive {
 // with the surviving records; the conversions follow its new features (ekf_batch_step).  NC: feature capacity (BNCAP or
 // BNCAP_L); one CTA covers every entry of n2 x n2 either way, and every record (N2 <= 128 <= BCMP_THREADS).
 // one >= 0 (grid of one CTA): removeFeature(one_idx) on filter `one` alone (ekf_batch_remove_feature): no other removal, no
-// max_features rule, no conversion; pending decisions move with the records as under hold.  ACT: CTA i works on filter act[i].
+// max_features rule, no conversion; pending decisions move with the records as under hold.  Otherwise CTA i works on filter act[i].
 // ROWS: the max_features rule takes the filter's min / max_features from its row.
 // With the archive on, every removed feature that removeFeature archives (XYZ, n_find > 5) is appended to the filter's archive
 // in the single filter's order: the flagged features in ascending index (ekf_update_after_match's victims), then the
 // removeFeature(0) victim.  The records are read from Sigma and mu before the pass overwrites them.  A conversion fused into
 // the same pass never touches a removed feature's block: the reference removes before it converts, the decisions exclude the
 // removed features, and J is the identity on every row but the converted feature's.
-template <int NC, bool ROWS, bool ACT>
+template <int NC, bool ROWS>
 __global__ void __launch_bounds__(BCMP_THREADS, 1) k_batch_compact(BatchView bv, double* __restrict__ scratch, int min_features,
                                                                 int max_features, int remove, const int* __restrict__ hold_stats,
                                                                 BatchArchive ar, int one, int one_idx, const int* __restrict__ act) {
@@ -1246,7 +1241,7 @@ __global__ void __launch_bounds__(BCMP_THREADS, 1) k_batch_compact(BatchView bv,
   __shared__ int2 rmap[EKF_CAM + 6 * NC + 2];
   __shared__ int s_N2, s_n2, s_narch, s_abase;
   const bool single = one >= 0;
-  const int b = single ? one : act_filter<ACT>(act, blockIdx.x), tid = threadIdx.x;
+  const int b = single ? one : act[blockIdx.x], tid = threadIdx.x;
   DevCtl* ctl = bv.ctl + b;
   const bool rem = single || (remove && ctl->n_remove > 0);
   const bool hold = single || (hold_stats && hold_stats[(size_t)b * EKF_BATCH_STAT_FIELDS + EKF_BSTAT_TOPUP] > 0);
@@ -1407,15 +1402,16 @@ __global__ void __launch_bounds__(BNCAP_L) k_batch_xyz_decide_large(BatchView bv
 // took for the filter's older features (adds change no entry their linearity test reads), for k_batch_compact to apply.
 // LARGE (capacity up to BNCAP_L): the corners sit at xy + 2 * BNCAP_L * b, the rows (n <= 776 before an add) are taken
 // BADD_THREADS at a time and the decisions one thread per feature.  Templates come from frame cam_of[b] of the stack fr
-// (cam_of null: frame 0).  ACT: CTA i works on filter act[i] (ekf_batch_step_filters).
+// (cam_of null: frame 0).  Otherwise CTA i works on filter act[i].
 #define BADD_THREADS 256
-template <bool LARGE, bool ROWS, bool ACT>
+template <bool LARGE, bool ROWS>
 __global__ void __launch_bounds__(BADD_THREADS) k_batch_add(BatchView bv, FrameView fr, DevCfg cfg, const float* __restrict__ xy,
                                                             const int* __restrict__ cnt, int one, float u, float v, int decide,
                                                             const int* __restrict__ cam_of, const int* __restrict__ act) {
   constexpr int CS = LARGE ? BNCAP_L : EKF_BATCH_MAX_CORNERS;   // corner stride of xy
   __shared__ double A[6 * 7], Ap[6 * 3], fnew[6], Tc[6 * 7];
-  const int b = one >= 0 ? one : (ACT ? act[blockIdx.x] : blockIdx.x), tid = threadIdx.x;
+  // the filter index selected as unsigned: an int-typed select moves spills
+  const int b = one >= 0 ? one : (unsigned)act[blockIdx.x], tid = threadIdx.x;
   const int k = one >= 0 ? 1 : cnt[b];
   if (k <= 0) return;
   if (cam_of) fr.px += (size_t)cam_of[b] * fr.h * fr.stride;
@@ -1723,6 +1719,7 @@ struct ekf_batch {
   std::vector<int> over_seen;                   // ar.overflow at the last check
   int *pts_dev = nullptr, *h_pts = nullptr;     // [2][B] row counts and archive sizes of ekf_batch_get_points_features; pinned mirror
   int2* rs_pairs = nullptr;                     // [2 * B] (destination, source) slot pairs of ekf_batch_resample's launches
+  int* iota = nullptr;                          // [B] 0 ... B - 1: the list of a launch over every filter
   cudaEvent_t ev[4] = {nullptr, nullptr, nullptr, nullptr};
   std::string err;
 };
@@ -1817,7 +1814,7 @@ int ekf_batch_destroy(ekf_batch* b) {
   if (b->h_n) cudaFreeHost(b->h_n);
   if (b->h_N) cudaFreeHost(b->h_N);
   cudaFree(b->ar.rec); cudaFree(b->ar.real_index); cudaFree(b->ar.count); cudaFree(b->ar.overflow); cudaFree(b->pts_dev);
-  cudaFree(b->rs_pairs);
+  cudaFree(b->rs_pairs); cudaFree(b->iota);
   if (b->h_over) cudaFreeHost(b->h_over);
   if (b->h_pts) cudaFreeHost(b->h_pts);
   for (auto& e : b->ev) if (e) cudaEventDestroy(e);
@@ -1893,19 +1890,15 @@ static int batch_create(const ekf_config* cfg, int n_filters, int feature_capaci
   TRY(cudaSetDevice(device))
   TRY(cudaStreamCreateWithFlags(&b->own_stream, cudaStreamNonBlocking))
   b->stream = b->own_stream;
-  for (void* k : {(void*)k_batch_update<false, false, false>, (void*)k_batch_update<true, false, false>,
-                  (void*)k_batch_update<false, true, false>, (void*)k_batch_update<true, true, false>,
-                  (void*)k_batch_update<false, false, true>, (void*)k_batch_update<true, false, true>,
-                  (void*)k_batch_update<false, true, true>, (void*)k_batch_update<true, true, true>})
+  for (void* k : {(void*)k_batch_update<false, false>, (void*)k_batch_update<true, false>,
+                  (void*)k_batch_update<false, true>, (void*)k_batch_update<true, true>})
     TRY(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kUpdSmemBytes))
   if (large) {
-    void* const cl[8] = {(void*)k_batch_update_cluster<false, false, false>, (void*)k_batch_update_cluster<true, false, false>,
-                         (void*)k_batch_update_cluster<false, true, false>, (void*)k_batch_update_cluster<true, true, false>,
-                         (void*)k_batch_update_cluster<false, false, true>, (void*)k_batch_update_cluster<true, false, true>,
-                         (void*)k_batch_update_cluster<false, true, true>, (void*)k_batch_update_cluster<true, true, true>};
+    void* const cl[4] = {(void*)k_batch_update_cluster<false, false>, (void*)k_batch_update_cluster<true, false>,
+                         (void*)k_batch_update_cluster<false, true>, (void*)k_batch_update_cluster<true, true>};
     for (void* k : cl) TRY(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kUpdSmemBytes))
     cudaLaunchAttribute attr[1];
-    for (int i = 0; i < 8; ++i) {   // forsePlane x per-filter rows x filter list
+    for (int i = 0; i < 4; ++i) {   // forsePlane x per-filter rows
       const cudaLaunchConfig_t lc = cluster_config(1, b->cl_ctas, nullptr, attr);
       int ncl = 0;
       TRY(cudaOccupancyMaxActiveClusters(&ncl, cl[i], &lc))
@@ -1948,6 +1941,10 @@ static int batch_create(const ekf_config* cfg, int n_filters, int feature_capaci
   TRY(cudaMemsetAsync(v.ctl, 0, sizeof(DevCtl) * Bn, b->stream))
   TRY(cudaMemsetAsync(v.n, 0, sizeof(int) * Bn, b->stream)) TRY(cudaMemsetAsync(v.N, 0, sizeof(int) * Bn, b->stream))
   TRY(cudaMemsetAsync(v.xyz_count, 0, sizeof(int) * Bn, b->stream))
+  std::vector<int> iota(Bn);
+  for (size_t i = 0; i < Bn; ++i) iota[i] = (int)i;
+  TRY(balloc(&b->iota, Bn))
+  TRY(cudaMemcpyAsync(b->iota, iota.data(), sizeof(int) * Bn, cudaMemcpyHostToDevice, b->stream))
   for (auto& evn : b->ev) TRY(cudaEventCreate(&evn))
   TRY(cudaStreamSynchronize(b->stream))
 #undef TRY
@@ -2469,21 +2466,20 @@ int ekf_batch_set_force_plane(ekf_batch* b, int on) {
   return b->bv.row ? upload_rows(b) : EKF_OK;   // the rows are whole configurations: they follow dcfg
 }
 
-// The filters a step works on: n_act of them listed at act (device) by ekf_batch_step_filters, or every filter (act null).
+// The filters a launch works on, n_act of them listed at act (device), ascending: ekf_batch_step_filters' list, or every filter
+// (iota).
 struct StepList {
-  const int* act = nullptr;
-  int n_act = 0;
+  const int* act;
+  int n_act;
 };
-static unsigned step_grid(const ekf_batch* b, const StepList& sl) { return (unsigned)(sl.act ? sl.n_act : b->B); }
+static StepList all_filters(const ekf_batch* b) { return {b->iota, b->B}; }
 
-// k_batch_compact at the batch's capacity on the step's filters; one >= 0: removeFeature(one_idx) on filter `one` alone (one CTA)
-static void launch_compact(ekf_batch* b, int remove, const int* hold_stats, int one = -1, int one_idx = -1, const StepList& sl = {}) {
-  const unsigned grid = one >= 0 ? 1u : step_grid(b, sl);
+// k_batch_compact at the batch's capacity on the listed filters; one >= 0: removeFeature(one_idx) on filter `one` alone (one CTA)
+static void launch_compact(ekf_batch* b, int remove, const int* hold_stats, const StepList& sl, int one = -1, int one_idx = -1) {
+  const unsigned grid = one >= 0 ? 1u : (unsigned)sl.n_act;
   const bool rows = b->bv.row != nullptr;
-  auto* const compact = b->large ? (sl.act ? (rows ? k_batch_compact<BNCAP_L, true, true> : k_batch_compact<BNCAP_L, false, true>)
-                                           : (rows ? k_batch_compact<BNCAP_L, true, false> : k_batch_compact<BNCAP_L, false, false>))
-                                 : (sl.act ? (rows ? k_batch_compact<BNCAP, true, true> : k_batch_compact<BNCAP, false, true>)
-                                           : (rows ? k_batch_compact<BNCAP, true, false> : k_batch_compact<BNCAP, false, false>));
+  auto* const compact = b->large ? (rows ? k_batch_compact<BNCAP_L, true> : k_batch_compact<BNCAP_L, false>)
+                                 : (rows ? k_batch_compact<BNCAP, true> : k_batch_compact<BNCAP, false>);
   compact<<<grid, BCMP_THREADS, 0, b->stream>>>(b->bv, b->scratch, b->cfg.min_features, b->cfg.max_features, remove, hold_stats, b->ar,
                                                 one, one_idx, sl.act);
   b->launches += 1;
@@ -2543,25 +2539,23 @@ static int batch_detect(ekf_batch* b, const int* num, const int* hnum, int num_s
   return EKF_OK;
 }
 
-// k_batch_add at the batch's capacity and intrinsics, with or without a list of filters
-static void (*add_kernel(const ekf_batch* b, bool act))(BatchView, FrameView, DevCfg, const float*, const int*, int, float, float, int,
-                                                        const int*, const int*) {
+// k_batch_add at the batch's capacity and intrinsics
+static void (*add_kernel(const ekf_batch* b))(BatchView, FrameView, DevCfg, const float*, const int*, int, float, float, int,
+                                              const int*, const int*) {
   const bool rows = b->bv.row != nullptr;
-  if (b->large) return act ? (rows ? k_batch_add<true, true, true> : k_batch_add<true, false, true>)
-                           : (rows ? k_batch_add<true, true, false> : k_batch_add<true, false, false>);
-  return act ? (rows ? k_batch_add<false, true, true> : k_batch_add<false, false, true>)
-             : (rows ? k_batch_add<false, true, false> : k_batch_add<false, false, false>);
+  if (b->large) return rows ? k_batch_add<true, true> : k_batch_add<true, false>;
+  return rows ? k_batch_add<false, true> : k_batch_add<false, false>;
 }
 
 // detection + adds for every filter, as batch_detect; decide: also take the new features' XYZ decisions (in-step top-up).
-// The detector runs on every filter (one that asks for nothing costs next to nothing), the adds on the step's filters.
+// The detector runs on every filter (one that asks for nothing costs next to nothing), the adds on the listed filters.
 // Enqueued only.
-static int batch_topup(ekf_batch* b, const int* num, const int* hnum, int num_stride, int decide, const StepList& sl = {}) {
+static int batch_topup(ekf_batch* b, const int* num, const int* hnum, int num_stride, int decide, const StepList& sl) {
   cudaStream_t st = b->stream;
   const int rc = batch_detect(b, num, hnum, num_stride, 1);
   if (rc) return rc;
-  add_kernel(b, sl.act)<<<step_grid(b, sl), BADD_THREADS, 0, st>>>(b->bv, b->fv, b->dcfg, b->det_xy, b->det_n, -1, 0.0f, 0.0f, decide,
-                                                                   b->cam_dev, sl.act);
+  add_kernel(b)<<<(unsigned)sl.n_act, BADD_THREADS, 0, st>>>(b->bv, b->fv, b->dcfg, b->det_xy, b->det_n, -1, 0.0f, 0.0f, decide,
+                                                             b->cam_dev, sl.act);
   b->launches += 1;
   BCHECK(cudaGetLastError());
   return EKF_OK;
@@ -2591,8 +2585,9 @@ static int need_frame(ekf_batch* b, int f, const char* what) {
 // n_filters x 3, vcontrol n_filters; null = zeros) and ekf_batch_step_filters (filters: the n_act listed filters, strictly
 // ascending, with per_filter controls in list order).  With one camera, shared controls and no list the picks go up alone;
 // otherwise the cameras' dT, the filters' controls, the list and the picks are staged together and go up in one copy (BatchStepIn).
-// With a list every per-filter kernel runs on the listed filters only; the counters of the others are zeroed on the device and
-// their camera rows gathered when they may be stale, so that ekf_batch_get_camera_states reports every filter as it stands.
+// Every per-filter kernel runs on the filters of a list: the caller's, or iota without one.  With the caller's list the counters
+// of the other filters are zeroed on the device and their camera rows gathered when they may be stale, so that
+// ekf_batch_get_camera_states reports every filter as it stands.
 static int batch_step(ekf_batch* b, const double* dv, const double* dw, int vcontrol, const int32_t* vcontrols, bool per_filter,
                       const uint32_t* picks, int n_picks, const int32_t* filters = nullptr, int n_act = 0) {
   if (!b || n_picks < 0 || (n_picks > 0 && !picks)) return EKF_ERR_ARG;
@@ -2613,8 +2608,8 @@ static int batch_step(ekf_batch* b, const double* dv, const double* dw, int vcon
   BCHECK(cudaSetDevice(b->device));
   cudaStream_t st = b->stream;
   const size_t Bn = (size_t)b->B;
-  BatchStepIn in{b->cam_dev, nullptr, nullptr, nullptr, b->fsize_on ? b->fsize_dev : nullptr, nullptr};
-  StepList sl;
+  BatchStepIn in{b->cam_dev, nullptr, nullptr, nullptr, b->fsize_on ? b->fsize_dev : nullptr, b->iota};
+  StepList sl = all_filters(b);
   const uint32_t* picks_dev = b->picks_dev;
   const double z3[3] = {0, 0, 0};
   const double* a = (dv && !per_filter) ? dv : z3; const double* w = (dw && !per_filter) ? dw : z3;
@@ -2659,12 +2654,12 @@ static int batch_step(ekf_batch* b, const double* dv, const double* dw, int vcon
     const int* di = reinterpret_cast<const int*>(dd + n_dT + n_ctl);
     if (n_dT) in.dT = dd;
     if (per_filter) { in.ctl = dd + n_dT; in.vcontrol = di; }
-    if (filters) { in.act = di + n_vc; sl.act = in.act; sl.n_act = n_act; }
+    if (filters) { in.act = di + n_vc; sl = {in.act, n_act}; }
     picks_dev = reinterpret_cast<const uint32_t*>(di + n_vc + n_al);
   }
-  const bool act = sl.act != nullptr, rows = b->bv.row != nullptr;
-  const unsigned grid = step_grid(b, sl);
-  if (act) {   // the others' counters read zero; their camera rows are gathered once a call changed some filter's
+  const bool rows = b->bv.row != nullptr;
+  const unsigned grid = (unsigned)sl.n_act;
+  if (filters) {   // the others' counters read zero; their camera rows are gathered once a call changed some filter's
     BCHECK(cudaMemsetAsync(b->out_stats, 0, sizeof(int) * Bn * EKF_BATCH_STAT_FIELDS, st));
     if (b->rows_stale) {
       k_batch_camera_rows<<<(unsigned)((Bn * 210 + 255) / 256), 256, 0, st>>>(b->bv, b->out_mu14, b->out_S14, b->B);
@@ -2672,17 +2667,12 @@ static int batch_step(ekf_batch* b, const double* dv, const double* dw, int vcon
     }
   }
   BCHECK(cudaEventRecord(b->ev[0], st));
-  auto* const predict = act ? (rows ? k_batch_predict<true, true> : k_batch_predict<false, true>)
-                            : (rows ? k_batch_predict<true, false> : k_batch_predict<false, false>);
-  predict<<<grid, BPRED_THREADS, 0, st>>>(b->bv, b->fv, b->dcfg, b->cam_dT[0], make_double3(a[0], a[1], a[2]),
-                                          make_double3(w[0], w[1], w[2]), vcontrol, in);
+  (rows ? k_batch_predict<true> : k_batch_predict<false>)<<<grid, BPRED_THREADS, 0, st>>>(
+      b->bv, b->fv, b->dcfg, b->cam_dT[0], make_double3(a[0], a[1], a[2]), make_double3(w[0], w[1], w[2]), vcontrol, in);
   b->launches += 1;
   if (b->blur) {   // matching_patch <- blurred patch where the prediction moves far enough (k_batch_predict copied patch)
-    void (*blur)(BatchView, DevCfg, double, int*, BatchStepIn);
-    if (b->large) blur = act ? (rows ? k_batch_predict_blur<BNCAP_L, true, true> : k_batch_predict_blur<BNCAP_L, false, true>)
-                             : (rows ? k_batch_predict_blur<BNCAP_L, true, false> : k_batch_predict_blur<BNCAP_L, false, false>);
-    else blur = act ? (rows ? k_batch_predict_blur<BNCAP, true, true> : k_batch_predict_blur<BNCAP, false, true>)
-                    : (rows ? k_batch_predict_blur<BNCAP, true, false> : k_batch_predict_blur<BNCAP, false, false>);
+    auto* const blur = b->large ? (rows ? k_batch_predict_blur<BNCAP_L, true> : k_batch_predict_blur<BNCAP_L, false>)
+                                : (rows ? k_batch_predict_blur<BNCAP, true> : k_batch_predict_blur<BNCAP, false>);
     blur<<<grid, BBLUR_WARPS * 32, 0, st>>>(b->bv, b->dcfg, b->cam_dT[0], b->blur_out, in);
     b->launches += 1;
   }
@@ -2695,19 +2685,13 @@ static int batch_step(ekf_batch* b, const double* dv, const double* dw, int vcon
   if (b->large) {   // one cluster of cl_ctas CTAs per filter
     cudaLaunchAttribute attr[1];
     const cudaLaunchConfig_t lc = cluster_config((int)grid, b->cl_ctas, st, attr);
-    void (*update)(BatchView, DevCfg, const uint32_t*, int, double*, double*, int*, int, int, int, const int*);
-    if (act) update = plane ? (rows ? k_batch_update_cluster<true, true, true> : k_batch_update_cluster<true, false, true>)
-                            : (rows ? k_batch_update_cluster<false, true, true> : k_batch_update_cluster<false, false, true>);
-    else update = plane ? (rows ? k_batch_update_cluster<true, true, false> : k_batch_update_cluster<true, false, false>)
-                        : (rows ? k_batch_update_cluster<false, true, false> : k_batch_update_cluster<false, false, false>);
+    auto* const update = plane ? (rows ? k_batch_update_cluster<true, true> : k_batch_update_cluster<true, false>)
+                               : (rows ? k_batch_update_cluster<false, true> : k_batch_update_cluster<false, false>);
     BCHECK(cudaLaunchKernelEx(&lc, update, b->bv, b->dcfg, picks_dev, n_picks, b->out_mu14, b->out_S14,
                               b->out_stats, (int)b->cfg.min_features, (int)b->cfg.max_features, (int)b->cfg.xyz_conversion, sl.act));
   } else {
-    void (*update)(BatchView, DevCfg, const uint32_t*, int, double*, double*, int*, int, int, int, const int*);
-    if (act) update = plane ? (rows ? k_batch_update<true, true, true> : k_batch_update<true, false, true>)
-                            : (rows ? k_batch_update<false, true, true> : k_batch_update<false, false, true>);
-    else update = plane ? (rows ? k_batch_update<true, true, false> : k_batch_update<true, false, false>)
-                        : (rows ? k_batch_update<false, true, false> : k_batch_update<false, false, false>);
+    auto* const update = plane ? (rows ? k_batch_update<true, true> : k_batch_update<true, false>)
+                               : (rows ? k_batch_update<false, true> : k_batch_update<false, false>);
     update<<<grid, BUPD_THREADS, kUpdSmemBytes, st>>>(b->bv, b->dcfg, picks_dev, n_picks, b->out_mu14, b->out_S14,
                                                       b->out_stats, b->cfg.min_features, b->cfg.max_features,
                                                       b->cfg.xyz_conversion, sl.act);
@@ -2722,7 +2706,7 @@ static int batch_step(ekf_batch* b, const double* dv, const double* dw, int vcon
   BCHECK(cudaStreamSynchronize(st));
   b->results_valid = true;
   b->rows_stale = false;
-  if (b->blur && act) {   // the kernel wrote list positions: scatter them to filters, zeros for the others
+  if (b->blur && filters) {   // the kernel wrote list positions: scatter them to filters, zeros for the others
     const std::vector<int> got(b->h_blur, b->h_blur + 2 * (size_t)n_act);
     std::fill(b->h_blur, b->h_blur + 2 * Bn, 0);
     for (int i = 0; i < n_act; ++i) { b->h_blur[filters[i]] = got[i]; b->h_blur[Bn + filters[i]] = got[n_act + i]; }
@@ -2738,7 +2722,7 @@ static int batch_step(ekf_batch* b, const double* dv, const double* dw, int vcon
   std::fill(b->h_added, b->h_added + Bn, 0);
   if (!b->topup || topups == 0) {
     if (removed > 0 || converted > 0) {   // removals, then convert2XYZ_ifLinearAll (V:1312-1317), in one pass
-      launch_compact(b, 1, nullptr, -1, -1, sl);
+      launch_compact(b, 1, nullptr, sl);
       BCHECK(cudaGetLastError());
       const int rc = batch_readback(b, false);
       if (rc) return rc;
@@ -2749,12 +2733,12 @@ static int batch_step(ekf_batch* b, const double* dv, const double* dw, int vcon
     // and converting first would give A (J Sigma[cam, f]), equal only up to rounding.  So its compaction removes only;
     // every other filter keeps the fused pass.
     if (removed > 0 || converted > 0) {
-      launch_compact(b, 1, b->out_stats, -1, -1, sl);
+      launch_compact(b, 1, b->out_stats, sl);
     }
     int rc = batch_topup(b, b->out_stats + EKF_BSTAT_TOPUP, b->h_stats + EKF_BSTAT_TOPUP, EKF_BATCH_STAT_FIELDS, b->cfg.xyz_conversion, sl);
     if (rc) return rc;
     if (b->cfg.xyz_conversion) {   // the held conversions and the new features' (filters with none return at once)
-      launch_compact(b, 0, nullptr, -1, -1, sl);
+      launch_compact(b, 0, nullptr, sl);
     }
     BCHECK(cudaGetLastError());
     rc = batch_readback(b, true);
@@ -2794,7 +2778,7 @@ int ekf_batch_convert2xyz_if_linear_all(ekf_batch* b) {
   long long converted = 0;
   for (size_t i = 0; i < Bn; ++i) converted += b->h_xyz_count[i];
   if (converted == 0) return EKF_OK;
-  launch_compact(b, 0, nullptr);
+  launch_compact(b, 0, nullptr, all_filters(b));
   BCHECK(cudaGetLastError());
   BCHECK(cudaMemcpyAsync(b->h_n, b->bv.n, sizeof(int) * Bn, cudaMemcpyDeviceToHost, st));
   BCHECK(cudaMemcpyAsync(b->h_N, b->bv.N, sizeof(int) * Bn, cudaMemcpyDeviceToHost, st));
@@ -2888,7 +2872,7 @@ int ekf_batch_add_feature(ekf_batch* b, int f, float u, float v) {
   const int fw = b->fsize_on ? b->fsize_host[4 * c + 2] : b->fv.w, fh = b->fsize_on ? b->fsize_host[4 * c + 3] : b->fv.h;
   if (!(x > half && y > half && x < fw - half && y < fh - half)) return 0;
   if (b->h_N[f] >= b->Ncap || b->h_n[f] + 6 > b->ncap) return bfail(b, EKF_ERR_CAPACITY, "feature capacity exceeded");
-  add_kernel(b, false)<<<1, BADD_THREADS, 0, b->stream>>>(b->bv, b->fv, b->dcfg, nullptr, nullptr, f, u, v, 0, b->cam_dev, nullptr);
+  add_kernel(b)<<<1, BADD_THREADS, 0, b->stream>>>(b->bv, b->fv, b->dcfg, nullptr, nullptr, f, u, v, 0, b->cam_dev, b->iota);
   b->launches += 1;
   BCHECK(cudaGetLastError());
   b->h_N[f] += 1;
@@ -2945,8 +2929,8 @@ int ekf_batch_find_new_features(ekf_batch* b, const int32_t* num, int32_t* added
   BCHECK(cudaSetDevice(b->device));
   rc = num ? batch_stage_num(b, num) : EKF_OK;
   if (rc) return rc;
-  rc = num ? batch_topup(b, b->det_num, b->h_num, 1, 0)
-           : batch_topup(b, b->out_stats + EKF_BSTAT_TOPUP, b->h_stats + EKF_BSTAT_TOPUP, EKF_BATCH_STAT_FIELDS, 0);
+  rc = num ? batch_topup(b, b->det_num, b->h_num, 1, 0, all_filters(b))
+           : batch_topup(b, b->out_stats + EKF_BSTAT_TOPUP, b->h_stats + EKF_BSTAT_TOPUP, EKF_BATCH_STAT_FIELDS, 0, all_filters(b));
   if (rc) return rc;
   rc = batch_readback(b, true);
   if (rc) return rc;
@@ -3026,7 +3010,7 @@ int ekf_batch_remove_feature(ekf_batch* b, int f, int index) {
   if (!b->seeded) return bfail(b, EKF_ERR_STATE, "removeFeature before ekf_batch_seed_from");
   if (index < 0 || index >= b->h_N[f]) return bfail(b, EKF_ERR_ARG, "feature index out of range");
   BCHECK(cudaSetDevice(b->device));
-  launch_compact(b, 0, nullptr, f, index);
+  launch_compact(b, 0, nullptr, all_filters(b), f, index);
   BCHECK(cudaGetLastError());
   const int rc = batch_readback(b, false);
   if (rc) return rc;

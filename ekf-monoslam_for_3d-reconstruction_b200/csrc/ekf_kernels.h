@@ -40,9 +40,9 @@ struct FilterRow {
 };
 void launch_match_filter_batch(cudaStream_t st, FeatTab base, int Ncap, const int* Nper, int B, FrameView fr, const DevCfg& cfg,
                                const EkfTensorMap* tmap, int* defer_list, int* defer_cnt, long long* launches,
-                               const int* cam_of = nullptr,    // cam_of [B]: filter b searches frame cam_of[b] of the stack fr
-                               const int* fsize = nullptr,     // [n_cameras][4] (in w, in h, w, h): camera c is the top-left w x h of its slot
-                               const int* act = nullptr,       // [B]: the pairs' filter i is filter act[i] (a list of B filters)
+                               const int* cam_of,    // cam_of [B]: filter b searches frame cam_of[b] of the stack fr
+                               const int* fsize,     // [n_cameras][4] (in w, in h, w, h): camera c is the top-left w x h of its slot
+                               const int* act,       // [B]: the pairs' filter i is filter act[i] (a list of B filters)
                                const FilterRow* rows = nullptr,    // [B]: filter b matches with rows[b].cfg's sigma_size, ncc_threshold and window
                                int windows = 0,    // MATCH_WIN_* of the rows' windows (rows only); 0: every filter at cfg.window
                                // rows only: the n_wmaps distinct windows of the filters and a tensor map of the stack for each (its box

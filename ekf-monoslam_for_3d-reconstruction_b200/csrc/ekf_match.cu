@@ -770,7 +770,7 @@ struct MatchWarp2Smem {
   int cnt;
 };
 
-template <int W, bool TSMEM, bool SLIDE>
+template <int W>
 __device__ bool match_one_warp2(const MatchJob& jb, float sigma_size, float clampv, MatchWarp2Smem<W>& sm, MatchResult& res) {
   constexpr int TW = (W + 3) / 4, W2 = W * W;
   const int lane = threadIdx.x & 31;
@@ -806,11 +806,6 @@ __device__ bool match_one_warp2(const MatchJob& jb, float sigma_size, float clam
   MTTop top;
   top.reset();
   {
-    unsigned Treg[TSMEM ? 1 : W * TW];   // TSMEM: the template words are shared-memory operands (broadcast loads) instead of 33 registers
-    if (!TSMEM) {
-#pragma unroll
-      for (int e = 0; e < W * TW; ++e) Treg[e] = sm.tpk[e];
-    }
     MTGate g;
     g.x2c = G.x_2_coeff; g.y2c = G.y_2_coeff; g.yxc = G.yx_coeff; g.sigma2 = G.sigma_2;
     g.du0 = G.ilo - G.uc; g.dv0 = G.jlo - G.vc; g.cw = cw; g.ch = ch; g.T = T; g.rd1f = (float)rd1;
@@ -818,8 +813,7 @@ __device__ bool match_one_warp2(const MatchJob& jb, float sigma_size, float clam
     int ty = lane / ntx, tx = lane - ty * ntx;
     const int dty = 32 / ntx, dtx = 32 - dty * ntx;
     while (ty < nty) {
-      if (TSMEM) mt_tile<W, MT_R, SLIDE>(sm.win, tx, ty, sm.tpk, g, top);
-      else mt_tile<W, MT_R, SLIDE>(sm.win, tx, ty, reinterpret_cast<const unsigned (&)[W * TW]>(Treg), g, top);
+      mt_tile<W, MT_R>(sm.win, tx, ty, sm.tpk, g, top);   // the template words as shared-memory operands (broadcast loads)
       tx += dtx; ty += dty;
       if (tx >= ntx) { tx -= ntx; ++ty; }
     }
@@ -1061,14 +1055,6 @@ __device__ __forceinline__ FrameView batch_frame_of(FrameView fr, const int* __r
   return fr;
 }
 
-// ACT (ekf_batch_step_filters): the pairs run over the B = n listed filters, the list's entry i being filter act[i]; the deferred
-// list keeps the pair of the filter itself, b * Ncap + f.  Without a list the kernels are the code they were before.
-template <bool ACT>
-__device__ __forceinline__ int batch_pair_filter(const int* __restrict__ act, int i) {
-  if constexpr (ACT) return act[i];
-  else return i;
-}
-
 // ROWS (a batch with per-filter rows, ekf_batch_set_filter_params / ekf_batch_set_intrinsics / ekf_batch_set_camera_settings):
 // filter b searches and accepts with its row's sigma_size and ncc_threshold, and with its row's window, its camera's.  Without
 // rows the kernels are the code they were before.
@@ -1078,9 +1064,12 @@ __device__ __forceinline__ const DevCfg& batch_filter_cfg(const DevCfg& cfg, con
   else return cfg;
 }
 
+// Pass 1 of the batched filters runs over (filter, feature) pairs of the B listed filters, the list's entry i being filter
+// act[i]; the deferred list keeps the pair of the filter itself, b * Ncap + f.
+
 // Batched filters, pass 1 with the full-window warp matcher (template side 11): one warp per (filter, feature)
-template <int MINB, bool TSMEM, bool SLIDE, bool CAMS, bool SIZES, bool ACT, bool ROWS>
-__global__ void __launch_bounds__(MW2_WARPS * 32, MINB) k_match_filter_batch_warp2(FeatTab base, int Ncap, const int* __restrict__ Nper, int B,
+template <bool CAMS, bool SIZES, bool ROWS>
+__global__ void __launch_bounds__(MW2_WARPS * 32, 2) k_match_filter_batch_warp2(FeatTab base, int Ncap, const int* __restrict__ Nper, int B,
                                                                                 FrameView fr, DevCfg cfg, int* __restrict__ defer_list,
                                                                                 int* __restrict__ defer_cnt, const int* __restrict__ cam_of,
                                                                                 const int* __restrict__ fsize, const int* __restrict__ act,
@@ -1089,8 +1078,8 @@ __global__ void __launch_bounds__(MW2_WARPS * 32, MINB) k_match_filter_batch_war
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const long long pair_i = (long long)blockIdx.x * MW2_WARPS + warp;
   if (pair_i >= (long long)B * Ncap) return;
-  const int i = (int)(pair_i / Ncap), f = (int)(pair_i - (long long)i * Ncap), b = batch_pair_filter<ACT>(act, i);
-  const long long pair = ACT ? (long long)b * Ncap + f : pair_i;
+  const int i = (int)(pair_i / Ncap), f = (int)(pair_i - (long long)i * Ncap), b = act[i];
+  const long long pair = (long long)b * Ncap + f;
   const FeatTab ft = feattab_slice(base, b, Ncap, cfg.tstride);
   if (f >= Nper[b] || !ft.innov[f]) return;
   MatchJob jb;
@@ -1107,7 +1096,7 @@ __global__ void __launch_bounds__(MW2_WARPS * 32, MINB) k_match_filter_batch_war
   if constexpr (ROWS) {
     if (fc.window != 11) return;   // a filter whose camera has another window takes k_match_filter_batch_warp
   }
-  if (!match_one_warp2<11, TSMEM, SLIDE>(jb, fc.sigma_size_f, cfg.search_clamp, wsm[warp], r)) {
+  if (!match_one_warp2<11>(jb, fc.sigma_size_f, cfg.search_clamp, wsm[warp], r)) {
     if (lane == 0) defer_list[atomicAdd(defer_cnt, 1)] = (int)pair;
     return;
   }
@@ -1117,7 +1106,7 @@ __global__ void __launch_bounds__(MW2_WARPS * 32, MINB) k_match_filter_batch_war
 
 // Batched filters, pass 1: one warp per (filter, feature); features that do not fit go to defer_list.  warp_path ==
 // MATCH_WARP_SKIP11 (rows only): the window-11 filters were matched by k_match_filter_batch_warp2 and are skipped here.
-template <bool CAMS, bool SIZES, bool ACT, bool ROWS>
+template <bool CAMS, bool SIZES, bool ROWS>
 __global__ void __launch_bounds__(MW_WARPS * 32) k_match_filter_batch_warp(FeatTab base, int Ncap, const int* __restrict__ Nper, int B,
                                                                            FrameView fr, DevCfg cfg, int* __restrict__ defer_list,
                                                                            int* __restrict__ defer_cnt, int warp_path,
@@ -1127,8 +1116,8 @@ __global__ void __launch_bounds__(MW_WARPS * 32) k_match_filter_batch_warp(FeatT
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const long long pair_i = (long long)blockIdx.x * MW_WARPS + warp;
   if (pair_i >= (long long)B * Ncap) return;
-  const int i = (int)(pair_i / Ncap), f = (int)(pair_i - (long long)i * Ncap), b = batch_pair_filter<ACT>(act, i);
-  const long long pair = ACT ? (long long)b * Ncap + f : pair_i;
+  const int i = (int)(pair_i / Ncap), f = (int)(pair_i - (long long)i * Ncap), b = act[i];
+  const long long pair = (long long)b * Ncap + f;
   const FeatTab ft = feattab_slice(base, b, Ncap, cfg.tstride);
   if (f >= Nper[b] || !ft.innov[f]) return;
   const DevCfg& fc = batch_filter_cfg<ROWS>(cfg, rows, b);
@@ -1228,8 +1217,7 @@ __global__ void __launch_bounds__(MATCH_THREADS) k_match_batch(const uint8_t* __
 // Stateless batch with the full-window warp matcher (template side 11): one warp per (frame, feature).  A feature that needs
 // the CTA matcher is MARKED in out_uv and worked off by the persistent grid of k_match_batch_marked.
 #define MATCH_MARK ((int32_t)0x80000000)
-template <int MINB, bool TSMEM, bool SLIDE>
-__global__ void __launch_bounds__(MW2_WARPS * 32, MINB) k_match_batch_warp2(const uint8_t* __restrict__ frames, int width, int height, int stride,
+__global__ void __launch_bounds__(MW2_WARPS * 32, 2) k_match_batch_warp2(const uint8_t* __restrict__ frames, int width, int height, int stride,
                                                                          const uint8_t* __restrict__ templates, int fpf,
                                                                          const double* __restrict__ hh, const double* __restrict__ Sm,
                                                                          float sigma_size, float thr, float clampv,
@@ -1248,7 +1236,7 @@ __global__ void __launch_bounds__(MW2_WARPS * 32, MINB) k_match_batch_warp2(cons
   if (lane == 0) wsm[warp].cnt = 0;
   __syncwarp();
   MatchResult r;
-  const bool done = match_one_warp2<11, TSMEM, SLIDE>(jb, sigma_size, clampv, wsm[warp], r);
+  const bool done = match_one_warp2<11>(jb, sigma_size, clampv, wsm[warp], r);
   if (lane == 0) {
     if (!done) {
       out_uv[2 * idx] = MATCH_MARK;
@@ -1289,16 +1277,6 @@ __global__ void __launch_bounds__(MATCH_THREADS) k_match_batch_marked(const uint
     }
     __syncthreads();
   }
-}
-
-// EKF_MATCH_W2VAR: build of the warp tile matcher — 0 template words in registers, 2 CTAs per SM (128 registers); 1 template
-// words as shared-memory operands, 2 CTAs; 2 shared-memory operands, 3 CTAs per SM (80 registers); + 4: window sums of the three
-// right-hand candidates by sliding (mt_tile SLIDE).  Measured (tools/match_ab.py, 12 800 features per launch): 0 / 1 / 2 / 4 / 5 / 6 =
-// 52.3 / 55.2 / 54.4 / 51.9 / 55.6 / 53.4 M matches/s — DP4A and IMAD share one pipe (tools/idp_rate_probe: 2 warp-instructions per
-// cycle per SM each and together), so sliding buys nothing; default 1.
-static int match_w2_variant() {
-  const char* e = getenv("EKF_MATCH_W2VAR");   // read per call: tools/match_ab.py switches it inside one process
-  return e ? atoi(e) : 1;
 }
 
 void launch_match_filter(cudaStream_t st, FeatTab ft, int N, FrameView fr, const DevCfg& cfg, const EkfTensorMap* tmap, long long* launches) {
@@ -1346,39 +1324,20 @@ void launch_match_filter_batch(cudaStream_t st, FeatTab base, int Ncap, const in
   const bool full = warp_path >= 2 && cfg.search_clamp <= 20.0f;
   if (full && has11) {
     const unsigned grid = (unsigned)((pairs + MW2_WARPS - 1) / MW2_WARPS);
-    const int var = match_w2_variant();
-#define MW2_LAUNCH_ACT(MINB, TS, SL, ACT, RW)                                                                                           \
-  if (fsize) k_match_filter_batch_warp2<MINB, TS, SL, true, true, ACT, RW><<<grid, MW2_WARPS * 32, 0, st>>>(base, Ncap, Nper, B, fr, cfg, defer_list, defer_cnt, cam_of, fsize, act, rows); \
-  else if (cam_of) k_match_filter_batch_warp2<MINB, TS, SL, true, false, ACT, RW><<<grid, MW2_WARPS * 32, 0, st>>>(base, Ncap, Nper, B, fr, cfg, defer_list, defer_cnt, cam_of, fsize, act, rows); \
-  else k_match_filter_batch_warp2<MINB, TS, SL, false, false, ACT, RW><<<grid, MW2_WARPS * 32, 0, st>>>(base, Ncap, Nper, B, fr, cfg, defer_list, defer_cnt, cam_of, fsize, act, rows)
-#define MW2_LAUNCH(MINB, TS, SL)                                        \
-  if (act && rows) { MW2_LAUNCH_ACT(MINB, TS, SL, true, true); }        \
-  else if (act) { MW2_LAUNCH_ACT(MINB, TS, SL, true, false); }          \
-  else if (rows) { MW2_LAUNCH_ACT(MINB, TS, SL, false, true); }         \
-  else { MW2_LAUNCH_ACT(MINB, TS, SL, false, false); }
-    switch (var) {
-      case 0: MW2_LAUNCH(2, false, false); break;
-      case 2: MW2_LAUNCH(3, true, false); break;
-      case 4: MW2_LAUNCH(2, false, true); break;
-      case 5: MW2_LAUNCH(2, true, true); break;
-      case 6: MW2_LAUNCH(3, true, true); break;
-      default: MW2_LAUNCH(2, true, false); break;   // 1
-    }
-#undef MW2_LAUNCH
-#undef MW2_LAUNCH_ACT
+    auto* const warp2 = rows ? (fsize ? k_match_filter_batch_warp2<true, true, true>
+                                      : cam_of ? k_match_filter_batch_warp2<true, false, true> : k_match_filter_batch_warp2<false, false, true>)
+                             : (fsize ? k_match_filter_batch_warp2<true, true, false>
+                                      : cam_of ? k_match_filter_batch_warp2<true, false, false> : k_match_filter_batch_warp2<false, false, false>);
+    warp2<<<grid, MW2_WARPS * 32, 0, st>>>(base, Ncap, Nper, B, fr, cfg, defer_list, defer_cnt, cam_of, fsize, act, rows);
   }
   if (!full || has_other) {
     const unsigned grid = (unsigned)((pairs + MW_WARPS - 1) / MW_WARPS);
     const int wp = (full && has11) ? MATCH_WARP_SKIP11 : warp_path;
-#define MW_LAUNCH(ACT, RW)                                                                                                            \
-  if (fsize) k_match_filter_batch_warp<true, true, ACT, RW><<<grid, MW_WARPS * 32, 0, st>>>(base, Ncap, Nper, B, fr, cfg, defer_list, defer_cnt, wp, cam_of, fsize, act, rows); \
-  else if (cam_of) k_match_filter_batch_warp<true, false, ACT, RW><<<grid, MW_WARPS * 32, 0, st>>>(base, Ncap, Nper, B, fr, cfg, defer_list, defer_cnt, wp, cam_of, fsize, act, rows); \
-  else k_match_filter_batch_warp<false, false, ACT, RW><<<grid, MW_WARPS * 32, 0, st>>>(base, Ncap, Nper, B, fr, cfg, defer_list, defer_cnt, wp, cam_of, fsize, act, rows)
-    if (act && rows) { MW_LAUNCH(true, true); }
-    else if (act) { MW_LAUNCH(true, false); }
-    else if (rows) { MW_LAUNCH(false, true); }
-    else { MW_LAUNCH(false, false); }
-#undef MW_LAUNCH
+    auto* const warp = rows ? (fsize ? k_match_filter_batch_warp<true, true, true>
+                                     : cam_of ? k_match_filter_batch_warp<true, false, true> : k_match_filter_batch_warp<false, false, true>)
+                            : (fsize ? k_match_filter_batch_warp<true, true, false>
+                                     : cam_of ? k_match_filter_batch_warp<true, false, false> : k_match_filter_batch_warp<false, false, false>);
+    warp<<<grid, MW_WARPS * 32, 0, st>>>(base, Ncap, Nper, B, fr, cfg, defer_list, defer_cnt, wp, cam_of, fsize, act, rows);
   }
   int dev = 0, sms = 148;
   if (cudaGetDevice(&dev) == cudaSuccess) cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
@@ -1429,18 +1388,9 @@ int launch_match_batch(cudaStream_t st, const uint8_t* frames, int n_frames, int
     static PerDeviceOnce once2;
     if (once2.ensure([] { return cudaFuncSetAttribute(k_match_batch_marked, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                                       (int)match_smem_bytes(MATCH_MAX_W, 20.0f)); }) != cudaSuccess) return -1;
-    const int grid2 = (total + MW2_WARPS - 1) / MW2_WARPS, var = match_w2_variant();
-#define MW2_LAUNCH(MINB, TS, SL) \
-  k_match_batch_warp2<MINB, TS, SL><<<grid2, MW2_WARPS * 32, 0, st>>>(frames, width, height, stride, templates, fpf, h, S, sigma_size, thr, clampv, out_uv, out_score, total)
-    switch (var) {
-      case 0: MW2_LAUNCH(2, false, false); break;
-      case 2: MW2_LAUNCH(3, true, false); break;
-      case 4: MW2_LAUNCH(2, false, true); break;
-      case 5: MW2_LAUNCH(2, true, true); break;
-      case 6: MW2_LAUNCH(3, true, true); break;
-      default: MW2_LAUNCH(2, true, false); break;   // 1
-    }
-#undef MW2_LAUNCH
+    const int grid2 = (total + MW2_WARPS - 1) / MW2_WARPS;
+    k_match_batch_warp2<<<grid2, MW2_WARPS * 32, 0, st>>>(frames, width, height, stride, templates, fpf, h, S, sigma_size, thr, clampv,
+                                                          out_uv, out_score, total);
     int dev = 0, sms = 148, per_sm = 4;
     if (cudaGetDevice(&dev) == cudaSuccess) cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
     if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_match_batch_marked, MATCH_THREADS, smem) != cudaSuccess || per_sm < 1) {

@@ -13,10 +13,9 @@ python bench.py --workload cfg3_batch4096 > $O/bench_cfg3_$TAG.json 2>/dev/null
 python bench.py --workload cfg4_n2000 --steps 8 --no-cpu-baseline > $O/bench_cfg4_$TAG.json 2>/dev/null
 python bench.py --workload cfg5_match > $O/bench_cfg5_$TAG.json 2>/dev/null
 python bench.py --full-square --no-cpu-baseline > $O/bench_full_$TAG.json 2>/dev/null
-# matcher evidence: DP4A / IMAD issue rates of this GPU and the builds of the tile matcher in one process
+# matcher evidence: DP4A / IMAD issue rates of this GPU
 [ -x tools/idp_rate_probe ] || nvcc -gencode arch=compute_100a,code=sm_100a -O3 -o tools/idp_rate_probe tools/idp_rate_probe.cu
 ./tools/idp_rate_probe > $O/idp_rate_probe_$TAG.txt 2>&1
-python tools/match_ab.py 0 1 2 4 5 6 >> $O/idp_rate_probe_$TAG.txt 2>&1
 ncu --metrics gpu__time_duration.sum --clock-control none -c 4000 --csv --log-file $O/launches_$TAG.csv \
     python bench.py --steps 2 --warmup 3 --no-cpu-baseline --no-sharded --no-parity > $O/ncu_$TAG.log 2>&1
 ncu --set full --clock-control none --import-source on \
